@@ -4,6 +4,7 @@ workloads, the point-source ray casting and the combined outer iteration on a ne
 
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched under torch.distributed.run)
     python bench.py --impl reference ...                      (CPU arm: the reference algorithm on the host cores)
+    python bench.py ... --dump-outputs DIR                    (one GPU: the last timed step's outputs as DIR/*.npy)
 
 One *step* of the default workload = one full diffuse solve (all 12*4**(nAngularLevel-1) = 192 directions) over one
 synthetic grid: computeOpacities + sweep + merge + diffuse photo-rates; on N > 1 GPUs the directions are sharded inside
@@ -33,6 +34,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 REAL_STDOUT = 1
 METRIC = "ray-cell segment updates/sec (diffuse sweep)"
@@ -198,6 +200,29 @@ def measured_peak():
 
 def rel_linf(a, b, floor=1e-290):
     return float(np.max(np.abs(a - b) / np.maximum(np.abs(b), floor))) if a.size else 0.0
+
+
+DUMP_BYTES = 64 * 10 ** 6            # what --dump-outputs writes at most
+
+
+def dump_outputs(path, arrays, nseg, nleaf, max_bytes=DUMP_BYTES, seed=0):
+    """writes the per-leaf outputs `arrays` (name -> [rows, nleaf], torch tensor or numpy) as path/<name>.npy in float64,
+    with segment_updates.npy = [nseg] and leaf_index.npy = the leaves written.  When all leaves would exceed `max_bytes`,
+    every array is cut to the same seeded sample of leaves (sorted), identical from run to run for a given nleaf."""
+    rows = sum(int(a.shape[0]) for a in arrays.values())
+    count = min(nleaf, (max_bytes - 4096 * (len(arrays) + 2)) // (8 * (rows + 1)))     # 4 KiB per file for the header
+    idx = np.arange(nleaf) if count == nleaf else \
+        np.sort(np.random.default_rng(seed).choice(nleaf, size=count, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "leaf_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(path, "segment_updates.npy"), np.array([nseg], dtype=np.float64))
+    for name, a in arrays.items():
+        if isinstance(a, np.ndarray):
+            a = a[:, idx]
+        else:
+            import torch
+            a = a[:, torch.from_numpy(idx).to(a.device)].cpu().numpy()
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -424,8 +449,10 @@ def set_grid(eng, g):
     eng.set_grid(g["nx"], g["level"], g["HI"], g["HeI"], g["HeII"], g["rho"], g["abun2"], g["box_size"])
 
 
-def run_workload(env, workload, steps, warmup, cpu_seconds, with_clocks=True, faithful_too=False, e2e_steps=3):
-    """times one workload on the process group `env`; returns the dict of measured fields (rank 0 uses it)"""
+def run_workload(env, workload, steps, warmup, cpu_seconds, with_clocks=True, faithful_too=False, e2e_steps=3,
+                 dump_dir=None):
+    """times one workload on the process group `env`; returns the dict of measured fields (rank 0 uses it).
+    `dump_dir` (one process only): the outputs of the last timed step go there (dump_outputs)."""
     import radiativetransfer_b200 as rt
     from radiativetransfer_b200 import workloads as Wk
     torch = env.torch
@@ -502,6 +529,22 @@ def run_workload(env, workload, steps, warmup, cpu_seconds, with_clocks=True, fa
 
     clock_samples = [] if with_clocks else None
     ms_per_step, nseg_rank = time_steps(env, step_resident, W, steps, clock_samples)
+    if dump_dir is not None:
+        # what a caller of the resident step holds after it: Jmean1..3 [3, N], the diffuse photo-rates k24, k25, k26
+        # [3, N], the point-source rates in the order of rtb200_point [6, N], the species HI, HeI, HeII [3, N]
+        outs = {} if kind == "point" else dict(jmean=J)
+        if kind == "diffuse":
+            # the rates call adds to K (rate fields the caller zeroes once per outer iteration) and the timed steps never
+            # zero it: K holds the sum over all steps, so the last step's photo-rates are evaluated again from its J
+            K.zero_()
+            eng.diffuse_rates_device(J.data_ptr(), bg["ksi24"], bg["ksi25"], bg["ksi26"], K[0].data_ptr(), K[1].data_ptr(),
+                                     K[2].data_ptr(), stream=stream)
+            outs["photo_rates"] = K
+        if kind in ("point", "combined"):
+            outs["rates"] = R
+        if kind in ("iterate", "combined"):
+            outs["species"] = np.stack(eng.get_species())
+        dump_outputs(dump_dir, outs, nseg_rank, N)
     if not with_clocks:   # secondary workloads (3 steps): a second pass, keep the better one (host jitter of a shared box)
         ms2, _ = time_steps(env, step_resident, 1, steps)
         ms_per_step = min(ms_per_step, ms2)
@@ -745,8 +788,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--secondary", default="diffuse-64^3-amr3-192dir,point-128^3-amr-100src,combined-64^3-amr3-192dir-64src")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float64, at most "
+                         f"{DUMP_BYTES // 10 ** 6} MB: a fixed seeded sample of leaves, DIR/leaf_index.npy, when larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
+    if args.dump_outputs is not None and (args.impl != "rtb200" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs writes the outputs of the rtb200 arm on one GPU (one process)")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -754,7 +804,7 @@ def main():
     env = Env()
     world = env.world
     cpu_s = 0.0 if args.no_cpu_baseline else args.cpu_seconds
-    res = run_workload(env, args.workload, args.steps, args.warmup, cpu_s, faithful_too=True)
+    res = run_workload(env, args.workload, args.steps, args.warmup, cpu_s, faithful_too=True, dump_dir=args.dump_outputs)
     kind = res["kind"]
     line = None
     if env.rank == 0:
