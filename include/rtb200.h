@@ -116,7 +116,7 @@ int rtb200_set_math(rtb200_ctx* ctx, int math_mode);
  *                  for all tasks, 1), "dirs_per_task" (0 = chosen from a wave model), "cells" (cells of a layer per thread: 1, 2, or 0 = by grid size and zone tasks per launch), "block_warps" (rows per block 8 / 4 / 2,
  *                  0 = by the number of blocks a launch has), "transpose_z" (z-major copy for
  *                  the zones sweeping along the contiguous axis, 1), "persistent" (1 = the whole sweep as ONE launch, tiles handed out by a counter and
- *                  ordered by per-tile progress words; bit-identical, measured no faster: 0 = per-layer launches is the default), "pdl" (programmatic dependent launch of layer
+ *                  ordered by per-tile progress words; bit-identical, measured no faster: 0 = per-layer launches is the default; an emissive sweep always runs per-layer launches of one-cell threads), "pdl" (programmatic dependent launch of layer
  *                  l+1 on layer l, also used by the nested-grid waves, 1), "l2_mb"
  *   nested grids   "force_amr" (general octree path on a uniform grid), "amr_batch" (directions per batch, 0 = as many
  *                  as fit in memory), "amr_stream" (2:1-balanced grids: 1 = the whole sweep as one launch whose work items wait
@@ -154,6 +154,26 @@ int rtb200_grid_set(rtb200_ctx* ctx, int nx, int64_t nleaf, const int8_t* level,
  * context's device (including what *_device calls put on the caller's streams), then copies, then returns when the
  * copies are complete -- work issued afterwards on any stream sees the new arrays. */
 int rtb200_grid_update_species(rtb200_ctx* ctx, const double* HI, const double* HeI, const double* HeII);
+
+/* Emission (an extension without a reference value, DESIGN.md 4.6): per leaf and frequency group an emission
+ * coefficient eta >= 0 in the units of uvb per cm, [3][nleaf] in the leaf order of rtb200_grid_set.  A segment of path
+ * dpath and optical depth tau = kappa dpath then leaves with
+ *     Iout = Iin e^-tau + eta t,   t = (1 - e^-tau) / kappa  if tau > (double)1.e-10f,  else dpath
+ * (the reference's `nemi` slot, transportRoutinesModule.f90:673-678, with nemi = eta dpath) and contributes to Jmean
+ *     J_seg = L(Iin) + eta dpath phi(tau),   phi(tau) = (tau - 1 + e^-tau) / tau^2,  phi(0) = 1/2,
+ * L(Iin) being what the math mode computes today for the attenuated part; J_seg is the exact path average.  With eta = 0
+ * every result is bit for bit the emission-free one.  rtb200_diffuse, rtb200_diffuse_device, the device-group host call
+ * and rtb200_multi_diffuse_resident honour the emission; the point-source path does not.  rtb200_grid_set clears it,
+ * rtb200_grid_update_species leaves it alone.  The intensity guard of refined leaves (status 7) still applies.
+ *   rtb200_grid_set_emission         eta = host [3][nleaf], copied; NULL clears the emission.  Ordering as
+ *                                    rtb200_grid_update_species.  A device group reads the array slab-wise in rank mode
+ *                                    (all-gathered on the devices, as the species) and every rank returns the same status.
+ *   rtb200_grid_set_emission_device  eta_device = device [3][nleaf], copied on `stream` (a cudaStream_t) and checked there;
+ *                                    returns after synchronising that stream.  Single contexts only (a group: ERR_ARG).
+ * An entry that is negative, NaN or Inf refuses the call with RTB200_ERR_ARG and the previous emission stays: the streamed
+ * nested-grid sweep marks its intensity records with the sign bit, which needs intensities >= 0 (DESIGN.md 4.4). */
+int rtb200_grid_set_emission(rtb200_ctx* ctx, const double* eta);
+int rtb200_grid_set_emission_device(rtb200_ctx* ctx, const double* eta_device, void* stream);
 
 /* Diffuse (UV background) sweep: replaces equiSources.f90:1372-1808 (computeOpacities :4956, the loop over
  * 12*4**(nAngularLevel-1) HEALPix directions, pattern set-up, neighbour threading, transport).
@@ -307,7 +327,7 @@ int rtb200_debug_fast_exp(rtb200_ctx* ctx, int64_t n, const double* tau, double*
 
 /* timing of the last rtb200_diffuse* call, from CUDA events on the launch stream: device milliseconds of the whole
  * call (opacities + sweep + merge) and of the sweep kernels alone, kernel launches issued (all / sweep kernel), and
- * the algorithmic bytes of the call (72 B per leaf per direction, SURVEY.md 8d). */
+ * the algorithmic bytes of the call (72 B per leaf per direction, SURVEY.md 8d; 96 B while emission is set). */
 int rtb200_last_stats(rtb200_ctx* ctx, double* device_ms, double* sweep_ms, int64_t* launches,
                       int64_t* sweep_launches, double* algorithmic_bytes);
 

@@ -61,6 +61,8 @@ static void free_grid(Context& c) {
   cudaFree(c.dKappa); cudaFree(c.tree.child); cudaFree(c.tree.leafX); cudaFree(c.tree.leafY); cudaFree(c.tree.leafZ);
   cudaFree(c.dJ); cudaFree(c.dRates); c.dRates = nullptr;
   cudaFree(c.dKappaT); c.dKappaT = nullptr; c.kappaTBytes = 0;
+  cudaFree(c.dEta); c.dEta = nullptr;
+  cudaFree(c.dEtaT); c.dEtaT = nullptr; c.etaTBytes = 0;
   cudaFree(c.dLogT); c.dLogT = nullptr;
   for (auto& sl : c.pointPool) cudaFree(sl.first);
   c.pointPool.clear();
@@ -174,9 +176,77 @@ int run_diffuse(Context& c, int nAngularLevel, const double* uvb, const double* 
   if (st) return st;
   RTB_CUDA(cudaEventRecord(c.evStop, s));
   if (nseg) *nseg = ns;
-  c.lastAlgBytes = 72.0 * (double)c.nleaf * (double)dirs.size();
+  // 72 B per leaf and direction (SURVEY.md 8d), 96 B with the emission coefficients of the 3 groups
+  c.lastAlgBytes = (c.dEta ? 96.0 : 72.0) * (double)c.nleaf * (double)dirs.size();
   c.statsPending = true;
   c.sweepTimed = uniformPath && !dirs.empty();
+  return RTB200_OK;
+}
+
+// number of entries that are negative, NaN or Inf (the emission check of rtb200_grid_set_emission_device)
+__global__ void count_bad_kernel(const double* __restrict__ x, int64_t n, int32_t* bad) {
+  int32_t mine = 0;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const double v = x[i];
+    if (!(v >= 0. && v <= 1.7976931348623157e308)) mine++;
+  }
+  if (mine) atomicAdd(bad, mine);
+}
+
+static bool host_eta_ok(const double* eta, int64_t n) {
+  for (int64_t i = 0; i < n; i++)
+    if (!(eta[i] >= 0. && eta[i] <= 1.7976931348623157e308)) return false;
+  return true;
+}
+
+int set_emission(Context& c, const double* eta, bool device, cudaStream_t s) {
+  if (c.nleaf == 0) return RTB200_ERR_ARG;
+  RTB_CUDA(cudaSetDevice(c.device));
+  // queued sweeps read the current array (as rtb200_grid_update_species)
+  RTB_CUDA(cudaDeviceSynchronize());
+  const int64_t n = 3 * c.nleaf;
+  const size_t bytes = (size_t)n * sizeof(double);
+  auto drop_plans = [&] {   // the sweeps' plans and graphs know whether emission is set
+    c.uniPlanKey.clear();
+    if (c.graphExec) { cudaGraphExecDestroy(c.graphExec); c.graphExec = nullptr; }
+  };
+  if (!eta) {
+    cudaFree(c.dEta); c.dEta = nullptr;
+    cudaFree(c.dEtaT); c.dEtaT = nullptr; c.etaTBytes = 0;
+    drop_plans();
+    return RTB200_OK;
+  }
+  if (!device && !host_eta_ok(eta, n)) return RTB200_ERR_ARG;
+  // the new array goes to a buffer of its own first: a refused array leaves the previous emission in place
+  double* fresh = nullptr;
+  cudaError_t e = cudaMalloc((void**)&fresh, bytes);
+  if (e != cudaSuccess) { set_cuda_error("cudaMalloc", e, __FILE__, __LINE__); return e == cudaErrorMemoryAllocation ? RTB200_ERR_NOMEM : RTB200_ERR_CUDA; }
+  int st = RTB200_OK;
+  if (!device) {
+    if (cudaMemcpyAsync(fresh, eta, bytes, cudaMemcpyHostToDevice, c.stream) != cudaSuccess ||
+        cudaStreamSynchronize(c.stream) != cudaSuccess)
+      st = RTB200_ERR_CUDA;
+  } else {
+    int32_t* dBad = c.dErr + 12;  // scratch word of the 64-byte error block (chemistry uses words 8..11)
+    int32_t bad = 0;
+    const int blocks = (int)std::min<int64_t>((n + 255) / 256, (int64_t)c.smCount * 8);
+    if (cudaMemcpyAsync(fresh, eta, bytes, cudaMemcpyDeviceToDevice, s) != cudaSuccess ||
+        cudaMemsetAsync(dBad, 0, sizeof(int32_t), s) != cudaSuccess)
+      st = RTB200_ERR_CUDA;
+    if (!st) {
+      count_bad_kernel<<<blocks, 256, 0, s>>>(fresh, n, dBad);
+      if (cudaGetLastError() != cudaSuccess || cudaMemcpyAsync(&bad, dBad, sizeof(int32_t), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
+          cudaStreamSynchronize(s) != cudaSuccess)
+        st = RTB200_ERR_CUDA;
+    }
+    if (!st && bad) st = RTB200_ERR_ARG;
+  }
+  if (st) { cudaFree(fresh); return st; }
+  const bool had = c.dEta != nullptr;
+  cudaFree(c.dEta);
+  c.dEta = fresh;
+  if (!had) drop_plans();
+  else if (c.graphExec) { cudaGraphExecDestroy(c.graphExec); c.graphExec = nullptr; }   // the graph holds the pointer
   return RTB200_OK;
 }
 
@@ -398,6 +468,17 @@ int rtb200_grid_update_species(rtb200_ctx* h, const double* HI, const double* He
   if (HeII) RTB_CUDA(cudaMemcpyAsync(c.dHeII, HeII, nb, cudaMemcpyHostToDevice, c.stream));
   RTB_CUDA(cudaStreamSynchronize(c.stream));
   return RTB200_OK;
+}
+
+int rtb200_grid_set_emission(rtb200_ctx* h, const double* eta) {
+  if (!h) return RTB200_ERR_ARG;
+  if (h->m) return multi_set_emission(h->m, eta);
+  return set_emission(h->c, eta, false, h->c.stream);
+}
+
+int rtb200_grid_set_emission_device(rtb200_ctx* h, const double* eta_device, void* stream) {
+  if (!h || h->m || !eta_device) return RTB200_ERR_ARG;   // a device group takes the host array (slab-wise)
+  return set_emission(h->c, eta_device, true, (cudaStream_t)stream);
 }
 
 int rtb200_diffuse_device(rtb200_ctx* h, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays,

@@ -96,7 +96,8 @@ struct AmrParams {
   uint8_t* code;           // debugging export only: [ndir][3][N] what to read from the upstream leaf
   int32_t* nbc;            // [group][slot][8][4] the same packed for the sweep: upstream SLOT << 3 | code (or -1 / -2) per ray, 16 B per item
   const int32_t* patIdx;   // [6][N] levelOff[level] + coordinate along physical axis a (a = 0..2), then reflected (3..5)
-  const double* kappaA;    // [N][6] leaf-major: opacity of the 3 groups, then 1 / max(opacity, floor) (FAST arithmetic)
+  const double* kappaA;    // [N][6] leaf-major: opacity of the 3 groups, then 1 / max(opacity, floor) (FAST arithmetic);
+                           // [N][9] with the emission coefficients of the 3 groups behind them when emission is set
   double* JA;              // [N][3] running sum over the groups, leaf-major, un-interleaved into J at the end
   double* JS;              // balanced grids: [group][N][4] sum over the 8 directions of a group per leaf (one sector)
   double* JI;              // unbalanced grids: [group][slot][8][3] contribution of every item
@@ -105,7 +106,7 @@ struct AmrParams {
   const int32_t* slotOf[8];  // per reflection combination: position of every leaf in the wave order
   const int32_t* sorted[8];  // ... and its inverse
   const int32_t* patIdxS;    // streamed sweep: [8 combos][3 axes][N] patIdx in wave order (slot) per reflection combination
-  const double* kappaS;      // streamed sweep: [8 combos][N][6] kappaA in wave order
+  const double* kappaS;      // streamed sweep: [8 combos][N][6 or 9] kappaA in wave order
   uint64_t epochSign;        // streamed sweep: sign bit this sweep's intensity records carry (0 or 1 << 63), see amr_stream_kernel
   int32_t* abortFlag;        // streamed sweep: set by the first poll that gave up, ends every other poll
   int noThin;                // experiments: FAST arithmetic on thin layers as well
@@ -230,13 +231,21 @@ __global__ void amr_neighbour_kernel(AmrParams P, int ngroups) {
 
 // leaf-major copies for the sweep's gathers
 constexpr double kAmrKappaFloor = 1e-100;  // FAST arithmetic: kappa = 0 is evaluated as this (every formula takes its limit)
-__global__ void interleave_kappa_kernel(const double* __restrict__ in, double* __restrict__ out, int64_t N) {
+// record length of the per-leaf inputs: opacity, 1 / opacity [, emission coefficient]
+template <bool EMIT>
+__host__ __device__ constexpr int kappa_record() { return EMIT ? 9 : 6; }
+
+template <bool EMIT = false>
+__global__ void interleave_kappa_kernel(const double* __restrict__ in, double* __restrict__ out, int64_t N,
+                                        const double* __restrict__ eta = nullptr) {
+  constexpr int R = kappa_record<EMIT>();
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < 3 * N; i += (int64_t)gridDim.x * blockDim.x) {
     const int64_t leaf = i / 3;
     const int g = (int)(i - 3 * leaf);
     const double k = in[g * N + leaf];
-    out[leaf * 6 + g] = k;
-    out[leaf * 6 + 3 + g] = 1.0 / (k > 0. ? k : kAmrKappaFloor);
+    out[leaf * R + g] = k;
+    out[leaf * R + 3 + g] = 1.0 / (k > 0. ? k : kAmrKappaFloor);
+    if (EMIT) out[leaf * R + 6 + g] = eta[g * N + leaf];
   }
 }
 __global__ void deinterleave3_kernel(const double* __restrict__ in, double* __restrict__ out, int64_t N) {
@@ -247,7 +256,10 @@ __global__ void deinterleave3_kernel(const double* __restrict__ in, double* __re
 }
 
 // streamed sweep: the same per-leaf inputs in wave order, one copy per reflection combination
-__global__ void kappa_slots_kernel(const double* __restrict__ in, double* __restrict__ out, AmrParams P) {
+template <bool EMIT = false>
+__global__ void kappa_slots_kernel(const double* __restrict__ in, double* __restrict__ out, AmrParams P,
+                                   const double* __restrict__ eta = nullptr) {
+  constexpr int R = kappa_record<EMIT>();
   const int64_t N = P.N;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < 8 * N; i += (int64_t)gridDim.x * blockDim.x) {
     const int combo = (int)(i / N);
@@ -255,8 +267,9 @@ __global__ void kappa_slots_kernel(const double* __restrict__ in, double* __rest
 #pragma unroll
     for (int g = 0; g < 3; g++) {
       const double k = in[g * N + leaf];
-      out[i * 6 + g] = k;
-      out[i * 6 + 3 + g] = 1.0 / (k > 0. ? k : kAmrKappaFloor);
+      out[i * R + g] = k;
+      out[i * R + 3 + g] = 1.0 / (k > 0. ? k : kAmrKappaFloor);
+      if (EMIT) out[i * R + 6 + g] = eta[g * N + leaf];
     }
   }
 }
@@ -331,9 +344,22 @@ __device__ __noinline__ ThinSeg amr_thin_segment(double i0, double i1, double i2
   }
   return o;
 }
+// the same with emission (segment_faithful_emit)
+__device__ __noinline__ ThinSeg amr_thin_segment_emit(double i0, double i1, double i2, double k0, double k1, double k2,
+                                                      double dpath, double e0, double e1, double e2) {
+  ThinSeg o;
+  const double Iin[3] = {i0, i1, i2}, kap[3] = {k0, k1, k2}, eta[3] = {e0, e1, e2};
+  for (int g = 0; g < 3; g++) {
+    const SegResult sr = segment_faithful_emit(Iin[g], kap[g], dpath, eta[g]);
+    o.out[g] = sr.Iout;
+    o.J[g] = sr.J;
+  }
+  return o;
+}
 
 // Jc = this direction's contribution to the leaf's mean intensity (the caller adds it up)
-template <bool FAITHFUL, int MODE>
+// EMIT: emission (DESIGN.md 4.6), the coefficients are words 6..8 of the opacity record
+template <bool FAITHFUL, int MODE, bool EMIT = false>
 __device__ __forceinline__ bool amr_transport_leaf(const AmrParams& P, const AmrDir& D, int gi, int lane, int64_t leaf,
                                                    int64_t slot, double (&Jc)[3], const double* __restrict__ sT) {
   const int64_t item = item_index(P, gi, lane, slot);
@@ -362,12 +388,14 @@ __device__ __forceinline__ bool amr_transport_leaf(const AmrParams& P, const Amr
   // (streamed sweep: from the copies in wave order -- no leaf number, nothing to wait for but the neighbour record)
   const int32_t pidx = MODE == 2 ? __ldg(P.patIdxS + ((int64_t)D.combo * 3 + D.patRow % 3) * P.N + slot)
                                  : P.patIdx[(int64_t)D.patRow * P.N + leaf];
-  const double* kA = MODE == 2 ? P.kappaS + ((int64_t)D.combo * P.N + slot) * 6 : P.kappaA + leaf * 6;
-  double kap[3], invk[3];
+  constexpr int R = kappa_record<EMIT>();
+  const double* kA = MODE == 2 ? P.kappaS + ((int64_t)D.combo * P.N + slot) * R : P.kappaA + leaf * R;
+  double kap[3], invk[3], eta[3];
 #pragma unroll
   for (int g = 0; g < 3; g++) {
     kap[g] = kA[g];
     invk[g] = FAITHFUL ? 0. : kA[3 + g];
+    eta[g] = EMIT ? kA[6 + g] : 0.;
   }
   // Programmatic dependent launch: everything above is geometry or per-sweep input; the upstream intensities below
   // come from the waves before this one (no-op for a grid launched without the attribute)
@@ -409,6 +437,9 @@ __device__ __forceinline__ bool amr_transport_leaf(const AmrParams& P, const Amr
   const int thinMask = (!FAITHFUL && !P.noThin) ? (patFlags >> 8) : 0;
   const double kapRaw[3] = {kap[0], kap[1], kap[2]};
   double Jthin[3] = {0., 0., 0.};   // thin segments: sum of the reference-formula segment means (divided by nseg, times w below)
+  double E[3] = {0., 0., 0.};       // emission, FAST arithmetic: sum of phi(tau) dpath w / nseg (times eta below)
+  const int nact = 1 + (nbl[1] != -2) + (nbl[2] != -2);
+  const double wn = EMIT && !FAITHFUL ? D.w * (nact == 1 ? 1.0 : (nact == 2 ? 0.5 : 1.0 / 3.0)) : 0.;
   if (!FAITHFUL) {
 #pragma unroll
     for (int g = 0; g < 3; g++) kap[g] = kap[g] > 0. ? kap[g] : kAmrKappaFloor;
@@ -423,18 +454,25 @@ __device__ __forceinline__ bool amr_transport_leaf(const AmrParams& P, const Amr
     if (FAITHFUL) {
 #pragma unroll
       for (int g = 0; g < 3; g++) {
-        SegResult sr = segment_update<true, 0>(Iin[ray][g], kap[g], dpath[ray], 0., nullptr);
+        SegResult sr = EMIT ? segment_faithful_emit(Iin[ray][g], kap[g], dpath[ray], eta[g])
+                            : segment_update<true, 0>(Iin[ray][g], kap[g], dpath[ray], 0., nullptr);
         out[g] = sr.Iout;
         Jm[g] = __dadd_rn(Jm[g], sr.J);
       }
     } else if (thinMask & (1 << ray)) {
-      const ThinSeg t = amr_thin_segment(Iin[ray][0], Iin[ray][1], Iin[ray][2], kapRaw[0], kapRaw[1], kapRaw[2], dpath[ray]);
+      const ThinSeg t =
+          EMIT ? amr_thin_segment_emit(Iin[ray][0], Iin[ray][1], Iin[ray][2], kapRaw[0], kapRaw[1], kapRaw[2], dpath[ray],
+                                       eta[0], eta[1], eta[2])
+               : amr_thin_segment(Iin[ray][0], Iin[ray][1], Iin[ray][2], kapRaw[0], kapRaw[1], kapRaw[2], dpath[ray]);
 #pragma unroll
       for (int g = 0; g < 3; g++) { out[g] = t.out[g]; Jthin[g] = __dadd_rn(Jthin[g], t.J[g]); }
     } else {
       const double cs = pat.cs[ray][lane];
 #pragma unroll
-      for (int g = 0; g < 3; g++) out[g] = segment_fast<1, true>(Iin[ray][g], kap[g] * dpath[ray], cs, sT, Jm[g]);
+      for (int g = 0; g < 3; g++)
+        out[g] = EMIT ? segment_fast_emit<1, true>(Iin[ray][g], kap[g] * dpath[ray], cs, sT, Jm[g], eta[g], invk[g],
+                                                   dpath[ray], dpath[ray] * wn, E[g])
+                      : segment_fast<1, true>(Iin[ray][g], kap[g] * dpath[ray], cs, sT, Jm[g]);
     }
     if (ray == 0) { xy[0] = out[0]; xy[1] = out[1]; xy[2] = out[2]; }
     imean++;
@@ -458,6 +496,7 @@ __device__ __forceinline__ bool amr_transport_leaf(const AmrParams& P, const Amr
     else {
       Jc[g] = Jm[g] * invk[g];
       if (thinMask) Jc[g] += __dmul_rn(__ddiv_rn(Jthin[g], (double)imean), D.w);   // the thin segments' share of sum(J) / nseg * w
+      if (EMIT) Jc[g] = fma(eta[g], E[g], Jc[g]);
     }
   }
   if (CHECK) {
@@ -476,7 +515,7 @@ struct WaveParams {
 };
 
 // block = 16 leaves of the wave x 8 direction lanes; blockIdx.y = group of the batch
-template <bool FAITHFUL, bool CHECK, int MINB = 8>
+template <bool FAITHFUL, bool CHECK, int MINB = 8, bool EMIT = false>
 __global__ void __launch_bounds__(128, MINB) amr_wave_kernel(AmrParams P, WaveParams Wp, int ngroups) {
   __shared__ double sT[kExpTableSize];
   asm volatile("griddepcontrol.launch_dependents;");               // the next wave may start its prologue early
@@ -499,7 +538,7 @@ __global__ void __launch_bounds__(128, MINB) amr_wave_kernel(AmrParams P, WavePa
   bool deferred = false;
   if (mine) {
     const int d = grp.x + lane;
-    if (!amr_transport_leaf<FAITHFUL, CHECK ? 1 : 0>(P, P.dirs[d], gi, lane, leaf, slot, Jc, sT)) {
+    if (!amr_transport_leaf<FAITHFUL, CHECK ? 1 : 0, EMIT>(P, P.dirs[d], gi, lane, leaf, slot, Jc, sT)) {
       deferred = true;
       int q = atomicAdd(Wp.deferredCount, 1);
       if (q < Wp.deferredCap) Wp.deferred[q] = ((int64_t)d << 32) | slot;
@@ -557,7 +596,7 @@ constexpr int kStreamDirs = 192;   // directions of a batch the streamed kernel 
 // (8.56 against 8.37 ms: the extra stores cost more than the avoided fills); the pause between two polls of a missing
 // record, 40 ns to 3 us (8.13 ms +- 0.02 throughout, profiles/r02y_amr_stream_poll_interval_*: waiting warps are not what
 // limits the kernel); and issuing the first attempt at all three upstream records before examining any (8.22 ms).)
-template <bool FAITHFUL, int MINB>
+template <bool FAITHFUL, int MINB, bool EMIT = false>
 __global__ void __launch_bounds__(128, MINB) amr_stream_kernel(AmrParams P, StreamParams Q, int ndirs, int ngroups) {
   __shared__ double sT[kExpTableSize];
   __shared__ AmrDir sDirs[kStreamDirs];
@@ -596,7 +635,7 @@ __global__ void __launch_bounds__(128, MINB) amr_stream_kernel(AmrParams P, Stre
     const bool have = i < count, mine = have && lane < grp.y;
     const int64_t slot = cur.y + i;
     double Jc[3] = {0., 0., 0.};
-    if (mine) amr_transport_leaf<FAITHFUL, 2>(P, sDirs[grp.x + lane], gi, lane, 0, slot, Jc, sT);
+    if (mine) amr_transport_leaf<FAITHFUL, 2, EMIT>(P, sDirs[grp.x + lane], gi, lane, 0, slot, Jc, sT);
     __syncwarp();
     double v[3];
 #pragma unroll
@@ -619,7 +658,7 @@ __global__ void __launch_bounds__(128, MINB) amr_stream_kernel(AmrParams P, Stre
   }
 }
 
-template <bool FAITHFUL>
+template <bool FAITHFUL, bool EMIT = false>
 __global__ void amr_retry_kernel(AmrParams P, const int64_t* in, const int32_t* inCount, int64_t* out, int32_t* outCount,
                                  int64_t cap) {
   __shared__ double sT[kExpTableSize];
@@ -634,7 +673,7 @@ __global__ void amr_retry_kernel(AmrParams P, const int64_t* in, const int32_t* 
     const int64_t slot = item & 0xffffffffLL;
     const int64_t leaf = P.slotIsLeaf ? slot : P.sorted[P.dirs[d].combo][slot];
     double Jc[3];
-    if (!amr_transport_leaf<FAITHFUL, 1>(P, P.dirs[d], P.dirs[d].group, P.dirs[d].lane, leaf, slot, Jc, sT)) {
+    if (!amr_transport_leaf<FAITHFUL, 1, EMIT>(P, P.dirs[d], P.dirs[d].group, P.dirs[d].lane, leaf, slot, Jc, sT)) {
       int q = atomicAdd(outCount, 1);
       if (q < cap) out[q] = item;
     } else {
@@ -871,7 +910,8 @@ struct AmrBuffers {
   uint8_t* code = nullptr;
   int32_t* nbc = nullptr;
   double* kappaA = nullptr;
-  double* kappaS = nullptr;     // streamed sweep: [8][N][6]
+  double* kappaS = nullptr;     // streamed sweep: [8][N][kappaSRecord]
+  int kappaSRecord = 0;
   double* JA = nullptr;
   double* JS = nullptr;
   double* JI = nullptr;
@@ -1047,7 +1087,7 @@ static int alloc_batch(AmrBuffers& B, const DirTables& T, int64_t N, int ngroups
     return RTB200_OK;
   }
   RTB_CUDA(cudaMalloc((void**)&B.nbc, slots * 4 * N * sizeof(int32_t)));
-  RTB_CUDA(cudaMalloc((void**)&B.kappaA, (size_t)6 * N * sizeof(double)));
+  RTB_CUDA(cudaMalloc((void**)&B.kappaA, (size_t)9 * N * sizeof(double)));   // room for the emission coefficients
   RTB_CUDA(cudaMalloc((void**)&B.JA, (size_t)3 * N * sizeof(double)));
   if (balanced) RTB_CUDA(cudaMalloc((void**)&B.JS, (size_t)ngroups * N * 4 * sizeof(double)));
   else RTB_CUDA(cudaMalloc((void**)&B.JI, slots * N * 3 * sizeof(double)));
@@ -1070,6 +1110,7 @@ static int choose_batch(Context& c, int ngroups) {
 }
 
 // groups [g0, g0 + ng) of the tables
+template <bool EMIT>
 static int run_batch(Context& c, AmrState& S, const DirTables& T, int g0, int ng, const double* uvb, double* dJ,
                      cudaStream_t s, bool faithful, AmrBuffers& B, int64_t defCap, int64_t* launches) {
   const int64_t N = c.nleaf;
@@ -1183,25 +1224,30 @@ static int run_batch(Context& c, AmrState& S, const DirTables& T, int g0, int ng
       patidx_slots_kernel<<<cb, 256, 0, s>>>(S.plan.dPatIdx, S.plan.dPatIdxS, P);
       (*launches)++;
     }
-    if (!B.kappaS) RTB_CUDA(cudaMalloc((void**)&B.kappaS, (size_t)8 * N * 6 * sizeof(double)));
-    kappa_slots_kernel<<<cb, 256, 0, s>>>(c.dKappa, B.kappaS, P);
+    constexpr int R = kappa_record<EMIT>();
+    if (B.kappaS && B.kappaSRecord < R) { cudaFree(B.kappaS); B.kappaS = nullptr; }
+    if (!B.kappaS) {
+      RTB_CUDA(cudaMalloc((void**)&B.kappaS, (size_t)8 * N * R * sizeof(double)));
+      B.kappaSRecord = R;
+    }
+    kappa_slots_kernel<EMIT><<<cb, 256, 0, s>>>(c.dKappa, B.kappaS, P, c.dEta);
     (*launches)++;
     P.patIdxS = S.plan.dPatIdxS; P.kappaS = B.kappaS;
     StreamParams Q;
     Q.items = B.items; Q.nitems = B.nitems; Q.counter = B.defCount;
     int perSm = 0;
     if (faithful) {
-      RTB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, amr_stream_kernel<true, 4>, 128, 0));
-      amr_stream_kernel<true, 4><<<std::min(perSm * c.smCount, (int)B.nitems), 128, 0, s>>>(P, Q, nd, ng);
+      RTB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, amr_stream_kernel<true, 4, EMIT>, 128, 0));
+      amr_stream_kernel<true, 4, EMIT><<<std::min(perSm * c.smCount, (int)B.nitems), 128, 0, s>>>(P, Q, nd, ng);
     } else if (c.tune.amrMinBlocks >= 8) {
-      RTB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, amr_stream_kernel<false, 8>, 128, 0));
-      amr_stream_kernel<false, 8><<<std::min(perSm * c.smCount, (int)B.nitems), 128, 0, s>>>(P, Q, nd, ng);
+      RTB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, amr_stream_kernel<false, 8, EMIT>, 128, 0));
+      amr_stream_kernel<false, 8, EMIT><<<std::min(perSm * c.smCount, (int)B.nitems), 128, 0, s>>>(P, Q, nd, ng);
     } else if (c.tune.amrMinBlocks == 5) {
-      RTB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, amr_stream_kernel<false, 5>, 128, 0));
-      amr_stream_kernel<false, 5><<<std::min(perSm * c.smCount, (int)B.nitems), 128, 0, s>>>(P, Q, nd, ng);
+      RTB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, amr_stream_kernel<false, 5, EMIT>, 128, 0));
+      amr_stream_kernel<false, 5, EMIT><<<std::min(perSm * c.smCount, (int)B.nitems), 128, 0, s>>>(P, Q, nd, ng);
     } else {
-      RTB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, amr_stream_kernel<false, 6>, 128, 0));
-      amr_stream_kernel<false, 6><<<std::min(perSm * c.smCount, (int)B.nitems), 128, 0, s>>>(P, Q, nd, ng);
+      RTB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, amr_stream_kernel<false, 6, EMIT>, 128, 0));
+      amr_stream_kernel<false, 6, EMIT><<<std::min(perSm * c.smCount, (int)B.nitems), 128, 0, s>>>(P, Q, nd, ng);
     }
     (*launches)++;
     const int blocks = (int)std::min<int64_t>((N + 127) / 128, (int64_t)c.smCount * 16);
@@ -1240,21 +1286,21 @@ static int run_batch(Context& c, AmrState& S, const DirTables& T, int g0, int ng
     cfg.attrs = at;
     cfg.numAttrs = (c.tune.pdl && prevWasWave) ? 1 : 0;
     if (faithful) {
-      if (check) RTB_CUDA(cudaLaunchKernelEx(&cfg, amr_wave_kernel<true, true>, P, Wp, ng));
-      else RTB_CUDA(cudaLaunchKernelEx(&cfg, amr_wave_kernel<true, false>, P, Wp, ng));
+      if (check) RTB_CUDA(cudaLaunchKernelEx(&cfg, amr_wave_kernel<true, true, 8, EMIT>, P, Wp, ng));
+      else RTB_CUDA(cudaLaunchKernelEx(&cfg, amr_wave_kernel<true, false, 8, EMIT>, P, Wp, ng));
     } else {
-      if (check) RTB_CUDA(cudaLaunchKernelEx(&cfg, amr_wave_kernel<false, true>, P, Wp, ng));
+      if (check) RTB_CUDA(cudaLaunchKernelEx(&cfg, amr_wave_kernel<false, true, 8, EMIT>, P, Wp, ng));
       else if (c.tune.amrMinBlocks > 0 ? c.tune.amrMinBlocks <= 6 : smallWaves)
-        RTB_CUDA(cudaLaunchKernelEx(&cfg, amr_wave_kernel<false, false, 6>, P, Wp, ng));
-      else RTB_CUDA(cudaLaunchKernelEx(&cfg, amr_wave_kernel<false, false, 8>, P, Wp, ng));
+        RTB_CUDA(cudaLaunchKernelEx(&cfg, amr_wave_kernel<false, false, 6, EMIT>, P, Wp, ng));
+      else RTB_CUDA(cudaLaunchKernelEx(&cfg, amr_wave_kernel<false, false, 8, EMIT>, P, Wp, ng));
     }
     prevWasWave = true;
     (*launches)++;
     if (check && (w & 15) == 15) {
       // retry what has been deferred so far (nothing on 2:1-balanced grids)
       RTB_CUDA(cudaMemsetAsync(B.defCount + (cur ^ 1), 0, sizeof(int32_t), s));
-      if (faithful) amr_retry_kernel<true><<<64, 128, 0, s>>>(P, lists[cur], B.defCount + cur, lists[cur ^ 1], B.defCount + (cur ^ 1), defCap);
-      else amr_retry_kernel<false><<<64, 128, 0, s>>>(P, lists[cur], B.defCount + cur, lists[cur ^ 1], B.defCount + (cur ^ 1), defCap);
+      if (faithful) amr_retry_kernel<true, EMIT><<<64, 128, 0, s>>>(P, lists[cur], B.defCount + cur, lists[cur ^ 1], B.defCount + (cur ^ 1), defCap);
+      else amr_retry_kernel<false, EMIT><<<64, 128, 0, s>>>(P, lists[cur], B.defCount + cur, lists[cur ^ 1], B.defCount + (cur ^ 1), defCap);
       (*launches)++;
       cur ^= 1;
       prevWasWave = false;
@@ -1268,8 +1314,8 @@ static int run_batch(Context& c, AmrState& S, const DirTables& T, int g0, int ng
     if (cnt == 0) break;
     if (cnt > defCap) return RTB200_ERR_NOMEM;
     RTB_CUDA(cudaMemsetAsync(B.defCount + (cur ^ 1), 0, sizeof(int32_t), s));
-    if (faithful) amr_retry_kernel<true><<<256, 128, 0, s>>>(P, lists[cur], B.defCount + cur, lists[cur ^ 1], B.defCount + (cur ^ 1), defCap);
-    else amr_retry_kernel<false><<<256, 128, 0, s>>>(P, lists[cur], B.defCount + cur, lists[cur ^ 1], B.defCount + (cur ^ 1), defCap);
+    if (faithful) amr_retry_kernel<true, EMIT><<<256, 128, 0, s>>>(P, lists[cur], B.defCount + cur, lists[cur ^ 1], B.defCount + (cur ^ 1), defCap);
+    else amr_retry_kernel<false, EMIT><<<256, 128, 0, s>>>(P, lists[cur], B.defCount + cur, lists[cur ^ 1], B.defCount + (cur ^ 1), defCap);
     (*launches)++;
     cur ^= 1;
     if (iter == 99999) return RTB200_ERR_ARG;
@@ -1329,14 +1375,17 @@ int diffuse_amr(Context& c, int nAngularLevel, const double* uvb, const std::vec
   }
   int64_t launches = 0;
   const bool faithful = c.mathMode == RTB200_MATH_FAITHFUL;
+  const bool emit = c.dEta != nullptr;   // emission set (rtb200_grid_set_emission): the sweep kernels' EMIT instantiations
   const int cpyBlocks = (int)std::min<int64_t>((3 * N + 255) / 256, (int64_t)c.smCount * 16);
   if (!st) {
-    interleave_kappa_kernel<<<cpyBlocks, 256, 0, s>>>(c.dKappa, B.kappaA, N);
+    if (emit) interleave_kappa_kernel<true><<<cpyBlocks, 256, 0, s>>>(c.dKappa, B.kappaA, N, c.dEta);
+    else interleave_kappa_kernel<false><<<cpyBlocks, 256, 0, s>>>(c.dKappa, B.kappaA, N);
     RTB_CUDA(cudaMemsetAsync(B.JA, 0, 3 * N * sizeof(double), s));
     launches += 1;
   }
   for (int g0 = 0; g0 < ngroups && !st; g0 += batch)
-    st = run_batch(c, S, T, g0, std::min(batch, ngroups - g0), uvb, dJout, s, faithful, B, defCap, &launches);
+    st = (emit ? run_batch<true> : run_batch<false>)(c, S, T, g0, std::min(batch, ngroups - g0), uvb, dJout, s, faithful, B,
+                                                     defCap, &launches);
   if (!st) {
     deinterleave3_kernel<<<cpyBlocks, 256, 0, s>>>(B.JA, dJout, N);
     launches += 1;

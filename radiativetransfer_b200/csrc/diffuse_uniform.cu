@@ -91,31 +91,53 @@ __global__ void fill_planes_kernel(double* __restrict__ planes, int64_t perGroup
 //
 // FAST arithmetic (segment_math.cuh: segment_fast): A[g] collects Iin (1 - e^-tau) cs over all segments and
 // directions of the layer; the caller multiplies by 2^-200 / kappa once per layer.
-template <int EXPV, int NSEG, bool SECL, bool GUARD>
+// Emission (EMIT, DESIGN.md 4.6): the cell's and the (b-1) cell's emission coefficients and 1 / kappa ride along in Em;
+// every segment also adds phi(tau) dpath weight / nseg to E[g], which the caller multiplies by eta once per layer.
+struct Em {
+  double eta[3], etaR[3];    // own cell, (b-1) cell (0 outside the domain)
+  double invk[3], invkR[3];  // FAST arithmetic: 1 / kappa with kappa floored as in the segment
+};
+
+template <int EXPV, bool GUARD, bool EMIT>
+__device__ __forceinline__ double seg_fast(double Iin, double kap, double d, double cs, const double* __restrict__ T,
+                                           double& A, double eta, double invk, double dw, double& E) {
+  if (EMIT) return segment_fast_emit<EXPV, GUARD>(Iin, kap * d, cs, T, A, eta, invk, d, dw, E);
+  return segment_fast<EXPV, GUARD>(Iin, kap * d, cs, T, A);
+}
+template <int EXPV, bool GUARD, bool EMIT>
+__device__ __forceinline__ double att_fast(double Iin, double kap, double d, const double* __restrict__ T, double eta,
+                                           double invk) {
+  if (EMIT) return attenuate_fast_emit<EXPV, GUARD>(Iin, kap * d, T, eta, invk, d);
+  return attenuate_fast<EXPV, GUARD>(Iin, kap * d, T);
+}
+
+template <int EXPV, int NSEG, bool SECL, bool GUARD, bool EMIT = false>
 __device__ __forceinline__ void direction_fast(const LayerSeg& P, const double (&cur)[3], const double (&upR)[3],
                                                const double (&kap)[3], const double (&kR)[3], double (&I)[3],
-                                               double (&A)[3], const double* __restrict__ T) {
+                                               double (&A)[3], const double* __restrict__ T, const Em& em,
+                                               double (&E)[3]) {
   const unsigned full = 0xffffffffu;
+  const double wn = EMIT ? P.w * (1.0 / NSEG) : 0.;
 #pragma unroll
   for (int g = 0; g < 3; g++) {
-    const double I1 = segment_fast<EXPV, GUARD>(cur[g], kap[g] * P.d[0], P.cs[0], T, A[g]);
+    const double I1 = seg_fast<EXPV, GUARD, EMIT>(cur[g], kap[g], P.d[0], P.cs[0], T, A[g], em.eta[g], em.invk[g], P.d[0] * wn, E[g]);
     I[g] = I1;
     if (NSEG >= 2) {
       double rup = 0.;  // xy-segment output of the (b-1) cell
-      if (!SECL || NSEG == 3) rup = attenuate_fast<EXPV, GUARD>(upR[g], kR[g] * P.d[0], T);
+      if (!SECL || NSEG == 3) rup = att_fast<EXPV, GUARD, EMIT>(upR[g], kR[g], P.d[0], T, em.etaR[g], em.invkR[g]);
       const double in2 = SECL ? __shfl_up_sync(full, I1, 1) : rup;
-      const double I2 = segment_fast<EXPV, GUARD>(in2, kap[g] * P.d[1], P.cs[1], T, A[g]);
+      const double I2 = seg_fast<EXPV, GUARD, EMIT>(in2, kap[g], P.d[1], P.cs[1], T, A[g], em.eta[g], em.invk[g], P.d[1] * wn, E[g]);
       I[g] = I2;
       if (NSEG == 3) {
         double in3;
         if (SECL) {
           // third segment from the (b-1) cell's SECOND segment, which was fed by the (b-1, a-1) cell's xy segment
           const double x = __shfl_up_sync(full, rup, 1);
-          in3 = attenuate_fast<EXPV, GUARD>(x, kR[g] * P.d[1], T);
+          in3 = att_fast<EXPV, GUARD, EMIT>(x, kR[g], P.d[1], T, em.etaR[g], em.invkR[g]);
         } else {
           in3 = __shfl_up_sync(full, I2, 1);  // the (a-1) cell's second segment
         }
-        I[g] = segment_fast<EXPV, GUARD>(in3, kap[g] * P.d[2], P.cs[2], T, A[g]);
+        I[g] = seg_fast<EXPV, GUARD, EMIT>(in3, kap[g], P.d[2], P.cs[2], T, A[g], em.eta[g], em.invk[g], P.d[2] * wn, E[g]);
       }
     }
   }
@@ -123,32 +145,43 @@ __device__ __forceinline__ void direction_fast(const LayerSeg& P, const double (
 
 // The reference's own operation sequence (RTB200_MATH_FAITHFUL, and the thin layers of FAST mode): adds
 // (sum of the segments' J) / nseg * weight to acc (transportRoutinesModule.f90:953-955).
-template <int NSEG, bool SECL>
+template <bool EMIT>
+__device__ __forceinline__ SegResult seg_faithful(double Iin, double kap, double d, double eta) {
+  if (EMIT) return segment_faithful_emit(Iin, kap, d, eta);
+  return segment_update<true, 0>(Iin, kap, d, 0., nullptr);
+}
+template <bool EMIT>
+__device__ __forceinline__ double att_faithful(double Iin, double kap, double d, double eta) {
+  if (EMIT) return attenuate_faithful_emit(Iin, kap, d, eta);
+  return __dmul_rn(Iin, exp(-__dmul_rn(kap, d)));
+}
+
+template <int NSEG, bool SECL, bool EMIT = false>
 __device__ __forceinline__ void direction_faithful(const LayerSeg& P, const double (&cur)[3], const double (&upR)[3],
                                                    const double (&kap)[3], const double (&kR)[3], double (&I)[3],
-                                                   double (&acc)[3]) {
+                                                   double (&acc)[3], const double (&eta)[3], const double (&etaR)[3]) {
   const unsigned full = 0xffffffffu;
 #pragma unroll
   for (int g = 0; g < 3; g++) {
-    SegResult r1 = segment_update<true, 0>(cur[g], kap[g], P.d[0], 0., nullptr);
+    SegResult r1 = seg_faithful<EMIT>(cur[g], kap[g], P.d[0], eta[g]);
     double Jsum = r1.J;
     I[g] = r1.Iout;
     if (NSEG >= 2) {
       double rup = 0.;
-      if (!SECL || NSEG == 3) rup = __dmul_rn(upR[g], exp(-__dmul_rn(kR[g], P.d[0])));
+      if (!SECL || NSEG == 3) rup = att_faithful<EMIT>(upR[g], kR[g], P.d[0], etaR[g]);
       const double in2 = SECL ? __shfl_up_sync(full, r1.Iout, 1) : rup;
-      SegResult r2 = segment_update<true, 0>(in2, kap[g], P.d[1], 0., nullptr);
+      SegResult r2 = seg_faithful<EMIT>(in2, kap[g], P.d[1], eta[g]);
       I[g] = r2.Iout;
       double J3 = 0.;
       if (NSEG == 3) {
         double in3;
         if (SECL) {
           const double x = __shfl_up_sync(full, rup, 1);
-          in3 = __dmul_rn(x, exp(-__dmul_rn(kR[g], P.d[1])));
+          in3 = att_faithful<EMIT>(x, kR[g], P.d[1], etaR[g]);
         } else {
           in3 = __shfl_up_sync(full, r2.Iout, 1);
         }
-        SegResult r3 = segment_update<true, 0>(in3, kap[g], P.d[2], 0., nullptr);
+        SegResult r3 = seg_faithful<EMIT>(in3, kap[g], P.d[2], eta[g]);
         I[g] = r3.Iout;
         J3 = r3.J;
       }
@@ -167,29 +200,29 @@ __device__ __forceinline__ void direction_faithful(const LayerSeg& P, const doub
 // dispatch on the layer's chain kind (warp-uniform).  kmax = the largest opacity this thread multiplies a path with.
 // If kmax * (longest segment of the layer) <= 64 for every lane of the warp, the overflow guards of segment_fast are
 // dropped (4 fewer instructions per segment update); `thick` warps take the guarded instantiation.
-template <int EXPV, bool GUARD>
+template <int EXPV, bool GUARD, bool EMIT>
 __device__ __forceinline__ void direction_kinds_fast(const LayerSeg& P, bool secL, const double (&cur)[3],
                                                      const double (&upR)[3], const double (&kap)[3],
                                                      const double (&kR)[3], double (&I)[3], double (&A)[3],
-                                                     const double* __restrict__ T) {
+                                                     const double* __restrict__ T, const Em& em, double (&E)[3]) {
   const int kind = P.kind;
-  if (kind == 0) direction_fast<EXPV, 1, true, GUARD>(P, cur, upR, kap, kR, I, A, T);
+  if (kind == 0) direction_fast<EXPV, 1, true, GUARD, EMIT>(P, cur, upR, kap, kR, I, A, T, em, E);
   else if (kind == 1 || kind == 3) {
-    if (secL) direction_fast<EXPV, 2, true, GUARD>(P, cur, upR, kap, kR, I, A, T);
-    else direction_fast<EXPV, 2, false, GUARD>(P, cur, upR, kap, kR, I, A, T);
+    if (secL) direction_fast<EXPV, 2, true, GUARD, EMIT>(P, cur, upR, kap, kR, I, A, T, em, E);
+    else direction_fast<EXPV, 2, false, GUARD, EMIT>(P, cur, upR, kap, kR, I, A, T, em, E);
   } else {
-    if (secL) direction_fast<EXPV, 3, true, GUARD>(P, cur, upR, kap, kR, I, A, T);
-    else direction_fast<EXPV, 3, false, GUARD>(P, cur, upR, kap, kR, I, A, T);
+    if (secL) direction_fast<EXPV, 3, true, GUARD, EMIT>(P, cur, upR, kap, kR, I, A, T, em, E);
+    else direction_fast<EXPV, 3, false, GUARD, EMIT>(P, cur, upR, kap, kR, I, A, T, em, E);
   }
 }
 
-template <int EXPV>
+template <int EXPV, bool EMIT>
 __device__ __forceinline__ void direction_dispatch_fast(const LayerSeg& P, bool secL, double kmax, const double (&cur)[3],
                                                         const double (&upR)[3], const double (&kap)[3],
                                                         const double (&kR)[3], double (&I)[3], double (&A)[3],
-                                                        const double* __restrict__ T) {
-  if (__any_sync(0xffffffffu, kmax * P.dmax > 64.)) direction_kinds_fast<EXPV, true>(P, secL, cur, upR, kap, kR, I, A, T);
-  else direction_kinds_fast<EXPV, false>(P, secL, cur, upR, kap, kR, I, A, T);
+                                                        const double* __restrict__ T, const Em& em, double (&E)[3]) {
+  if (__any_sync(0xffffffffu, kmax * P.dmax > 64.)) direction_kinds_fast<EXPV, true, EMIT>(P, secL, cur, upR, kap, kR, I, A, T, em, E);
+  else direction_kinds_fast<EXPV, false, EMIT>(P, secL, cur, upR, kap, kR, I, A, T, em, E);
 }
 
 // Out of line and by value: the rare faithful branch must not force the fast path's per-direction arrays into
@@ -205,32 +238,53 @@ struct FaithOut {
 #else
 #define RTB_FAITHFUL_CALL __forceinline__
 #endif
-__device__ RTB_FAITHFUL_CALL FaithOut direction_call_faithful(double d0, double d1, double d2, double w, int kind,
-                                                              bool secL, Tri cur_, Tri upR_, Tri kap_, Tri kR_, Tri acc_) {
+template <bool EMIT>
+__device__ __forceinline__ FaithOut direction_faithful_kinds(double d0, double d1, double d2, double w, int kind, bool secL,
+                                                             const Tri& cur_, const Tri& upR_, const Tri& kap_,
+                                                             const Tri& kR_, const Tri& acc_, const Tri& eta_,
+                                                             const Tri& etaR_) {
   LayerSeg P;
   P.d[0] = d0; P.d[1] = d1; P.d[2] = d2; P.w = w; P.kind = kind;
   double cur[3] = {cur_.v[0], cur_.v[1], cur_.v[2]}, upR[3] = {upR_.v[0], upR_.v[1], upR_.v[2]};
   double kap[3] = {kap_.v[0], kap_.v[1], kap_.v[2]}, kR[3] = {kR_.v[0], kR_.v[1], kR_.v[2]};
   double acc[3] = {acc_.v[0], acc_.v[1], acc_.v[2]}, I[3] = {0., 0., 0.};
-  if (kind == 0) direction_faithful<1, true>(P, cur, upR, kap, kR, I, acc);
+  double eta[3] = {eta_.v[0], eta_.v[1], eta_.v[2]}, etaR[3] = {etaR_.v[0], etaR_.v[1], etaR_.v[2]};
+  if (kind == 0) direction_faithful<1, true, EMIT>(P, cur, upR, kap, kR, I, acc, eta, etaR);
   else if (kind == 1 || kind == 3) {
-    if (secL) direction_faithful<2, true>(P, cur, upR, kap, kR, I, acc);
-    else direction_faithful<2, false>(P, cur, upR, kap, kR, I, acc);
+    if (secL) direction_faithful<2, true, EMIT>(P, cur, upR, kap, kR, I, acc, eta, etaR);
+    else direction_faithful<2, false, EMIT>(P, cur, upR, kap, kR, I, acc, eta, etaR);
   } else {
-    if (secL) direction_faithful<3, true>(P, cur, upR, kap, kR, I, acc);
-    else direction_faithful<3, false>(P, cur, upR, kap, kR, I, acc);
+    if (secL) direction_faithful<3, true, EMIT>(P, cur, upR, kap, kR, I, acc, eta, etaR);
+    else direction_faithful<3, false, EMIT>(P, cur, upR, kap, kR, I, acc, eta, etaR);
   }
   FaithOut o;
 #pragma unroll
   for (int g = 0; g < 3; g++) { o.I.v[g] = I[g]; o.acc.v[g] = acc[g]; }
   return o;
 }
+__device__ RTB_FAITHFUL_CALL FaithOut direction_call_faithful(double d0, double d1, double d2, double w, int kind,
+                                                              bool secL, Tri cur_, Tri upR_, Tri kap_, Tri kR_, Tri acc_) {
+  const Tri zero = {{0., 0., 0.}};
+  return direction_faithful_kinds<false>(d0, d1, d2, w, kind, secL, cur_, upR_, kap_, kR_, acc_, zero, zero);
+}
+__device__ RTB_FAITHFUL_CALL FaithOut direction_call_faithful_emit(double d0, double d1, double d2, double w, int kind,
+                                                                   bool secL, Tri cur_, Tri upR_, Tri kap_, Tri kR_,
+                                                                   Tri acc_, Tri eta_, Tri etaR_) {
+  return direction_faithful_kinds<true>(d0, d1, d2, w, kind, secL, cur_, upR_, kap_, kR_, acc_, eta_, etaR_);
+}
+template <bool EMIT = false>
 __device__ __forceinline__ void direction_dispatch_faithful(const LayerSeg& P, bool secL, const double (&cur)[3],
                                                             const double (&upR)[3], const double (&kap)[3],
-                                                            const double (&kR)[3], double (&I)[3], double (&acc)[3]) {
-  const FaithOut o = direction_call_faithful(P.d[0], P.d[1], P.d[2], P.w, P.kind, secL, Tri{{cur[0], cur[1], cur[2]}},
-                                             Tri{{upR[0], upR[1], upR[2]}}, Tri{{kap[0], kap[1], kap[2]}},
-                                             Tri{{kR[0], kR[1], kR[2]}}, Tri{{acc[0], acc[1], acc[2]}});
+                                                            const double (&kR)[3], double (&I)[3], double (&acc)[3],
+                                                            const double* eta = nullptr, const double* etaR = nullptr) {
+  const FaithOut o =
+      EMIT ? direction_call_faithful_emit(P.d[0], P.d[1], P.d[2], P.w, P.kind, secL, Tri{{cur[0], cur[1], cur[2]}},
+                                          Tri{{upR[0], upR[1], upR[2]}}, Tri{{kap[0], kap[1], kap[2]}},
+                                          Tri{{kR[0], kR[1], kR[2]}}, Tri{{acc[0], acc[1], acc[2]}},
+                                          Tri{{eta[0], eta[1], eta[2]}}, Tri{{etaR[0], etaR[1], etaR[2]}})
+           : direction_call_faithful(P.d[0], P.d[1], P.d[2], P.w, P.kind, secL, Tri{{cur[0], cur[1], cur[2]}},
+                                     Tri{{upR[0], upR[1], upR[2]}}, Tri{{kap[0], kap[1], kap[2]}},
+                                     Tri{{kR[0], kR[1], kR[2]}}, Tri{{acc[0], acc[1], acc[2]}});
 #pragma unroll
   for (int g = 0; g < 3; g++) { I[g] = o.I.v[g]; acc[g] = o.acc.v[g]; }
 }
@@ -254,9 +308,14 @@ static_assert(sizeof(BatchParams) + 64 <= 32764, "kernel parameter space");
 // pairs) is evaluated with the reference's own operation sequence even in FAST mode: there tau is tiny and the
 // rounding noise of the reference's (Iin-Iout)/log(Iin/Iout), ~1.1e-16/tau, would otherwise show up as a parity
 // difference.  That branch is warp-uniform (P.thin is a per-layer table entry) and kept out of line.
-template <bool FAITHFUL, int EXPV, int MINB>
-__global__ void __launch_bounds__(256, MINB)
-sweep_cell_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1, int npl3) {
+// Emission (DESIGN.md 4.6): the emission coefficients of every task, in the layout of its kappa (leaf order or z-major)
+struct EtaParams {
+  const double* eta[kMaxBatch];
+};
+
+template <bool FAITHFUL, int EXPV, bool EMIT>
+__device__ __forceinline__ void sweep_cell_body(const BatchParams& bp, const double* __restrict__ etaTask, int N, int n,
+                                                int np1, int npl3) {
   // n, np1 = n + 1 and npl3 = 3 (n+1)^2 are the same for every task: as top-level parameters they are constant-bank
   // operands instead of values re-derived from the task table for every direction
   const StepParams& sp = bp.t[blockIdx.z];
@@ -287,6 +346,18 @@ sweep_cell_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1,
   }
   const double kmax = fmax(fmax(fmax(kap[0], kap[1]), fmax(kap[2], kR[0])), fmax(kR[1], kR[2]));
   double A[3] = {0., 0., 0.}, acc[3] = {0., 0., 0.};
+  Em em;
+  double E[3] = {0., 0., 0.};
+  if (EMIT) {
+#pragma unroll
+    for (int g = 0; g < 3; g++) {
+      const double* eg = etaTask + (int64_t)g * N + leaf;
+      em.eta[g] = cell ? eg[0] : 0.;
+      em.etaR[g] = (cell && b > 0) ? eg[-sB] : 0.;                // the pad row and column emit nothing
+      em.invk[g] = FAITHFUL ? 0. : 1.0 / kap[g];
+      em.invkR[g] = FAITHFUL ? 0. : 1.0 / (kR[g] > 0. ? kR[g] : kKappaFloor);   // as the (b-1) cell's own thread
+    }
+  }
   const int pidx = (b + 1) * np1 + (inRow ? a + 1 : 0);
   const int ndir = sp.ndir;
   const int dstride = npl3;                                    // one direction's plane (3 groups per cell)
@@ -313,8 +384,8 @@ sweep_cell_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1,
 #pragma unroll
       for (int g = 0; g < 3; g++) upR[g] = pin[g - up];
     }
-    if (FAITHFUL || P.thin) direction_dispatch_faithful(P, secL, cur, upR, kapF, kR, I, acc);
-    else direction_dispatch_fast<EXPV>(P, secL, kmax, cur, upR, kap, kR, I, A, sT);
+    if (FAITHFUL || P.thin) direction_dispatch_faithful<EMIT>(P, secL, cur, upR, kapF, kR, I, acc, em.eta, em.etaR);
+    else direction_dispatch_fast<EXPV, EMIT>(P, secL, kmax, cur, upR, kap, kR, I, A, sT, em, E);
     if (writer) {
 #pragma unroll
       for (int g = 0; g < 3; g++) pout[g] = I[g];
@@ -324,10 +395,25 @@ sweep_cell_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1,
 #pragma unroll
     for (int g = 0; g < 3; g++) {
       if (!FAITHFUL) acc[g] = fma(A[g], kTwoM200 / kap[g], acc[g]);
+      if (EMIT && !FAITHFUL) acc[g] = fma(em.eta[g], E[g], acc[g]);
       double* p = sp.acc + (int64_t)g * N + leaf;
       *p = sp.firstInSlot ? acc[g] : __dadd_rn(*p, acc[g]);
     }
   }
+}
+
+template <bool FAITHFUL, int EXPV, int MINB>
+__global__ void __launch_bounds__(256, MINB)
+sweep_cell_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1, int npl3) {
+  sweep_cell_body<FAITHFUL, EXPV, false>(bp, nullptr, N, n, np1, npl3);
+}
+
+// the emissive sweep: one cell per thread, 2 blocks of 256 threads per SM (the emission terms need registers)
+template <bool FAITHFUL, int EXPV>
+__global__ void __launch_bounds__(256, 2)
+sweep_cell_emit_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1, int npl3,
+                       const __grid_constant__ EtaParams ep) {
+  sweep_cell_body<FAITHFUL, EXPV, true>(bp, ep.eta[blockIdx.z], N, n, np1, npl3);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -777,9 +863,9 @@ static LayerSeg make_layer_seg(const RayPattern& p, double cellSize, double weig
 // `warps` = rows of the layer a block covers with one warp each (8, 4 or 2): small direction shards (multi-GPU ranks) put
 // only a few hundred 8-warp blocks on the device per layer, 1.5 "waves" of which cost as much as 2; smaller blocks
 // spread the same rows evenly over the SMs
-template <class Kernel>
+template <class Kernel, class... Extra>
 static cudaError_t launch_layer(Kernel kern, dim3 grid, cudaStream_t s, bool pdl, const BatchParams& bp, int N, int n,
-                                int warps = 8) {
+                                int warps, const Extra&... extra) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid;
   cfg.blockDim = dim3(32, warps);
@@ -790,19 +876,21 @@ static cudaError_t launch_layer(Kernel kern, dim3 grid, cudaStream_t s, bool pdl
   at[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
   cfg.numAttrs = pdl ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kern, bp, N, n, n + 1, 3 * (n + 1) * (n + 1));
+  return cudaLaunchKernelEx(&cfg, kern, bp, N, n, n + 1, 3 * (n + 1) * (n + 1), extra...);
 }
 
 // `pdl`: programmatic dependent launch on the previous launch of the stream (only for a layer whose predecessor in
 // the stream is the previous layer's sweep kernel)
+// `ep` != nullptr: the emissive sweep (sweep_cell_emit_kernel: one cell per thread, "dense" does not apply)
 static cudaError_t launch_cells(int dense, int expv, bool faithful, bool pdl, dim3 grid, cudaStream_t s,
-                                const BatchParams& bp, int N, int n, int cells, int warps, int smCount) {
+                                const BatchParams& bp, int N, int n, int cells, int warps, int smCount,
+                                const EtaParams* ep = nullptr) {
   // `dense`: 0 = compiler's choice of registers (2 blocks per SM), 1 = cap for 3 blocks, 2 = cap for 4 blocks
   // automatic: two cells per thread pay (1-2%) when the launch has many zone tasks; a small direction shard (3 zone
   // tasks on each of 8 GPUs) is 1.3 waves of two-cell threads but fills the device evenly with one-cell threads
   // (measured on the shards of an 8-GPU run: 7.03 against 7.21 ms mean, 7.31 against 7.93 ms for the slowest rank)
   if (cells == 0) cells = (n >= 192 && grid.z >= 6) ? 2 : 1;
-  if (faithful || expv != 1) cells = 1;
+  if (faithful || expv != 1 || ep) cells = 1;
   const int rowsTotal = cells == 2 ? (n + 1) / 2 : n;           // rows of threads per task and layer
   if (warps != 8 && warps != 4 && warps != 2) {
     // automatic: the largest block that still gives the device ~6 blocks per resident 8-warp slot
@@ -811,6 +899,11 @@ static cudaError_t launch_cells(int dense, int expv, bool faithful, bool pdl, di
     while (warps > 2 && (long long)grid.x * ((rowsTotal + warps - 1) / warps) * grid.z < 6 * slots) warps /= 2;
   }
   grid.y = (unsigned)((rowsTotal + warps - 1) / warps);
+  if (ep) {
+    if (faithful) return launch_layer(sweep_cell_emit_kernel<true, 0>, grid, s, pdl, bp, N, n, warps, *ep);
+    if (expv == 1) return launch_layer(sweep_cell_emit_kernel<false, 1>, grid, s, pdl, bp, N, n, warps, *ep);
+    return launch_layer(sweep_cell_emit_kernel<false, 0>, grid, s, pdl, bp, N, n, warps, *ep);
+  }
   if (faithful) return launch_layer(sweep_cell_kernel<true, 0, 2>, grid, s, pdl, bp, N, n, warps);
   if (cells == 2) {   // two cells per thread
     // register budget: default 2 blocks of 256 threads per SM (119 registers, no spills; as many cells in flight as
@@ -910,6 +1003,7 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
   const int64_t nraysTotal = 12LL << (2 * (nAngularLevel - 1));
   const double weight = (double)(1.f / (float)nraysTotal);  // equiSources.f90:1386 (single-precision division)
   const double cellSize = c.boxSize / (double)n;             // equiSources.f90:1570
+  const bool emit = c.dEta != nullptr;                       // emission set (rtb200_grid_set_emission)
 
   // ---- plan: pattern tables and zone tasks.  Depends only on the grid size and the direction list, so it is
   //      cached across the outer transport<->chemistry iterations. ----
@@ -917,7 +1011,7 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
   {
     char buf[128];
     snprintf(buf, sizeof(buf), "%d:%a:%d:%d:%d:%d:%d:%d:%d:", n, c.boxSize, nAngularLevel, c.tune.slots, c.tune.lockstep, c.tune.dirsPerTask,
-             c.tune.transposeZ, 0, c.tune.blockWarps);
+             c.tune.transposeZ, (int)emit, c.tune.blockWarps);
     planKey = buf;
     for (const auto& d : dirs) { snprintf(buf, sizeof(buf), "%lld,", (long long)d.iray); planKey += buf; }
   }
@@ -1026,8 +1120,11 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
         T.transposed = 1;
       }
       c.uniStdSlots = nStd;
-      if (nStd < ntask)
+      if (nStd < ntask) {
         if (int st = ensure_buffer((void**)&c.dKappaT, &c.kappaTBytes, (size_t)3 * N * sizeof(double))) return st;
+        if (emit)
+          if (int st = ensure_buffer((void**)&c.dEtaT, &c.etaTBytes, (size_t)3 * N * sizeof(double))) return st;
+      }
     }
     for (int t = 0; t < ntask; t++) {  // first task of a slot (in issue order) overwrites the accumulator
       c.uniTasks[t].firstInSlot = !seen[c.uniTasks[t].slot];
@@ -1056,7 +1153,8 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
     // 8-GPU run take 6.99-7.22 ms mean / 7.26-7.50 ms max against 7.03 / 7.31 ms with per-layer launches of one-cell
     // threads, and 4-, 2- and 1-GPU shards are 9-16% SLOWER (the layer tables come from shared memory instead of the
     // constant bank, 128 registers with spills, an L1 invalidation per tile), so per-layer launches stay the default
-    const bool fast = c.mathMode != RTB200_MATH_FAITHFUL && c.tune.expVariant == 1 && c.tune.lockstep;
+    // (an emissive sweep always runs per-layer launches: the persistent kernel has no emission terms)
+    const bool fast = c.mathMode != RTB200_MATH_FAITHFUL && c.tune.expVariant == 1 && c.tune.lockstep && !emit;
     const bool want = c.tune.persistent == 1 || (c.tune.persistent < 0 && ntask <= 6 && n >= 64);
     if (fast && want) {
       const int pst = run_persistent(c, n, uvb, dJout, s, ndir);
@@ -1086,6 +1184,7 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
     if (c.uniStdSlots < (int)c.uniTasks.size() && c.uniStdSlots < c.uniSlots) {
       dim3 tg((n + 31) / 32, (n + 31) / 32, 3 * n);
       transpose_kappa_kernel<<<tg, dim3(32, 8), 0, st>>>(c.dKappa, c.dKappaT, n);
+      if (emit) transpose_kappa_kernel<<<tg, dim3(32, 8), 0, st>>>(c.dEta, c.dEtaT, n);
     }
     {  // both plane buffers start as "boundary intensity everywhere": first-layer input and the permanent pads
       const int64_t total = (int64_t)2 * ndir * 3 * npl;
@@ -1107,6 +1206,9 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
       return T.ndir;
     };
     static thread_local BatchParams bp;
+    static thread_local EtaParams ep;
+    const EtaParams* epp = emit ? &ep : nullptr;
+    auto etaOf = [&](const UniTaskHost& T) -> const double* { return T.transposed ? c.dEtaT : c.dEta; };
     if (lockstep) {
       // all tasks of a batch advance one layer per launch; each task of a batch has its own accumulator slot
       for (int base = 0; base < ntask; base += slots) {
@@ -1115,10 +1217,11 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
           for (int z = 0; z < nb; z++) {
             const UniTaskHost& T = c.uniTasks[base + z];
             fill(bp.t[z], T, step, T.firstInSlot);  // every layer touches its own cells once per task
+            ep.eta[z] = etaOf(T);
           }
           dim3 gz = grid;
           gz.z = nb;
-          RTB_CUDA(launch_cells(c.tune.minBlocks, c.tune.expVariant, faithful, c.tune.pdl && step > 0, gz, st, bp, (int)N, n, c.tune.cells, c.tune.blockWarps, c.smCount));
+          RTB_CUDA(launch_cells(c.tune.minBlocks, c.tune.expVariant, faithful, c.tune.pdl && step > 0, gz, st, bp, (int)N, n, c.tune.cells, c.tune.blockWarps, c.smCount, epp));
           nLaunched++;
         }
       }
@@ -1133,7 +1236,8 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
         if (T.slot != k) continue;
         for (int step = 0; step < n; step++) {
           fill(bp.t[0], T, step, T.firstInSlot);
-          RTB_CUDA(launch_cells(c.tune.minBlocks, c.tune.expVariant, faithful, c.tune.pdl && step > 0, grid, cs, bp, (int)N, n, c.tune.cells, c.tune.blockWarps, c.smCount));
+          ep.eta[0] = etaOf(T);
+          RTB_CUDA(launch_cells(c.tune.minBlocks, c.tune.expVariant, faithful, c.tune.pdl && step > 0, grid, cs, bp, (int)N, n, c.tune.cells, c.tune.blockWarps, c.smCount, epp));
           nLaunched++;
         }
       }
@@ -1148,10 +1252,10 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
   if (c.tune.useGraph) {
     // The launch sequence depends only on the plan, the mode and the buffers: capture once, replay afterwards.
     char key[256];
-    snprintf(key, sizeof(key), "u:%d:%d:%d:%d:%p:%p:%p:%a:%a:%a", n, ntask, slots,
+    snprintf(key, sizeof(key), "u:%d:%d:%d:%d:%p:%p:%p:%a:%a:%a:%p:%p", n, ntask, slots,
              (int)faithful * 64 + c.tune.minBlocks * 4 + c.tune.expVariant + 1000 * c.tune.lockstep + 10000 * c.tune.pdl +
                  100000 * c.tune.cells + 1000000 * c.tune.blockWarps,
-             (void*)c.dAcc, (void*)c.dPlanes, (void*)c.dKappa, uvb[0], uvb[1], uvb[2]);
+             (void*)c.dAcc, (void*)c.dPlanes, (void*)c.dKappa, uvb[0], uvb[1], uvb[2], (void*)c.dEta, (void*)c.dEtaT);
     if (!c.graphExec || c.graphKey != key) {
       if (c.graphExec) { cudaGraphExecDestroy(c.graphExec); c.graphExec = nullptr; }
       cudaGraph_t graph;

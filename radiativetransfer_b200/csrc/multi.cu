@@ -778,6 +778,72 @@ int multi_update_species(Multi* m, const double* HI, const double* HeI, const do
 }
 
 // the species are identical on every member after each step: every rank returns its slab (one process: the whole array)
+// Emission of a device group: every rank checks its slab of the caller's array, the ranks agree on the status (an
+// all-gather of one word each in rank mode), then every rank uploads its slab and all-gathers the three fields on the
+// devices, as multi_update_species does for the species.  NULL clears the emission everywhere.
+int multi_set_emission(Multi* m, const double* eta) {
+  if (m->nleaf == 0) return RTB200_ERR_ARG;
+  if (!eta) return for_each_member(*m, [&](Member& q, int) { return set_emission(q.c, nullptr, false, q.c.stream); });
+  const int64_t N = m->nleaf;
+  bool ok = true;
+  for (Member* q : m->mem) {
+    const int64_t off = slab_off(*m, q->rank), cnt = slab_cnt(*m, q->rank);
+    for (int g = 0; g < 3 && ok; g++)
+      for (int64_t i = off; i < off + cnt; i++) {
+        const double v = eta[g * N + i];
+        if (!(v >= 0. && v <= 1.7976931348623157e308)) { ok = false; break; }
+      }
+  }
+  return for_each_member(*m, [&](Member& q, int) -> int {
+    Context& c = q.c;
+    RTB_CUDA(cudaSetDevice(c.device));
+    RTB_CUDA(cudaDeviceSynchronize());   // queued sweeps read the current array
+    const int64_t off = slab_off(*m, q.rank), cnt = slab_cnt(*m, q.rank);
+    double* stage = nullptr;             // [3 fields][npad]: slab copies, completed in place by the all-gather
+    RTB_CUDA(cudaMalloc((void**)&stage, (size_t)3 * m->npad * sizeof(double)));
+    auto done = [&](int st) { cudaStreamSynchronize(c.stream); cudaFree(stage); return st; };
+    if (m->nranks > 1) {                 // every rank learns every rank's verdict
+      const double mine = ok ? 0. : 1.;
+      RTB_CUDA(cudaMemcpyAsync(stage + q.rank, &mine, sizeof(double), cudaMemcpyHostToDevice, c.stream));
+      if (int st = [&]() -> int {
+            RTB_NCCL(nccl().AllGather(stage + q.rank, stage, 1, kNcclFloat64, q.comm, c.stream));
+            return RTB200_OK;
+          }())
+        return done(st);
+      std::vector<double> all((size_t)m->nranks);
+      RTB_CUDA(cudaMemcpyAsync(all.data(), stage, all.size() * sizeof(double), cudaMemcpyDeviceToHost, c.stream));
+      RTB_CUDA(cudaStreamSynchronize(c.stream));
+      for (double v : all)
+        if (v != 0.) return done(RTB200_ERR_ARG);
+    } else if (!ok) {
+      return done(RTB200_ERR_ARG);
+    }
+    for (int g = 0; g < 3; g++) {
+      double* f = stage + (size_t)g * m->npad;
+      if (cnt > 0) RTB_CUDA(cudaMemcpyAsync(f + off, eta + g * N + off, (size_t)cnt * sizeof(double), cudaMemcpyHostToDevice, c.stream));
+      if (m->nranks > 1) {
+        if (int st = [&]() -> int {
+              RTB_NCCL(nccl().AllGather(f + (size_t)q.rank * m->slab, f, (size_t)m->slab, kNcclFloat64, q.comm, c.stream));
+              return RTB200_OK;
+            }())
+          return done(st);
+      }
+    }
+    // the fields side by side, [3][nleaf] as the sweeps read them
+    double* packed = nullptr;
+    RTB_CUDA(cudaMalloc((void**)&packed, (size_t)3 * N * sizeof(double)));
+    int st = RTB200_OK;
+    for (int g = 0; g < 3 && !st; g++)
+      if (cudaMemcpyAsync(packed + (size_t)g * N, stage + (size_t)g * m->npad, (size_t)N * sizeof(double),
+                          cudaMemcpyDeviceToDevice, c.stream) != cudaSuccess)
+        st = RTB200_ERR_CUDA;
+    if (!st) st = set_emission(c, packed, true, c.stream);
+    cudaStreamSynchronize(c.stream);
+    cudaFree(packed);
+    return done(st);
+  });
+}
+
 int multi_get_species(Multi* m, double* HI, double* HeI, double* HeII) {
   if (m->nleaf == 0) return RTB200_ERR_ARG;
   return for_each_member(*m, [&](Member& q, int) -> int {

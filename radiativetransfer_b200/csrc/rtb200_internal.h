@@ -154,6 +154,10 @@ struct Context {
   double* dKappa = nullptr;  // [3][nleaf]
   double* dKappaT = nullptr; // [3][nleaf] z-major copy (index (z*n + x)*n + y) for the uniform sweep, lazily allocated
   size_t kappaTBytes = 0;
+  // emission coefficient per leaf and frequency group (rtb200_grid_set_emission): [3][nleaf], nullptr = no emission
+  double* dEta = nullptr;
+  double* dEtaT = nullptr;   // z-major copy of dEta for the uniform sweep (like dKappaT), lazily allocated
+  size_t etaTBytes = 0;
   int uniStdSlots = 0;       // slots [0, uniStdSlots) are in leaf order, the rest z-major
   DevTree tree;
   std::vector<int32_t> hChild;               // host copy of the linear octree
@@ -209,6 +213,9 @@ void context_destroy(Context& c);
 int grid_set(Context& c, int nx, int64_t nleaf, const int8_t* level, const double* HI, const double* HeI, const double* HeII,
              const double* rho, const double* abun2, double physicalBoxSize);
 int set_tuning(Context& c, const char* key, double value);
+// emission: eta = host [3][nleaf] (nullptr clears), or a device array on stream s (device = true); negative, NaN or
+// Inf entries are refused with RTB200_ERR_ARG and leave the previous emission in place
+int set_emission(Context& c, const double* eta, bool device, cudaStream_t s);
 int run_diffuse(Context& c, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays, int32_t nrays,
                 double* dJ, cudaStream_t s, int64_t* nseg);
 
@@ -252,6 +259,7 @@ int multi_set_tuning(Multi* m, const char* key, double value);
 int multi_grid_set(Multi* m, int nx, int64_t nleaf, const int8_t* level, const double* HI, const double* HeI,
                    const double* HeII, const double* rho, const double* abun2, double physicalBoxSize);
 int multi_update_species(Multi* m, const double* HI, const double* HeI, const double* HeII);
+int multi_set_emission(Multi* m, const double* eta);
 int multi_get_species(Multi* m, double* HI, double* HeI, double* HeII);
 int multi_diffuse_host(Multi* m, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays,
                        int32_t nrays, double* J1, double* J2, double* J3, int64_t* nseg);

@@ -246,4 +246,85 @@ __device__ __forceinline__ SegResult segment_update(double Iin, double kappa, do
   return r;
 }
 
+// ---- emission (DESIGN.md 4.6) -------------------------------------------------------------------------------------
+// A segment of an emitting leaf (coefficient eta >= 0, units of uvb per cm) adds to the attenuated intensity
+//   Iout = Iin e^-tau + eta t,   t = (1 - e^-tau) / kappa  if tau > (double)1.e-10f  else dpath
+// (the reference's nemi slot with nemi = eta dpath, transportRoutinesModule.f90:673-678), and to its mean intensity
+//   J_seg = L(Iin) + eta dpath phi(tau),   phi(tau) = (tau - 1 + e^-tau) / tau^2,  phi(0) = 1/2,
+// L = what the mode computes for pure attenuation: the exact path average of Iin e^-kappa s + eta (1 - e^-kappa s) / kappa.
+// Below kPhiSeries phi is its series (through tau^6: truncation < 3e-20), above it (tau - (1 - e^-tau)) / tau^2 from the
+// exponential pieces the mode already has (relative rounding ~2e-16 / tau <= 2e-14).  An opacity of exactly 0 (or the
+// FAST floor) gives exactly t = dpath and phi = 1/2.
+constexpr double kPhiSeries = 1e-2;
+__device__ __forceinline__ double emission_phi(double tau, double ome) {
+  double s = fma(tau, 1. / 40320., -1. / 5040.);
+  s = fma(s, tau, 1. / 720.);
+  s = fma(s, tau, -1. / 120.);
+  s = fma(s, tau, 1. / 24.);
+  s = fma(s, tau, -1. / 6.);
+  s = fma(s, tau, 0.5);
+  return tau < kPhiSeries ? s : (tau - ome) / (tau * tau);
+}
+__device__ __forceinline__ double emission_t(double tau, double ome, double invk, double dpath) {
+  return tau > (double)1.e-10f ? ome * invk : dpath;
+}
+
+// FAST-mode segment with emission: as segment_fast, plus E += phi(tau) * dw (dw = dpath * weight / nseg; the caller
+// adds eta * E to the cell's sum once per layer) and the emitted part of Iout.  invk = 1 / kappa (kappa floored).
+template <int EXPV, bool GUARD = true>
+__device__ __forceinline__ double segment_fast_emit(double Iin, double tau, double cs, const double* __restrict__ T, double& A,
+                                                    double eta, double invk, double d, double dw, double& E) {
+  double Ts, p;
+  if (EXPV == 1) exp_neg_parts32<GUARD>(tau, T, Ts, p);
+  else exp_neg_parts_poly(tau, Ts, p);
+  const double X = Iin * Ts;
+  const double Iatt = fma(X, p, X);
+  const double Z = fma(-X, p, Iin - X);
+  if (!GUARD || ((__double2hiint(Iatt) << 1) | __double2loint(Iatt)) != 0) A = fma(Z, cs, A);
+  const double ome = fma(-Ts, p, 1.0 - Ts);
+  E = fma(emission_phi(tau, ome), dw, E);
+  return fma(eta, emission_t(tau, ome, invk, d), Iatt);
+}
+
+// the outgoing intensity alone, bit for bit what segment_fast_emit returns for the same arguments
+template <int EXPV, bool GUARD = true>
+__device__ __forceinline__ double attenuate_fast_emit(double Iin, double tau, const double* __restrict__ T, double eta,
+                                                      double invk, double d) {
+  double Ts, p;
+  if (EXPV == 1) exp_neg_parts32<GUARD>(tau, T, Ts, p);
+  else exp_neg_parts_poly(tau, Ts, p);
+  const double X = Iin * Ts;
+  const double Iatt = fma(X, p, X);
+  const double ome = fma(-Ts, p, 1.0 - Ts);
+  return fma(eta, emission_t(tau, ome, invk, d), Iatt);
+}
+
+// FAITHFUL-mode segment with emission: L is segment_update<true>'s operation sequence on the attenuated part, the eta
+// terms are one FMA each, so eta = 0 reproduces segment_update<true> bit for bit
+__device__ __forceinline__ SegResult segment_faithful_emit(double Iin, double kappa, double dpath, double eta) {
+  SegResult r;
+  const double tau = __dmul_rn(kappa, dpath);
+  const double a = exp(-tau);
+  const double Iatt = __dmul_rn(Iin, a);
+  double L;
+  if (Iatt < Iin) L = __ddiv_rn(__dsub_rn(Iin, Iatt), log(__ddiv_rn(Iin, Iatt)));
+  else L = __dmul_rn(0.5, __dadd_rn(Iin, Iatt));
+  const double ome = __dsub_rn(1.0, a);
+  const double t = tau > (double)1.e-10f ? __ddiv_rn(ome, kappa) : dpath;
+  double phi = 0.5;
+  if (tau >= kPhiSeries) phi = __ddiv_rn(__dsub_rn(tau, ome), __dmul_rn(tau, tau));
+  else phi = emission_phi(tau, ome);
+  r.Iout = fma(eta, t, Iatt);
+  r.J = fma(__dmul_rn(eta, dpath), phi, L);
+  return r;
+}
+// the outgoing intensity alone (the recomputed upstream cell of the uniform sweep)
+__device__ __forceinline__ double attenuate_faithful_emit(double Iin, double kappa, double dpath, double eta) {
+  const double tau = __dmul_rn(kappa, dpath);
+  const double a = exp(-tau);
+  const double ome = __dsub_rn(1.0, a);
+  const double t = tau > (double)1.e-10f ? __ddiv_rn(ome, kappa) : dpath;
+  return fma(eta, t, __dmul_rn(Iin, a));
+}
+
 }  // namespace rtb

@@ -50,6 +50,10 @@ module rtb200_shim
        import :: c_int, c_ptr
        type(c_ptr), value :: ctx, HI, HeI, HeII
      end function rtb200_grid_update_species
+     integer(c_int) function rtb200_grid_set_emission(ctx, eta) bind(C, name='rtb200_grid_set_emission')
+       import :: c_ptr, c_int
+       type(c_ptr), value :: ctx, eta
+     end function rtb200_grid_set_emission
      integer(c_int) function rtb200_diffuse(ctx, nAngularLevel, uvb, beta, rays, nrays, J1, J2, J3, nseg) &
           bind(C, name='rtb200_diffuse')
        import :: c_int, c_int32_t, c_ptr
@@ -406,5 +410,17 @@ contains
     cosmicSpectrum = cosmicSpectrum / float(nStarsSpecificAge)
     deallocate(srcLeaf, srcWeight, highestLevel, remaining, boundary, spectrum, dustEscape)
   end subroutine rtbPoint
+
+  ! Emission coefficients per leaf (extension, DESIGN.md 4.6): eta(leaf, group) in the leaf order of rtbSetGrid, i.e.
+  ! [3][nleaf] in C; the driver flattens its per-cell emissivities in the same writeCell pre-order as the species.
+  ! Without the argument the emission is cleared.  Negative, NaN or Inf entries stop with RTB200_ERR_ARG.
+  subroutine rtbSetEmission(eta)
+    real(c_double), dimension(:,:), target, contiguous, intent(in), optional :: eta
+    if (present(eta)) then
+       call rtbCheck(rtb200_grid_set_emission(rtbContext, c_loc(eta)), 'rtb200_grid_set_emission')
+    else
+       call rtbCheck(rtb200_grid_set_emission(rtbContext, c_null_ptr), 'rtb200_grid_set_emission')
+    endif
+  end subroutine rtbSetEmission
 
 end module rtb200_shim

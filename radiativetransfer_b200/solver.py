@@ -198,6 +198,23 @@ class Transport:
         a = [_f64(HI), _f64(HeI), _f64(HeII)]
         _lib.check(self.L.rtb200_grid_update_species(self.h, *[_ptr(x) for x in a]), "rtb200_grid_update_species")
 
+    def set_emission(self, eta):
+        """Emission coefficient per leaf and frequency group, [3, nleaf] in the units of uvb per cm (DESIGN.md 4.6);
+        None clears it.  Negative, NaN or Inf entries raise and keep the previous emission."""
+        if eta is None:
+            _lib.check(self.L.rtb200_grid_set_emission(self.h, None), "rtb200_grid_set_emission")
+            return
+        e = np.ascontiguousarray(eta, dtype=np.float64)
+        if e.size != 3 * self.nleaf:
+            raise ValueError("eta must have 3 * nleaf entries ([3][nleaf])")
+        _lib.check(self.L.rtb200_grid_set_emission(self.h, _ptr(e)), "rtb200_grid_set_emission")
+
+    def set_emission_device(self, eta_ptr, stream=0):
+        """The same from a device pointer to [3][nleaf] doubles (e.g. torch tensor .data_ptr()), copied and checked on
+        `stream`; returns after synchronising it.  Single-GPU handles only."""
+        st = self.L.rtb200_grid_set_emission_device(self.h, C.c_void_p(int(eta_ptr)), C.c_void_p(int(stream)))
+        _lib.check(st, "rtb200_grid_set_emission_device")
+
     def diffuse(self, uvb, beta, n_angular_level=3, rays=None, out=None):
         """Host-buffer call (H2D of nothing but tables, D2H of J): returns (J[3, nleaf], nseg)."""
         uvb, beta = _f64(uvb), _f64(np.asarray(beta).reshape(9))
