@@ -111,12 +111,11 @@ int rtb200_multi_slab_get(rtb200_ctx* ctx, int local, double* J3, double* K3, do
 
 int rtb200_set_math(rtb200_ctx* ctx, int math_mode);
 /* Launch tuning knobs; results do not depend on them (tests/test_diffuse_gpu.py, test_point_gpu.py).  Keys:
- *   uniform sweep  "slots" (zone tasks per launch, 0 = all), "graph" (CUDA graph replay, 1), "dense" (register cap:
- *                  0/1/2 = 2/3/4 blocks per SM, 2), "expv" (1 = table exponential), "lockstep" (one launch per layer
- *                  for all tasks, 1), "dirs_per_task" (0 = chosen from a wave model), "cells" (cells of a layer per thread: 1, 2, or 0 = by grid size and zone tasks per launch), "block_warps" (rows per block 8 / 4 / 2,
+ *   uniform sweep  "slots" (zone tasks per launch, 0 = all), "graph" (CUDA graph replay, 1), "dirs_per_task" (0 = chosen
+ *                  from a wave model), "cells" (cells of a layer per thread: 1, 2, or 0 = by grid size and zone tasks per
+ *                  launch; an emissive sweep always runs one-cell threads), "block_warps" (rows per block 8 / 4 / 2,
  *                  0 = by the number of blocks a launch has), "transpose_z" (z-major copy for
- *                  the zones sweeping along the contiguous axis, 1), "persistent" (1 = the whole sweep as ONE launch, tiles handed out by a counter and
- *                  ordered by per-tile progress words; bit-identical, measured no faster: 0 = per-layer launches is the default; an emissive sweep always runs per-layer launches of one-cell threads), "pdl" (programmatic dependent launch of layer
+ *                  the zones sweeping along the contiguous axis, 1), "pdl" (programmatic dependent launch of layer
  *                  l+1 on layer l, also used by the nested-grid waves, 1), "l2_mb"
  *   nested grids   "force_amr" (general octree path on a uniform grid), "amr_batch" (directions per batch, 0 = as many
  *                  as fit in memory), "amr_stream" (2:1-balanced grids: 1 = the whole sweep as one launch whose work items wait

@@ -9,7 +9,6 @@ CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "librtb200.so")
 SOURCES = ["api.cu", "diffuse_uniform.cu", "diffuse_amr.cu", "point_source.cu", "chemistry.cu", "multi.cu", "octree_build.cu", "geometry.cpp", "point_host.cpp", "uvb_host.cpp"]
 NVCC_FLAGS = [
-    "-DRTB_FAITHFUL_INLINE",
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "--use_fast_math=false", "-Xcompiler", "-fPIC,-O2,-ffp-contract=off,-fno-fast-math", "-Xptxas", "-v",
 ]

@@ -263,10 +263,8 @@ int context_init(Context& c, int device) {
   RTB_CUDA(cudaEventCreate(&c.evStop));
   RTB_CUDA(cudaEventCreate(&c.evSweep0));
   RTB_CUDA(cudaEventCreate(&c.evSweep1));
-  RTB_CUDA(cudaEventCreateWithFlags(&c.evFork, cudaEventDisableTiming));
   RTB_CUDA(cudaMalloc((void**)&c.dErr, 64));
   RTB_CUDA(cudaMemset(c.dErr, 0, 64));
-  if (const char* v = getenv("RTB200_DENSE")) c.tune.minBlocks = atoi(v);
   if (const char* v = getenv("RTB200_SLOTS")) c.tune.slots = atoi(v);
   if (const char* v = getenv("RTB200_GRAPH")) c.tune.useGraph = atoi(v);
   if (const char* v = getenv("RTB200_L2_MB")) c.tune.l2BudgetMB = atof(v);
@@ -279,15 +277,12 @@ void context_destroy(Context& c) {
   free_grid(c);
   cudaFree(c.dChemK);
   cudaFree(c.dMassPart);
-  cudaFree(c.dAcc); cudaFree(c.dPlanes); cudaFree(c.dAmrScratch); cudaFree(c.dErr); cudaFree(c.dMarchSeg); cudaFree(c.dMarchProg);
+  cudaFree(c.dAcc); cudaFree(c.dPlanes); cudaFree(c.dAmrScratch); cudaFree(c.dErr);
   if (c.hPinned) cudaFreeHost(c.hPinned);
   if (c.evStart) cudaEventDestroy(c.evStart);
   if (c.evStop) cudaEventDestroy(c.evStop);
   if (c.evSweep0) cudaEventDestroy(c.evSweep0);
   if (c.evSweep1) cudaEventDestroy(c.evSweep1);
-  if (c.evFork) cudaEventDestroy(c.evFork);
-  for (auto e : c.chainEvents) cudaEventDestroy(e);
-  for (auto st : c.chainStreams) cudaStreamDestroy(st);
   if (c.stream) cudaStreamDestroy(c.stream);
   c = Context();
 }
@@ -308,10 +303,7 @@ int set_math(Context& c, int mode) {
 
 int set_tuning(Context& c, const char* key, double value) {
   std::string k(key);
-  if (k == "dense") c.tune.minBlocks = (int)value;
-  else if (k == "expv") c.tune.expVariant = (int)value;
-  else if (k == "lockstep") c.tune.lockstep = (int)value;
-  else if (k == "amr_batch") c.tune.amrBatch = (int)value;
+  if (k == "amr_batch") c.tune.amrBatch = (int)value;
   else if (k == "force_amr") c.tune.forceAmr = (int)value;
   else if (k == "amr_slots") c.tune.amrSlots = (int)value;
   else if (k == "amr_thin") c.tune.amrThin = (int)value;
@@ -324,7 +316,6 @@ int set_tuning(Context& c, const char* key, double value) {
   else if (k == "transpose_z") c.tune.transposeZ = (int)value;
   else if (k == "cells") c.tune.cells = (int)value;
   else if (k == "block_warps") c.tune.blockWarps = (int)value;
-  else if (k == "persistent") c.tune.persistent = (int)value;
   else if (k == "pdl") c.tune.pdl = (int)value;
   else if (k == "dirs_per_task") c.tune.dirsPerTask = (int)value;
   else if (k == "portable_math") c.tune.portableMath = (int)value;

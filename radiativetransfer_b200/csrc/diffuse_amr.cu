@@ -338,7 +338,7 @@ __device__ __noinline__ ThinSeg amr_thin_segment(double i0, double i1, double i2
   ThinSeg o;
   const double Iin[3] = {i0, i1, i2}, kap[3] = {k0, k1, k2};
   for (int g = 0; g < 3; g++) {
-    const SegResult sr = segment_update<true, 0>(Iin[g], kap[g], dpath, 0., nullptr);
+    const SegResult sr = segment_faithful(Iin[g], kap[g], dpath);
     o.out[g] = sr.Iout;
     o.J[g] = sr.J;
   }
@@ -455,7 +455,7 @@ __device__ __forceinline__ bool amr_transport_leaf(const AmrParams& P, const Amr
 #pragma unroll
       for (int g = 0; g < 3; g++) {
         SegResult sr = EMIT ? segment_faithful_emit(Iin[ray][g], kap[g], dpath[ray], eta[g])
-                            : segment_update<true, 0>(Iin[ray][g], kap[g], dpath[ray], 0., nullptr);
+                            : segment_faithful(Iin[ray][g], kap[g], dpath[ray]);
         out[g] = sr.Iout;
         Jm[g] = __dadd_rn(Jm[g], sr.J);
       }
@@ -470,9 +470,9 @@ __device__ __forceinline__ bool amr_transport_leaf(const AmrParams& P, const Amr
       const double cs = pat.cs[ray][lane];
 #pragma unroll
       for (int g = 0; g < 3; g++)
-        out[g] = EMIT ? segment_fast_emit<1, true>(Iin[ray][g], kap[g] * dpath[ray], cs, sT, Jm[g], eta[g], invk[g],
-                                                   dpath[ray], dpath[ray] * wn, E[g])
-                      : segment_fast<1, true>(Iin[ray][g], kap[g] * dpath[ray], cs, sT, Jm[g]);
+        out[g] = EMIT ? segment_fast_emit<true>(Iin[ray][g], kap[g] * dpath[ray], cs, sT, Jm[g], eta[g], invk[g],
+                                                dpath[ray], dpath[ray] * wn, E[g])
+                      : segment_fast<true>(Iin[ray][g], kap[g] * dpath[ray], cs, sT, Jm[g]);
     }
     if (ray == 0) { xy[0] = out[0]; xy[1] = out[1]; xy[2] = out[2]; }
     imean++;

@@ -17,7 +17,8 @@
 //    ("slot"), so no atomics and a fixed summation order.  Final kernels sum the slot accumulators into J.
 //  * Zones that sweep along the contiguous axis of the leaf order read a z-major copy of kappa and accumulate in
 //    that layout (transpose_kappa_kernel / merge_transposed_kernel) so that their lanes stay coalesced.
-//  * sweep_persistent_kernel runs the whole layer loop in one launch (tiles ordered by progress words); off by default.
+//  * Layer kernels: sweep_cell_kernel (one cell per thread, FAST or FAITHFUL), sweep_cell2_kernel (two cells per
+//    thread, FAST) and sweep_cell_emit_kernel (one cell per thread, with emission); launch_cells picks one per launch.
 
 #include <algorithm>
 #include <cmath>
@@ -98,20 +99,20 @@ struct Em {
   double invk[3], invkR[3];  // FAST arithmetic: 1 / kappa with kappa floored as in the segment
 };
 
-template <int EXPV, bool GUARD, bool EMIT>
+template <bool GUARD, bool EMIT>
 __device__ __forceinline__ double seg_fast(double Iin, double kap, double d, double cs, const double* __restrict__ T,
                                            double& A, double eta, double invk, double dw, double& E) {
-  if (EMIT) return segment_fast_emit<EXPV, GUARD>(Iin, kap * d, cs, T, A, eta, invk, d, dw, E);
-  return segment_fast<EXPV, GUARD>(Iin, kap * d, cs, T, A);
+  if (EMIT) return segment_fast_emit<GUARD>(Iin, kap * d, cs, T, A, eta, invk, d, dw, E);
+  return segment_fast<GUARD>(Iin, kap * d, cs, T, A);
 }
-template <int EXPV, bool GUARD, bool EMIT>
+template <bool GUARD, bool EMIT>
 __device__ __forceinline__ double att_fast(double Iin, double kap, double d, const double* __restrict__ T, double eta,
                                            double invk) {
-  if (EMIT) return attenuate_fast_emit<EXPV, GUARD>(Iin, kap * d, T, eta, invk, d);
-  return attenuate_fast<EXPV, GUARD>(Iin, kap * d, T);
+  if (EMIT) return attenuate_fast_emit<GUARD>(Iin, kap * d, T, eta, invk, d);
+  return attenuate_fast<GUARD>(Iin, kap * d, T);
 }
 
-template <int EXPV, int NSEG, bool SECL, bool GUARD, bool EMIT = false>
+template <int NSEG, bool SECL, bool GUARD, bool EMIT = false>
 __device__ __forceinline__ void direction_fast(const LayerSeg& P, const double (&cur)[3], const double (&upR)[3],
                                                const double (&kap)[3], const double (&kR)[3], double (&I)[3],
                                                double (&A)[3], const double* __restrict__ T, const Em& em,
@@ -120,24 +121,24 @@ __device__ __forceinline__ void direction_fast(const LayerSeg& P, const double (
   const double wn = EMIT ? P.w * (1.0 / NSEG) : 0.;
 #pragma unroll
   for (int g = 0; g < 3; g++) {
-    const double I1 = seg_fast<EXPV, GUARD, EMIT>(cur[g], kap[g], P.d[0], P.cs[0], T, A[g], em.eta[g], em.invk[g], P.d[0] * wn, E[g]);
+    const double I1 = seg_fast<GUARD, EMIT>(cur[g], kap[g], P.d[0], P.cs[0], T, A[g], em.eta[g], em.invk[g], P.d[0] * wn, E[g]);
     I[g] = I1;
     if (NSEG >= 2) {
       double rup = 0.;  // xy-segment output of the (b-1) cell
-      if (!SECL || NSEG == 3) rup = att_fast<EXPV, GUARD, EMIT>(upR[g], kR[g], P.d[0], T, em.etaR[g], em.invkR[g]);
+      if (!SECL || NSEG == 3) rup = att_fast<GUARD, EMIT>(upR[g], kR[g], P.d[0], T, em.etaR[g], em.invkR[g]);
       const double in2 = SECL ? __shfl_up_sync(full, I1, 1) : rup;
-      const double I2 = seg_fast<EXPV, GUARD, EMIT>(in2, kap[g], P.d[1], P.cs[1], T, A[g], em.eta[g], em.invk[g], P.d[1] * wn, E[g]);
+      const double I2 = seg_fast<GUARD, EMIT>(in2, kap[g], P.d[1], P.cs[1], T, A[g], em.eta[g], em.invk[g], P.d[1] * wn, E[g]);
       I[g] = I2;
       if (NSEG == 3) {
         double in3;
         if (SECL) {
           // third segment from the (b-1) cell's SECOND segment, which was fed by the (b-1, a-1) cell's xy segment
           const double x = __shfl_up_sync(full, rup, 1);
-          in3 = att_fast<EXPV, GUARD, EMIT>(x, kR[g], P.d[1], T, em.etaR[g], em.invkR[g]);
+          in3 = att_fast<GUARD, EMIT>(x, kR[g], P.d[1], T, em.etaR[g], em.invkR[g]);
         } else {
           in3 = __shfl_up_sync(full, I2, 1);  // the (a-1) cell's second segment
         }
-        I[g] = seg_fast<EXPV, GUARD, EMIT>(in3, kap[g], P.d[2], P.cs[2], T, A[g], em.eta[g], em.invk[g], P.d[2] * wn, E[g]);
+        I[g] = seg_fast<GUARD, EMIT>(in3, kap[g], P.d[2], P.cs[2], T, A[g], em.eta[g], em.invk[g], P.d[2] * wn, E[g]);
       }
     }
   }
@@ -148,7 +149,7 @@ __device__ __forceinline__ void direction_fast(const LayerSeg& P, const double (
 template <bool EMIT>
 __device__ __forceinline__ SegResult seg_faithful(double Iin, double kap, double d, double eta) {
   if (EMIT) return segment_faithful_emit(Iin, kap, d, eta);
-  return segment_update<true, 0>(Iin, kap, d, 0., nullptr);
+  return segment_faithful(Iin, kap, d);
 }
 template <bool EMIT>
 __device__ __forceinline__ double att_faithful(double Iin, double kap, double d, double eta) {
@@ -200,44 +201,38 @@ __device__ __forceinline__ void direction_faithful(const LayerSeg& P, const doub
 // dispatch on the layer's chain kind (warp-uniform).  kmax = the largest opacity this thread multiplies a path with.
 // If kmax * (longest segment of the layer) <= 64 for every lane of the warp, the overflow guards of segment_fast are
 // dropped (4 fewer instructions per segment update); `thick` warps take the guarded instantiation.
-template <int EXPV, bool GUARD, bool EMIT>
+template <bool GUARD, bool EMIT>
 __device__ __forceinline__ void direction_kinds_fast(const LayerSeg& P, bool secL, const double (&cur)[3],
                                                      const double (&upR)[3], const double (&kap)[3],
                                                      const double (&kR)[3], double (&I)[3], double (&A)[3],
                                                      const double* __restrict__ T, const Em& em, double (&E)[3]) {
   const int kind = P.kind;
-  if (kind == 0) direction_fast<EXPV, 1, true, GUARD, EMIT>(P, cur, upR, kap, kR, I, A, T, em, E);
+  if (kind == 0) direction_fast<1, true, GUARD, EMIT>(P, cur, upR, kap, kR, I, A, T, em, E);
   else if (kind == 1 || kind == 3) {
-    if (secL) direction_fast<EXPV, 2, true, GUARD, EMIT>(P, cur, upR, kap, kR, I, A, T, em, E);
-    else direction_fast<EXPV, 2, false, GUARD, EMIT>(P, cur, upR, kap, kR, I, A, T, em, E);
+    if (secL) direction_fast<2, true, GUARD, EMIT>(P, cur, upR, kap, kR, I, A, T, em, E);
+    else direction_fast<2, false, GUARD, EMIT>(P, cur, upR, kap, kR, I, A, T, em, E);
   } else {
-    if (secL) direction_fast<EXPV, 3, true, GUARD, EMIT>(P, cur, upR, kap, kR, I, A, T, em, E);
-    else direction_fast<EXPV, 3, false, GUARD, EMIT>(P, cur, upR, kap, kR, I, A, T, em, E);
+    if (secL) direction_fast<3, true, GUARD, EMIT>(P, cur, upR, kap, kR, I, A, T, em, E);
+    else direction_fast<3, false, GUARD, EMIT>(P, cur, upR, kap, kR, I, A, T, em, E);
   }
 }
 
-template <int EXPV, bool EMIT>
+template <bool EMIT>
 __device__ __forceinline__ void direction_dispatch_fast(const LayerSeg& P, bool secL, double kmax, const double (&cur)[3],
                                                         const double (&upR)[3], const double (&kap)[3],
                                                         const double (&kR)[3], double (&I)[3], double (&A)[3],
                                                         const double* __restrict__ T, const Em& em, double (&E)[3]) {
-  if (__any_sync(0xffffffffu, kmax * P.dmax > 64.)) direction_kinds_fast<EXPV, true, EMIT>(P, secL, cur, upR, kap, kR, I, A, T, em, E);
-  else direction_kinds_fast<EXPV, false, EMIT>(P, secL, cur, upR, kap, kR, I, A, T, em, E);
+  if (__any_sync(0xffffffffu, kmax * P.dmax > 64.)) direction_kinds_fast<true, EMIT>(P, secL, cur, upR, kap, kR, I, A, T, em, E);
+  else direction_kinds_fast<false, EMIT>(P, secL, cur, upR, kap, kR, I, A, T, em, E);
 }
 
-// Out of line and by value: the rare faithful branch must not force the fast path's per-direction arrays into
-// local memory (a by-reference call would).
+// By value: the rare faithful branch must not force the fast path's per-direction arrays into local memory.
 struct Tri {
   double v[3];
 };
 struct FaithOut {
   Tri I, acc;
 };
-#ifndef RTB_FAITHFUL_INLINE
-#define RTB_FAITHFUL_CALL __noinline__
-#else
-#define RTB_FAITHFUL_CALL __forceinline__
-#endif
 template <bool EMIT>
 __device__ __forceinline__ FaithOut direction_faithful_kinds(double d0, double d1, double d2, double w, int kind, bool secL,
                                                              const Tri& cur_, const Tri& upR_, const Tri& kap_,
@@ -262,14 +257,14 @@ __device__ __forceinline__ FaithOut direction_faithful_kinds(double d0, double d
   for (int g = 0; g < 3; g++) { o.I.v[g] = I[g]; o.acc.v[g] = acc[g]; }
   return o;
 }
-__device__ RTB_FAITHFUL_CALL FaithOut direction_call_faithful(double d0, double d1, double d2, double w, int kind,
-                                                              bool secL, Tri cur_, Tri upR_, Tri kap_, Tri kR_, Tri acc_) {
+__device__ __forceinline__ FaithOut direction_call_faithful(double d0, double d1, double d2, double w, int kind,
+                                                            bool secL, Tri cur_, Tri upR_, Tri kap_, Tri kR_, Tri acc_) {
   const Tri zero = {{0., 0., 0.}};
   return direction_faithful_kinds<false>(d0, d1, d2, w, kind, secL, cur_, upR_, kap_, kR_, acc_, zero, zero);
 }
-__device__ RTB_FAITHFUL_CALL FaithOut direction_call_faithful_emit(double d0, double d1, double d2, double w, int kind,
-                                                                   bool secL, Tri cur_, Tri upR_, Tri kap_, Tri kR_,
-                                                                   Tri acc_, Tri eta_, Tri etaR_) {
+__device__ __forceinline__ FaithOut direction_call_faithful_emit(double d0, double d1, double d2, double w, int kind,
+                                                                 bool secL, Tri cur_, Tri upR_, Tri kap_, Tri kR_,
+                                                                 Tri acc_, Tri eta_, Tri etaR_) {
   return direction_faithful_kinds<true>(d0, d1, d2, w, kind, secL, cur_, upR_, kap_, kR_, acc_, eta_, etaR_);
 }
 template <bool EMIT = false>
@@ -307,13 +302,13 @@ static_assert(sizeof(BatchParams) + 64 <= 32764, "kernel parameter space");
 // A layer whose pattern has a very short segment (a corner clip, len < 1e-2 cell; 1.7% of the (direction, layer)
 // pairs) is evaluated with the reference's own operation sequence even in FAST mode: there tau is tiny and the
 // rounding noise of the reference's (Iin-Iout)/log(Iin/Iout), ~1.1e-16/tau, would otherwise show up as a parity
-// difference.  That branch is warp-uniform (P.thin is a per-layer table entry) and kept out of line.
+// difference.  That branch is warp-uniform (P.thin is a per-layer table entry).
 // Emission (DESIGN.md 4.6): the emission coefficients of every task, in the layout of its kappa (leaf order or z-major)
 struct EtaParams {
   const double* eta[kMaxBatch];
 };
 
-template <bool FAITHFUL, int EXPV, bool EMIT>
+template <bool FAITHFUL, bool EMIT>
 __device__ __forceinline__ void sweep_cell_body(const BatchParams& bp, const double* __restrict__ etaTask, int N, int n,
                                                 int np1, int npl3) {
   // n, np1 = n + 1 and npl3 = 3 (n+1)^2 are the same for every task: as top-level parameters they are constant-bank
@@ -385,7 +380,7 @@ __device__ __forceinline__ void sweep_cell_body(const BatchParams& bp, const dou
       for (int g = 0; g < 3; g++) upR[g] = pin[g - up];
     }
     if (FAITHFUL || P.thin) direction_dispatch_faithful<EMIT>(P, secL, cur, upR, kapF, kR, I, acc, em.eta, em.etaR);
-    else direction_dispatch_fast<EXPV, EMIT>(P, secL, kmax, cur, upR, kap, kR, I, A, sT, em, E);
+    else direction_dispatch_fast<EMIT>(P, secL, kmax, cur, upR, kap, kR, I, A, sT, em, E);
     if (writer) {
 #pragma unroll
       for (int g = 0; g < 3; g++) pout[g] = I[g];
@@ -402,18 +397,20 @@ __device__ __forceinline__ void sweep_cell_body(const BatchParams& bp, const dou
   }
 }
 
-template <bool FAITHFUL, int EXPV, int MINB>
-__global__ void __launch_bounds__(256, MINB)
+// register budget: FAST arithmetic 4 blocks of 256 threads per SM (64 registers; 2 or 3 blocks measured slower,
+// DESIGN.md 4.2), FAITHFUL 2
+template <bool FAITHFUL>
+__global__ void __launch_bounds__(256, FAITHFUL ? 2 : 4)
 sweep_cell_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1, int npl3) {
-  sweep_cell_body<FAITHFUL, EXPV, false>(bp, nullptr, N, n, np1, npl3);
+  sweep_cell_body<FAITHFUL, false>(bp, nullptr, N, n, np1, npl3);
 }
 
 // the emissive sweep: one cell per thread, 2 blocks of 256 threads per SM (the emission terms need registers)
-template <bool FAITHFUL, int EXPV>
+template <bool FAITHFUL>
 __global__ void __launch_bounds__(256, 2)
 sweep_cell_emit_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1, int npl3,
                        const __grid_constant__ EtaParams ep) {
-  sweep_cell_body<FAITHFUL, EXPV, true>(bp, ep.eta[blockIdx.z], N, n, np1, npl3);
+  sweep_cell_body<FAITHFUL, true>(bp, ep.eta[blockIdx.z], N, n, np1, npl3);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -425,7 +422,7 @@ sweep_cell_emit_kernel(const __grid_constant__ BatchParams bp, int N, int n, int
 // of every cell is unchanged: the handed-over value is bit for bit what the single-cell kernel recomputes.
 //   r01 ncu of the single-cell kernel: 318 warp instructions per direction, 194 of them not FP64 (issue-bound).
 // ---------------------------------------------------------------------------------------------------------
-template <int EXPV, int NSEG, bool SECL, bool GUARD>
+template <int NSEG, bool SECL, bool GUARD>
 __device__ __forceinline__ void direction_fast2(const LayerSeg& P, const double (&cur0)[3], const double (&cur1)[3],
                                                 const double (&upR)[3], const double (&kap0)[3], const double (&kap1)[3],
                                                 const double (&kR)[3], double (&I0)[3], double (&I1)[3], double (&A0)[3],
@@ -433,54 +430,54 @@ __device__ __forceinline__ void direction_fast2(const LayerSeg& P, const double 
   const unsigned full = 0xffffffffu;
 #pragma unroll
   for (int g = 0; g < 3; g++) {
-    const double a1 = segment_fast<EXPV, GUARD>(cur0[g], kap0[g] * P.d[0], P.cs[0], T, A0[g]);
-    const double b1 = segment_fast<EXPV, GUARD>(cur1[g], kap1[g] * P.d[0], P.cs[0], T, A1[g]);
+    const double a1 = segment_fast<GUARD>(cur0[g], kap0[g] * P.d[0], P.cs[0], T, A0[g]);
+    const double b1 = segment_fast<GUARD>(cur1[g], kap1[g] * P.d[0], P.cs[0], T, A1[g]);
     I0[g] = a1; I1[g] = b1;
     if (NSEG >= 2) {
       double rup = 0.;  // xy-segment output of the (b0 - 1) cell, recomputed (lower cell only)
-      if (!SECL || NSEG == 3) rup = attenuate_fast<EXPV, GUARD>(upR[g], kR[g] * P.d[0], T);
+      if (!SECL || NSEG == 3) rup = attenuate_fast<GUARD>(upR[g], kR[g] * P.d[0], T);
       const double a_in2 = SECL ? __shfl_up_sync(full, a1, 1) : rup;
       const double b_in2 = SECL ? __shfl_up_sync(full, b1, 1) : a1;   // the lower cell's own xy output
-      const double a2 = segment_fast<EXPV, GUARD>(a_in2, kap0[g] * P.d[1], P.cs[1], T, A0[g]);
-      const double b2 = segment_fast<EXPV, GUARD>(b_in2, kap1[g] * P.d[1], P.cs[1], T, A1[g]);
+      const double a2 = segment_fast<GUARD>(a_in2, kap0[g] * P.d[1], P.cs[1], T, A0[g]);
+      const double b2 = segment_fast<GUARD>(b_in2, kap1[g] * P.d[1], P.cs[1], T, A1[g]);
       I0[g] = a2; I1[g] = b2;
       if (NSEG == 3) {
         double a_in3, b_in3;
         if (SECL) {
           const double x = __shfl_up_sync(full, rup, 1);
-          a_in3 = attenuate_fast<EXPV, GUARD>(x, kR[g] * P.d[1], T);
+          a_in3 = attenuate_fast<GUARD>(x, kR[g] * P.d[1], T);
           b_in3 = a2;                                                 // the lower cell's second segment
         } else {
           a_in3 = __shfl_up_sync(full, a2, 1);
           b_in3 = __shfl_up_sync(full, b2, 1);
         }
-        I0[g] = segment_fast<EXPV, GUARD>(a_in3, kap0[g] * P.d[2], P.cs[2], T, A0[g]);
-        I1[g] = segment_fast<EXPV, GUARD>(b_in3, kap1[g] * P.d[2], P.cs[2], T, A1[g]);
+        I0[g] = segment_fast<GUARD>(a_in3, kap0[g] * P.d[2], P.cs[2], T, A0[g]);
+        I1[g] = segment_fast<GUARD>(b_in3, kap1[g] * P.d[2], P.cs[2], T, A1[g]);
       }
     }
   }
 }
 
-template <int EXPV, bool GUARD>
+template <bool GUARD>
 __device__ __forceinline__ void direction_kinds_fast2(const LayerSeg& P, bool secL, const double (&cur0)[3],
                                                       const double (&cur1)[3], const double (&upR)[3],
                                                       const double (&kap0)[3], const double (&kap1)[3],
                                                       const double (&kR)[3], double (&I0)[3], double (&I1)[3],
                                                       double (&A0)[3], double (&A1)[3], const double* __restrict__ T) {
   const int kind = P.kind;
-  if (kind == 0) direction_fast2<EXPV, 1, true, GUARD>(P, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, T);
+  if (kind == 0) direction_fast2<1, true, GUARD>(P, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, T);
   else if (kind == 1 || kind == 3) {
-    if (secL) direction_fast2<EXPV, 2, true, GUARD>(P, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, T);
-    else direction_fast2<EXPV, 2, false, GUARD>(P, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, T);
+    if (secL) direction_fast2<2, true, GUARD>(P, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, T);
+    else direction_fast2<2, false, GUARD>(P, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, T);
   } else {
-    if (secL) direction_fast2<EXPV, 3, true, GUARD>(P, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, T);
-    else direction_fast2<EXPV, 3, false, GUARD>(P, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, T);
+    if (secL) direction_fast2<3, true, GUARD>(P, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, T);
+    else direction_fast2<3, false, GUARD>(P, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, T);
   }
 }
 
-// block = 8 warps; a warp covers 31 cells (+ the recomputed halo cell in lane 0) of TWO rows
-template <int EXPV, int MINB>
-__global__ void __launch_bounds__(256, MINB)
+// block = 8 warps; a warp covers 31 cells (+ the recomputed halo cell in lane 0) of TWO rows.  Register budget: 2 blocks of
+// 256 threads per SM (124 registers, no spills; as many cells in flight as the one-cell kernel at 4 blocks).
+__global__ void __launch_bounds__(256, 2)
 sweep_cell2_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1, int npl3) {
   const StepParams& sp = bp.t[blockIdx.z];
   const double* __restrict__ kappa = sp.kappa;
@@ -540,9 +537,9 @@ sweep_cell2_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1
       direction_dispatch_faithful(P, secL, cur0, upR, kF0, kR, I0, acc0);
       direction_dispatch_faithful(P, secL, cur1, cur0, kF1, kF0, I1, acc1);
     } else if (__any_sync(0xffffffffu, kmax * P.dmax > 64.)) {
-      direction_kinds_fast2<EXPV, true>(P, secL, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, sT);
+      direction_kinds_fast2<true>(P, secL, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, sT);
     } else {
-      direction_kinds_fast2<EXPV, false>(P, secL, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, sT);
+      direction_kinds_fast2<false>(P, secL, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, sT);
     }
     if (writer0) {
 #pragma unroll
@@ -568,176 +565,6 @@ sweep_cell2_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1
       double* p = sp.acc + (int64_t)g * N + leaf0 + sB;
       *p = sp.firstInSlot ? v : __dadd_rn(*p, v);
     }
-  }
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// Persistent layer loop (FAST arithmetic; set_tuning "persistent": 1 on, 0 off, -1 = for small direction shards).
-//
-// A multi-GPU rank sweeps 3 zones: a layer launch of 3 zone tasks is ~16 us of fp64 work, but costs ~28 us -- its
-// 98K threads are 1.3 "waves" of the 75K the device holds, and the hand-over from one launch to the next (drain of
-// the whole grid, ramp-up of the next) is paid 256 times per sweep.  Here ONE launch runs the whole sweep: blocks
-// take work items (layer, task, tile) in that order from a counter; a tile of layer L waits until the tiles it
-// exchanges plane values with -- itself and its 8 neighbours in the task -- have completed layer L-1 (one progress
-// word per tile, release/acquire), so layers overlap wherever the dependencies allow and the device stays full.  Items are handed out in dependency order, so the
-// oldest unfinished item never waits: no co-residency requirement, no grid-wide barrier.  The planes stay in global
-// memory (L2-resident for a shard's ~24 directions); a plane buffer is rewritten every second layer, and the
-// acquire load that ends the wait is what makes the SM's L1 forget the older contents.  The per-cell code and the
-// order of every sum are those of sweep_cell2_kernel: results are bit-identical to the per-layer launches.
-// ---------------------------------------------------------------------------------------------------------
-struct PersistTask {
-  const double* kappa;   // [3][N] in the task's layout
-  double* acc;           // slot accumulator [3][N]
-  int64_t planeOff;      // offset of the task's first direction in a plane buffer (doubles)
-  int32_t origin, si, sj, sk, ndir, laneIsK, firstInSlot, tileBase;   // tileBase: first work item of the task in a layer
-};
-struct PersistParams {
-  PersistTask t[kMaxBatch];
-  const LayerSeg* seg;   // [task][layer][kMaxDirPerTask]
-  double *planeA, *planeB;
-  int32_t* counters;     // [0] work counter, [1 + task * tilesPerTask + tile] layers the tile has completed; zero at launch
-  int32_t ntask, n, np1, npl3, N, gx, gyT, itemsPerLayer, tilesPerTask;
-};
-
-template <int EXPV>
-__device__ __forceinline__ void persistent_tile(const PersistParams& pp, const PersistTask& T, const LayerSeg* __restrict__ sP,
-                                                int layer, int bx, int byWarp, const double* __restrict__ sT) {
-  const int n = pp.n, np1 = pp.np1, N = pp.N;
-  const int a = bx * 31 - 1 + (int)threadIdx.x, b0 = 2 * byWarp;
-  if (b0 >= n) return;                                         // warp-uniform
-  const bool row1 = b0 + 1 < n;
-  const bool inRow = a < n;
-  const bool writer0 = inRow && threadIdx.x >= 1, writer1 = writer0 && row1;
-  const bool cell0 = inRow && a >= 0, cell1 = cell0 && row1;
-  const int laneIsK = T.laneIsK;
-  const int sA = laneIsK ? T.sk : T.sj, sB = laneIsK ? T.sj : T.sk;
-  const int leaf0 = T.origin + layer * T.si + a * sA + b0 * sB;
-  double kap0[3], kap1[3], kF0[3], kF1[3], kR[3];
-#pragma unroll
-  for (int g = 0; g < 3; g++) {
-    const double* kg = T.kappa + (int64_t)g * N + leaf0;
-    kF0[g] = cell0 ? __ldg(kg) : 0.;
-    kF1[g] = cell1 ? __ldg(kg + sB) : 0.;
-    kR[g] = (cell0 && b0 > 0) ? __ldg(kg - sB) : 0.;
-    kap0[g] = kF0[g] > 0. ? kF0[g] : kKappaFloor;
-    kap1[g] = kF1[g] > 0. ? kF1[g] : kKappaFloor;
-  }
-  const double kmax = fmax(fmax(fmax(fmax(kap0[0], kap0[1]), fmax(kap0[2], kR[0])), fmax(kR[1], kR[2])),
-                           fmax(fmax(kap1[0], kap1[1]), kap1[2]));
-  double A0[3] = {0., 0., 0.}, A1[3] = {0., 0., 0.}, acc0[3] = {0., 0., 0.}, acc1[3] = {0., 0., 0.};
-  const int pidx = (b0 + 1) * np1 + (inRow ? a + 1 : 0);
-  const int ndir = T.ndir;
-  const int dstride = pp.npl3;
-  const int up = 3 * np1;
-  const int up1 = row1 ? up : 0;
-  const double* pin = ((layer & 1) ? pp.planeA : pp.planeB) + T.planeOff + 3 * pidx;
-  double* pout = ((layer & 1) ? pp.planeB : pp.planeA) + T.planeOff + 3 * pidx;
-  for (int q = 0; q < ndir; q++, pin += dstride, pout += dstride) {
-    const LayerSeg& P = sP[q];
-    const int kind = P.kind;
-    if (q + 1 < ndir) {
-      prefetch_l1(pin + dstride);
-      prefetch_l1(pin + dstride + up1);
-      prefetch_l1(pin + dstride - up);
-    }
-    double cur0[3], cur1[3], upR[3] = {0., 0., 0.}, I0[3], I1[3];
-#pragma unroll
-    for (int g = 0; g < 3; g++) { cur0[g] = pin[g]; cur1[g] = pin[g + up1]; }
-    const bool secL = (kind <= 2) == (laneIsK != 0);
-    if (kind == 2 || kind == 4 || (kind != 0 && !secL)) {
-#pragma unroll
-      for (int g = 0; g < 3; g++) upR[g] = pin[g - up];
-    }
-    if (P.thin) {
-      direction_dispatch_faithful(P, secL, cur0, upR, kF0, kR, I0, acc0);
-      direction_dispatch_faithful(P, secL, cur1, cur0, kF1, kF0, I1, acc1);
-    } else if (__any_sync(0xffffffffu, kmax * P.dmax > 64.)) {
-      direction_kinds_fast2<EXPV, true>(P, secL, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, sT);
-    } else {
-      direction_kinds_fast2<EXPV, false>(P, secL, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, sT);
-    }
-    if (writer0) {
-#pragma unroll
-      for (int g = 0; g < 3; g++) pout[g] = I0[g];
-    }
-    if (writer1) {
-#pragma unroll
-      for (int g = 0; g < 3; g++) pout[g + up] = I1[g];
-    }
-  }
-  if (writer0) {
-#pragma unroll
-    for (int g = 0; g < 3; g++) {
-      const double v = fma(A0[g], kTwoM200 / kap0[g], acc0[g]);
-      double* p = T.acc + (int64_t)g * N + leaf0;
-      *p = T.firstInSlot ? v : __dadd_rn(*p, v);
-    }
-  }
-  if (writer1) {
-#pragma unroll
-    for (int g = 0; g < 3; g++) {
-      const double v = fma(A1[g], kTwoM200 / kap1[g], acc1[g]);
-      double* p = T.acc + (int64_t)g * N + leaf0 + sB;
-      *p = T.firstInSlot ? v : __dadd_rn(*p, v);
-    }
-  }
-}
-
-__device__ __forceinline__ int ld_relaxed_gpu(const int32_t* p) {
-  int v;
-  asm volatile("ld.relaxed.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-
-template <int MINB>
-__global__ void __launch_bounds__(256, MINB) sweep_persistent_kernel(const __grid_constant__ PersistParams pp, int32_t* err) {
-  extern __shared__ double smem[];
-  double* sT = smem;                                           // exp table (kExpTableSize entries)
-  LayerSeg* sSeg = reinterpret_cast<LayerSeg*>(smem + kExpTableSize);     // [kMaxDirPerTask] tables of the item's task and layer
-  __shared__ int sItem;
-  const int tid = threadIdx.y * 32 + threadIdx.x;
-  if (tid < kExpTableSize) sT[tid] = kExpTable32[tid];
-  constexpr int segDoubles = (int)(sizeof(LayerSeg) / sizeof(double)) * kMaxDirPerTask;
-  const int warps = blockDim.y;
-  const int total = pp.n * pp.itemsPerLayer;
-  int32_t* prog = pp.counters + 1;
-  for (;;) {
-    if (tid == 0) sItem = atomicAdd(pp.counters, 1);
-    __syncthreads();
-    const int item = sItem;
-    if (item >= total) break;
-    const int layer = item / pp.itemsPerLayer, inLayer = item - layer * pp.itemsPerLayer;
-    int task = 0;
-    while (task + 1 < pp.ntask && inLayer >= pp.t[task + 1].tileBase) task++;
-    const int local = inLayer - pp.t[task].tileBase;
-    const int bx = local % pp.gx, by = local / pp.gx;
-    for (int i = tid; i < segDoubles; i += blockDim.x * blockDim.y)
-      reinterpret_cast<double*>(sSeg)[i] =
-          __ldg(reinterpret_cast<const double*>(pp.seg + ((size_t)task * pp.n + layer) * kMaxDirPerTask) + i);
-    if (threadIdx.y == 0 && layer > 0) {
-      // the tile's inputs are the previous layer's planes of itself and its upstream neighbours, and the buffer it
-      // writes was read in the previous layer by itself and its downstream neighbours: wait until those (up to) 9
-      // tiles have completed `layer` layers.  Polls are relaxed loads (they leave the SM's L1 alone); the acquire
-      // fence after them is what invalidates it.
-      if (threadIdx.x < 9) {
-        const int nx = bx + (int)(threadIdx.x % 3) - 1, ny = by + (int)(threadIdx.x / 3) - 1;
-        if (nx >= 0 && nx < pp.gx && ny >= 0 && ny < pp.gyT) {
-          const int32_t* flag = prog + task * pp.tilesPerTask + ny * pp.gx + nx;
-          unsigned spins = 0;
-          while (ld_relaxed_gpu(flag) < layer) {
-            __nanosleep(32);
-            if (++spins > (1u << 26)) { atomicExch(err, RTB200_ERR_CUDA); break; }
-          }
-        }
-      }
-      __syncwarp();
-      asm volatile("fence.acq_rel.gpu;" ::: "memory");
-    }
-    __syncthreads();
-    persistent_tile<1>(pp, pp.t[task], sSeg, layer, bx, by * warps + (int)threadIdx.y, sT);
-    __syncthreads();                       // every thread's plane and accumulator stores are issued
-    if (tid == 0)
-      asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(prog + task * pp.tilesPerTask + local), "r"(layer + 1) : "memory");
   }
 }
 
@@ -881,16 +708,14 @@ static cudaError_t launch_layer(Kernel kern, dim3 grid, cudaStream_t s, bool pdl
 
 // `pdl`: programmatic dependent launch on the previous launch of the stream (only for a layer whose predecessor in
 // the stream is the previous layer's sweep kernel)
-// `ep` != nullptr: the emissive sweep (sweep_cell_emit_kernel: one cell per thread, "dense" does not apply)
-static cudaError_t launch_cells(int dense, int expv, bool faithful, bool pdl, dim3 grid, cudaStream_t s,
-                                const BatchParams& bp, int N, int n, int cells, int warps, int smCount,
-                                const EtaParams* ep = nullptr) {
-  // `dense`: 0 = compiler's choice of registers (2 blocks per SM), 1 = cap for 3 blocks, 2 = cap for 4 blocks
+// `ep` != nullptr: the emissive sweep (sweep_cell_emit_kernel: one cell per thread)
+static cudaError_t launch_cells(bool faithful, bool pdl, dim3 grid, cudaStream_t s, const BatchParams& bp, int N, int n,
+                                int cells, int warps, int smCount, const EtaParams* ep = nullptr) {
   // automatic: two cells per thread pay (1-2%) when the launch has many zone tasks; a small direction shard (3 zone
   // tasks on each of 8 GPUs) is 1.3 waves of two-cell threads but fills the device evenly with one-cell threads
   // (measured on the shards of an 8-GPU run: 7.03 against 7.21 ms mean, 7.31 against 7.93 ms for the slowest rank)
   if (cells == 0) cells = (n >= 192 && grid.z >= 6) ? 2 : 1;
-  if (faithful || expv != 1 || ep) cells = 1;
+  if (faithful || ep) cells = 1;
   const int rowsTotal = cells == 2 ? (n + 1) / 2 : n;           // rows of threads per task and layer
   if (warps != 8 && warps != 4 && warps != 2) {
     // automatic: the largest block that still gives the device ~6 blocks per resident 8-warp slot
@@ -900,99 +725,12 @@ static cudaError_t launch_cells(int dense, int expv, bool faithful, bool pdl, di
   }
   grid.y = (unsigned)((rowsTotal + warps - 1) / warps);
   if (ep) {
-    if (faithful) return launch_layer(sweep_cell_emit_kernel<true, 0>, grid, s, pdl, bp, N, n, warps, *ep);
-    if (expv == 1) return launch_layer(sweep_cell_emit_kernel<false, 1>, grid, s, pdl, bp, N, n, warps, *ep);
-    return launch_layer(sweep_cell_emit_kernel<false, 0>, grid, s, pdl, bp, N, n, warps, *ep);
+    if (faithful) return launch_layer(sweep_cell_emit_kernel<true>, grid, s, pdl, bp, N, n, warps, *ep);
+    return launch_layer(sweep_cell_emit_kernel<false>, grid, s, pdl, bp, N, n, warps, *ep);
   }
-  if (faithful) return launch_layer(sweep_cell_kernel<true, 0, 2>, grid, s, pdl, bp, N, n, warps);
-  if (cells == 2) {   // two cells per thread
-    // register budget: default 2 blocks of 256 threads per SM (119 registers, no spills; as many cells in flight as
-    // the single-cell kernel at 4 blocks); "dense" 3 / 4 cap the registers for 3 / 4 blocks
-    if (dense >= 4) return launch_layer(sweep_cell2_kernel<1, 4>, grid, s, pdl, bp, N, n, warps);
-    if (dense == 3) return launch_layer(sweep_cell2_kernel<1, 3>, grid, s, pdl, bp, N, n, warps);
-    return launch_layer(sweep_cell2_kernel<1, 2>, grid, s, pdl, bp, N, n, warps);
-  }
-#define RTB_LAUNCH(E)                                                                                    \
-  if (dense == 1) return launch_layer(sweep_cell_kernel<false, E, 3>, grid, s, pdl, bp, N, n, warps);    \
-  else if (dense >= 2) return launch_layer(sweep_cell_kernel<false, E, 4>, grid, s, pdl, bp, N, n, warps); \
-  else return launch_layer(sweep_cell_kernel<false, E, 2>, grid, s, pdl, bp, N, n, warps)
-  if (expv == 1) { RTB_LAUNCH(1); } else { RTB_LAUNCH(0); }
-#undef RTB_LAUNCH
-}
-
-
-// Runs the sweep as one launch (see sweep_persistent_kernel).  Returns -1 when it does not apply.
-static int run_persistent(Context& c, int n, const double* uvb, double* dJout, cudaStream_t s, int ndir) {
-  const int64_t N = c.nleaf, npl = (int64_t)(n + 1) * (n + 1);
-  const int ntask = (int)c.uniTasks.size();
-  if (ntask < 1 || ntask > kMaxBatch || c.uniSlots < ntask) return -1;   // every task needs its own accumulator slot
-  const int warps = (c.tune.blockWarps == 8 || c.tune.blockWarps == 4) ? c.tune.blockWarps : 2;   // small tiles by default
-  const int gx = (n + 30) / 31, rowsTotal = (n + 1) / 2, gyT = (rowsTotal + warps - 1) / warps;
-  static thread_local PersistParams pp;
-  // per-layer tables of all tasks on the device (kept while the plan is the same)
-  const size_t segPerTask = (size_t)n * kMaxDirPerTask;
-  if (c.marchSegKey != c.uniPlanKey) {
-    if (int e = ensure_buffer((void**)&c.dMarchSeg, &c.marchSegBytes, (size_t)ntask * segPerTask * sizeof(LayerSeg))) return e;
-    for (int t = 0; t < ntask; t++)
-      RTB_CUDA(cudaMemcpyAsync((LayerSeg*)c.dMarchSeg + (size_t)t * segPerTask, c.uniTasks[t].seg.data(),
-                               segPerTask * sizeof(LayerSeg), cudaMemcpyHostToDevice, s));
-    RTB_CUDA(cudaStreamSynchronize(s));
-    c.marchSegKey = c.uniPlanKey;
-  }
-  const size_t counterBytes = ((size_t)ntask * gx * gyT + 1) * sizeof(int32_t);
-  if (int e = ensure_buffer((void**)&c.dMarchProg, &c.marchProgBytes, counterBytes)) return e;
-  const size_t smemBytes = kExpTableSize * sizeof(double) + (size_t)kMaxDirPerTask * sizeof(LayerSeg);
-  auto kern = sweep_persistent_kernel<2>;
-  if (smemBytes > 48 * 1024) RTB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smemBytes));
-  int perSm = 0;
-  RTB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSm, kern, 32 * warps, smemBytes));
-  if (perSm < 1) return -1;
-  int items = 0;
-  for (int t = 0; t < ntask; t++) {
-    const UniTaskHost& T = c.uniTasks[t];
-    PersistTask& q = pp.t[t];
-    q.kappa = T.transposed ? c.dKappaT : c.dKappa;
-    q.acc = c.dAcc + (size_t)T.slot * 3 * N;
-    q.planeOff = (int64_t)T.planeFirst * 3 * npl;
-    q.origin = (int32_t)T.origin; q.si = (int32_t)T.si; q.sj = (int32_t)T.sj; q.sk = (int32_t)T.sk;
-    q.ndir = T.ndir; q.laneIsK = T.laneIsK; q.firstInSlot = T.firstInSlot; q.tileBase = items;
-    items += gx * gyT;
-  }
-  pp.seg = (const LayerSeg*)c.dMarchSeg;
-  pp.planeA = c.dPlanes; pp.planeB = c.dPlanes + (size_t)ndir * 3 * npl;
-  pp.counters = c.dMarchProg;
-  pp.ntask = ntask; pp.n = n; pp.np1 = n + 1; pp.npl3 = (int32_t)(3 * npl); pp.N = (int32_t)N; pp.gx = gx; pp.gyT = gyT;
-  pp.itemsPerLayer = items;
-  pp.tilesPerTask = gx * gyT;
-  const int blocks = (int)std::min<int64_t>((int64_t)perSm * c.smCount, (int64_t)items * n);
-  RTB_CUDA(cudaEventRecord(c.evSweep0, s));
-  if (c.uniStdSlots < ntask && c.uniStdSlots < c.uniSlots) {
-    dim3 tg((n + 31) / 32, (n + 31) / 32, 3 * n);
-    transpose_kappa_kernel<<<tg, dim3(32, 8), 0, s>>>(c.dKappa, c.dKappaT, n);
-  }
-  {
-    const int64_t total = (int64_t)2 * ndir * 3 * npl;
-    int fb = (int)std::min<int64_t>((total + 255) / 256, (int64_t)c.smCount * 16);
-    fill_planes_kernel<<<fb, 256, 0, s>>>(c.dPlanes, npl, total, uvb[0], uvb[1], uvb[2]);
-  }
-  RTB_CUDA(cudaMemsetAsync(c.dMarchProg, 0, counterBytes, s));
-  kern<<<dim3(blocks), dim3(32, warps), smemBytes, s>>>(pp, c.dErr);
-  RTB_CUDA(cudaEventRecord(c.evSweep1, s));
-  {
-    const int nStd = std::min(c.uniStdSlots, c.uniSlots);
-    int mb = std::min<int64_t>((3 * N + 255) / 256, (int64_t)c.smCount * 16);
-    if (nStd > 0) merge_slots_kernel<<<mb, 256, 0, s>>>(c.dAcc, nStd, 3 * N, dJout);
-    else RTB_CUDA(cudaMemsetAsync(dJout, 0, 3 * N * sizeof(double), s));
-    if (nStd < c.uniSlots) {
-      dim3 tg((n + 31) / 32, (n + 31) / 32, 3 * n);
-      merge_transposed_kernel<<<tg, dim3(32, 8), 0, s>>>(c.dAcc, nStd, c.uniSlots - nStd, n, dJout);
-    }
-  }
-  RTB_CUDA(cudaGetLastError());
-  c.uniLaunches = 4;
-  c.lastSweepLaunches = 1;
-  c.lastLaunches = 7;
-  return RTB200_OK;
+  if (faithful) return launch_layer(sweep_cell_kernel<true>, grid, s, pdl, bp, N, n, warps);
+  if (cells == 2) return launch_layer(sweep_cell2_kernel, grid, s, pdl, bp, N, n, warps);
+  return launch_layer(sweep_cell_kernel<false>, grid, s, pdl, bp, N, n, warps);
 }
 
 int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std::vector<Direction>& dirs,
@@ -1010,7 +748,7 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
   std::string planKey;
   {
     char buf[128];
-    snprintf(buf, sizeof(buf), "%d:%a:%d:%d:%d:%d:%d:%d:%d:", n, c.boxSize, nAngularLevel, c.tune.slots, c.tune.lockstep, c.tune.dirsPerTask,
+    snprintf(buf, sizeof(buf), "%d:%a:%d:%d:%d:%d:%d:%d:", n, c.boxSize, nAngularLevel, c.tune.slots, c.tune.dirsPerTask,
              c.tune.transposeZ, (int)emit, c.tune.blockWarps);
     planKey = buf;
     for (const auto& d : dirs) { snprintf(buf, sizeof(buf), "%lld,", (long long)d.iray); planKey += buf; }
@@ -1028,7 +766,7 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
       int perZone[25] = {0};
       for (int d = 0; d < ndir; d++) perZone[dirs[d].izone]++;
       const int64_t bpt = (int64_t)((n + 30) / 31) * ((n + 7) / 8);
-      const int64_t cap = (int64_t)c.smCount * (c.tune.minBlocks >= 2 ? 4 : (c.tune.minBlocks == 1 ? 3 : 2));
+      const int64_t cap = (int64_t)c.smCount * 4;   // resident blocks: 4 per SM (sweep_cell_kernel's register budget)
       double best = 1e300;
       for (int d = kMaxDirPerTask; d >= 2; d--) {
         int64_t T = 0;
@@ -1082,28 +820,13 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
       }
     }
     const int ntask = (int)c.uniTasks.size();
-    // slots = zones in flight, each an independent stream / graph branch with a private J accumulator;
-    // longest-processing-time-first assignment of the tasks to the slots
-    int slots = c.tune.slots;
-    if (slots <= 0) slots = c.tune.lockstep ? kMaxBatch : 24;
-    slots = std::max(1, std::min(slots, ntask));
-    std::vector<int> order(ntask), load(slots, 0), seen(slots, 0);
-    for (int t = 0; t < ntask; t++) order[t] = t;
-    std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return c.uniTasks[x].ndir > c.uniTasks[y].ndir; });
-    if (c.tune.lockstep) {
-      slots = std::min(slots, kMaxBatch);
-      for (int t = 0; t < ntask; t++) c.uniTasks[t].slot = t % slots;   // batch b = tasks [b*slots, (b+1)*slots)
-    } else {
-      for (int t : order) {
-        int best = 0;
-        for (int k = 1; k < slots; k++)
-          if (load[k] < load[best]) best = k;
-        c.uniTasks[t].slot = best;
-        load[best] += c.uniTasks[t].ndir;
-      }
-    }
+    // slots = zone tasks per launch, each with a private J accumulator; batch b = tasks [b*slots, (b+1)*slots)
+    int slots = c.tune.slots > 0 ? c.tune.slots : kMaxBatch;
+    slots = std::min(std::max(1, std::min(slots, ntask)), kMaxBatch);
+    std::vector<int> seen(slots, 0);
+    for (int t = 0; t < ntask; t++) c.uniTasks[t].slot = t % slots;
     c.uniStdSlots = slots;
-    if (c.tune.transposeZ && c.tune.lockstep && ntask <= slots && n >= 32) {
+    if (c.tune.transposeZ && ntask <= slots && n >= 32) {
       // every task owns its slot: tasks sweeping along the contiguous axis switch to the z-major layout (see
       // transpose_kappa_kernel) and are moved behind the others so that their slots form one range
       std::stable_partition(c.uniTasks.begin(), c.uniTasks.end(), [](const UniTaskHost& T) { return T.si != 1 && T.si != -1; });
@@ -1148,38 +871,15 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
 
   if (int st = ensure_buffer((void**)&c.dAcc, &c.accBytes, (size_t)c.uniSlots * 3 * N * sizeof(double))) return st;
   if (int st = ensure_buffer((void**)&c.dPlanes, &c.planeBytes, (size_t)2 * std::max(ndir, 1) * 3 * npl * sizeof(double))) return st;
-  {
-    // one launch for the whole sweep: on request only.  Measured on one B200 (profiles/r02h_*): the shards of an
-    // 8-GPU run take 6.99-7.22 ms mean / 7.26-7.50 ms max against 7.03 / 7.31 ms with per-layer launches of one-cell
-    // threads, and 4-, 2- and 1-GPU shards are 9-16% SLOWER (the layer tables come from shared memory instead of the
-    // constant bank, 128 registers with spills, an L1 invalidation per tile), so per-layer launches stay the default
-    // (an emissive sweep always runs per-layer launches: the persistent kernel has no emission terms)
-    const bool fast = c.mathMode != RTB200_MATH_FAITHFUL && c.tune.expVariant == 1 && c.tune.lockstep && !emit;
-    const bool want = c.tune.persistent == 1 || (c.tune.persistent < 0 && ntask <= 6 && n >= 64);
-    if (fast && want) {
-      const int pst = run_persistent(c, n, uvb, dJout, s, ndir);
-      if (pst >= 0) return pst;
-    }
-  }
-
   dim3 grid((n + 30) / 31, (n + 7) / 8, 1);
   double* planeA = c.dPlanes;
   double* planeB = c.dPlanes + (size_t)ndir * 3 * npl;
   const bool faithful = c.mathMode == RTB200_MATH_FAITHFUL;
-  while ((int)c.chainStreams.size() < slots) {
-    cudaStream_t cs;
-    RTB_CUDA(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
-    cudaEvent_t ce;
-    RTB_CUDA(cudaEventCreateWithFlags(&ce, cudaEventDisableTiming));
-    c.chainStreams.push_back(cs);
-    c.chainEvents.push_back(ce);
-  }
   int64_t nLaunched = 1;
-  const bool lockstep = c.tune.lockstep != 0;
 
-  // Every task (zone) is a chain of n layer steps; the tasks of one slot run back to back because they share the
-  // slot's J accumulator.  Each slot is an independent stream (a parallel branch of the captured graph), so the
-  // hardware block scheduler balances the zones and there is no device-wide barrier between layers.
+  // Every task (zone) is a chain of n layer steps.  The tasks of a batch advance one layer per launch, each into its own
+  // accumulator slot; the batches run one after the other, so task t shares slot t % slots with the tasks of the
+  // earlier batches.
   auto issue = [&](cudaStream_t st) -> int {
     if (c.uniStdSlots < (int)c.uniTasks.size() && c.uniStdSlots < c.uniSlots) {
       dim3 tg((n + 31) / 32, (n + 31) / 32, 3 * n);
@@ -1209,41 +909,18 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
     static thread_local EtaParams ep;
     const EtaParams* epp = emit ? &ep : nullptr;
     auto etaOf = [&](const UniTaskHost& T) -> const double* { return T.transposed ? c.dEtaT : c.dEta; };
-    if (lockstep) {
-      // all tasks of a batch advance one layer per launch; each task of a batch has its own accumulator slot
-      for (int base = 0; base < ntask; base += slots) {
-        const int nb = std::min(slots, ntask - base);
-        for (int step = 0; step < n; step++) {
-          for (int z = 0; z < nb; z++) {
-            const UniTaskHost& T = c.uniTasks[base + z];
-            fill(bp.t[z], T, step, T.firstInSlot);  // every layer touches its own cells once per task
-            ep.eta[z] = etaOf(T);
-          }
-          dim3 gz = grid;
-          gz.z = nb;
-          RTB_CUDA(launch_cells(c.tune.minBlocks, c.tune.expVariant, faithful, c.tune.pdl && step > 0, gz, st, bp, (int)N, n, c.tune.cells, c.tune.blockWarps, c.smCount, epp));
-          nLaunched++;
+    for (int base = 0; base < ntask; base += slots) {
+      const int nb = std::min(slots, ntask - base);
+      for (int step = 0; step < n; step++) {
+        for (int z = 0; z < nb; z++) {
+          const UniTaskHost& T = c.uniTasks[base + z];
+          fill(bp.t[z], T, step, T.firstInSlot);  // every layer touches its own cells once per task
+          ep.eta[z] = etaOf(T);
         }
-      }
-      return RTB200_OK;
-    }
-    RTB_CUDA(cudaEventRecord(c.evFork, st));
-    for (int k = 0; k < slots; k++) {
-      cudaStream_t cs = slots > 1 ? c.chainStreams[k] : st;
-      if (slots > 1) RTB_CUDA(cudaStreamWaitEvent(cs, c.evFork, 0));
-      for (int t = 0; t < ntask; t++) {
-        const UniTaskHost& T = c.uniTasks[t];
-        if (T.slot != k) continue;
-        for (int step = 0; step < n; step++) {
-          fill(bp.t[0], T, step, T.firstInSlot);
-          ep.eta[0] = etaOf(T);
-          RTB_CUDA(launch_cells(c.tune.minBlocks, c.tune.expVariant, faithful, c.tune.pdl && step > 0, grid, cs, bp, (int)N, n, c.tune.cells, c.tune.blockWarps, c.smCount, epp));
-          nLaunched++;
-        }
-      }
-      if (slots > 1) {
-        RTB_CUDA(cudaEventRecord(c.chainEvents[k], cs));
-        RTB_CUDA(cudaStreamWaitEvent(st, c.chainEvents[k], 0));
+        dim3 gz = grid;
+        gz.z = nb;
+        RTB_CUDA(launch_cells(faithful, c.tune.pdl && step > 0, gz, st, bp, (int)N, n, c.tune.cells, c.tune.blockWarps, c.smCount, epp));
+        nLaunched++;
       }
     }
     return RTB200_OK;
@@ -1253,8 +930,7 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
     // The launch sequence depends only on the plan, the mode and the buffers: capture once, replay afterwards.
     char key[256];
     snprintf(key, sizeof(key), "u:%d:%d:%d:%d:%p:%p:%p:%a:%a:%a:%p:%p", n, ntask, slots,
-             (int)faithful * 64 + c.tune.minBlocks * 4 + c.tune.expVariant + 1000 * c.tune.lockstep + 10000 * c.tune.pdl +
-                 100000 * c.tune.cells + 1000000 * c.tune.blockWarps,
+             (int)faithful * 64 + 10000 * c.tune.pdl + 100000 * c.tune.cells + 1000000 * c.tune.blockWarps,
              (void*)c.dAcc, (void*)c.dPlanes, (void*)c.dKappa, uvb[0], uvb[1], uvb[2], (void*)c.dEta, (void*)c.dEtaT);
     if (!c.graphExec || c.graphKey != key) {
       if (c.graphExec) { cudaGraphExecDestroy(c.graphExec); c.graphExec = nullptr; }

@@ -61,7 +61,7 @@ struct UniTaskHost {
 };
 
 struct Tuning {
-  int slots = 0;         // zones swept concurrently (independent streams), each with its own J accumulator (0 = 24)
+  int slots = 0;         // uniform sweep: zone tasks per launch, each with its own J accumulator (0 = 40, the most a launch takes)
   int useGraph = 1;
   int forceAmr = 0;      // route uniform grids through the general (AMR) path as well (cross-check)
   int amrSlots = 1;      // nested grids: per-item arrays indexed by the leaf's position in the wave order (1) or by leaf number (0)
@@ -73,13 +73,8 @@ struct Tuning {
                          // 2:1-balanced grids and the depth elsewhere (-1)
   int amrThin = 1;       // nested grids, FAST arithmetic: thin layers use the reference's operation sequence (1)
   int amrBatch = 0;      // directions per AMR batch (0 = as many as fit in half of the free memory)
-  int lockstep = 1;      // 1: one launch per layer for all zones of a batch; 0: every slot an independent stream
-  int minBlocks = 2;     // 0: compiler's register choice (2 blocks per SM); 1: cap for 3 blocks; 2: cap for 4 blocks
-  int expVariant = 1;    // exp(-tau) of the fast path: 0 = polynomial, 1 = 16-entry shared-memory table
   double l2BudgetMB = 96.0;
   int pdl = 1;           // uniform sweep: programmatic dependent launch of layer l+1 on layer l (its prologue overlaps the tail)
-  int persistent = 0;    // uniform sweep, FAST arithmetic: 1 = the whole sweep as one launch (sweep_persistent_kernel),
-                         // -1 = for small direction shards only, 0 = per-layer launches (measured: not slower)
   int blockWarps = 0;    // uniform sweep: rows (warps) per block: 8, 4, 2, or 0 = chosen from the number of blocks per launch
   int cells = 0;         // uniform sweep, FAST arithmetic: cells of a layer per thread (2: two rows per warp, see
                          // sweep_cell2_kernel; 0 = 2 from n = 192 on, where it measured 1-2% faster, else 1: 6% faster at 128^3)
@@ -129,9 +124,7 @@ struct Context {
   int mathMode = RTB200_MATH_FAST;
   Tuning tune;
   cudaStream_t stream = nullptr;  // internal stream for host-buffer calls
-  cudaEvent_t evStart = nullptr, evStop = nullptr, evSweep0 = nullptr, evSweep1 = nullptr, evFork = nullptr;
-  std::vector<cudaStream_t> chainStreams;
-  std::vector<cudaEvent_t> chainEvents;
+  cudaEvent_t evStart = nullptr, evStop = nullptr, evSweep0 = nullptr, evSweep1 = nullptr;
   int smCount = 148;
   size_t l2Bytes = 0;
 
@@ -178,11 +171,6 @@ struct Context {
   size_t accBytes = 0;
   double* dPlanes = nullptr;   // ping-pong top-exit planes
   size_t planeBytes = 0;
-  void* dMarchSeg = nullptr;   // per-task layer tables of the persistent uniform sweep
-  size_t marchSegBytes = 0;
-  std::string marchSegKey;
-  int32_t* dMarchProg = nullptr;   // work counter + per-tile progress words of the persistent uniform sweep
-  size_t marchProgBytes = 0;
   void* dAmrScratch = nullptr;
   size_t amrScratchBytes = 0;
   int32_t* dErr = nullptr;     // device error flag

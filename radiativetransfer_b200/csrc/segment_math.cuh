@@ -72,34 +72,7 @@ __device__ __forceinline__ void exp_neg_parts(double tau, const double* __restri
 // Measured at 256^3 on one box, 20 solves back to back under the power cap: 16 entries / r^7 53.8 ms, 32 / r^5
 // 50.7 ms, 64 / r^4 49.8 ms (the 4-way bank conflicts of the larger table cost less than the DFMA saves).
 // (The point-source kernels keep the 16-entry / r^7 version above: their deposits are differences of exponentials.)
-#ifndef RTB_EXP_TABLE
-#define RTB_EXP_TABLE 64
-#endif
-constexpr int kExpTableSize = RTB_EXP_TABLE;
-#if RTB_EXP_TABLE == 32   // 32 entries, |r| <= ln2/64, polynomial through r^5
-static __constant__ double kExpC32[12] = {
-    -8.33333333333333333333e-03,  // [0] -1/5!
-    4.16666666666666666667e-02,   // [1]  1/4!
-    -1.66666666666666666667e-01,  // [2] -1/3!
-    0.5,                          // [3]
-    -1.0,                         // [4]
-    46.16624130844683,            // [5]  32/ln2
-    6755399441055744.0,           // [6]  1.5 * 2^52
-    -0.02166084898635745,         // [7]  -ln2/32, high part (28 trailing zero bits)
-    -4.06140840434059e-10,        // [8]  -ln2/32, low part
-    0., 0., 0.};
-constexpr int kExpDeg = 4;       // Horner steps after the leading coefficient
-constexpr int kExpShift = 5;
-static __constant__ double kExpTable32[32] = {
-    1.00000000000000000000e+00, 9.78572062087700089705e-01, 9.57603280698573700036e-01, 9.37083817055149981279e-01,
-    9.17004043204671215328e-01, 8.97354537501553584100e-01, 8.78126080186649726755e-01, 8.59309649061238967072e-01,
-    8.40896415253714502036e-01, 8.22877739076982472888e-01, 8.05245165974627141736e-01, 7.87990422553943248296e-01,
-    7.71105412703970372057e-01, 7.54582213796711420706e-01, 7.38413072969749673113e-01, 7.22590403488523325137e-01,
-    7.07106781186547572737e-01, 6.91954940981916011289e-01, 6.77127773468446325644e-01, 6.62618321579870661608e-01,
-    6.48419777325504820276e-01, 6.34525478595866609943e-01, 6.20928906036742001007e-01, 6.07623679990234477621e-01,
-    5.94603557501360513449e-01, 5.81862429388788737761e-01, 5.69394317378345782288e-01, 5.57193371297946216103e-01,
-    5.45253866332628844837e-01, 5.33570200338411848584e-01, 5.22136891213706877402e-01, 5.10948574327058313571e-01};
-#else   // 64 entries, |r| <= ln2/128, polynomial through r^4 (default)
+constexpr int kExpTableSize = 64;   // |r| <= ln2/128, polynomial through r^4
 static __constant__ double kExpC32[12] = {
     0., 4.16666666666666666667e-02, -1.66666666666666666667e-01, 0.5, -1.0,
     92.33248261689366,            // [5]  64/ln2
@@ -126,7 +99,6 @@ static __constant__ double kExpTable32[64] = {
     5.69394317378345782288e-01, 5.63260809304120924068e-01, 5.57193371297946216103e-01, 5.51191291653920445448e-01,
     5.45253866332628844837e-01, 5.39380398878559930154e-01, 5.33570200338411848584e-01, 5.27822589180278578525e-01,
     5.22136891213706877402e-01, 5.16512439510614207450e-01, 5.10948574327058313571e-01, 5.05444643025850237628e-01};
-#endif
 
 template <bool GUARD = true>
 __device__ __forceinline__ void exp_neg_parts32(double tau, const double* __restrict__ T, double& Ts, double& p) {
@@ -144,48 +116,6 @@ __device__ __forceinline__ void exp_neg_parts32(double tau, const double* __rest
   Ts = __hiloint2double(__double2hiint(Tj) - ((k >> kExpShift) << 20), __double2loint(Tj));
 }
 
-// Table-free variant (T == nullptr at compile time is not needed: chosen by the EXPV template parameter):
-// exp(-tau) = 2^n * exp(r), n = round(-tau/ln2), |r| <= ln2/2, Taylor through r^12.  ~20 FP64 instructions.
-static __constant__ double kExpP[16] = {
-    2.08767569878680989792e-09, 2.50521083854417187751e-08, 2.75573192239858906526e-07, 2.75573192239858906526e-06,
-    2.48015873015873015873e-05, 1.98412698412698412698e-04, 1.38888888888888888889e-03, 8.33333333333333333333e-03,
-    4.16666666666666666667e-02, 1.66666666666666666667e-01, 0.5,
-    -1.4426950408889634074,       // [11] -log2(e)
-    6755399441055744.0,           // [12]
-    -6.93147180369123816490e-01,  // [13] -ln2 hi
-    -1.90821492927058770002e-10,  // [14] -ln2 lo
-    707.0};
-__device__ __forceinline__ void exp_neg_parts_poly(double tau, double& Ts, double& p) {
-  tau = __hiloint2double(min(__double2hiint(tau), 0x40861800), __double2loint(tau));
-  double t = fma(tau, kExpP[11], kExpP[12]);
-  int n = __double2loint(t);
-  double fn = t - kExpP[12];
-  double r = fma(fn, kExpP[13], -tau);
-  r = fma(fn, kExpP[14], r);
-  double q = kExpP[0];
-#pragma unroll
-  for (int i = 1; i <= 10; i++) q = fma(q, r, kExpP[i]);
-  p = fma(r * r, q, r);                                       // exp(r) - 1
-  Ts = __hiloint2double(0x3ff00000 + (n << 20), 0);           // 2^n
-}
-
-template <int EXPV>
-__device__ __forceinline__ void exp_neg(double tau, const double* __restrict__ T, double& e, double& ome) {
-  double Ts, p;
-  if (EXPV == 1) exp_neg_parts(tau, T, Ts, p);
-  else exp_neg_parts_poly(tau, Ts, p);
-  e = fma(Ts, p, Ts);
-  ome = fma(-Ts, p, 1.0 - Ts);
-}
-
-template <int EXPV>
-__device__ __forceinline__ double exp_neg_only(double tau, const double* __restrict__ T) {
-  double Ts, p;
-  if (EXPV == 1) exp_neg_parts(tau, T, Ts, p);
-  else exp_neg_parts_poly(tau, Ts, p);
-  return fma(Ts, p, Ts);
-}
-
 // FAST-mode segment: Iout = Iin e^-tau and the segment's contribution to the cell's mean intensity,
 //   J_seg * weight/nseg = Iin (1 - e^-tau) / (kappa d) * wn = [Iin (1 - e^-tau)] * cs * (2^-200 / kappa),
 // cs = 2^200 wn / d a per-(layer, direction, segment) constant from the host and 2^-200/kappa a per-cell constant that
@@ -196,11 +126,10 @@ __device__ __forceinline__ double exp_neg_only(double tau, const double* __restr
 // GUARD = false (tau <= 64 for every segment of the warp): no clamp, and no test for Iout underflowing to 0 -- with
 // tau <= 64 that can only happen where Iin < 5e-324 e^64 = 3e-296, i.e. where the segment's contribution to Jmean
 // (< Iin) is itself below every tolerance floor (the parity tests compare with a floor of 1e-290).
-template <int EXPV, bool GUARD = true>
+template <bool GUARD = true>
 __device__ __forceinline__ double segment_fast(double Iin, double tau, double cs, const double* __restrict__ T, double& A) {
   double Ts, p;
-  if (EXPV == 1) exp_neg_parts32<GUARD>(tau, T, Ts, p);
-  else exp_neg_parts_poly(tau, Ts, p);
+  exp_neg_parts32<GUARD>(tau, T, Ts, p);
   const double X = Iin * Ts;
   const double Iout = fma(X, p, X);
   const double Z = fma(-X, p, Iin - X);
@@ -209,11 +138,10 @@ __device__ __forceinline__ double segment_fast(double Iin, double tau, double cs
   return Iout;
 }
 
-template <int EXPV, bool GUARD = true>
+template <bool GUARD = true>
 __device__ __forceinline__ double attenuate_fast(double Iin, double tau, const double* __restrict__ T) {
   double Ts, p;
-  if (EXPV == 1) exp_neg_parts32<GUARD>(tau, T, Ts, p);
-  else exp_neg_parts_poly(tau, Ts, p);
+  exp_neg_parts32<GUARD>(tau, T, Ts, p);
   const double X = Iin * Ts;
   return fma(X, p, X);
 }
@@ -222,27 +150,14 @@ struct SegResult {
   double Iout, J;
 };
 
-// FAST mode expects kappa > 0 (callers replace an exact zero by a tiny positive number, for which every formula
-// below returns the kappa = 0 limits Iout = Iin, J = Iin) and invtau = 1 / (kappa * dpath).
-template <bool FAITHFUL, int EXPV>
-__device__ __forceinline__ SegResult segment_update(double Iin, double kappa, double dpath, double invtau,
-                                                    const double* __restrict__ T) {
+// FAITHFUL-mode segment: the reference's operation sequence (CUDA libm exp / log, IEEE arithmetic, no contraction)
+__device__ __forceinline__ SegResult segment_faithful(double Iin, double kappa, double dpath) {
   SegResult r;
-  if (FAITHFUL) {
-    double tau = __dmul_rn(kappa, dpath);
-    double a = exp(-tau);
-    r.Iout = __dmul_rn(Iin, a);
-    if (r.Iout < Iin) r.J = __ddiv_rn(__dsub_rn(Iin, r.Iout), log(__ddiv_rn(Iin, r.Iout)));
-    else r.J = __dmul_rn(0.5, __dadd_rn(Iin, r.Iout));
-  } else {
-    double tau = kappa * dpath, e, ome;
-    exp_neg<EXPV>(tau, T, e, ome);
-    r.Iout = Iin * e;
-    // Iout == 0 (underflow): the reference gets (Iin - 0)/log(Iin/0) = 0.  (Where Iout is a non-zero SUBNORMAL,
-    // i.e. per-segment tau of ~650-745, the reference's log sees only the few bits Iout has left; FAST mode returns
-    // the smooth value there -- use FAITHFUL mode to reproduce that artefact.)
-    r.J = ((__double_as_longlong(r.Iout) << 1) == 0) ? 0.0 : Iin * (ome * invtau);
-  }
+  double tau = __dmul_rn(kappa, dpath);
+  double a = exp(-tau);
+  r.Iout = __dmul_rn(Iin, a);
+  if (r.Iout < Iin) r.J = __ddiv_rn(__dsub_rn(Iin, r.Iout), log(__ddiv_rn(Iin, r.Iout)));
+  else r.J = __dmul_rn(0.5, __dadd_rn(Iin, r.Iout));
   return r;
 }
 
@@ -271,12 +186,11 @@ __device__ __forceinline__ double emission_t(double tau, double ome, double invk
 
 // FAST-mode segment with emission: as segment_fast, plus E += phi(tau) * dw (dw = dpath * weight / nseg; the caller
 // adds eta * E to the cell's sum once per layer) and the emitted part of Iout.  invk = 1 / kappa (kappa floored).
-template <int EXPV, bool GUARD = true>
+template <bool GUARD = true>
 __device__ __forceinline__ double segment_fast_emit(double Iin, double tau, double cs, const double* __restrict__ T, double& A,
                                                     double eta, double invk, double d, double dw, double& E) {
   double Ts, p;
-  if (EXPV == 1) exp_neg_parts32<GUARD>(tau, T, Ts, p);
-  else exp_neg_parts_poly(tau, Ts, p);
+  exp_neg_parts32<GUARD>(tau, T, Ts, p);
   const double X = Iin * Ts;
   const double Iatt = fma(X, p, X);
   const double Z = fma(-X, p, Iin - X);
@@ -287,20 +201,19 @@ __device__ __forceinline__ double segment_fast_emit(double Iin, double tau, doub
 }
 
 // the outgoing intensity alone, bit for bit what segment_fast_emit returns for the same arguments
-template <int EXPV, bool GUARD = true>
+template <bool GUARD = true>
 __device__ __forceinline__ double attenuate_fast_emit(double Iin, double tau, const double* __restrict__ T, double eta,
                                                       double invk, double d) {
   double Ts, p;
-  if (EXPV == 1) exp_neg_parts32<GUARD>(tau, T, Ts, p);
-  else exp_neg_parts_poly(tau, Ts, p);
+  exp_neg_parts32<GUARD>(tau, T, Ts, p);
   const double X = Iin * Ts;
   const double Iatt = fma(X, p, X);
   const double ome = fma(-Ts, p, 1.0 - Ts);
   return fma(eta, emission_t(tau, ome, invk, d), Iatt);
 }
 
-// FAITHFUL-mode segment with emission: L is segment_update<true>'s operation sequence on the attenuated part, the eta
-// terms are one FMA each, so eta = 0 reproduces segment_update<true> bit for bit
+// FAITHFUL-mode segment with emission: L is segment_faithful's operation sequence on the attenuated part, the eta
+// terms are one FMA each, so eta = 0 reproduces segment_faithful bit for bit
 __device__ __forceinline__ SegResult segment_faithful_emit(double Iin, double kappa, double dpath, double eta) {
   SegResult r;
   const double tau = __dmul_rn(kappa, dpath);

@@ -1,5 +1,5 @@
-"""small end-to-end calls of every path for compute-sanitizer (memcheck): uniform sweep (per-layer kernels with one and
-two cells per thread, the one-launch layer loop, both math modes), nested-grid sweep (per-wave launches and the streamed
+"""small end-to-end calls of every path for compute-sanitizer (memcheck): uniform sweep (one and two cells per thread,
+block sizes, both math modes), nested-grid sweep (per-wave launches and the streamed
 one-launch path, several sweeps), point sources (three deposition modes, trace), a device group of one, octree build"""
 import os, sys
 import numpy as np
@@ -16,11 +16,11 @@ for mode in (rt.MATH_FAST, rt.MATH_FAITHFUL):
     J, nseg = t.diffuse(bg["uvb"], bg["beta"], rays=list(range(0, 192, 5)))
     print("uniform", mode, nseg, float(J.sum()))
 t.set_math(rt.MATH_FAST)
-for kw in (dict(cells=1), dict(cells=2), dict(cells=2, block_warps=2), dict(persistent=1), dict(persistent=1, block_warps=8)):
-    t.set_tuning(cells=0, block_warps=0, persistent=0); t.set_tuning(**kw)
+for kw in (dict(cells=1), dict(cells=2), dict(cells=2, block_warps=2)):
+    t.set_tuning(cells=0, block_warps=0); t.set_tuning(**kw)
     J, nseg = t.diffuse(bg["uvb"], bg["beta"], rays=list(range(0, 192, 5)))
     print("uniform", kw, nseg, float(J.sum()), t.device_error())
-t.set_tuning(cells=0, block_warps=0, persistent=0)
+t.set_tuning(cells=0, block_warps=0)
 gb = W.nested_grid(8, 1, W.central_box_refine(0.25, 0.75), seed=3)      # 2:1 balanced: streamed path
 t.set_grid(gb["nx"], gb["level"], gb["HI"], gb["HeI"], gb["HeII"], gb["rho"], gb["abun2"], gb["box_size"])
 for stream in (1, 1, 1, 0, 1):

@@ -9,7 +9,7 @@ import radiativetransfer_b200 as rt
 from radiativetransfer_b200 import sharding, workloads as W
 n = 256
 world = int(sys.argv[1]) if len(sys.argv) > 1 else 8
-variants = sys.argv[2:] or ["0"]          # block_warps[:lockstep[:slots[:persistent]]] or key=value,key=value (set_tuning keys)
+variants = sys.argv[2:] or ["0"]          # block_warps[:slots] or key=value,key=value (set_tuning keys)
 bg = W.uvb_background(3.0)
 g = W.uniform_grid(n, seed=1)
 t = rt.Transport(device=0)
@@ -18,15 +18,14 @@ J = torch.zeros(3, n ** 3, dtype=torch.float64, device="cuda:0")
 s = torch.cuda.current_stream().cuda_stream
 shards = sharding.shard_directions(world, n_angular_level=3, nx=n)
 zone, cost = sharding.direction_costs(3, 64)
-DEFAULTS = dict(block_warps=0, lockstep=1, slots=0, persistent=0, dense=0, cells=0, dirs_per_task=0)
+DEFAULTS = dict(block_warps=0, slots=0, cells=0, dirs_per_task=0)
 for v in variants:
     if "=" in v:                 # k=v,k=v
         kv = {k: int(x) for k, x in (f.split("=") for f in v.split(","))}
-    else:                        # block_warps[:lockstep[:slots[:persistent]]]
+    else:                        # block_warps[:slots]
         f = [int(x) for x in v.split(":")]
-        kv = dict(zip(("block_warps", "lockstep", "slots", "persistent"), f))
+        kv = dict(zip(("block_warps", "slots"), f))
     cfg = dict(DEFAULTS); cfg.update(kv)
-    persistent = cfg["persistent"]
     t.set_tuning(**cfg)
     times, totals = [], []
     for rank in range(world):
@@ -34,13 +33,6 @@ for v in variants:
             t.diffuse_device(bg["uvb"], bg["beta"], J.data_ptr(), rays=shards[rank], stream=s)
             torch.cuda.synchronize()
             st = t.last_stats()
-        if persistent == 1:         # the layer loop in one launch must reproduce the per-layer launches bit for bit
-            Jp = J.clone()
-            t.set_tuning(persistent=0)
-            t.diffuse_device(bg["uvb"], bg["beta"], J.data_ptr(), rays=shards[rank], stream=s)
-            torch.cuda.synchronize()
-            t.set_tuning(persistent=1)
-            print(f"   persistent vs per-layer launches: max |dJ| {float((Jp - J).abs().max()):.3e}", flush=True)
         zs = sorted(set(int(zone[r]) for r in shards[rank]))
         times.append(st["sweep_ms"]); totals.append(st["device_ms"])
         print(f"world {world} block_warps {v} rank {rank} ndir {len(shards[rank])} zones {zs} segs/col {cost[shards[rank]].sum():.0f}: "

@@ -1,4 +1,4 @@
-"""GPU experiment: single-cell vs two-cells-per-thread uniform sweep (set_tuning cells / dense), 256^3 and 128^3, with a
+"""GPU experiment: single-cell vs two-cells-per-thread uniform sweep (set_tuning cells), 256^3 and 128^3, with a
 bit-for-bit comparison of the results"""
 import os, sys
 import numpy as np
@@ -14,8 +14,8 @@ for n in (255, 128, 256):
     J = torch.zeros(3, n ** 3, dtype=torch.float64, device="cuda:0")
     s = torch.cuda.current_stream().cuda_stream
     ref = None
-    for cells, dense in ((1, 2), (2, 2), (2, 3), (2, 4), (1, 2), (2, 2)):
-        t.set_tuning(cells=cells, dense=dense)
+    for cells in (1, 2, 1, 2):
+        t.set_tuning(cells=cells)
         ms = []
         for rep in range(5):
             nseg = t.diffuse_device(bg["uvb"], bg["beta"], J.data_ptr(), stream=s)
@@ -27,6 +27,6 @@ for n in (255, 128, 256):
             ref = Jh
         same = bool(np.array_equal(Jh, ref))
         best = min(ms[1:])
-        print(f"n={n} cells={cells} dense={dense}: sweep ms {['%.2f' % m for m in ms]} best {best:.2f} total {st['device_ms']:.2f} "
+        print(f"n={n} cells={cells}: sweep ms {['%.2f' % m for m in ms]} best {best:.2f} total {st['device_ms']:.2f} "
               f"alg GB/s {st['algorithmic_bytes'] / best / 1e6:.0f} identical_to_first={same}", flush=True)
     t.close()

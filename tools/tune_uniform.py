@@ -14,9 +14,8 @@ from radiativetransfer_b200 import workloads as W  # noqa: E402
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--n", type=int, nargs="+", default=[128, 256])
-# slots:dense:expv:lockstep:math[:-:-:dirs_per_task:pdl]   (fields 6 and 7 were the removed round-1 march kernel's)
-ap.add_argument("--variants", nargs="+", default=["0:2:1:1:fast", "0:2:0:1:fast", "0:1:1:1:fast", "0:0:1:1:fast", "16:2:1:1:fast",
-                                                   "8:2:1:1:fast", "24:2:1:0:fast", "0:0:0:1:faithful"])
+# slots:math[:dirs_per_task:pdl]
+ap.add_argument("--variants", nargs="+", default=["0:fast", "16:fast", "8:fast", "0:faithful"])
 ap.add_argument("--reps", type=int, default=3)
 args = ap.parse_args()
 bg = W.uvb_background(3.0)
@@ -28,11 +27,11 @@ for n in args.n:
     s = torch.cuda.current_stream().cuda_stream
     for v in args.variants:
         f = v.split(":")
-        slots, dense, expv, lockstep, mode = f[:5]
-        dpt = int(f[7]) if len(f) > 7 else 0
-        pdl = int(f[8]) if len(f) > 8 else 0
+        slots, mode = f[:2]
+        dpt = int(f[2]) if len(f) > 2 else 0
+        pdl = int(f[3]) if len(f) > 3 else 0
         t.set_math(rt.MATH_FAST if mode == "fast" else rt.MATH_FAITHFUL)
-        t.set_tuning(slots=int(slots), dense=int(dense), expv=int(expv), lockstep=int(lockstep), dirs_per_task=dpt, pdl=pdl)
+        t.set_tuning(slots=int(slots), dirs_per_task=dpt, pdl=pdl)
         ms = []
         for rep in range(args.reps + 1):
             nseg = t.diffuse_device(bg["uvb"], bg["beta"], J.data_ptr(), stream=s)
@@ -40,7 +39,7 @@ for n in args.n:
             st = t.last_stats()
             ms.append(st["sweep_ms"])
         best = min(ms[1:])
-        print(f"n={n} slots={slots} dense={dense} expv={expv} lockstep={lockstep} dpt={dpt} pdl={pdl} math={mode}: ms={['%.2f' % m for m in ms]} "
+        print(f"n={n} slots={slots} dpt={dpt} pdl={pdl} math={mode}: ms={['%.2f' % m for m in ms]} "
               f"seg/s={nseg / best * 1e3:.3e} alg GB/s={st['algorithmic_bytes'] / best / 1e6:.1f} "
               f"total_ms={st['device_ms']:.2f} launches={st['launches']}", flush=True)
     t.close()
