@@ -174,6 +174,30 @@ int rtb200_grid_update_species(rtb200_ctx* ctx, const double* HI, const double* 
 int rtb200_grid_set_emission(rtb200_ctx* ctx, const double* eta);
 int rtb200_grid_set_emission_device(rtb200_ctx* ctx, const double* eta_device, void* stream);
 
+/* Scattering (an extension without a reference value, DESIGN.md 4.7): per leaf and frequency group a scattering
+ * coefficient sigma >= 0 in the units of kappa (1/cm), [3][nleaf] in the leaf order of rtb200_grid_set; coherent within a
+ * group and isotropic.  The sweep then uses the extinction kappa_ext = kappa_abs + sigma (sigma added last, rounded
+ * once) and solves by source iteration: sweep k runs with the emission coefficient
+ *     eta_k = eta_th + sigma * J_{k-1}     (two roundings, no FMA),   J_0 = 0,
+ * eta_th being the emission of rtb200_grid_set_emission (0 if none) and J the full Jmean of the previous sweep.  The
+ * residual of sweep k is r_k = max over (group, leaf) of |J_k - J_{k-1}| / J_k (0 where J_k == J_{k-1}, +inf where
+ * J_k == 0 != J_{k-1}); with tolerance > 0 the solve stops after the first k with r_k <= tolerance or at maxIterations,
+ * with tolerance == 0 it runs exactly maxIterations sweeps without reading anything back in between (so it stays
+ * asynchronous on the stream of the *_device calls).  Not converging is not an error: the call returns J_k.
+ * rtb200_diffuse, rtb200_diffuse_device, the device-group host call and rtb200_multi_diffuse_resident (whose photo-rates
+ * are those of the last iteration, its chemistry runs once after it) solve this way; a direction subset (rays != NULL)
+ * returns RTB200_ERR_ARG, because a shard's J is not the mean intensity.  The point-source path ignores scattering.
+ * nseg and rtb200_last_stats count all sweeps of the call (algorithmic bytes 96 B per leaf, direction and iteration; the
+ * device time covers the whole call, the sweep time is the last sweep's).  sigma = 0 gives the results of no scattering
+ * bit for bit (with tolerance > 0 after 2 sweeps, residual 0).  rtb200_grid_set clears the scattering,
+ * rtb200_grid_update_species keeps it; a device group reads sigma slab-wise as the emission.
+ *   rtb200_grid_set_scattering  sigma = host [3][nleaf], copied (NULL clears); maxIterations >= 1; tolerance >= 0 and
+ *                               finite.  A negative, NaN or Inf entry or a bad count or tolerance is refused with
+ *                               RTB200_ERR_ARG and the previous state stays.  Queued work completes before the copy.
+ *   rtb200_last_scattering      sweeps done and the last residual of the latest diffuse call (0 / 0 without scattering). */
+int rtb200_grid_set_scattering(rtb200_ctx* ctx, const double* sigma, int32_t maxIterations, double tolerance);
+int rtb200_last_scattering(rtb200_ctx* ctx, int32_t* iterations, double* residual);
+
 /* Diffuse (UV background) sweep: replaces equiSources.f90:1372-1808 (computeOpacities :4956, the loop over
  * 12*4**(nAngularLevel-1) HEALPix directions, pattern set-up, neighbour threading, transport).
  *   uvb[3]      boundary intensities uvb1..3 (definitionsModule.f90:53)

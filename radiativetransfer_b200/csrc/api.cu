@@ -63,6 +63,10 @@ static void free_grid(Context& c) {
   cudaFree(c.dKappaT); c.dKappaT = nullptr; c.kappaTBytes = 0;
   cudaFree(c.dEta); c.dEta = nullptr;
   cudaFree(c.dEtaT); c.dEtaT = nullptr; c.etaTBytes = 0;
+  cudaFree(c.dSigma); c.dSigma = nullptr;
+  cudaFree(c.dEtaEff); c.dEtaEff = nullptr;
+  cudaFree(c.dScatScratch); c.dScatScratch = nullptr; c.scatScratchBytes = 0;
+  c.scatMaxIter = 1; c.scatTol = 0.; c.lastScatIter = 0; c.lastScatResid = 0.; c.scatResidPending = false;
   cudaFree(c.dLogT); c.dLogT = nullptr;
   for (auto& sl : c.pointPool) cudaFree(sl.first);
   c.pointPool.clear();
@@ -160,15 +164,22 @@ static int resolve_directions(int nAngularLevel, const int32_t* rays, int32_t nr
   return RTB200_OK;
 }
 
-int run_diffuse(Context& c, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays,
-                       int32_t nrays, double* dJ, cudaStream_t s, int64_t* nseg) {
+int run_sweep(Context& c, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays, int32_t nrays,
+              double* dJ, cudaStream_t s, int64_t* nseg, int iter) {
   if (!uvb || !beta || !dJ) return RTB200_ERR_ARG;
   if (c.nleaf == 0) return RTB200_ERR_ARG;
   std::vector<Direction> dirs;
   if (int st = resolve_directions(nAngularLevel, rays, nrays, dirs)) return st;
   RTB_CUDA(cudaSetDevice(c.device));
-  RTB_CUDA(cudaEventRecord(c.evStart, s));
-  if (int st = launch_compute_opacities(c, beta, s)) return st;
+  // the later sweeps of a source iteration add their counts to the earlier ones
+  const int64_t launches0 = iter > 1 ? c.lastLaunches : 0, sweepLaunches0 = iter > 1 ? c.lastSweepLaunches : 0;
+  const double bytes0 = iter > 1 ? c.lastAlgBytes : 0.;
+  if (iter <= 1) {
+    RTB_CUDA(cudaEventRecord(c.evStart, s));
+    if (int st = launch_compute_opacities(c, beta, s)) return st;
+    if (c.dSigma)
+      if (int st = launch_add_scattering(c, s)) return st;
+  }
   int64_t ns = 0;
   const bool uniformPath = c.uniform && !c.tune.forceAmr;
   int st = uniformPath ? diffuse_uniform(c, nAngularLevel, uvb, dirs, dJ, s, &ns)
@@ -177,10 +188,22 @@ int run_diffuse(Context& c, int nAngularLevel, const double* uvb, const double* 
   RTB_CUDA(cudaEventRecord(c.evStop, s));
   if (nseg) *nseg = ns;
   // 72 B per leaf and direction (SURVEY.md 8d), 96 B with the emission coefficients of the 3 groups
-  c.lastAlgBytes = (c.dEta ? 96.0 : 72.0) * (double)c.nleaf * (double)dirs.size();
+  c.lastAlgBytes = bytes0 + (c.sweepEta() ? 96.0 : 72.0) * (double)c.nleaf * (double)dirs.size();
+  c.lastLaunches += launches0;
+  c.lastSweepLaunches += sweepLaunches0;
   c.statsPending = true;
   c.sweepTimed = uniformPath && !dirs.empty();
   return RTB200_OK;
+}
+
+int run_diffuse(Context& c, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays,
+                int32_t nrays, double* dJ, cudaStream_t s, int64_t* nseg) {
+  c.lastScatIter = 0;
+  c.lastScatResid = 0.;
+  c.scatResidPending = false;
+  if (!c.dSigma) return run_sweep(c, nAngularLevel, uvb, beta, rays, nrays, dJ, s, nseg, 0);
+  if (rays) return RTB200_ERR_ARG;   // the J of a direction subset is not the mean intensity the source needs
+  return scatter_solve(c, nAngularLevel, uvb, beta, dJ, s, nseg);
 }
 
 // number of entries that are negative, NaN or Inf (the emission check of rtb200_grid_set_emission_device)
@@ -199,38 +222,29 @@ static bool host_eta_ok(const double* eta, int64_t n) {
   return true;
 }
 
-int set_emission(Context& c, const double* eta, bool device, cudaStream_t s) {
-  if (c.nleaf == 0) return RTB200_ERR_ARG;
-  RTB_CUDA(cudaSetDevice(c.device));
-  // queued sweeps read the current array (as rtb200_grid_update_species)
-  RTB_CUDA(cudaDeviceSynchronize());
+void drop_sweep_plans(Context& c) {
+  c.uniPlanKey.clear();
+  if (c.graphExec) { cudaGraphExecDestroy(c.graphExec); c.graphExec = nullptr; }
+}
+
+int replace_leaf_field(Context& c, double** field, const double* src, bool device, cudaStream_t s) {
   const int64_t n = 3 * c.nleaf;
   const size_t bytes = (size_t)n * sizeof(double);
-  auto drop_plans = [&] {   // the sweeps' plans and graphs know whether emission is set
-    c.uniPlanKey.clear();
-    if (c.graphExec) { cudaGraphExecDestroy(c.graphExec); c.graphExec = nullptr; }
-  };
-  if (!eta) {
-    cudaFree(c.dEta); c.dEta = nullptr;
-    cudaFree(c.dEtaT); c.dEtaT = nullptr; c.etaTBytes = 0;
-    drop_plans();
-    return RTB200_OK;
-  }
-  if (!device && !host_eta_ok(eta, n)) return RTB200_ERR_ARG;
-  // the new array goes to a buffer of its own first: a refused array leaves the previous emission in place
+  if (!device && !host_eta_ok(src, n)) return RTB200_ERR_ARG;
+  // the new array goes to a buffer of its own first: a refused array leaves the previous one in place
   double* fresh = nullptr;
   cudaError_t e = cudaMalloc((void**)&fresh, bytes);
   if (e != cudaSuccess) { set_cuda_error("cudaMalloc", e, __FILE__, __LINE__); return e == cudaErrorMemoryAllocation ? RTB200_ERR_NOMEM : RTB200_ERR_CUDA; }
   int st = RTB200_OK;
   if (!device) {
-    if (cudaMemcpyAsync(fresh, eta, bytes, cudaMemcpyHostToDevice, c.stream) != cudaSuccess ||
+    if (cudaMemcpyAsync(fresh, src, bytes, cudaMemcpyHostToDevice, c.stream) != cudaSuccess ||
         cudaStreamSynchronize(c.stream) != cudaSuccess)
       st = RTB200_ERR_CUDA;
   } else {
     int32_t* dBad = c.dErr + 12;  // scratch word of the 64-byte error block (chemistry uses words 8..11)
     int32_t bad = 0;
     const int blocks = (int)std::min<int64_t>((n + 255) / 256, (int64_t)c.smCount * 8);
-    if (cudaMemcpyAsync(fresh, eta, bytes, cudaMemcpyDeviceToDevice, s) != cudaSuccess ||
+    if (cudaMemcpyAsync(fresh, src, bytes, cudaMemcpyDeviceToDevice, s) != cudaSuccess ||
         cudaMemsetAsync(dBad, 0, sizeof(int32_t), s) != cudaSuccess)
       st = RTB200_ERR_CUDA;
     if (!st) {
@@ -242,10 +256,25 @@ int set_emission(Context& c, const double* eta, bool device, cudaStream_t s) {
     if (!st && bad) st = RTB200_ERR_ARG;
   }
   if (st) { cudaFree(fresh); return st; }
+  cudaFree(*field);
+  *field = fresh;
+  return RTB200_OK;
+}
+
+int set_emission(Context& c, const double* eta, bool device, cudaStream_t s) {
+  if (c.nleaf == 0) return RTB200_ERR_ARG;
+  RTB_CUDA(cudaSetDevice(c.device));
+  // queued sweeps read the current array (as rtb200_grid_update_species)
+  RTB_CUDA(cudaDeviceSynchronize());
+  if (!eta) {
+    cudaFree(c.dEta); c.dEta = nullptr;
+    cudaFree(c.dEtaT); c.dEtaT = nullptr; c.etaTBytes = 0;
+    drop_sweep_plans(c);   // the sweeps' plans and graphs know whether emission is set
+    return RTB200_OK;
+  }
   const bool had = c.dEta != nullptr;
-  cudaFree(c.dEta);
-  c.dEta = fresh;
-  if (!had) drop_plans();
+  if (int st = replace_leaf_field(c, &c.dEta, eta, device, s)) return st;
+  if (!had) drop_sweep_plans(c);
   else if (c.graphExec) { cudaGraphExecDestroy(c.graphExec); c.graphExec = nullptr; }   // the graph holds the pointer
   return RTB200_OK;
 }
@@ -465,6 +494,18 @@ int rtb200_grid_set_emission(rtb200_ctx* h, const double* eta) {
   if (!h) return RTB200_ERR_ARG;
   if (h->m) return multi_set_emission(h->m, eta);
   return set_emission(h->c, eta, false, h->c.stream);
+}
+
+int rtb200_grid_set_scattering(rtb200_ctx* h, const double* sigma, int32_t maxIterations, double tolerance) {
+  if (!h) return RTB200_ERR_ARG;
+  if (h->m) return multi_set_scattering(h->m, sigma, maxIterations, tolerance);
+  return set_scattering(h->c, sigma, false, maxIterations, tolerance);
+}
+
+int rtb200_last_scattering(rtb200_ctx* h, int32_t* iterations, double* residual) {
+  if (!h) return RTB200_ERR_ARG;
+  if (h->m) return multi_last_scattering(h->m, iterations, residual);
+  return last_scattering(h->c, iterations, residual);
 }
 
 int rtb200_grid_set_emission_device(rtb200_ctx* h, const double* eta_device, void* stream) {

@@ -1230,7 +1230,7 @@ static int run_batch(Context& c, AmrState& S, const DirTables& T, int g0, int ng
       RTB_CUDA(cudaMalloc((void**)&B.kappaS, (size_t)8 * N * R * sizeof(double)));
       B.kappaSRecord = R;
     }
-    kappa_slots_kernel<EMIT><<<cb, 256, 0, s>>>(c.dKappa, B.kappaS, P, c.dEta);
+    kappa_slots_kernel<EMIT><<<cb, 256, 0, s>>>(c.dKappa, B.kappaS, P, c.sweepEta());
     (*launches)++;
     P.patIdxS = S.plan.dPatIdxS; P.kappaS = B.kappaS;
     StreamParams Q;
@@ -1375,10 +1375,11 @@ int diffuse_amr(Context& c, int nAngularLevel, const double* uvb, const std::vec
   }
   int64_t launches = 0;
   const bool faithful = c.mathMode == RTB200_MATH_FAITHFUL;
-  const bool emit = c.dEta != nullptr;   // emission set (rtb200_grid_set_emission): the sweep kernels' EMIT instantiations
+  const double* etaSrc = c.sweepEta();   // emission or the scattering source: the sweep kernels' EMIT instantiations
+  const bool emit = etaSrc != nullptr;
   const int cpyBlocks = (int)std::min<int64_t>((3 * N + 255) / 256, (int64_t)c.smCount * 16);
   if (!st) {
-    if (emit) interleave_kappa_kernel<true><<<cpyBlocks, 256, 0, s>>>(c.dKappa, B.kappaA, N, c.dEta);
+    if (emit) interleave_kappa_kernel<true><<<cpyBlocks, 256, 0, s>>>(c.dKappa, B.kappaA, N, etaSrc);
     else interleave_kappa_kernel<false><<<cpyBlocks, 256, 0, s>>>(c.dKappa, B.kappaA, N);
     RTB_CUDA(cudaMemsetAsync(B.JA, 0, 3 * N * sizeof(double), s));
     launches += 1;

@@ -741,7 +741,8 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
   const int64_t nraysTotal = 12LL << (2 * (nAngularLevel - 1));
   const double weight = (double)(1.f / (float)nraysTotal);  // equiSources.f90:1386 (single-precision division)
   const double cellSize = c.boxSize / (double)n;             // equiSources.f90:1570
-  const bool emit = c.dEta != nullptr;                       // emission set (rtb200_grid_set_emission)
+  const double* etaSrc = c.sweepEta();                       // emission or the scattering source (scattering.cu)
+  const bool emit = etaSrc != nullptr;
 
   // ---- plan: pattern tables and zone tasks.  Depends only on the grid size and the direction list, so it is
   //      cached across the outer transport<->chemistry iterations. ----
@@ -884,7 +885,7 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
     if (c.uniStdSlots < (int)c.uniTasks.size() && c.uniStdSlots < c.uniSlots) {
       dim3 tg((n + 31) / 32, (n + 31) / 32, 3 * n);
       transpose_kappa_kernel<<<tg, dim3(32, 8), 0, st>>>(c.dKappa, c.dKappaT, n);
-      if (emit) transpose_kappa_kernel<<<tg, dim3(32, 8), 0, st>>>(c.dEta, c.dEtaT, n);
+      if (emit) transpose_kappa_kernel<<<tg, dim3(32, 8), 0, st>>>(etaSrc, c.dEtaT, n);
     }
     {  // both plane buffers start as "boundary intensity everywhere": first-layer input and the permanent pads
       const int64_t total = (int64_t)2 * ndir * 3 * npl;
@@ -908,7 +909,7 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
     static thread_local BatchParams bp;
     static thread_local EtaParams ep;
     const EtaParams* epp = emit ? &ep : nullptr;
-    auto etaOf = [&](const UniTaskHost& T) -> const double* { return T.transposed ? c.dEtaT : c.dEta; };
+    auto etaOf = [&](const UniTaskHost& T) -> const double* { return T.transposed ? c.dEtaT : etaSrc; };
     for (int base = 0; base < ntask; base += slots) {
       const int nb = std::min(slots, ntask - base);
       for (int step = 0; step < n; step++) {
@@ -931,7 +932,7 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
     char key[256];
     snprintf(key, sizeof(key), "u:%d:%d:%d:%d:%p:%p:%p:%a:%a:%a:%p:%p", n, ntask, slots,
              (int)faithful * 64 + 10000 * c.tune.pdl + 100000 * c.tune.cells + 1000000 * c.tune.blockWarps,
-             (void*)c.dAcc, (void*)c.dPlanes, (void*)c.dKappa, uvb[0], uvb[1], uvb[2], (void*)c.dEta, (void*)c.dEtaT);
+             (void*)c.dAcc, (void*)c.dPlanes, (void*)c.dKappa, uvb[0], uvb[1], uvb[2], (const void*)etaSrc, (void*)c.dEtaT);
     if (!c.graphExec || c.graphKey != key) {
       if (c.graphExec) { cudaGraphExecDestroy(c.graphExec); c.graphExec = nullptr; }
       cudaGraph_t graph;

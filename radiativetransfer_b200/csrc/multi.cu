@@ -28,6 +28,7 @@
 
 #include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -276,6 +277,10 @@ struct Member {                     // one local device
   cudaStream_t copyStream = nullptr;                    // slab uploads of update_species, one event per species
   cudaEvent_t evCopy[3] = {nullptr, nullptr, nullptr};
   int64_t nsegLast = 0;
+  // source iteration (scattering set): [3][npad] all-gather stage of the source | [3][slab] J of the previous
+  // iteration | [kMaxRanks] slab residuals of every rank | this rank's residual word
+  double* scat = nullptr;
+  size_t scatBytes = 0;
 };
 
 struct Multi {
@@ -320,6 +325,7 @@ void free_exchange(Multi& m) {
     q->ipcOpened.clear();
     cudaFree(q->exch[0]); cudaFree(q->exch[1]); cudaFree(q->flags);
     cudaFree(q->Jslab); cudaFree(q->Kslab); cudaFree(q->Rslab); cudaFree(q->Rbase);
+    cudaFree(q->scat); q->scat = nullptr; q->scatBytes = 0;
     q->exch[0] = q->exch[1] = nullptr; q->flags = nullptr;
     q->Jslab = q->Kslab = q->Rslab = q->Rbase = nullptr;
     q->haveR = false;
@@ -585,17 +591,18 @@ struct Epilogue {
 };
 
 // `nf` fields of exch[buf] (this rank's partial results, complete on stream s) -> out [nf][slab] = sum over the ranks
-int reduce_member(Multi& m, Member& q, int buf, int nf, double* out, const Epilogue& ep, cudaStream_t s) {
+// step = the exchange step of this reduction (its parity selects buf); a source iteration takes one step per iteration
+int reduce_member(Multi& m, Member& q, int buf, unsigned long long step, int nf, double* out, const Epilogue& ep, cudaStream_t s) {
   const int64_t off = slab_off(m, q.rank), cnt = slab_cnt(m, q.rank);
   const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>((cnt / 2 + 255) / 256, (int64_t)q.c.smCount * 8));
   const bool usePeer = m.reduceMode == 1 && m.peerOk;
   if (usePeer) {
     PeerFlagPtrs F{};
     for (int p = 0; p < m.nranks; p++) F.p[p] = q.peerFlags[p];
-    peer_signal_kernel_v<<<1, 32, 0, s>>>(F, m.nranks, q.rank, m.step);
+    peer_signal_kernel_v<<<1, 32, 0, s>>>(F, m.nranks, q.rank, step);
     PeerReduceParams P{};
     for (int p = 0; p < m.nranks; p++) P.src[p] = q.peerExch[buf][p];
-    P.flags = q.flags; P.step = m.step; P.err = q.c.dErr; P.nranks = m.nranks;
+    P.flags = q.flags; P.step = step; P.err = q.c.dErr; P.nranks = m.nranks;
     P.off = off; P.cnt = cnt; P.gstride = m.npad; P.slab = m.slab; P.out = out;
     P.kout = ep.ksi ? q.Kslab : nullptr; P.kAccumulate = ep.kAccumulate; P.base = ep.base;
     P.fourPi = 4. * kPi;
@@ -631,13 +638,14 @@ int reduce_member(Multi& m, Member& q, int buf, int nf, double* out, const Epilo
   return RTB200_OK;
 }
 
-// sweep of this member's direction shard into exch[buf][0..2] (padded layout)
-int sweep_member(Multi& m, Member& q, int buf, int nAngularLevel, const double* uvb, const double* beta, cudaStream_t s) {
+// sweep of this member's direction shard into exch[buf][0..2] (padded layout); iter: see run_sweep
+int sweep_member(Multi& m, Member& q, int buf, int nAngularLevel, const double* uvb, const double* beta, cudaStream_t s,
+                 int iter = 0) {
   const std::vector<int32_t>& mine = m.shards[(size_t)q.rank];
   static const int32_t none = 0;
   double* target = m.npad == m.nleaf ? q.exch[buf] : q.c.dJ;
   int64_t ns = 0;
-  int st = run_diffuse(q.c, nAngularLevel, uvb, beta, mine.empty() ? &none : mine.data(), (int32_t)mine.size(), target, s, &ns);
+  int st = run_sweep(q.c, nAngularLevel, uvb, beta, mine.empty() ? &none : mine.data(), (int32_t)mine.size(), target, s, &ns, iter);
   if (st) return st;
   q.nsegLast = ns;
   if (target != q.exch[buf]) {
@@ -777,13 +785,12 @@ int multi_update_species(Multi* m, const double* HI, const double* HeI, const do
   });
 }
 
-// the species are identical on every member after each step: every rank returns its slab (one process: the whole array)
-// Emission of a device group: every rank checks its slab of the caller's array, the ranks agree on the status (an
-// all-gather of one word each in rank mode), then every rank uploads its slab and all-gathers the three fields on the
-// devices, as multi_update_species does for the species.  NULL clears the emission everywhere.
-int multi_set_emission(Multi* m, const double* eta) {
-  if (m->nleaf == 0) return RTB200_ERR_ARG;
-  if (!eta) return for_each_member(*m, [&](Member& q, int) { return set_emission(q.c, nullptr, false, q.c.stream); });
+// A per-leaf [3][nleaf] field of a device group (emission, scattering): every rank checks its slab of the caller's
+// array, the ranks agree on the status (an all-gather of one word each in rank mode), then every rank uploads its slab
+// and all-gathers the three fields on the devices, as multi_update_species does for the species.  `apply(c, packed)`
+// installs the complete device copy [3][nleaf] in a member's context.
+template <class Apply>
+static int multi_set_field(Multi* m, const double* eta, Apply apply) {
   const int64_t N = m->nleaf;
   bool ok = true;
   for (Member* q : m->mem) {
@@ -837,11 +844,44 @@ int multi_set_emission(Multi* m, const double* eta) {
       if (cudaMemcpyAsync(packed + (size_t)g * N, stage + (size_t)g * m->npad, (size_t)N * sizeof(double),
                           cudaMemcpyDeviceToDevice, c.stream) != cudaSuccess)
         st = RTB200_ERR_CUDA;
-    if (!st) st = set_emission(c, packed, true, c.stream);
+    if (!st) st = apply(c, packed);
     cudaStreamSynchronize(c.stream);
     cudaFree(packed);
     return done(st);
   });
+}
+
+// NULL clears the emission everywhere
+int multi_set_emission(Multi* m, const double* eta) {
+  if (m->nleaf == 0) return RTB200_ERR_ARG;
+  if (!eta) return for_each_member(*m, [&](Member& q, int) { return set_emission(q.c, nullptr, false, q.c.stream); });
+  return multi_set_field(m, eta, [](Context& c, const double* packed) { return set_emission(c, packed, true, c.stream); });
+}
+
+// NULL clears the scattering everywhere
+int multi_set_scattering(Multi* m, const double* sigma, int32_t maxIterations, double tolerance) {
+  if (m->nleaf == 0) return RTB200_ERR_ARG;
+  if (!sigma) return for_each_member(*m, [&](Member& q, int) { return set_scattering(q.c, nullptr, false, 1, 0.); });
+  if (maxIterations < 1 || !(tolerance >= 0.) || std::isinf(tolerance)) return RTB200_ERR_ARG;
+  return multi_set_field(m, sigma, [&](Context& c, const double* packed) {
+    return set_scattering(c, packed, true, maxIterations, tolerance);
+  });
+}
+
+int multi_last_scattering(Multi* m, int32_t* iterations, double* residual) {
+  Member& q = *m->mem[0];
+  Context& c = q.c;
+  if (c.scatResidPending) {   // tolerance 0: every rank's slab residual was all-gathered on the devices
+    RTB_CUDA(cudaSetDevice(c.device));
+    RTB_CUDA(cudaDeviceSynchronize());
+    std::vector<double> all((size_t)m->nranks);
+    RTB_CUDA(cudaMemcpy(all.data(), q.scat + 3 * m->npad + 3 * m->slab, all.size() * sizeof(double), cudaMemcpyDeviceToHost));
+    c.lastScatResid = *std::max_element(all.begin(), all.end());
+    c.scatResidPending = false;
+  }
+  if (iterations) *iterations = c.lastScatIter;
+  if (residual) *residual = c.lastScatResid;
+  return RTB200_OK;
 }
 
 int multi_get_species(Multi* m, double* HI, double* HeI, double* HeII) {
@@ -877,16 +917,94 @@ int multi_device_error(Multi* m) {
   return first;
 }
 
+// Source iteration of one member (scattering set), iterations k = 1, 2, ...  Every iteration is an exchange step of its
+// own, step0 + k, so that the peer reduction's double buffering (DESIGN.md 5) keeps its parity:
+//   1. the sweep of the shard with the current source (opacities and sigma once, in the first),
+//   2. the reduction into Jslab (with the epilogue ep: photo-rates are overwritten, so the last iteration's stay),
+//   3. the slab's source pass: eta_th + sigma * J into this rank's part of the stage, the slab residual,
+//   4. the all-gather of the three source fields, copied into the effective buffer [3][nleaf],
+//   5. with a tolerance, an all-gather of the slab residuals: every rank takes the same max and stops after the same k.
+// Returns the number of iterations in *iters.
+static int scatter_member(Multi& m, Member& q, unsigned long long step0, int nAngularLevel, const double* uvb,
+                          const double* beta, const Epilogue& ep, cudaStream_t s, int* iters) {
+  Context& c = q.c;
+  const int64_t N = m.nleaf, off = slab_off(m, q.rank), cnt = slab_cnt(m, q.rank);
+  const size_t need = (size_t)(3 * m.npad + 3 * m.slab + kMaxRanks + 1) * sizeof(double);
+  if (int st = ensure_buffer((void**)&q.scat, &q.scatBytes, need)) return st;
+  double* stage = q.scat;
+  double* Jprev = stage + 3 * m.npad;
+  double* all = Jprev + 3 * m.slab;
+  unsigned long long* resid = (unsigned long long*)(all + kMaxRanks);
+  const size_t nb = (size_t)3 * N * sizeof(double);
+  // J_0 = 0, eta_1 = eta_th
+  RTB_CUDA(cudaMemsetAsync(Jprev, 0, (size_t)3 * m.slab * sizeof(double), s));
+  if (c.dEta) RTB_CUDA(cudaMemcpyAsync(c.dEtaEff, c.dEta, nb, cudaMemcpyDeviceToDevice, s));
+  else RTB_CUDA(cudaMemsetAsync(c.dEtaEff, 0, nb, s));
+  auto gather_resid = [&]() -> int {   // every rank's slab residual into all[0 .. nranks)
+    RTB_CUDA(cudaMemcpyAsync(all + q.rank, resid, sizeof(double), cudaMemcpyDeviceToDevice, s));
+    if (m.nranks > 1) RTB_NCCL(nccl().AllGather(all + q.rank, all, 1, kNcclFloat64, q.comm, s));
+    return RTB200_OK;
+  };
+  int64_t nsTotal = 0;
+  int k = 1;
+  double r = 0.;
+  for (;; k++) {
+    const unsigned long long step = step0 + (unsigned long long)k;
+    const int buf = (int)(step & 1);
+    if (int st = sweep_member(m, q, buf, nAngularLevel, uvb, beta, s, k)) return st;
+    nsTotal += q.nsegLast;
+    if (int st = reduce_member(m, q, buf, step, 3, q.Jslab, ep, s)) return st;
+    RTB_CUDA(cudaMemsetAsync(resid, 0, sizeof(unsigned long long), s));
+    if (int st = launch_scatter_source(c, cnt, q.Jslab, Jprev, m.slab, c.dSigma + off, c.dEta ? c.dEta + off : nullptr, N,
+                                       stage + (size_t)q.rank * m.slab, m.npad, resid, s))
+      return st;
+    if (m.nranks > 1) {
+      RTB_NCCL(nccl().GroupStart());
+      for (int g = 0; g < 3; g++) {
+        double* f = stage + (size_t)g * m.npad;
+        RTB_NCCL(nccl().AllGather(f + (size_t)q.rank * m.slab, f, (size_t)m.slab, kNcclFloat64, q.comm, s));
+      }
+      RTB_NCCL(nccl().GroupEnd());
+    }
+    for (int g = 0; g < 3; g++)
+      RTB_CUDA(cudaMemcpyAsync(c.dEtaEff + (size_t)g * N, stage + (size_t)g * m.npad, (size_t)N * sizeof(double),
+                               cudaMemcpyDeviceToDevice, s));
+    c.lastLaunches += 1;
+    if (c.scatTol > 0.) {
+      if (int st = gather_resid()) return st;
+      std::vector<double> v((size_t)m.nranks);
+      RTB_CUDA(cudaMemcpyAsync(v.data(), all, v.size() * sizeof(double), cudaMemcpyDeviceToHost, s));
+      RTB_CUDA(cudaStreamSynchronize(s));
+      r = *std::max_element(v.begin(), v.end());
+      if (r <= c.scatTol) break;
+    }
+    if (k == c.scatMaxIter) break;
+  }
+  if (c.scatTol == 0.)   // read by rtb200_last_scattering: no host round trip in the call
+    if (int st = gather_resid()) return st;
+  RTB_CUDA(cudaEventRecord(c.evStop, s));
+  q.nsegLast = nsTotal;
+  c.lastScatIter = k;
+  c.lastScatResid = r;
+  c.scatResidPending = c.scatTol == 0.;
+  *iters = k;
+  return RTB200_OK;
+}
+
 // resident step of one member on stream s: opacities + sweep of the shard + reduce-scatter (+ photo-rates)
 // (+ ionisation equilibrium on the slab + all-gather of the new species)
 static int diffuse_resident_member(Multi& m, Member& q, int nAngularLevel, const double* uvb, const double* beta,
-                                   const double* ksi6, int chemistry, cudaStream_t s) {
-  const int buf = (int)(m.step & 1);
-  if (int st = sweep_member(m, q, buf, nAngularLevel, uvb, beta, s)) return st;
+                                   const double* ksi6, int chemistry, cudaStream_t s, int* iters) {
   Epilogue ep;
   ep.ksi = ksi6;
   ep.kAccumulate = 0;
-  if (int st = reduce_member(m, q, buf, 3, q.Jslab, ep, s)) return st;
+  if (q.c.dSigma) {   // source iteration, steps m.step .. m.step + iterations - 1; chemistry once, after it
+    if (int st = scatter_member(m, q, m.step - 1, nAngularLevel, uvb, beta, ep, s, iters)) return st;
+  } else {
+    const int buf = (int)(m.step & 1);
+    if (int st = sweep_member(m, q, buf, nAngularLevel, uvb, beta, s)) return st;
+    if (int st = reduce_member(m, q, buf, m.step, 3, q.Jslab, ep, s)) return st;
+  }
   if (chemistry) {
     if (!ksi6) return RTB200_ERR_ARG;
     const int64_t off = slab_off(m, q.rank), cnt = slab_cnt(m, q.rank);
@@ -903,11 +1021,14 @@ int multi_diffuse_resident(Multi* m, int nAngularLevel, const double* uvb, const
   if (m->nleaf == 0 || !uvb || !beta) return RTB200_ERR_ARG;
   if (int st = build_shards(*m, nAngularLevel, nullptr, 0, multi_primary(m).nx)) return st;
   m->step++;
+  std::vector<int> iters((size_t)m->nlocal, 1);
+  for (Member* q : m->mem) q->c.lastScatIter = 0, q->c.lastScatResid = 0., q->c.scatResidPending = false;
   int st = for_each_member(*m, [&](Member& q, int i) -> int {
     RTB_CUDA(cudaSetDevice(q.c.device));
     return diffuse_resident_member(*m, q, nAngularLevel, uvb, beta, ksi6, chemistry,
-                                   streams ? (cudaStream_t)streams[i] : q.c.stream);
+                                   streams ? (cudaStream_t)streams[i] : q.c.stream, &iters[(size_t)i]);
   });
+  m->step += (unsigned long long)(iters[0] - 1);   // the ranks agree on the iteration count
   if (nseg) {
     *nseg = 0;
     for (Member* q : m->mem) *nseg += q->nsegLast;
@@ -918,17 +1039,26 @@ int multi_diffuse_resident(Multi* m, int nAngularLevel, const double* uvb, const
 int multi_diffuse_host(Multi* m, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays,
                        int32_t nrays, double* J1, double* J2, double* J3, int64_t* nseg) {
   if (m->nleaf == 0 || !uvb || !beta) return RTB200_ERR_ARG;
+  const bool scatter = multi_primary(m).dSigma != nullptr;
+  if (scatter && rays) return RTB200_ERR_ARG;   // the J of a direction subset is not the mean intensity the source needs
   if (int st = build_shards(*m, nAngularLevel, rays, nrays, multi_primary(m).nx)) return st;
   m->step++;
-  int st = for_each_member(*m, [&](Member& q, int) -> int {
+  std::vector<int> iters((size_t)m->nlocal, 1);
+  for (Member* q : m->mem) q->c.lastScatIter = 0, q->c.lastScatResid = 0., q->c.scatResidPending = false;
+  int st = for_each_member(*m, [&](Member& q, int i) -> int {
     Context& c = q.c;
     RTB_CUDA(cudaSetDevice(c.device));
     const int buf = (int)(m->step & 1);
     PhaseTimer tm("diffuse", q.rank, c.stream);
-    if (int e = sweep_member(*m, q, buf, nAngularLevel, uvb, beta, c.stream)) return e;
-    tm.mark("opacities+sweep+merge");
-    if (int e = reduce_member(*m, q, buf, 3, q.Jslab, Epilogue(), c.stream)) return e;
-    tm.mark("reduce-scatter");
+    if (scatter) {
+      if (int e = scatter_member(*m, q, m->step - 1, nAngularLevel, uvb, beta, Epilogue(), c.stream, &iters[(size_t)i])) return e;
+      tm.mark("source iteration");
+    } else {
+      if (int e = sweep_member(*m, q, buf, nAngularLevel, uvb, beta, c.stream)) return e;
+      tm.mark("opacities+sweep+merge");
+      if (int e = reduce_member(*m, q, buf, m->step, 3, q.Jslab, Epilogue(), c.stream)) return e;
+      tm.mark("reduce-scatter");
+    }
     const int64_t off = slab_off(*m, q.rank), cnt = slab_cnt(*m, q.rank);
     const size_t nb = (size_t)cnt * sizeof(double);
     if (cnt > 0) {
@@ -942,6 +1072,7 @@ int multi_diffuse_host(Multi* m, int nAngularLevel, const double* uvb, const dou
     tm.mark("status");
     return de;
   });
+  m->step += (unsigned long long)(iters[0] - 1);   // the ranks agree on the iteration count
   if (nseg) {
     *nseg = 0;
     for (Member* q : m->mem) *nseg += q->nsegLast;
@@ -1015,7 +1146,7 @@ int multi_point_host(Multi* m, const PointInputs& in, double* const k[6], double
     if (int e = point_member(*m, q, buf, in, idx, diag, c.stream)) return e;
     Epilogue ep;
     ep.base = q.Rbase;
-    if (int e = reduce_member(*m, q, buf, 6, q.Rslab, ep, c.stream)) return e;
+    if (int e = reduce_member(*m, q, buf, m->step, 6, q.Rslab, ep, c.stream)) return e;
     q.haveR = true;
     if (cnt > 0)
       for (int f = 0; f < 6; f++)
@@ -1043,7 +1174,7 @@ int multi_point_resident(Multi* m, const PointInputs& in, void* const* streams, 
     std::vector<int> idx;
     std::vector<double> diag;
     if (int e = point_member(*m, q, buf, in, idx, diag, s)) return e;
-    if (int e = reduce_member(*m, q, buf, 6, q.Rslab, Epilogue(), s)) return e;
+    if (int e = reduce_member(*m, q, buf, m->step, 6, q.Rslab, Epilogue(), s)) return e;
     q.haveR = true;
     scatter_diag(idx, diag, rem, bnd, dust, spec, hpl);
     return RTB200_OK;

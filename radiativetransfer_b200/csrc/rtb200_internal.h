@@ -151,7 +151,21 @@ struct Context {
   double* dEta = nullptr;
   double* dEtaT = nullptr;   // z-major copy of dEta for the uniform sweep (like dKappaT), lazily allocated
   size_t etaTBytes = 0;
-  int uniStdSlots = 0;       // slots [0, uniStdSlots) are in leaf order, the rest z-major
+  // isotropic scattering (rtb200_grid_set_scattering, scattering.cu): sigma [3][nleaf], nullptr = no scattering.  While
+  // it is set the sweeps read dEtaEff = eta_th + sigma * J of the previous iteration, one fixed buffer, so that the
+  // uniform plan and the captured graph stay valid across the iterations and the calls
+  double* dSigma = nullptr;
+  double* dEtaEff = nullptr;
+  double* dScatScratch = nullptr;   // J of the previous iteration [3][nleaf] + the residual word (lazily allocated)
+  size_t scatScratchBytes = 0;
+  int32_t scatMaxIter = 1;
+  double scatTol = 0;
+  int32_t lastScatIter = 0;         // sweeps and last residual of the latest diffuse call
+  double lastScatResid = 0;
+  bool scatResidPending = false;    // tolerance 0: the residual is still on the device (read by last_scattering)
+  // the source the sweeps read: the effective one while scattering is set, else the emission (nullptr: none)
+  const double* sweepEta() const { return dSigma ? dEtaEff : dEta; }
+  int uniStdSlots = 0;      // slots [0, uniStdSlots) are in leaf order, the rest z-major
   DevTree tree;
   std::vector<int32_t> hChild;               // host copy of the linear octree
   std::vector<int32_t> hLeafX, hLeafY, hLeafZ;
@@ -204,8 +218,31 @@ int set_tuning(Context& c, const char* key, double value);
 // emission: eta = host [3][nleaf] (nullptr clears), or a device array on stream s (device = true); negative, NaN or
 // Inf entries are refused with RTB200_ERR_ARG and leave the previous emission in place
 int set_emission(Context& c, const double* eta, bool device, cudaStream_t s);
+// per-leaf field of the 3 groups, [3][nleaf] on the host or (device = true) on the device on stream s: checked (>= 0,
+// finite) and copied into a fresh buffer that replaces *field only on success (set_emission, set_scattering)
+int replace_leaf_field(Context& c, double** field, const double* src, bool device, cudaStream_t s);
+// forget the uniform plan and the captured graph (they know which source the sweeps read)
+void drop_sweep_plans(Context& c);
+// scattering: sigma = host [3][nleaf] (nullptr clears), or a device array (device = true, device groups) on c.stream
+int set_scattering(Context& c, const double* sigma, bool device, int32_t maxIterations, double tolerance);
+// the diffuse call: one sweep, or the source iteration while scattering is set (a direction subset is refused then)
 int run_diffuse(Context& c, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays, int32_t nrays,
                 double* dJ, cudaStream_t s, int64_t* nseg);
+// one sweep of the given directions with the context's current source.  iter <= 1: opacities first (+ sigma while
+// scattering is set) and the call's timing starts; iter > 1: stats add up to the earlier sweeps of the call
+int run_sweep(Context& c, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays, int32_t nrays,
+              double* dJ, cudaStream_t s, int64_t* nseg, int iter);
+// scattering.cu: source iteration of a single context over the full direction set
+int scatter_solve(Context& c, int nAngularLevel, const double* uvb, const double* beta, double* dJ, cudaStream_t s,
+                  int64_t* nseg);
+// eta_out[g * oStride + i] = eta_th + sigma * J, Jprev = J and the residual max |J - Jprev| / J folded into *resid (the
+// bits of a non-negative double) for i < cnt, g < 3; J and Jprev with stride jStride, sigma / eta_th (may be nullptr)
+// with stride sStride
+int launch_scatter_source(const Context& c, int64_t cnt, const double* J, double* Jprev, int64_t jStride, const double* sigma,
+                          const double* etaTh, int64_t sStride, double* etaOut, int64_t oStride, unsigned long long* resid,
+                          cudaStream_t s);
+int launch_add_scattering(Context& c, cudaStream_t s);
+int last_scattering(Context& c, int32_t* iterations, double* residual);
 
 // kernels / launchers --------------------------------------------------------------------------------
 int launch_compute_opacities(Context& c, const double* beta, cudaStream_t s);
@@ -248,6 +285,8 @@ int multi_grid_set(Multi* m, int nx, int64_t nleaf, const int8_t* level, const d
                    const double* HeII, const double* rho, const double* abun2, double physicalBoxSize);
 int multi_update_species(Multi* m, const double* HI, const double* HeI, const double* HeII);
 int multi_set_emission(Multi* m, const double* eta);
+int multi_set_scattering(Multi* m, const double* sigma, int32_t maxIterations, double tolerance);
+int multi_last_scattering(Multi* m, int32_t* iterations, double* residual);
 int multi_get_species(Multi* m, double* HI, double* HeI, double* HeII);
 int multi_diffuse_host(Multi* m, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays,
                        int32_t nrays, double* J1, double* J2, double* J3, int64_t* nseg);

@@ -54,6 +54,19 @@ module rtb200_shim
        import :: c_ptr, c_int
        type(c_ptr), value :: ctx, eta
      end function rtb200_grid_set_emission
+     integer(c_int) function rtb200_grid_set_scattering(ctx, sigma, maxIterations, tolerance) &
+          bind(C, name='rtb200_grid_set_scattering')
+       import :: c_ptr, c_int, c_int32_t, c_double
+       type(c_ptr), value :: ctx, sigma
+       integer(c_int32_t), value :: maxIterations
+       real(c_double), value :: tolerance
+     end function rtb200_grid_set_scattering
+     integer(c_int) function rtb200_last_scattering(ctx, iterations, residual) bind(C, name='rtb200_last_scattering')
+       import :: c_ptr, c_int, c_int32_t, c_double
+       type(c_ptr), value :: ctx
+       integer(c_int32_t), intent(out) :: iterations
+       real(c_double), intent(out) :: residual
+     end function rtb200_last_scattering
      integer(c_int) function rtb200_diffuse(ctx, nAngularLevel, uvb, beta, rays, nrays, J1, J2, J3, nseg) &
           bind(C, name='rtb200_diffuse')
        import :: c_int, c_int32_t, c_ptr
@@ -422,5 +435,31 @@ contains
        call rtbCheck(rtb200_grid_set_emission(rtbContext, c_null_ptr), 'rtb200_grid_set_emission')
     endif
   end subroutine rtbSetEmission
+
+  ! Isotropic scattering (extension, DESIGN.md 4.7): sigma(leaf, group) in 1/cm, in the leaf order of rtbSetGrid as
+  ! rtbSetEmission.  The diffuse sweep then solves by source iteration, at most maxIterations sweeps, stopping once the
+  ! relative change of J is <= tolerance (0: exactly maxIterations sweeps).  Without sigma the scattering is cleared.
+  ! Negative, NaN or Inf entries, maxIterations < 1 or a negative tolerance stop with RTB200_ERR_ARG.
+  subroutine rtbSetScattering(sigma, maxIterations, tolerance)
+    real(c_double), dimension(:,:), target, contiguous, intent(in), optional :: sigma
+    integer, intent(in) :: maxIterations
+    real(c_double), intent(in) :: tolerance
+    if (present(sigma)) then
+       call rtbCheck(rtb200_grid_set_scattering(rtbContext, c_loc(sigma), int(maxIterations, c_int32_t), tolerance), &
+            'rtb200_grid_set_scattering')
+    else
+       call rtbCheck(rtb200_grid_set_scattering(rtbContext, c_null_ptr, int(maxIterations, c_int32_t), tolerance), &
+            'rtb200_grid_set_scattering')
+    endif
+  end subroutine rtbSetScattering
+
+  ! sweeps done and the last residual of the latest diffuse call (0 / 0 without scattering)
+  subroutine rtbScatteringStatus(iterations, residual)
+    integer, intent(out) :: iterations
+    real(c_double), intent(out) :: residual
+    integer(c_int32_t) :: it
+    call rtbCheck(rtb200_last_scattering(rtbContext, it, residual), 'rtb200_last_scattering')
+    iterations = int(it)
+  end subroutine rtbScatteringStatus
 
 end module rtb200_shim

@@ -215,6 +215,27 @@ class Transport:
         st = self.L.rtb200_grid_set_emission_device(self.h, C.c_void_p(int(eta_ptr)), C.c_void_p(int(stream)))
         _lib.check(st, "rtb200_grid_set_emission_device")
 
+    def set_scattering(self, sigma, max_iterations=100, tolerance=1e-9):
+        """Isotropic scattering coefficient per leaf and frequency group, [3, nleaf] in 1/cm (DESIGN.md 4.7); None clears
+        it.  The diffuse calls then solve by source iteration: at most `max_iterations` sweeps, stopping after the first
+        whose largest relative change of J is <= `tolerance` (0: exactly `max_iterations` sweeps, no host round trip).
+        Negative, NaN or Inf entries, a count < 1 or a negative tolerance raise and keep the previous state."""
+        if sigma is None:
+            _lib.check(self.L.rtb200_grid_set_scattering(self.h, None, 1, 0.0), "rtb200_grid_set_scattering")
+            return
+        s = np.ascontiguousarray(sigma, dtype=np.float64)
+        if s.size != 3 * self.nleaf:
+            raise ValueError("sigma must have 3 * nleaf entries ([3][nleaf])")
+        st = self.L.rtb200_grid_set_scattering(self.h, _ptr(s), int(max_iterations), float(tolerance))
+        _lib.check(st, "rtb200_grid_set_scattering")
+
+    def last_scattering(self):
+        """Sweeps done and the last residual of the latest diffuse call: {"iterations", "residual"} (0 / 0 without
+        scattering)."""
+        it, r = C.c_int32(0), C.c_double(0)
+        _lib.check(self.L.rtb200_last_scattering(self.h, C.byref(it), C.byref(r)), "rtb200_last_scattering")
+        return {"iterations": it.value, "residual": r.value}
+
     def diffuse(self, uvb, beta, n_angular_level=3, rays=None, out=None):
         """Host-buffer call (H2D of nothing but tables, D2H of J): returns (J[3, nleaf], nseg)."""
         uvb, beta = _f64(uvb), _f64(np.asarray(beta).reshape(9))
