@@ -198,6 +198,28 @@ int rtb200_grid_set_emission_device(rtb200_ctx* ctx, const double* eta_device, v
 int rtb200_grid_set_scattering(rtb200_ctx* ctx, const double* sigma, int32_t maxIterations, double tolerance);
 int rtb200_last_scattering(rtb200_ctx* ctx, int32_t* iterations, double* residual);
 
+/* Dust in the diffuse sweep (an extension without a reference value, DESIGN.md 4.8): the dust model of the point-source
+ * path (dustModule.f90:30-73) as an opacity of the diffuse field.  betaDust[3] is a band-mean dust cross-section per
+ * frequency group in cm^2 per H (rtb200_uvb_dust_beta).  Per leaf and group the diffuse calls compute, on the device
+ * and from the current species of every call (no FMA, every step rounded):
+ *     mode 1:  kd_g = ((HI * betaDust[g]) * abun2) / (double)0.2f
+ *     mode 2:  kd_g = (((((double)0.76f * rho) / (double)1.6726231e-24f) * betaDust[g]) * abun2) / (double)0.2f
+ * (the dust column of the point path, point_source.cu), the extinction kappa_g = kappa_abs,g + kd_g (rounded once; a
+ * per-leaf sigma of rtb200_grid_set_scattering is added after it) and, while albedo[g] > 0, the scattering source
+ * sigma_g = albedo[g] * kd_g of the source iteration of rtb200_grid_set_scattering (same residual, stopping rule, stats
+ * and rtb200_last_scattering), with this call's maxIterations / tolerance.  Mode 0 is no dust.  One scattering medium at
+ * a time: dust with an albedo > 0 is refused while a per-leaf sigma is set, and rtb200_grid_set_scattering(sigma !=
+ * NULL) is refused while dust scatters; dust that only absorbs combines with emission and a per-leaf sigma.  A direction
+ * subset is refused while dust scatters.  The point-source path ignores this setting (it has its own dustApproximation).
+ * rtb200_grid_set clears the dust, rtb200_grid_update_species keeps it (the next call follows the new HI).  A device
+ * group stores the scalars on every member; each computes the dust of the whole grid from its complete species.
+ *   rtb200_grid_set_dust  mode 0..2; betaDust[3] >= 0 and finite; albedo[3] in [0, 1] (both may be NULL for mode 0);
+ *                         mode 1 needs abun2, mode 2 rho and abun2 in rtb200_grid_set; with an albedo > 0,
+ *                         maxIterations >= 1 and tolerance >= 0 and finite.  Anything else, or a conflict above, is
+ *                         refused with RTB200_ERR_ARG and the previous state stays.  Queued work completes first. */
+int rtb200_grid_set_dust(rtb200_ctx* ctx, int dustApproximation, const double* betaDust3, const double* albedo3,
+                         int32_t maxIterations, double tolerance);
+
 /* Diffuse (UV background) sweep: replaces equiSources.f90:1372-1808 (computeOpacities :4956, the loop over
  * 12*4**(nAngularLevel-1) HEALPix directions, pattern set-up, neighbour threading, transport).
  *   uvb[3]      boundary intensities uvb1..3 (definitionsModule.f90:53)
@@ -231,7 +253,14 @@ int rtb200_diffuse_rates_device(rtb200_ctx* ctx, const double* J_device, const d
  *   rtb200_uvb_background   both, returned in the shapes the calls above take: beta[9] = [group][beta24, beta26,
  *                           beta25], ksi24[3], ksi25[1] (group 3), ksi26[2] (groups 2, 3); any output may be NULL.
  * nfreq = nfbins = 400, freqdel = frequencyBinWidth = (double)0.02f in the reference (definitionsModule.f90:239-241).
- * Returns RTB200_ERR_ARG where powerSpectrumIndex prints 'wrong sign' and stops. */
+ * Returns RTB200_ERR_ARG where powerSpectrumIndex prints 'wrong sign' and stops.
+ *   rtb200_uvb_dust_beta    betaDust3[g] = band mean of the dust cross-section over group g with the weights of beta24:
+ *                           sum over the in-band bins i >= 1 of dt * sD(e_i) / (shape_g * nu_g), dt = (e_i/nu_g)^-alpha_g
+ *                           * (e_i - e_{i-1}), sD = the 7-term fit of aDust[7][5] (dustModule.f90:30-73) at the bin's
+ *                           wavelength, as the point path evaluates it.  Group 3 runs to wavelengths below the fit's
+ *                           range (down to ~1e-4 A at nfreq 400); the fit is extrapolated there as in the point tables.
+ *                           Input to rtb200_grid_set_dust.  ERR_ARG for NULL pointers or nfreq < 2. */
+int rtb200_uvb_dust_beta(int nfreq, double freqdel, const double* alpha, const double* aDust, double* betaDust3);
 int rtb200_uvb_amplitudes(double currentRedshift, double uvbCoefficient, double* uvb, double* alpha);
 int rtb200_uvb_beta_table(int nfreq, double freqdel, const double* alpha, double* table57);
 int rtb200_uvb_background(double currentRedshift, double uvbCoefficient, int nfreq, double freqdel, double* uvb,

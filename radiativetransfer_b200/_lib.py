@@ -40,11 +40,13 @@ SIGNATURES = {
     "rtb200_grid_set_emission_device": (C.c_int, [P, P, P]),
     "rtb200_grid_set_scattering": (C.c_int, [P, P, C.c_int32, C.c_double]),
     "rtb200_last_scattering": (C.c_int, [P, C.POINTER(C.c_int32), C.POINTER(C.c_double)]),
+    "rtb200_grid_set_dust": (C.c_int, [P, C.c_int, P, P, C.c_int32, C.c_double]),
     "rtb200_diffuse": (C.c_int, [P, C.c_int, P, P, P, C.c_int32, P, P, P, C.POINTER(C.c_int64)]),
     "rtb200_diffuse_device": (C.c_int, [P, C.c_int, P, P, P, C.c_int32, P, P, C.POINTER(C.c_int64)]),
     "rtb200_diffuse_rates_device": (C.c_int, [P, P, P, P, P, P, P, P, P]),
     "rtb200_uvb_amplitudes": (C.c_int, [C.c_double, C.c_double, P, P]),
     "rtb200_uvb_beta_table": (C.c_int, [C.c_int, C.c_double, P, P]),
+    "rtb200_uvb_dust_beta": (C.c_int, [C.c_int, C.c_double, P, P, P]),
     "rtb200_uvb_background": (C.c_int, [C.c_double, C.c_double, C.c_int, C.c_double, P, P, P, P, P, P, P]),
     "rtb200_point": (C.c_int, [P, C.c_int, P, P, P, C.c_double, P, C.c_int, C.c_int, C.c_int32, P, P, P, P, P, P, P, P,
                               P, P, P, P, P, C.POINTER(C.c_int64)]),

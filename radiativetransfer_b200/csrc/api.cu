@@ -67,6 +67,9 @@ static void free_grid(Context& c) {
   cudaFree(c.dEtaEff); c.dEtaEff = nullptr;
   cudaFree(c.dScatScratch); c.dScatScratch = nullptr; c.scatScratchBytes = 0;
   c.scatMaxIter = 1; c.scatTol = 0.; c.lastScatIter = 0; c.lastScatResid = 0.; c.scatResidPending = false;
+  cudaFree(c.dDustSigma); c.dDustSigma = nullptr;
+  c.dustMode = 0;
+  for (int g = 0; g < 3; g++) c.dustBeta[g] = c.dustAlbedo[g] = 0.;
   cudaFree(c.dLogT); c.dLogT = nullptr;
   for (auto& sl : c.pointPool) cudaFree(sl.first);
   c.pointPool.clear();
@@ -176,7 +179,7 @@ int run_sweep(Context& c, int nAngularLevel, const double* uvb, const double* be
   const double bytes0 = iter > 1 ? c.lastAlgBytes : 0.;
   if (iter <= 1) {
     RTB_CUDA(cudaEventRecord(c.evStart, s));
-    if (int st = launch_compute_opacities(c, beta, s)) return st;
+    if (int st = c.dustMode ? launch_compute_opacities_dust(c, beta, s) : launch_compute_opacities(c, beta, s)) return st;
     if (c.dSigma)
       if (int st = launch_add_scattering(c, s)) return st;
   }
@@ -201,7 +204,7 @@ int run_diffuse(Context& c, int nAngularLevel, const double* uvb, const double* 
   c.lastScatIter = 0;
   c.lastScatResid = 0.;
   c.scatResidPending = false;
-  if (!c.dSigma) return run_sweep(c, nAngularLevel, uvb, beta, rays, nrays, dJ, s, nseg, 0);
+  if (!c.scatterSigma()) return run_sweep(c, nAngularLevel, uvb, beta, rays, nrays, dJ, s, nseg, 0);
   if (rays) return RTB200_ERR_ARG;   // the J of a direction subset is not the mean intensity the source needs
   return scatter_solve(c, nAngularLevel, uvb, beta, dJ, s, nseg);
 }
@@ -500,6 +503,13 @@ int rtb200_grid_set_scattering(rtb200_ctx* h, const double* sigma, int32_t maxIt
   if (!h) return RTB200_ERR_ARG;
   if (h->m) return multi_set_scattering(h->m, sigma, maxIterations, tolerance);
   return set_scattering(h->c, sigma, false, maxIterations, tolerance);
+}
+
+int rtb200_grid_set_dust(rtb200_ctx* h, int dustApproximation, const double* betaDust3, const double* albedo3,
+                         int32_t maxIterations, double tolerance) {
+  if (!h) return RTB200_ERR_ARG;
+  if (h->m) return multi_set_dust(h->m, dustApproximation, betaDust3, albedo3, maxIterations, tolerance);
+  return set_dust(h->c, dustApproximation, betaDust3, albedo3, maxIterations, tolerance);
 }
 
 int rtb200_last_scattering(rtb200_ctx* h, int32_t* iterations, double* residual) {

@@ -863,9 +863,17 @@ int multi_set_scattering(Multi* m, const double* sigma, int32_t maxIterations, d
   if (m->nleaf == 0) return RTB200_ERR_ARG;
   if (!sigma) return for_each_member(*m, [&](Member& q, int) { return set_scattering(q.c, nullptr, false, 1, 0.); });
   if (maxIterations < 1 || !(tolerance >= 0.) || std::isinf(tolerance)) return RTB200_ERR_ARG;
+  if (multi_primary(m).dDustSigma) return RTB200_ERR_ARG;   // one scattering medium at a time (dust.cu)
   return multi_set_field(m, sigma, [&](Context& c, const double* packed) {
     return set_scattering(c, packed, true, maxIterations, tolerance);
   });
+}
+
+// scalars only: every member stores them and computes the dust of the whole grid from its complete species and its
+// complete rho / abun2 (grid_set uploads the caller's full arrays on every member, in rank mode too)
+int multi_set_dust(Multi* m, int mode, const double* betaDust, const double* albedo, int32_t maxIterations, double tolerance) {
+  if (m->nleaf == 0 || !dust_args_ok(mode, betaDust, albedo, maxIterations, tolerance)) return RTB200_ERR_ARG;
+  return for_each_member(*m, [&](Member& q, int) { return set_dust(q.c, mode, betaDust, albedo, maxIterations, tolerance); });
 }
 
 int multi_last_scattering(Multi* m, int32_t* iterations, double* residual) {
@@ -955,7 +963,7 @@ static int scatter_member(Multi& m, Member& q, unsigned long long step0, int nAn
     nsTotal += q.nsegLast;
     if (int st = reduce_member(m, q, buf, step, 3, q.Jslab, ep, s)) return st;
     RTB_CUDA(cudaMemsetAsync(resid, 0, sizeof(unsigned long long), s));
-    if (int st = launch_scatter_source(c, cnt, q.Jslab, Jprev, m.slab, c.dSigma + off, c.dEta ? c.dEta + off : nullptr, N,
+    if (int st = launch_scatter_source(c, cnt, q.Jslab, Jprev, m.slab, c.scatterSigma() + off, c.dEta ? c.dEta + off : nullptr, N,
                                        stage + (size_t)q.rank * m.slab, m.npad, resid, s))
       return st;
     if (m.nranks > 1) {
@@ -998,7 +1006,7 @@ static int diffuse_resident_member(Multi& m, Member& q, int nAngularLevel, const
   Epilogue ep;
   ep.ksi = ksi6;
   ep.kAccumulate = 0;
-  if (q.c.dSigma) {   // source iteration, steps m.step .. m.step + iterations - 1; chemistry once, after it
+  if (q.c.scatterSigma()) {   // source iteration, steps m.step .. m.step + iterations - 1; chemistry once, after it
     if (int st = scatter_member(m, q, m.step - 1, nAngularLevel, uvb, beta, ep, s, iters)) return st;
   } else {
     const int buf = (int)(m.step & 1);
@@ -1039,7 +1047,7 @@ int multi_diffuse_resident(Multi* m, int nAngularLevel, const double* uvb, const
 int multi_diffuse_host(Multi* m, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays,
                        int32_t nrays, double* J1, double* J2, double* J3, int64_t* nseg) {
   if (m->nleaf == 0 || !uvb || !beta) return RTB200_ERR_ARG;
-  const bool scatter = multi_primary(m).dSigma != nullptr;
+  const bool scatter = multi_primary(m).scatterSigma() != nullptr;
   if (scatter && rays) return RTB200_ERR_ARG;   // the J of a direction subset is not the mean intensity the source needs
   if (int st = build_shards(*m, nAngularLevel, rays, nrays, multi_primary(m).nx)) return st;
   m->step++;

@@ -16,7 +16,7 @@ static const double kHp = (double)6.6260693e-27f, kClight = (double)2.99792458e1
 static const double kEvToErg = 1.60217646e-12, kEvToHz = kEvToErg / kHp;
 static const double kNu[3] = {(double)13.598f, (double)24.587f, (double)54.418f};  // HI, HeI, HeII thresholds [eV]
 
-static double smc_dust_sigma(double lambdaMicron, const double* a) {  // dustModule.f90:36-50, 7-term fit
+double smc_dust_sigma(double lambdaMicron, const double* a) {  // dustModule.f90:36-50, 7-term fit
   double sum = 0;
   for (int t = 0; t < 7; t++) {
     const double* row = a + 5 * t;

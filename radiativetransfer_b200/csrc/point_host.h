@@ -16,6 +16,8 @@ struct PointFreq {
   double out24[kNenergy], out26[kNenergy], out25[kNenergy], outD[kNenergy];  // same ratios on the 300 output energies
 };
 
+// dust cross-section of the 7-term extinction fit a[7][5] at lambdaMicron, in units of 1e-22 cm^2 (dustModule.f90:36-50)
+double smc_dust_sigma(double lambdaMicron, const double* a);
 void point_frequency_tables(const double* aDust, PointFreq& F);
 void point_source_spectrum(const PointFreq& F, int nWave, const double* wavelength, const double* lum,
                            double coefSpectrum, int iMetal, double coefMetal, double* dtmp);

@@ -163,8 +163,15 @@ struct Context {
   int32_t lastScatIter = 0;         // sweeps and last residual of the latest diffuse call
   double lastScatResid = 0;
   bool scatResidPending = false;    // tolerance 0: the residual is still on the device (read by last_scattering)
-  // the source the sweeps read: the effective one while scattering is set, else the emission (nullptr: none)
-  const double* sweepEta() const { return dSigma ? dEtaEff : dEta; }
+  // dust (rtb200_grid_set_dust, dust.cu): mode 0 = none.  compute_opacities_dust_kernel adds kd to the opacities of every
+  // call and, while an albedo is > 0, writes the scattering source albedo * kd into dDustSigma [3][nleaf]
+  int dustMode = 0;
+  double dustBeta[3] = {0, 0, 0}, dustAlbedo[3] = {0, 0, 0};
+  double* dDustSigma = nullptr;     // allocated while dust scatters
+  // the scattering coefficient of the source iteration: the per-leaf sigma or the dust's (nullptr: no scattering)
+  const double* scatterSigma() const { return dSigma ? dSigma : dDustSigma; }
+  // the source the sweeps read: the effective one while the context scatters, else the emission (nullptr: none)
+  const double* sweepEta() const { return scatterSigma() ? dEtaEff : dEta; }
   int uniStdSlots = 0;      // slots [0, uniStdSlots) are in leaf order, the rest z-major
   DevTree tree;
   std::vector<int32_t> hChild;               // host copy of the linear octree
@@ -242,6 +249,12 @@ int launch_scatter_source(const Context& c, int64_t cnt, const double* J, double
                           const double* etaTh, int64_t sStride, double* etaOut, int64_t oStride, unsigned long long* resid,
                           cudaStream_t s);
 int launch_add_scattering(Context& c, cudaStream_t s);
+// dust.cu: dust (mode 0 clears; albedo may make it scatter) and the opacities with dust, in place of
+// launch_compute_opacities while a mode is set
+int set_dust(Context& c, int mode, const double* betaDust, const double* albedo, int32_t maxIterations, double tolerance);
+// the argument checks of set_dust that need no context (the device group runs them once for all members)
+bool dust_args_ok(int mode, const double* betaDust, const double* albedo, int32_t maxIterations, double tolerance);
+int launch_compute_opacities_dust(Context& c, const double* beta, cudaStream_t s);
 int last_scattering(Context& c, int32_t* iterations, double* residual);
 
 // kernels / launchers --------------------------------------------------------------------------------
@@ -287,6 +300,7 @@ int multi_update_species(Multi* m, const double* HI, const double* HeI, const do
 int multi_set_emission(Multi* m, const double* eta);
 int multi_set_scattering(Multi* m, const double* sigma, int32_t maxIterations, double tolerance);
 int multi_last_scattering(Multi* m, int32_t* iterations, double* residual);
+int multi_set_dust(Multi* m, int mode, const double* betaDust, const double* albedo, int32_t maxIterations, double tolerance);
 int multi_get_species(Multi* m, double* HI, double* HeI, double* HeII);
 int multi_diffuse_host(Multi* m, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays,
                        int32_t nrays, double* J1, double* J2, double* J3, int64_t* nseg);

@@ -80,12 +80,15 @@ int launch_scatter_source(const Context& c, int64_t cnt, const double* J, double
 int set_scattering(Context& c, const double* sigma, bool device, int32_t maxIterations, double tolerance) {
   if (c.nleaf == 0) return RTB200_ERR_ARG;
   if (sigma && (maxIterations < 1 || !(tolerance >= 0.) || std::isinf(tolerance))) return RTB200_ERR_ARG;
+  if (sigma && c.dDustSigma) return RTB200_ERR_ARG;   // one scattering medium at a time (dust.cu)
   RTB_CUDA(cudaSetDevice(c.device));
   RTB_CUDA(cudaDeviceSynchronize());   // queued sweeps read the current arrays
   if (!sigma) {
     cudaFree(c.dSigma); c.dSigma = nullptr;
-    cudaFree(c.dEtaEff); c.dEtaEff = nullptr;
-    cudaFree(c.dScatScratch); c.dScatScratch = nullptr; c.scatScratchBytes = 0;
+    if (!c.dDustSigma) {   // scattering dust keeps the buffers of its source iteration
+      cudaFree(c.dEtaEff); c.dEtaEff = nullptr;
+      cudaFree(c.dScatScratch); c.dScatScratch = nullptr; c.scatScratchBytes = 0;
+    }
     drop_sweep_plans(c);
     return RTB200_OK;
   }
@@ -142,7 +145,7 @@ int scatter_solve(Context& c, int nAngularLevel, const double* uvb, const double
     if (int st = run_sweep(c, nAngularLevel, uvb, beta, nullptr, 0, dJ, s, &ns, k)) return st;
     total += ns;
     RTB_CUDA(cudaMemsetAsync(resid, 0, sizeof(unsigned long long), s));
-    if (int st = launch_scatter_source(c, N, dJ, Jprev, N, c.dSigma, c.dEta, N, c.dEtaEff, N, resid, s)) return st;
+    if (int st = launch_scatter_source(c, N, dJ, Jprev, N, c.scatterSigma(), c.dEta, N, c.dEtaEff, N, resid, s)) return st;
     c.lastLaunches += 1;
     if (c.scatTol > 0.) {   // the stopping test reads the residual back; tolerance 0 runs on without a host round trip
       RTB_CUDA(cudaMemcpyAsync(&r, resid, sizeof(double), cudaMemcpyDeviceToHost, s));

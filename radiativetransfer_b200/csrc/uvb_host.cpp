@@ -2,6 +2,7 @@
 //   * band amplitudes uvb1..3 and the effective slopes alpha(3)      equiSources.f90:198-246, powerSpectrumIndex :4985-5043
 //   * group cross-sections beta24..31, rate weights ksi24..31 and heating weights gammaHI/HeI/HeII of the three
 //     frequency groups                                               uvbBetaTable.f90:31-296
+//   * band-mean dust cross-sections of the groups with the same weights (an extension, DESIGN.md 4.8)
 // They are what computeOpacities (equiSources.f90:4956-4983) and the diffuse photo-rates (:3546-3553) consume, i.e.
 // the `beta[9]` / `ksi*` arguments of rtb200_diffuse* and rtb200_chemistry_device.
 // Every Fortran real literal without a d-exponent is single precision and is widened where it meets a double; integer
@@ -10,6 +11,7 @@
 #include <vector>
 
 #include "../../include/rtb200.h"
+#include "point_host.h"
 
 namespace rtb {
 namespace {
@@ -86,6 +88,16 @@ int effective_slope(double u1, double a1, double u2, double a2, double nug, doub
   return RTB200_OK;
 }
 
+// the frequency groups' bins (uvbBetaTable.f90:171-257): [nu_g, nu_g+1] for groups 1, 2, from nu_3 on for group 3
+bool in_band(int g, double freq) { return g < 2 ? (freq >= kNu[g] && freq <= kNu[g + 1]) : freq >= kNu[2]; }
+
+// band integral of (e / nu_g)^-alpha_g in units of nu_g, the normalisation of beta24 (:259-293)
+void band_shapes(const double* alpha, double shape[3]) {
+  shape[0] = (1. - std::pow(kNu[1] / kNu[0], 1. - alpha[0])) / (alpha[0] - 1.);
+  shape[1] = (1. - std::pow(kNu[2] / kNu[1], 1. - alpha[1])) / (alpha[1] - 1.);
+  shape[2] = 1. / (alpha[2] - 1.);
+}
+
 }  // namespace
 }  // namespace rtb
 
@@ -138,8 +150,7 @@ int rtb200_uvb_beta_table(int nfreq, double freqdel, const double* alpha, double
     const double freq = e[i], dnu = e[i] - e[i - 1];
     const double* s = &sig[(size_t)i * 8];
     for (int g = 0; g < 3; g++) {
-      const bool inBand = g < 2 ? (freq >= kNu[g] && freq <= kNu[g + 1]) : freq >= kNu[2];
-      if (!inBand) continue;
+      if (!in_band(g, freq)) continue;
       double* G = table57 + 19 * g;
       const double dt = std::pow(freq / kNu[g], -alpha[g]) * dnu;
       const double dtE = dt * kEvToHz / (freq * kEvToErg);
@@ -153,12 +164,35 @@ int rtb200_uvb_beta_table(int nfreq, double freqdel, const double* alpha, double
       if (g == 2) G[18] = G[18] + dtE * (freq - kNu[2]) * kEvToErg * s[1];
     }
   }
-  const double shape[3] = {(1. - std::pow(kNu[1] / kNu[0], 1. - alpha[0])) / (alpha[0] - 1.),
-                           (1. - std::pow(kNu[2] / kNu[1], 1. - alpha[1])) / (alpha[1] - 1.), 1. / (alpha[2] - 1.)};
+  double shape[3];
+  band_shapes(alpha, shape);
   for (int g = 0; g < 3; g++) {                                     // :259-293
     const double energyShape = shape[g] * kNu[g];
     for (int k = 0; k < 8; k++) table57[19 * g + k] = table57[19 * g + k] / energyShape;
   }
+  return RTB200_OK;
+}
+
+int rtb200_uvb_dust_beta(int nfreq, double freqdel, const double* alpha, const double* aDust, double* betaDust3) {
+  if (nfreq < 2 || !alpha || !aDust || !betaDust3) return RTB200_ERR_ARG;
+  const double clight = w(2.99792458e10f);
+  double G[3] = {0., 0., 0.};
+  double prev = 1.;                                                 // e_0 = 10^0
+  for (int i = 1; i < nfreq; i++) {                                 // the bins and weights of beta24 above
+    const double freq = std::pow(10.0, (double)i * freqdel), dnu = freq - prev;
+    prev = freq;
+    // the dust cross-section as point_frequency_tables evaluates it: wavelength in A, the fit in micron
+    const double lambda = clight / (freq * kEvToHz) * w(1.e8f);
+    const double sD = smc_dust_sigma(lambda / w(1.e4f), aDust) * w(1.e-22f);
+    for (int g = 0; g < 3; g++) {
+      if (!in_band(g, freq)) continue;
+      const double dt = std::pow(freq / kNu[g], -alpha[g]) * dnu;
+      G[g] = G[g] + dt * sD;
+    }
+  }
+  double shape[3];
+  band_shapes(alpha, shape);
+  for (int g = 0; g < 3; g++) betaDust3[g] = G[g] / (shape[g] * kNu[g]);
   return RTB200_OK;
 }
 

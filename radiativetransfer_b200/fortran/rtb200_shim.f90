@@ -67,6 +67,20 @@ module rtb200_shim
        integer(c_int32_t), intent(out) :: iterations
        real(c_double), intent(out) :: residual
      end function rtb200_last_scattering
+     integer(c_int) function rtb200_grid_set_dust(ctx, dustApproximation, betaDust, albedo, maxIterations, tolerance) &
+          bind(C, name='rtb200_grid_set_dust')
+       import :: c_ptr, c_int, c_int32_t, c_double
+       type(c_ptr), value :: ctx, betaDust, albedo
+       integer(c_int), value :: dustApproximation
+       integer(c_int32_t), value :: maxIterations
+       real(c_double), value :: tolerance
+     end function rtb200_grid_set_dust
+     integer(c_int) function rtb200_uvb_dust_beta(nfreq, freqdel, alpha, aDust, betaDust) bind(C, name='rtb200_uvb_dust_beta')
+       import :: c_ptr, c_int, c_double
+       integer(c_int), value :: nfreq
+       real(c_double), value :: freqdel
+       type(c_ptr), value :: alpha, aDust, betaDust
+     end function rtb200_uvb_dust_beta
      integer(c_int) function rtb200_diffuse(ctx, nAngularLevel, uvb, beta, rays, nrays, J1, J2, J3, nseg) &
           bind(C, name='rtb200_diffuse')
        import :: c_int, c_int32_t, c_ptr
@@ -461,5 +475,25 @@ contains
     call rtbCheck(rtb200_last_scattering(rtbContext, it, residual), 'rtb200_last_scattering')
     iterations = int(it)
   end subroutine rtbScatteringStatus
+
+  ! Dust in the diffuse sweep (extension, DESIGN.md 4.8): the dust model of the point-source path (a_smc, dustModule.f90)
+  ! as an opacity of the UV background, recomputed from the current species in every rtbDiffuse.  dustApproximation
+  ! 1 / 2 as for the point sources, 0 clears it.  The band-mean dust cross-sections of the three groups come from
+  ! alpha(3) and a_smc with the weights of uvbBetaTable (nfbins bins of frequencyBinWidth).  albedo(g) > 0 makes the
+  ! dust scatter (source iteration, maxIterations / tolerance as rtbSetScattering; not together with rtbSetScattering).
+  subroutine rtbSetDust(dustApproximation, albedo, maxIterations, tolerance)
+    integer, intent(in) :: dustApproximation, maxIterations
+    real(c_double), dimension(3), intent(in) :: albedo
+    real(c_double), intent(in) :: tolerance
+    real(c_double), dimension(3), target :: alphaC, betaDust, albedoC
+    real(c_double), dimension(5,7), target :: dustPack                         ! = C [7][5]
+    alphaC = real(alpha(1:3), c_double)
+    dustPack = transpose(real(a_smc, c_double))
+    albedoC = albedo
+    call rtbCheck(rtb200_uvb_dust_beta(int(nfbins, c_int), real(frequencyBinWidth, c_double), c_loc(alphaC), &
+         c_loc(dustPack), c_loc(betaDust)), 'rtb200_uvb_dust_beta')
+    call rtbCheck(rtb200_grid_set_dust(rtbContext, int(dustApproximation, c_int), c_loc(betaDust), c_loc(albedoC), &
+         int(maxIterations, c_int32_t), tolerance), 'rtb200_grid_set_dust')
+  end subroutine rtbSetDust
 
 end module rtb200_shim

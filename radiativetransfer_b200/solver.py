@@ -229,6 +229,20 @@ class Transport:
         st = self.L.rtb200_grid_set_scattering(self.h, _ptr(s), int(max_iterations), float(tolerance))
         _lib.check(st, "rtb200_grid_set_scattering")
 
+    def set_dust(self, approximation, beta_dust=None, albedo=(0.0, 0.0, 0.0), max_iterations=100, tolerance=1e-9):
+        """Dust in the diffuse sweep (DESIGN.md 4.8): `approximation` 1 (dust column from HI) or 2 (from rho) with the
+        band-mean cross-sections `beta_dust[3]` of workloads.uvb_dust_beta, 0 clears it.  The opacity follows the current
+        species in every diffuse call; an `albedo[3]` > 0 makes the dust scatter, solved by source iteration with
+        `max_iterations` / `tolerance` as set_scattering.  Bad values, a missing rho / abun2, or scattering dust while a
+        per-leaf sigma is set raise and keep the previous state."""
+        bd = None if beta_dust is None else _f64(beta_dust)
+        al = _f64(albedo)
+        if (bd is not None and bd.size != 3) or al.size != 3:
+            raise ValueError("beta_dust and albedo take one value per frequency group")
+        st = self.L.rtb200_grid_set_dust(self.h, int(approximation), None if bd is None else _ptr(bd), _ptr(al),
+                                         int(max_iterations), float(tolerance))
+        _lib.check(st, "rtb200_grid_set_dust")
+
     def last_scattering(self):
         """Sweeps done and the last residual of the latest diffuse call: {"iterations", "residual"} (0 / 0 without
         scattering)."""

@@ -58,6 +58,23 @@ def uvb_background(redshift=3.0, uvb_coefficient=1.0, nfreq=400, freqdel=None):
     return dict(uvb=uvb, beta=beta, alpha=alpha, ksi24=k24, ksi25=k25, ksi26=k26, table=tab)
 
 
+def uvb_dust_beta(alpha, a_dust, nfreq=400, freqdel=None):
+    """betaD[3]: band-mean dust cross-section of each frequency group [cm^2 per H] from the extinction fit a_dust[7, 5]
+    with the weights of beta24 (rtb200_uvb_dust_beta, DESIGN.md 4.8), the input of Transport.set_dust.  alpha[3] are the
+    background's effective slopes (uvb_background()["alpha"])."""
+    import ctypes as C
+
+    from . import _lib
+    if freqdel is None:
+        freqdel = float(_f(0.02))
+    al = np.ascontiguousarray(alpha, dtype=np.float64).reshape(3)
+    ad = np.ascontiguousarray(a_dust, dtype=np.float64).reshape(7, 5)
+    out = np.zeros(3)
+    p = lambda a: a.ctypes.data_as(C.c_void_p)
+    _lib.check(_lib.lib().rtb200_uvb_dust_beta(int(nfreq), float(freqdel), p(al), p(ad), p(out)), "rtb200_uvb_dust_beta")
+    return out
+
+
 # ------------------------------------------------------------------------------------------------------
 # grids
 # ------------------------------------------------------------------------------------------------------
