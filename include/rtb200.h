@@ -220,6 +220,36 @@ int rtb200_last_scattering(rtb200_ctx* ctx, int32_t* iterations, double* residua
 int rtb200_grid_set_dust(rtb200_ctx* ctx, int dustApproximation, const double* betaDust3, const double* albedo3,
                          int32_t maxIterations, double tolerance);
 
+/* Acceleration of the source iteration (DESIGN.md 4.9), for whichever medium scatters (a per-leaf sigma or dust with an
+ * albedo > 0).  In a diffuse call, x_{k-1} is the J that forms the source of sweep k (eta_k = eta_th + sigma * x_{k-1})
+ * and y_k the J that sweep k returns; the residual is r_k = maxrel(y_k, x_{k-1}) as above, the stopping rule is
+ * unchanged, and the call returns y_k (a sweep output, never an extrapolated J).  Flags 0 is plain source iteration.
+ *   RTB200_SCATTER_WARM_START  x_0 = the J the previous diffuse call of this context returned, if that call completed a
+ *                              scattering solve; else x_0 = 0.  The stored J survives rtb200_grid_update_species, new
+ *                              emission, sigma, dust and iteration settings (it is only a starting guess); it is dropped
+ *                              by rtb200_grid_set, by clearing every scattering medium and by a call that fails.
+ *   RTB200_SCATTER_NG          Ng extrapolation of order 2 (Auer 1987).  After every fourth sweep counted from the call's
+ *                              start or from the last attempted extrapolation, except on the sweep that stops the call,
+ *                              with I0..I3 = y_k .. y_{k-3}: w = 1/I0 where I0 > 0 (else 0), d0 = (I0-I1) w,
+ *                              d1 = (I1-I2) w, d2 = (I2-I3) w, q1 = d0-d1, q2 = d0-d2, the sums over (group, leaf)
+ *                              A11 = <q1,q1>, A12 = <q1,q2>, A22 = <q2,q2>, c1 = <d0,q1>, c2 = <d0,q2>,
+ *                              det = A11 A22 - A12^2, a = (c1 A22 - c2 A12) / det, b = (c2 A11 - c1 A12) / det; if
+ *                              det > 1e-14 A11 A22 and a, b are finite, x_k = max(0, (1-a-b) I0 + a I1 + b I2), else
+ *                              the step is skipped (x_k = y_k).  The sums are taken in a fixed order (bit-identical
+ *                              from run to run; a device group sums its ranks' partials in rank order, so all ranks
+ *                              take the same step) and stay on the device: no host round trip is added.  While set, the
+ *                              history costs three more [3][nleaf] fields (a device group: [3][slab] per rank).
+ *   rtb200_grid_set_scattering_acceleration  flags = a combination of the two (0 = none); unknown bits are refused with
+ *                              RTB200_ERR_ARG and the previous flags stay.  Queued work completes first.  A device
+ *                              group calls it collectively (every rank returns the same status).  rtb200_grid_set
+ *                              resets it to 0.
+ *   rtb200_last_scattering_acceleration  extrapolations the latest diffuse call applied (skipped ones not counted) and
+ *                              whether it started warm (1) or from J = 0 (0). */
+#define RTB200_SCATTER_NG 1
+#define RTB200_SCATTER_WARM_START 2
+int rtb200_grid_set_scattering_acceleration(rtb200_ctx* ctx, int32_t flags);
+int rtb200_last_scattering_acceleration(rtb200_ctx* ctx, int32_t* extrapolations, int32_t* warmStarted);
+
 /* Diffuse (UV background) sweep: replaces equiSources.f90:1372-1808 (computeOpacities :4956, the loop over
  * 12*4**(nAngularLevel-1) HEALPix directions, pattern set-up, neighbour threading, transport).
  *   uvb[3]      boundary intensities uvb1..3 (definitionsModule.f90:53)

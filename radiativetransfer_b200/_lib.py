@@ -40,6 +40,8 @@ SIGNATURES = {
     "rtb200_grid_set_emission_device": (C.c_int, [P, P, P]),
     "rtb200_grid_set_scattering": (C.c_int, [P, P, C.c_int32, C.c_double]),
     "rtb200_last_scattering": (C.c_int, [P, C.POINTER(C.c_int32), C.POINTER(C.c_double)]),
+    "rtb200_grid_set_scattering_acceleration": (C.c_int, [P, C.c_int32]),
+    "rtb200_last_scattering_acceleration": (C.c_int, [P, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "rtb200_grid_set_dust": (C.c_int, [P, C.c_int, P, P, C.c_int32, C.c_double]),
     "rtb200_diffuse": (C.c_int, [P, C.c_int, P, P, P, C.c_int32, P, P, P, C.POINTER(C.c_int64)]),
     "rtb200_diffuse_device": (C.c_int, [P, C.c_int, P, P, P, C.c_int32, P, P, C.POINTER(C.c_int64)]),

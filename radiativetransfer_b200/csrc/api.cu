@@ -67,6 +67,8 @@ static void free_grid(Context& c) {
   cudaFree(c.dEtaEff); c.dEtaEff = nullptr;
   cudaFree(c.dScatScratch); c.dScatScratch = nullptr; c.scatScratchBytes = 0;
   c.scatMaxIter = 1; c.scatTol = 0.; c.lastScatIter = 0; c.lastScatResid = 0.; c.scatResidPending = false;
+  cudaFree(c.dNg); c.dNg = nullptr; c.ngBytes = 0;
+  c.scatAccel = 0; c.scatWarm = false; c.lastNgCount = 0; c.lastWarm = false; c.ngPending = false; c.dWarmTaken = nullptr;
   cudaFree(c.dDustSigma); c.dDustSigma = nullptr;
   c.dustMode = 0;
   for (int g = 0; g < 3; g++) c.dustBeta[g] = c.dustAlbedo[g] = 0.;
@@ -204,8 +206,14 @@ int run_diffuse(Context& c, int nAngularLevel, const double* uvb, const double* 
   c.lastScatIter = 0;
   c.lastScatResid = 0.;
   c.scatResidPending = false;
+  c.lastNgCount = 0;
+  c.lastWarm = false;
+  c.ngPending = false;
   if (!c.scatterSigma()) return run_sweep(c, nAngularLevel, uvb, beta, rays, nrays, dJ, s, nseg, 0);
-  if (rays) return RTB200_ERR_ARG;   // the J of a direction subset is not the mean intensity the source needs
+  if (rays) {   // the J of a direction subset is not the mean intensity the source needs
+    c.scatWarm = false;
+    return RTB200_ERR_ARG;
+  }
   return scatter_solve(c, nAngularLevel, uvb, beta, dJ, s, nseg);
 }
 
@@ -518,6 +526,17 @@ int rtb200_last_scattering(rtb200_ctx* h, int32_t* iterations, double* residual)
   return last_scattering(h->c, iterations, residual);
 }
 
+int rtb200_grid_set_scattering_acceleration(rtb200_ctx* h, int32_t flags) {
+  if (!h) return RTB200_ERR_ARG;
+  if (h->m) return multi_set_scattering_acceleration(h->m, flags);
+  return set_scattering_acceleration(h->c, flags);
+}
+
+int rtb200_last_scattering_acceleration(rtb200_ctx* h, int32_t* extrapolations, int32_t* warmStarted) {
+  if (!h) return RTB200_ERR_ARG;
+  return last_scattering_acceleration(h->m ? multi_primary(h->m) : h->c, extrapolations, warmStarted);
+}
+
 int rtb200_grid_set_emission_device(rtb200_ctx* h, const double* eta_device, void* stream) {
   if (!h || h->m || !eta_device) return RTB200_ERR_ARG;   // a device group takes the host array (slab-wise)
   return set_emission(h->c, eta_device, true, (cudaStream_t)stream);
@@ -543,7 +562,11 @@ int rtb200_diffuse(rtb200_ctx* h, int nAngularLevel, const double* uvb, const do
   RTB_CUDA(cudaStreamSynchronize(c.stream));
   int32_t err = 0;
   RTB_CUDA(cudaMemcpy(&err, c.dErr, sizeof(err), cudaMemcpyDeviceToHost));
-  if (err) { cudaMemset(c.dErr, 0, 64); return err; }
+  if (err) {
+    cudaMemset(c.dErr, 0, 64);
+    c.scatWarm = false;   // a failed solve is no starting guess
+    return err;
+  }
   return RTB200_OK;
 }
 

@@ -89,6 +89,7 @@ int set_dust(Context& c, int mode, const double* betaDust, const double* albedo,
     c.scatTol = tolerance;
   } else if (c.dDustSigma) {   // dust stops scattering: the source iteration's buffers go unless a per-leaf sigma needs them
     cudaFree(c.dDustSigma); c.dDustSigma = nullptr;
+    release_acceleration(c);
     cudaFree(c.dEtaEff); c.dEtaEff = nullptr;
     cudaFree(c.dScatScratch); c.dScatScratch = nullptr; c.scatScratchBytes = 0;
   }

@@ -108,6 +108,7 @@ int nccl_load() {
   } while (0)
 
 constexpr int kMaxRanks = 16;
+static_assert(kMaxRanks <= kNgMaxRanks, "room for every rank's Ng sums");
 constexpr double kZoneCostX = 1.0, kZoneCostY = 1.03, kZoneCostZ = 1.10;
 
 // ---- peer-memory reduce-scatter with fused epilogue -------------------------------------------------------------------
@@ -326,6 +327,7 @@ void free_exchange(Multi& m) {
     cudaFree(q->exch[0]); cudaFree(q->exch[1]); cudaFree(q->flags);
     cudaFree(q->Jslab); cudaFree(q->Kslab); cudaFree(q->Rslab); cudaFree(q->Rbase);
     cudaFree(q->scat); q->scat = nullptr; q->scatBytes = 0;
+    q->c.dWarmTaken = nullptr;
     q->exch[0] = q->exch[1] = nullptr; q->flags = nullptr;
     q->Jslab = q->Kslab = q->Rslab = q->Rbase = nullptr;
     q->haveR = false;
@@ -869,6 +871,12 @@ int multi_set_scattering(Multi* m, const double* sigma, int32_t maxIterations, d
   });
 }
 
+// flags only: every member keeps its own history and its own slab of the stored J
+int multi_set_scattering_acceleration(Multi* m, int32_t flags) {
+  if (m->nleaf == 0) return RTB200_ERR_ARG;
+  return for_each_member(*m, [&](Member& q, int) { return set_scattering_acceleration(q.c, flags); });
+}
+
 // scalars only: every member stores them and computes the dust of the whole grid from its complete species and its
 // complete rho / abun2 (grid_set uploads the caller's full arrays on every member, in rank mode too)
 int multi_set_dust(Multi* m, int mode, const double* betaDust, const double* albedo, int32_t maxIterations, double tolerance) {
@@ -925,6 +933,12 @@ int multi_device_error(Multi* m) {
   return first;
 }
 
+// the stored J of the warm start goes on every local member (in rank mode the other ranks learn it from the holding
+// flags all-gathered at the start of their next call)
+static void drop_stored_j(Multi& m) {
+  for (Member* q : m.mem) q->c.scatWarm = false;
+}
+
 // Source iteration of one member (scattering set), iterations k = 1, 2, ...  Every iteration is an exchange step of its
 // own, step0 + k, so that the peer reduction's double buffering (DESIGN.md 5) keeps its parity:
 //   1. the sweep of the shard with the current source (opacities and sigma once, in the first),
@@ -932,40 +946,37 @@ int multi_device_error(Multi* m) {
 //   3. the slab's source pass: eta_th + sigma * J into this rank's part of the stage, the slab residual,
 //   4. the all-gather of the three source fields, copied into the effective buffer [3][nleaf],
 //   5. with a tolerance, an all-gather of the slab residuals: every rank takes the same max and stops after the same k.
+// With the acceleration flags (ng.cu) the warm start takes x_0 from the rank's Jprev slab, and an Ng step runs between
+// 5 and 4: the slab's five sums, their all-gather, the same solve on every rank and the slab's combine pass.
 // Returns the number of iterations in *iters.
 static int scatter_member(Multi& m, Member& q, unsigned long long step0, int nAngularLevel, const double* uvb,
                           const double* beta, const Epilogue& ep, cudaStream_t s, int* iters) {
   Context& c = q.c;
+  // with the flag, every rank takes the same path below; whether x_0 is the stored J is decided on the devices from
+  // every rank's holding of one, so a rank that lost its J (a failed call) turns the whole group cold
+  const bool warm = (c.scatAccel & RTB200_SCATTER_WARM_START) != 0;
+  const bool ng = (c.scatAccel & RTB200_SCATTER_NG) != 0;
+  const double holds = c.scatWarm ? 1. : 0.;
+  c.scatWarm = false;   // the Jprev slab holds a returned J again only when this call completes
   const int64_t N = m.nleaf, off = slab_off(m, q.rank), cnt = slab_cnt(m, q.rank);
-  const size_t need = (size_t)(3 * m.npad + 3 * m.slab + kMaxRanks + 1) * sizeof(double);
+  // + one word: whether the warm start was taken
+  const size_t need = (size_t)(3 * m.npad + 3 * m.slab + kMaxRanks + 2) * sizeof(double);
   if (int st = ensure_buffer((void**)&q.scat, &q.scatBytes, need)) return st;
   double* stage = q.scat;
   double* Jprev = stage + 3 * m.npad;
   double* all = Jprev + 3 * m.slab;
   unsigned long long* resid = (unsigned long long*)(all + kMaxRanks);
+  int32_t* warmTaken = (int32_t*)(resid + 1);
   const size_t nb = (size_t)3 * N * sizeof(double);
-  // J_0 = 0, eta_1 = eta_th
-  RTB_CUDA(cudaMemsetAsync(Jprev, 0, (size_t)3 * m.slab * sizeof(double), s));
-  if (c.dEta) RTB_CUDA(cudaMemcpyAsync(c.dEtaEff, c.dEta, nb, cudaMemcpyDeviceToDevice, s));
-  else RTB_CUDA(cudaMemsetAsync(c.dEtaEff, 0, nb, s));
-  auto gather_resid = [&]() -> int {   // every rank's slab residual into all[0 .. nranks)
-    RTB_CUDA(cudaMemcpyAsync(all + q.rank, resid, sizeof(double), cudaMemcpyDeviceToDevice, s));
-    if (m.nranks > 1) RTB_NCCL(nccl().AllGather(all + q.rank, all, 1, kNcclFloat64, q.comm, s));
-    return RTB200_OK;
-  };
-  int64_t nsTotal = 0;
-  int k = 1;
-  double r = 0.;
-  for (;; k++) {
-    const unsigned long long step = step0 + (unsigned long long)k;
-    const int buf = (int)(step & 1);
-    if (int st = sweep_member(m, q, buf, nAngularLevel, uvb, beta, s, k)) return st;
-    nsTotal += q.nsegLast;
-    if (int st = reduce_member(m, q, buf, step, 3, q.Jslab, ep, s)) return st;
-    RTB_CUDA(cudaMemsetAsync(resid, 0, sizeof(unsigned long long), s));
-    if (int st = launch_scatter_source(c, cnt, q.Jslab, Jprev, m.slab, c.scatterSigma() + off, c.dEta ? c.dEta + off : nullptr, N,
-                                       stage + (size_t)q.rank * m.slab, m.npad, resid, s))
-      return st;
+  NgBuffers ngb{};
+  if (ng) {
+    if (int st = ng_buffers(c, m.slab, &ngb)) return st;
+    RTB_CUDA(cudaMemsetAsync(ngb.count, 0, sizeof(int32_t), s));
+  }
+  const double* sigmaSlab = nullptr;   // set after the dust (if any) is computed for this call
+  const double* etaThSlab = c.dEta ? c.dEta + off : nullptr;
+  double* stageSlab = stage + (size_t)q.rank * m.slab;
+  auto share_eta = [&]() -> int {      // the ranks' source slabs into every rank's effective buffer
     if (m.nranks > 1) {
       RTB_NCCL(nccl().GroupStart());
       for (int g = 0; g < 3; g++) {
@@ -977,6 +988,52 @@ static int scatter_member(Multi& m, Member& q, unsigned long long step0, int nAn
     for (int g = 0; g < 3; g++)
       RTB_CUDA(cudaMemcpyAsync(c.dEtaEff + (size_t)g * N, stage + (size_t)g * m.npad, (size_t)N * sizeof(double),
                                cudaMemcpyDeviceToDevice, s));
+    return RTB200_OK;
+  };
+  if (warm) {
+    // every rank's holding into all[0 .. nranks), then x_0 = the Jprev slab if all hold one, else 0 (eta_1 = eta_th then,
+    // bit for bit); eta_1 = eta_th + sigma * x_0 by the slab's source pass (Jslab, overwritten by the first reduction,
+    // takes its copy of x_0), then shared as in every iteration; dust computes its sigma from the current species first
+    RTB_CUDA(cudaMemcpyAsync(all + q.rank, &holds, sizeof(double), cudaMemcpyHostToDevice, s));
+    if (m.nranks > 1) RTB_NCCL(nccl().AllGather(all + q.rank, all, 1, kNcclFloat64, q.comm, s));
+    if (int st = launch_warm_start_agree(c, all, m.nranks, Jprev, 3 * m.slab, warmTaken, s)) return st;
+    if (c.dustMode && c.dDustSigma)
+      if (int st = launch_compute_opacities_dust(c, beta, s)) return st;
+    sigmaSlab = c.scatterSigma() + off;
+    if (int st = launch_scatter_source(c, cnt, Jprev, q.Jslab, m.slab, sigmaSlab, etaThSlab, N, stageSlab, m.npad, resid, s))
+      return st;
+    if (int st = share_eta()) return st;
+  } else {
+    // J_0 = 0, eta_1 = eta_th
+    RTB_CUDA(cudaMemsetAsync(Jprev, 0, (size_t)3 * m.slab * sizeof(double), s));
+    if (c.dEta) RTB_CUDA(cudaMemcpyAsync(c.dEtaEff, c.dEta, nb, cudaMemcpyDeviceToDevice, s));
+    else RTB_CUDA(cudaMemsetAsync(c.dEtaEff, 0, nb, s));
+  }
+  auto gather_resid = [&]() -> int {   // every rank's slab residual into all[0 .. nranks)
+    RTB_CUDA(cudaMemcpyAsync(all + q.rank, resid, sizeof(double), cudaMemcpyDeviceToDevice, s));
+    if (m.nranks > 1) RTB_NCCL(nccl().AllGather(all + q.rank, all, 1, kNcclFloat64, q.comm, s));
+    return RTB200_OK;
+  };
+  int64_t nsTotal = 0;
+  int k = 1;
+  int cycle = 0;   // sweeps since the call's start or the last attempted extrapolation
+  double r = 0.;
+  for (;; k++) {
+    const unsigned long long step = step0 + (unsigned long long)k;
+    const int buf = (int)(step & 1);
+    if (int st = sweep_member(m, q, buf, nAngularLevel, uvb, beta, s, k)) return st;
+    nsTotal += q.nsegLast;
+    if (int st = reduce_member(m, q, buf, step, 3, q.Jslab, ep, s)) return st;
+    sigmaSlab = c.scatterSigma() + off;
+    cycle++;
+    const bool extrapolate = ng && cycle == 4 && k < c.scatMaxIter;
+    if (ng && cycle >= 2)   // Ng keeps y of the cycle's sweeps 1..3: the Jprev slab holds y_{k-1} until the source pass
+      RTB_CUDA(cudaMemcpyAsync(ngb.hist[cycle - 2], Jprev, (size_t)3 * m.slab * sizeof(double), cudaMemcpyDeviceToDevice, s));
+    RTB_CUDA(cudaMemsetAsync(resid, 0, sizeof(unsigned long long), s));
+    if (int st = launch_scatter_source(c, cnt, q.Jslab, Jprev, m.slab, sigmaSlab, etaThSlab, N, stageSlab, m.npad, resid, s))
+      return st;
+    if (!extrapolate)
+      if (int st = share_eta()) return st;
     c.lastLaunches += 1;
     if (c.scatTol > 0.) {
       if (int st = gather_resid()) return st;
@@ -985,6 +1042,16 @@ static int scatter_member(Multi& m, Member& q, unsigned long long step0, int nAn
       RTB_CUDA(cudaStreamSynchronize(s));
       r = *std::max_element(v.begin(), v.end());
       if (r <= c.scatTol) break;
+    }
+    if (extrapolate) {   // I0..I3 = y_k (Jslab), y_{k-1}, y_{k-2}, y_{k-3} of the slab; every rank solves with all sums
+      if (int st = launch_ng_partials(ngb, cnt, q.Jslab, m.slab, q.rank, s)) return st;
+      if (m.nranks > 1) RTB_NCCL(nccl().AllGather(ngb.sums + 5 * q.rank, ngb.sums, 5, kNcclFloat64, q.comm, s));
+      if (int st = launch_ng_apply(c, ngb, m.nranks, cnt, q.Jslab, Jprev, m.slab, sigmaSlab, etaThSlab, N, stageSlab,
+                                   m.npad, s))
+        return st;
+      if (int st = share_eta()) return st;
+      c.lastLaunches += 4;
+      cycle = 0;
     }
     if (k == c.scatMaxIter) break;
   }
@@ -995,6 +1062,10 @@ static int scatter_member(Multi& m, Member& q, unsigned long long step0, int nAn
   c.lastScatIter = k;
   c.lastScatResid = r;
   c.scatResidPending = c.scatTol == 0.;
+  c.lastWarm = false;
+  c.dWarmTaken = warm ? warmTaken : nullptr;   // rtb200_last_scattering_acceleration reads it once the call's work is done
+  c.ngPending = ng;
+  c.scatWarm = true;   // the source pass left y_k in the Jprev slab
   *iters = k;
   return RTB200_OK;
 }
@@ -1030,12 +1101,14 @@ int multi_diffuse_resident(Multi* m, int nAngularLevel, const double* uvb, const
   if (int st = build_shards(*m, nAngularLevel, nullptr, 0, multi_primary(m).nx)) return st;
   m->step++;
   std::vector<int> iters((size_t)m->nlocal, 1);
-  for (Member* q : m->mem) q->c.lastScatIter = 0, q->c.lastScatResid = 0., q->c.scatResidPending = false;
+  for (Member* q : m->mem) q->c.lastScatIter = 0, q->c.lastScatResid = 0., q->c.scatResidPending = false, q->c.lastNgCount = 0,
+      q->c.lastWarm = false, q->c.ngPending = false, q->c.dWarmTaken = nullptr;
   int st = for_each_member(*m, [&](Member& q, int i) -> int {
     RTB_CUDA(cudaSetDevice(q.c.device));
     return diffuse_resident_member(*m, q, nAngularLevel, uvb, beta, ksi6, chemistry,
                                    streams ? (cudaStream_t)streams[i] : q.c.stream, &iters[(size_t)i]);
   });
+  if (st) drop_stored_j(*m);   // a failed solve is no starting guess, on any member
   m->step += (unsigned long long)(iters[0] - 1);   // the ranks agree on the iteration count
   if (nseg) {
     *nseg = 0;
@@ -1048,11 +1121,15 @@ int multi_diffuse_host(Multi* m, int nAngularLevel, const double* uvb, const dou
                        int32_t nrays, double* J1, double* J2, double* J3, int64_t* nseg) {
   if (m->nleaf == 0 || !uvb || !beta) return RTB200_ERR_ARG;
   const bool scatter = multi_primary(m).scatterSigma() != nullptr;
-  if (scatter && rays) return RTB200_ERR_ARG;   // the J of a direction subset is not the mean intensity the source needs
+  if (scatter && rays) {   // the J of a direction subset is not the mean intensity the source needs
+    drop_stored_j(*m);
+    return RTB200_ERR_ARG;
+  }
   if (int st = build_shards(*m, nAngularLevel, rays, nrays, multi_primary(m).nx)) return st;
   m->step++;
   std::vector<int> iters((size_t)m->nlocal, 1);
-  for (Member* q : m->mem) q->c.lastScatIter = 0, q->c.lastScatResid = 0., q->c.scatResidPending = false;
+  for (Member* q : m->mem) q->c.lastScatIter = 0, q->c.lastScatResid = 0., q->c.scatResidPending = false, q->c.lastNgCount = 0,
+      q->c.lastWarm = false, q->c.ngPending = false, q->c.dWarmTaken = nullptr;
   int st = for_each_member(*m, [&](Member& q, int i) -> int {
     Context& c = q.c;
     RTB_CUDA(cudaSetDevice(c.device));
@@ -1080,6 +1157,7 @@ int multi_diffuse_host(Multi* m, int nAngularLevel, const double* uvb, const dou
     tm.mark("status");
     return de;
   });
+  if (st) drop_stored_j(*m);   // a failed solve is no starting guess, on any member
   m->step += (unsigned long long)(iters[0] - 1);   // the ranks agree on the iteration count
   if (nseg) {
     *nseg = 0;

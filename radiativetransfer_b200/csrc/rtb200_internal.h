@@ -163,6 +163,14 @@ struct Context {
   int32_t lastScatIter = 0;         // sweeps and last residual of the latest diffuse call
   double lastScatResid = 0;
   bool scatResidPending = false;    // tolerance 0: the residual is still on the device (read by last_scattering)
+  // acceleration of the source iteration (rtb200_grid_set_scattering_acceleration, ng.cu): RTB200_SCATTER_* flags
+  int32_t scatAccel = 0;
+  bool scatWarm = false;            // the J of the previous iteration (Jprev) is the J the latest completed solve returned
+  double* dNg = nullptr;            // Ng history and sums (ng_buffers), allocated while the NG flag is set and a solve runs
+  size_t ngBytes = 0;
+  int32_t lastNgCount = 0;          // extrapolations applied by the latest diffuse call (on the device while ngPending)
+  bool lastWarm = false, ngPending = false;
+  const int32_t* dWarmTaken = nullptr;   // device group: the device's word saying whether the latest call started warm
   // dust (rtb200_grid_set_dust, dust.cu): mode 0 = none.  compute_opacities_dust_kernel adds kd to the opacities of every
   // call and, while an albedo is > 0, writes the scattering source albedo * kd into dDustSigma [3][nleaf]
   int dustMode = 0;
@@ -257,6 +265,34 @@ bool dust_args_ok(int mode, const double* betaDust, const double* albedo, int32_
 int launch_compute_opacities_dust(Context& c, const double* beta, cudaStream_t s);
 int last_scattering(Context& c, int32_t* iterations, double* residual);
 
+// ng.cu: acceleration of the source iteration (DESIGN.md 4.9)
+constexpr int kNgBlocks = 1024;    // fixed grid of the partial-sum pass: its sums do not depend on the device
+constexpr int kNgMaxRanks = 64;
+// views into Context::dNg for fields of `stride` entries per group: hist[j] = y of sweep j + 1 of the current cycle of
+// four, the block partials [kNgBlocks][5], every rank's five sums [kNgMaxRanks][5], coef = {1 - a - b, a, b, apply}
+// and the count of applied extrapolations
+struct NgBuffers {
+  double* hist[3];
+  double* part;
+  double* sums;
+  double* coef;
+  int32_t* count;
+};
+int ng_buffers(Context& c, int64_t stride, NgBuffers* b);
+int set_scattering_acceleration(Context& c, int32_t flags);
+void release_acceleration(Context& c);   // drops the stored J and the Ng history (scattering cleared)
+// the five sums of this rank's cnt entries of I0..I3 (stride jStride) into b.sums[5 * rank ..]
+int launch_ng_partials(const NgBuffers& b, int64_t cnt, const double* I0, int64_t jStride, int rank, cudaStream_t s);
+// from the sums of nranks ranks: a, b and the decision; when it applies, x = max(0, (1-a-b) I0 + a I1 + b I2) into
+// Jprev and eta_th + sigma * x into etaOut (strides as launch_scatter_source), else nothing changes
+int launch_ng_apply(const Context& c, const NgBuffers& b, int nranks, int64_t cnt, const double* I0, double* Jprev,
+                    int64_t jStride, const double* sigma, const double* etaTh, int64_t sStride, double* etaOut,
+                    int64_t oStride, cudaStream_t s);
+int last_scattering_acceleration(Context& c, int32_t* extrapolations, int32_t* warmStarted);
+// device group, warm start: *used = 1 if flags[r] != 0 for every r < nranks, else Jprev[0 .. n) = 0 and *used = 0
+int launch_warm_start_agree(const Context& c, const double* flags, int nranks, double* Jprev, int64_t n, int32_t* used,
+                            cudaStream_t s);
+
 // kernels / launchers --------------------------------------------------------------------------------
 int launch_compute_opacities(Context& c, const double* beta, cudaStream_t s);
 int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std::vector<Direction>& dirs,
@@ -300,6 +336,7 @@ int multi_update_species(Multi* m, const double* HI, const double* HeI, const do
 int multi_set_emission(Multi* m, const double* eta);
 int multi_set_scattering(Multi* m, const double* sigma, int32_t maxIterations, double tolerance);
 int multi_last_scattering(Multi* m, int32_t* iterations, double* residual);
+int multi_set_scattering_acceleration(Multi* m, int32_t flags);
 int multi_set_dust(Multi* m, int mode, const double* betaDust, const double* albedo, int32_t maxIterations, double tolerance);
 int multi_get_species(Multi* m, double* HI, double* HeI, double* HeII);
 int multi_diffuse_host(Multi* m, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays,

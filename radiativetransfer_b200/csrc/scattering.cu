@@ -86,6 +86,7 @@ int set_scattering(Context& c, const double* sigma, bool device, int32_t maxIter
   if (!sigma) {
     cudaFree(c.dSigma); c.dSigma = nullptr;
     if (!c.dDustSigma) {   // scattering dust keeps the buffers of its source iteration
+      release_acceleration(c);
       cudaFree(c.dEtaEff); c.dEtaEff = nullptr;
       cudaFree(c.dScatScratch); c.dScatScratch = nullptr; c.scatScratchBytes = 0;
     }
@@ -123,27 +124,50 @@ int last_scattering(Context& c, int32_t* iterations, double* residual) {
   return RTB200_OK;
 }
 
-// Source iteration of a single context over all directions of nAngularLevel, into dJ (J_k, the last iteration's).
+// Source iteration of a single context over all directions of nAngularLevel, into dJ (J_k, the last iteration's).  With
+// the acceleration flags (ng.cu): the warm start takes x_0 from Jprev, which holds the J the previous completed solve
+// returned, and Ng extrapolates after every fourth sweep of a cycle; the plain source pass runs after every sweep.
 int scatter_solve(Context& c, int nAngularLevel, const double* uvb, const double* beta, double* dJ, cudaStream_t s,
                   int64_t* nseg) {
   if (!uvb || !beta || !dJ || c.nleaf == 0) return RTB200_ERR_ARG;
+  const bool warm = (c.scatAccel & RTB200_SCATTER_WARM_START) && c.scatWarm;
+  const bool ng = (c.scatAccel & RTB200_SCATTER_NG) != 0;
+  c.scatWarm = false;   // Jprev holds a returned J again only when this call completes
   RTB_CUDA(cudaSetDevice(c.device));
   const int64_t N = c.nleaf;
   // [3][N] J of the previous iteration, then the residual word
   if (int st = ensure_buffer((void**)&c.dScatScratch, &c.scatScratchBytes, (size_t)(3 * N + 1) * sizeof(double))) return st;
   double* Jprev = c.dScatScratch;
   unsigned long long* resid = (unsigned long long*)(c.dScatScratch + 3 * N);
-  // J_0 = 0, eta_1 = eta_th (+ sigma * 0)
-  RTB_CUDA(cudaMemsetAsync(Jprev, 0, (size_t)3 * N * sizeof(double), s));
-  if (c.dEta) RTB_CUDA(cudaMemcpyAsync(c.dEtaEff, c.dEta, (size_t)3 * N * sizeof(double), cudaMemcpyDeviceToDevice, s));
-  else RTB_CUDA(cudaMemsetAsync(c.dEtaEff, 0, (size_t)3 * N * sizeof(double), s));
+  NgBuffers nb{};
+  if (ng) {
+    if (int st = ng_buffers(c, N, &nb)) return st;
+    RTB_CUDA(cudaMemsetAsync(nb.count, 0, sizeof(int32_t), s));
+  }
+  if (warm) {
+    // eta_1 = eta_th + sigma * x_0 by the source pass (dJ, overwritten by the first sweep, takes its copy of x_0); dust
+    // computes its sigma from the current species first
+    if (c.dustMode && c.dDustSigma)
+      if (int st = launch_compute_opacities_dust(c, beta, s)) return st;
+    if (int st = launch_scatter_source(c, N, Jprev, dJ, N, c.scatterSigma(), c.dEta, N, c.dEtaEff, N, resid, s)) return st;
+  } else {
+    // J_0 = 0, eta_1 = eta_th (+ sigma * 0)
+    RTB_CUDA(cudaMemsetAsync(Jprev, 0, (size_t)3 * N * sizeof(double), s));
+    if (c.dEta) RTB_CUDA(cudaMemcpyAsync(c.dEtaEff, c.dEta, (size_t)3 * N * sizeof(double), cudaMemcpyDeviceToDevice, s));
+    else RTB_CUDA(cudaMemsetAsync(c.dEtaEff, 0, (size_t)3 * N * sizeof(double), s));
+  }
   int64_t total = 0;
   int k = 0;
+  int cycle = 0;   // sweeps since the call's start or the last attempted extrapolation
   double r = 0.;
   for (k = 1; k <= c.scatMaxIter; k++) {
     int64_t ns = 0;
     if (int st = run_sweep(c, nAngularLevel, uvb, beta, nullptr, 0, dJ, s, &ns, k)) return st;
     total += ns;
+    cycle++;
+    // Ng keeps y of the cycle's sweeps 1..3: Jprev holds y_{k-1} until the source pass overwrites it
+    if (ng && cycle >= 2)
+      RTB_CUDA(cudaMemcpyAsync(nb.hist[cycle - 2], Jprev, (size_t)3 * N * sizeof(double), cudaMemcpyDeviceToDevice, s));
     RTB_CUDA(cudaMemsetAsync(resid, 0, sizeof(unsigned long long), s));
     if (int st = launch_scatter_source(c, N, dJ, Jprev, N, c.scatterSigma(), c.dEta, N, c.dEtaEff, N, resid, s)) return st;
     c.lastLaunches += 1;
@@ -152,6 +176,12 @@ int scatter_solve(Context& c, int nAngularLevel, const double* uvb, const double
       RTB_CUDA(cudaStreamSynchronize(s));
       if (r <= c.scatTol) break;
     }
+    if (ng && cycle == 4 && k < c.scatMaxIter) {   // I0..I3 = y_k (dJ), y_{k-1}, y_{k-2}, y_{k-3}
+      if (int st = launch_ng_partials(nb, N, dJ, N, 0, s)) return st;
+      if (int st = launch_ng_apply(c, nb, 1, N, dJ, Jprev, N, c.scatterSigma(), c.dEta, N, c.dEtaEff, N, s)) return st;
+      c.lastLaunches += 4;
+      cycle = 0;
+    }
   }
   if (k > c.scatMaxIter) k = c.scatMaxIter;
   RTB_CUDA(cudaEventRecord(c.evStop, s));   // device time of the whole call, source passes included
@@ -159,6 +189,9 @@ int scatter_solve(Context& c, int nAngularLevel, const double* uvb, const double
   c.lastScatIter = k;
   c.lastScatResid = r;
   c.scatResidPending = c.scatTol == 0.;     // rtb200_last_scattering reads it once the call's work is done
+  c.lastWarm = warm;
+  c.ngPending = ng;                         // rtb200_last_scattering_acceleration reads the count likewise
+  c.scatWarm = true;                        // the source pass left y_k in Jprev
   return RTB200_OK;
 }
 

@@ -67,6 +67,12 @@ module rtb200_shim
        integer(c_int32_t), intent(out) :: iterations
        real(c_double), intent(out) :: residual
      end function rtb200_last_scattering
+     integer(c_int) function rtb200_grid_set_scattering_acceleration(ctx, flags) &
+          bind(C, name='rtb200_grid_set_scattering_acceleration')
+       import :: c_ptr, c_int, c_int32_t
+       type(c_ptr), value :: ctx
+       integer(c_int32_t), value :: flags
+     end function rtb200_grid_set_scattering_acceleration
      integer(c_int) function rtb200_grid_set_dust(ctx, dustApproximation, betaDust, albedo, maxIterations, tolerance) &
           bind(C, name='rtb200_grid_set_dust')
        import :: c_ptr, c_int, c_int32_t, c_double
@@ -475,6 +481,19 @@ contains
     call rtbCheck(rtb200_last_scattering(rtbContext, it, residual), 'rtb200_last_scattering')
     iterations = int(it)
   end subroutine rtbScatteringStatus
+
+  ! Acceleration of the source iteration (extension, DESIGN.md 4.9) of rtbSetScattering / rtbSetDust: ng extrapolates
+  ! after every fourth sweep (Ng, order 2), warmStart starts each solve from the J the previous rtbDiffuse returned
+  ! instead of 0 (the case of an outer transport <-> chemistry loop).  Both .false. is plain source iteration; rtbSetGrid
+  ! resets it.
+  subroutine rtbSetScatteringAcceleration(ng, warmStart)
+    logical, intent(in) :: ng, warmStart
+    integer(c_int32_t) :: flags
+    flags = 0
+    if (ng) flags = flags + 1_c_int32_t
+    if (warmStart) flags = flags + 2_c_int32_t
+    call rtbCheck(rtb200_grid_set_scattering_acceleration(rtbContext, flags), 'rtb200_grid_set_scattering_acceleration')
+  end subroutine rtbSetScatteringAcceleration
 
   ! Dust in the diffuse sweep (extension, DESIGN.md 4.8): the dust model of the point-source path (a_smc, dustModule.f90)
   ! as an opacity of the UV background, recomputed from the current species in every rtbDiffuse.  dustApproximation

@@ -250,6 +250,22 @@ class Transport:
         _lib.check(self.L.rtb200_last_scattering(self.h, C.byref(it), C.byref(r)), "rtb200_last_scattering")
         return {"iterations": it.value, "residual": r.value}
 
+    def set_scattering_acceleration(self, ng=False, warm_start=False):
+        """Acceleration of the source iteration of set_scattering / set_dust (DESIGN.md 4.9): `ng` extrapolates after
+        every fourth sweep (Ng, order 2), `warm_start` starts from the J the previous completed solve returned instead
+        of J = 0.  Both off is plain source iteration.  A device group sets it on every rank (collectively in rank mode).
+        set_grid resets it."""
+        flags = (1 if ng else 0) | (2 if warm_start else 0)
+        _lib.check(self.L.rtb200_grid_set_scattering_acceleration(self.h, flags), "rtb200_grid_set_scattering_acceleration")
+
+    def last_scattering_acceleration(self):
+        """Of the latest diffuse call: {"extrapolations": Ng steps applied (skipped ones not counted), "warm_start": whether
+        it started from the previous call's J}."""
+        n, w = C.c_int32(0), C.c_int32(0)
+        _lib.check(self.L.rtb200_last_scattering_acceleration(self.h, C.byref(n), C.byref(w)),
+                   "rtb200_last_scattering_acceleration")
+        return {"extrapolations": n.value, "warm_start": bool(w.value)}
+
     def diffuse(self, uvb, beta, n_angular_level=3, rays=None, out=None):
         """Host-buffer call (H2D of nothing but tables, D2H of J): returns (J[3, nleaf], nseg)."""
         uvb, beta = _f64(uvb), _f64(np.asarray(beta).reshape(9))
