@@ -64,11 +64,9 @@ static void free_grid(Context& c) {
   cudaFree(c.dEta); c.dEta = nullptr;
   cudaFree(c.dEtaT); c.dEtaT = nullptr; c.etaTBytes = 0;
   cudaFree(c.dSigma); c.dSigma = nullptr;
-  cudaFree(c.dEtaEff); c.dEtaEff = nullptr;
-  cudaFree(c.dScatScratch); c.dScatScratch = nullptr; c.scatScratchBytes = 0;
-  c.scatMaxIter = 1; c.scatTol = 0.; c.lastScatIter = 0; c.lastScatResid = 0.; c.scatResidPending = false;
-  cudaFree(c.dNg); c.dNg = nullptr; c.ngBytes = 0;
-  c.scatAccel = 0; c.scatWarm = false; c.lastNgCount = 0; c.lastWarm = false; c.ngPending = false; c.dWarmTaken = nullptr;
+  release_source_iteration(c);
+  c.scatMaxIter = 1; c.scatTol = 0.; c.scatAccel = 0;
+  reset_call_results(c);
   cudaFree(c.dDustSigma); c.dDustSigma = nullptr;
   c.dustMode = 0;
   for (int g = 0; g < 3; g++) c.dustBeta[g] = c.dustAlbedo[g] = 0.;
@@ -201,14 +199,19 @@ int run_sweep(Context& c, int nAngularLevel, const double* uvb, const double* be
   return RTB200_OK;
 }
 
-int run_diffuse(Context& c, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays,
-                int32_t nrays, double* dJ, cudaStream_t s, int64_t* nseg) {
+void reset_call_results(Context& c) {
   c.lastScatIter = 0;
   c.lastScatResid = 0.;
-  c.scatResidPending = false;
+  c.dScatResid = nullptr;
   c.lastNgCount = 0;
   c.lastWarm = false;
   c.ngPending = false;
+  c.dWarmTaken = nullptr;
+}
+
+int run_diffuse(Context& c, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays,
+                int32_t nrays, double* dJ, cudaStream_t s, int64_t* nseg) {
+  reset_call_results(c);
   if (!c.scatterSigma()) return run_sweep(c, nAngularLevel, uvb, beta, rays, nrays, dJ, s, nseg, 0);
   if (rays) {   // the J of a direction subset is not the mean intensity the source needs
     c.scatWarm = false;
@@ -221,15 +224,14 @@ int run_diffuse(Context& c, int nAngularLevel, const double* uvb, const double* 
 __global__ void count_bad_kernel(const double* __restrict__ x, int64_t n, int32_t* bad) {
   int32_t mine = 0;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-    const double v = x[i];
-    if (!(v >= 0. && v <= 1.7976931348623157e308)) mine++;
+    if (!finite_nonneg(x[i])) mine++;
   }
   if (mine) atomicAdd(bad, mine);
 }
 
 static bool host_eta_ok(const double* eta, int64_t n) {
   for (int64_t i = 0; i < n; i++)
-    if (!(eta[i] >= 0. && eta[i] <= 1.7976931348623157e308)) return false;
+    if (!finite_nonneg(eta[i])) return false;
   return true;
 }
 
@@ -405,6 +407,29 @@ int grid_set(Context& c, int nx, int64_t nleaf, const int8_t* level, const doubl
   return RTB200_OK;
 }
 
+PointInputs make_point_inputs(int nWave, const double* wavelength, const double* lum, const double* metallicity,
+                              double coefSpectrum, const double* aDust, int dust, int maxPixelLevel, int nsrc,
+                              const int32_t* srcLeaf, const int32_t* srcWeight) {
+  PointInputs in;
+  in.nWave = nWave; in.wavelength = wavelength; in.lum = lum; in.metallicity = metallicity;
+  in.coefSpectrum = coefSpectrum; in.aDust = aDust; in.dust = dust; in.maxPixelLevel = maxPixelLevel;
+  in.nsrc = nsrc; in.srcLeaf = srcLeaf; in.srcWeight = srcWeight;
+  return in;
+}
+
+void split_diag(const double* d, size_t n, const int* idx, double* rem, double* bnd, double* dust, double* spec,
+                int32_t* hpl) {
+  for (size_t i = 0; i < n; i++) {
+    const double* p = d + i * 320;
+    const size_t s = idx ? (size_t)idx[i] : i;
+    if (rem) memcpy(rem + s * 7, p, 56);
+    if (bnd) memcpy(bnd + s * 7, p + 7, 56);
+    if (dust) dust[s] = p[14];
+    if (spec) memcpy(spec + s * 300, p + 16, 2400);
+    if (hpl) hpl[s] = (int32_t)p[15];
+  }
+}
+
 }  // namespace rtb
 
 using namespace rtb;
@@ -522,8 +547,7 @@ int rtb200_grid_set_dust(rtb200_ctx* h, int dustApproximation, const double* bet
 
 int rtb200_last_scattering(rtb200_ctx* h, int32_t* iterations, double* residual) {
   if (!h) return RTB200_ERR_ARG;
-  if (h->m) return multi_last_scattering(h->m, iterations, residual);
-  return last_scattering(h->c, iterations, residual);
+  return last_scattering(h->m ? multi_primary(h->m) : h->c, iterations, residual);
 }
 
 int rtb200_grid_set_scattering_acceleration(rtb200_ctx* h, int32_t flags) {
@@ -577,28 +601,6 @@ int rtb200_diffuse_rates_device(rtb200_ctx* h, const double* J, const double* ks
   return launch_diffuse_rates(h->c, J, ksi24, ksi25, ksi26, k24, k25, k26, (cudaStream_t)stream);
 }
 
-static PointInputs make_point_inputs(int nWave, const double* wavelength, const double* lum, const double* metallicity,
-                                     double coefSpectrum, const double* aDust, int dust, int maxPixelLevel, int nsrc,
-                                     const int32_t* srcLeaf, const int32_t* srcWeight) {
-  PointInputs in;
-  in.nWave = nWave; in.wavelength = wavelength; in.lum = lum; in.metallicity = metallicity;
-  in.coefSpectrum = coefSpectrum; in.aDust = aDust; in.dust = dust; in.maxPixelLevel = maxPixelLevel;
-  in.nsrc = nsrc; in.srcLeaf = srcLeaf; in.srcWeight = srcWeight;
-  return in;
-}
-
-static void split_diag(const std::vector<double>& d, int nsrc, double* rem, double* bnd, double* dust, double* spec,
-                       int32_t* hpl) {
-  for (int s = 0; s < nsrc; s++) {
-    const double* p = d.data() + (size_t)s * 320;
-    if (rem) memcpy(rem + (size_t)s * 7, p, 56);
-    if (bnd) memcpy(bnd + (size_t)s * 7, p + 7, 56);
-    if (dust) dust[s] = p[14];
-    if (spec) memcpy(spec + (size_t)s * 300, p + 16, 2400);
-    if (hpl) hpl[s] = (int32_t)p[15];
-  }
-}
-
 int rtb200_point_device(rtb200_ctx* h, int nWave, const double* wavelength, const double* lum, const double* metallicity,
                         double coefSpectrum, const double* aDust, int dustApproximation, int maxPixelLevel, int32_t nsrc,
                         const int32_t* srcLeaf, const int32_t* srcWeight, double* rates_device, void* stream,
@@ -612,7 +614,9 @@ int rtb200_point_device(rtb200_ctx* h, int nWave, const double* wavelength, cons
   int st = point_solve(h->c, in, rates_device, wantDiag ? diag.data() : nullptr, nseg, nullptr, 0, nullptr, nullptr,
                        (cudaStream_t)stream);
   if (st) return st;
-  if (wantDiag) split_diag(diag, nsrc, ndotRemaining, ndotBoundary, ndotDust, ndotSpectrum, highestPixelLevel);
+  if (wantDiag)
+    split_diag(diag.data(), (size_t)std::max(nsrc, 0), nullptr, ndotRemaining, ndotBoundary, ndotDust, ndotSpectrum,
+               highestPixelLevel);
   return RTB200_OK;
 }
 
@@ -631,7 +635,7 @@ static int point_host_call(Context& c, const PointInputs& in, double* const k[6]
   if (st) return st;
   for (int i = 0; i < 6; i++) RTB_CUDA(cudaMemcpyAsync(k[i], c.dRates + (size_t)i * c.nleaf, nb, cudaMemcpyDeviceToHost, c.stream));
   RTB_CUDA(cudaStreamSynchronize(c.stream));
-  split_diag(diag, in.nsrc, rem, bnd, dust, spec, hpl);
+  split_diag(diag.data(), (size_t)std::max(in.nsrc, 0), nullptr, rem, bnd, dust, spec, hpl);
   return RTB200_OK;
 }
 

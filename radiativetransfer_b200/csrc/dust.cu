@@ -58,7 +58,7 @@ bool dust_args_ok(int mode, const double* betaDust, const double* albedo, int32_
   if (mode == 0) return true;
   if (!betaDust || !albedo) return false;
   for (int g = 0; g < 3; g++) {
-    if (!(betaDust[g] >= 0. && betaDust[g] <= 1.7976931348623157e308)) return false;   // negative, NaN, Inf
+    if (!finite_nonneg(betaDust[g])) return false;
     if (!(albedo[g] >= 0. && albedo[g] <= 1.)) return false;
   }
   if (scatters(albedo) && (maxIterations < 1 || !(tolerance >= 0.) || std::isinf(tolerance))) return false;
@@ -87,11 +87,9 @@ int set_dust(Context& c, int mode, const double* betaDust, const double* albedo,
     }
     c.scatMaxIter = maxIterations;
     c.scatTol = tolerance;
-  } else if (c.dDustSigma) {   // dust stops scattering: the source iteration's buffers go unless a per-leaf sigma needs them
+  } else if (c.dDustSigma) {   // dust stops scattering (a per-leaf sigma cannot be set while it scatters)
     cudaFree(c.dDustSigma); c.dDustSigma = nullptr;
-    release_acceleration(c);
-    cudaFree(c.dEtaEff); c.dEtaEff = nullptr;
-    cudaFree(c.dScatScratch); c.dScatScratch = nullptr; c.scatScratchBytes = 0;
+    release_source_iteration(c);
   }
   c.dustMode = mode;
   for (int g = 0; g < 3; g++) {

@@ -278,10 +278,6 @@ struct Member {                     // one local device
   cudaStream_t copyStream = nullptr;                    // slab uploads of update_species, one event per species
   cudaEvent_t evCopy[3] = {nullptr, nullptr, nullptr};
   int64_t nsegLast = 0;
-  // source iteration (scattering set): [3][npad] all-gather stage of the source | [3][slab] J of the previous
-  // iteration | [kMaxRanks] slab residuals of every rank | this rank's residual word
-  double* scat = nullptr;
-  size_t scatBytes = 0;
 };
 
 struct Multi {
@@ -326,8 +322,6 @@ void free_exchange(Multi& m) {
     q->ipcOpened.clear();
     cudaFree(q->exch[0]); cudaFree(q->exch[1]); cudaFree(q->flags);
     cudaFree(q->Jslab); cudaFree(q->Kslab); cudaFree(q->Rslab); cudaFree(q->Rbase);
-    cudaFree(q->scat); q->scat = nullptr; q->scatBytes = 0;
-    q->c.dWarmTaken = nullptr;
     q->exch[0] = q->exch[1] = nullptr; q->flags = nullptr;
     q->Jslab = q->Kslab = q->Rslab = q->Rbase = nullptr;
     q->haveR = false;
@@ -798,10 +792,8 @@ static int multi_set_field(Multi* m, const double* eta, Apply apply) {
   for (Member* q : m->mem) {
     const int64_t off = slab_off(*m, q->rank), cnt = slab_cnt(*m, q->rank);
     for (int g = 0; g < 3 && ok; g++)
-      for (int64_t i = off; i < off + cnt; i++) {
-        const double v = eta[g * N + i];
-        if (!(v >= 0. && v <= 1.7976931348623157e308)) { ok = false; break; }
-      }
+      for (int64_t i = off; i < off + cnt; i++)
+        if (!finite_nonneg(eta[g * N + i])) { ok = false; break; }
   }
   return for_each_member(*m, [&](Member& q, int) -> int {
     Context& c = q.c;
@@ -884,22 +876,6 @@ int multi_set_dust(Multi* m, int mode, const double* betaDust, const double* alb
   return for_each_member(*m, [&](Member& q, int) { return set_dust(q.c, mode, betaDust, albedo, maxIterations, tolerance); });
 }
 
-int multi_last_scattering(Multi* m, int32_t* iterations, double* residual) {
-  Member& q = *m->mem[0];
-  Context& c = q.c;
-  if (c.scatResidPending) {   // tolerance 0: every rank's slab residual was all-gathered on the devices
-    RTB_CUDA(cudaSetDevice(c.device));
-    RTB_CUDA(cudaDeviceSynchronize());
-    std::vector<double> all((size_t)m->nranks);
-    RTB_CUDA(cudaMemcpy(all.data(), q.scat + 3 * m->npad + 3 * m->slab, all.size() * sizeof(double), cudaMemcpyDeviceToHost));
-    c.lastScatResid = *std::max_element(all.begin(), all.end());
-    c.scatResidPending = false;
-  }
-  if (iterations) *iterations = c.lastScatIter;
-  if (residual) *residual = c.lastScatResid;
-  return RTB200_OK;
-}
-
 int multi_get_species(Multi* m, double* HI, double* HeI, double* HeII) {
   if (m->nleaf == 0) return RTB200_ERR_ARG;
   return for_each_member(*m, [&](Member& q, int) -> int {
@@ -939,44 +915,29 @@ static void drop_stored_j(Multi& m) {
   for (Member* q : m.mem) q->c.scatWarm = false;
 }
 
-// Source iteration of one member (scattering set), iterations k = 1, 2, ...  Every iteration is an exchange step of its
-// own, step0 + k, so that the peer reduction's double buffering (DESIGN.md 5) keeps its parity:
-//   1. the sweep of the shard with the current source (opacities and sigma once, in the first),
-//   2. the reduction into Jslab (with the epilogue ep: photo-rates are overwritten, so the last iteration's stay),
-//   3. the slab's source pass: eta_th + sigma * J into this rank's part of the stage, the slab residual,
-//   4. the all-gather of the three source fields, copied into the effective buffer [3][nleaf],
-//   5. with a tolerance, an all-gather of the slab residuals: every rank takes the same max and stops after the same k.
-// With the acceleration flags (ng.cu) the warm start takes x_0 from the rank's Jprev slab, and an Ng step runs between
-// 5 and 4: the slab's five sums, their all-gather, the same solve on every rank and the slab's combine pass.
-// Returns the number of iterations in *iters.
+// Source iteration of one member (scattering set) over its slab: the loop of source_iteration (scattering.cu), with
+// the sweep of the shard reduced into Jslab and the exchanges over NCCL.  Iteration k is the exchange step step0 + k,
+// so that the peer reduction's double buffering (DESIGN.md 5) keeps its parity; the reduction applies the epilogue ep
+// (photo-rates are overwritten, so the last iteration's stay).  Returns the number of iterations in *iters.
 static int scatter_member(Multi& m, Member& q, unsigned long long step0, int nAngularLevel, const double* uvb,
                           const double* beta, const Epilogue& ep, cudaStream_t s, int* iters) {
   Context& c = q.c;
-  // with the flag, every rank takes the same path below; whether x_0 is the stored J is decided on the devices from
-  // every rank's holding of one, so a rank that lost its J (a failed call) turns the whole group cold
-  const bool warm = (c.scatAccel & RTB200_SCATTER_WARM_START) != 0;
-  const bool ng = (c.scatAccel & RTB200_SCATTER_NG) != 0;
-  const double holds = c.scatWarm ? 1. : 0.;
-  c.scatWarm = false;   // the Jprev slab holds a returned J again only when this call completes
-  const int64_t N = m.nleaf, off = slab_off(m, q.rank), cnt = slab_cnt(m, q.rank);
-  // + one word: whether the warm start was taken
-  const size_t need = (size_t)(3 * m.npad + 3 * m.slab + kMaxRanks + 2) * sizeof(double);
-  if (int st = ensure_buffer((void**)&q.scat, &q.scatBytes, need)) return st;
-  double* stage = q.scat;
-  double* Jprev = stage + 3 * m.npad;
-  double* all = Jprev + 3 * m.slab;
-  unsigned long long* resid = (unsigned long long*)(all + kMaxRanks);
-  int32_t* warmTaken = (int32_t*)(resid + 1);
-  const size_t nb = (size_t)3 * N * sizeof(double);
-  NgBuffers ngb{};
-  if (ng) {
-    if (int st = ng_buffers(c, m.slab, &ngb)) return st;
-    RTB_CUDA(cudaMemsetAsync(ngb.count, 0, sizeof(int32_t), s));
-  }
-  const double* sigmaSlab = nullptr;   // set after the dust (if any) is computed for this call
-  const double* etaThSlab = c.dEta ? c.dEta + off : nullptr;
-  double* stageSlab = stage + (size_t)q.rank * m.slab;
-  auto share_eta = [&]() -> int {      // the ranks' source slabs into every rank's effective buffer
+  SourcePart p;
+  p.rank = q.rank; p.nranks = m.nranks;
+  p.off = slab_off(m, q.rank); p.cnt = slab_cnt(m, q.rank);
+  p.J = q.Jslab; p.jStride = m.slab; p.stageStride = m.npad;
+  p.sweep = [&](int k, int64_t* ns) -> int {
+    const unsigned long long step = step0 + (unsigned long long)k;
+    const int buf = (int)(step & 1);
+    if (int st = sweep_member(m, q, buf, nAngularLevel, uvb, beta, s, k)) return st;
+    *ns = q.nsegLast;
+    return reduce_member(m, q, buf, step, 3, q.Jslab, ep, s);
+  };
+  p.allgather = [&](double* words, int n) -> int {
+    if (m.nranks > 1) RTB_NCCL(nccl().AllGather(words + (size_t)n * q.rank, words, (size_t)n, kNcclFloat64, q.comm, s));
+    return RTB200_OK;
+  };
+  p.share_source = [&](double* stage) -> int {
     if (m.nranks > 1) {
       RTB_NCCL(nccl().GroupStart());
       for (int g = 0; g < 3; g++) {
@@ -986,88 +947,11 @@ static int scatter_member(Multi& m, Member& q, unsigned long long step0, int nAn
       RTB_NCCL(nccl().GroupEnd());
     }
     for (int g = 0; g < 3; g++)
-      RTB_CUDA(cudaMemcpyAsync(c.dEtaEff + (size_t)g * N, stage + (size_t)g * m.npad, (size_t)N * sizeof(double),
+      RTB_CUDA(cudaMemcpyAsync(c.dEtaEff + (size_t)g * m.nleaf, stage + (size_t)g * m.npad, (size_t)m.nleaf * sizeof(double),
                                cudaMemcpyDeviceToDevice, s));
     return RTB200_OK;
   };
-  if (warm) {
-    // every rank's holding into all[0 .. nranks), then x_0 = the Jprev slab if all hold one, else 0 (eta_1 = eta_th then,
-    // bit for bit); eta_1 = eta_th + sigma * x_0 by the slab's source pass (Jslab, overwritten by the first reduction,
-    // takes its copy of x_0), then shared as in every iteration; dust computes its sigma from the current species first
-    RTB_CUDA(cudaMemcpyAsync(all + q.rank, &holds, sizeof(double), cudaMemcpyHostToDevice, s));
-    if (m.nranks > 1) RTB_NCCL(nccl().AllGather(all + q.rank, all, 1, kNcclFloat64, q.comm, s));
-    if (int st = launch_warm_start_agree(c, all, m.nranks, Jprev, 3 * m.slab, warmTaken, s)) return st;
-    if (c.dustMode && c.dDustSigma)
-      if (int st = launch_compute_opacities_dust(c, beta, s)) return st;
-    sigmaSlab = c.scatterSigma() + off;
-    if (int st = launch_scatter_source(c, cnt, Jprev, q.Jslab, m.slab, sigmaSlab, etaThSlab, N, stageSlab, m.npad, resid, s))
-      return st;
-    if (int st = share_eta()) return st;
-  } else {
-    // J_0 = 0, eta_1 = eta_th
-    RTB_CUDA(cudaMemsetAsync(Jprev, 0, (size_t)3 * m.slab * sizeof(double), s));
-    if (c.dEta) RTB_CUDA(cudaMemcpyAsync(c.dEtaEff, c.dEta, nb, cudaMemcpyDeviceToDevice, s));
-    else RTB_CUDA(cudaMemsetAsync(c.dEtaEff, 0, nb, s));
-  }
-  auto gather_resid = [&]() -> int {   // every rank's slab residual into all[0 .. nranks)
-    RTB_CUDA(cudaMemcpyAsync(all + q.rank, resid, sizeof(double), cudaMemcpyDeviceToDevice, s));
-    if (m.nranks > 1) RTB_NCCL(nccl().AllGather(all + q.rank, all, 1, kNcclFloat64, q.comm, s));
-    return RTB200_OK;
-  };
-  int64_t nsTotal = 0;
-  int k = 1;
-  int cycle = 0;   // sweeps since the call's start or the last attempted extrapolation
-  double r = 0.;
-  for (;; k++) {
-    const unsigned long long step = step0 + (unsigned long long)k;
-    const int buf = (int)(step & 1);
-    if (int st = sweep_member(m, q, buf, nAngularLevel, uvb, beta, s, k)) return st;
-    nsTotal += q.nsegLast;
-    if (int st = reduce_member(m, q, buf, step, 3, q.Jslab, ep, s)) return st;
-    sigmaSlab = c.scatterSigma() + off;
-    cycle++;
-    const bool extrapolate = ng && cycle == 4 && k < c.scatMaxIter;
-    if (ng && cycle >= 2)   // Ng keeps y of the cycle's sweeps 1..3: the Jprev slab holds y_{k-1} until the source pass
-      RTB_CUDA(cudaMemcpyAsync(ngb.hist[cycle - 2], Jprev, (size_t)3 * m.slab * sizeof(double), cudaMemcpyDeviceToDevice, s));
-    RTB_CUDA(cudaMemsetAsync(resid, 0, sizeof(unsigned long long), s));
-    if (int st = launch_scatter_source(c, cnt, q.Jslab, Jprev, m.slab, sigmaSlab, etaThSlab, N, stageSlab, m.npad, resid, s))
-      return st;
-    if (!extrapolate)
-      if (int st = share_eta()) return st;
-    c.lastLaunches += 1;
-    if (c.scatTol > 0.) {
-      if (int st = gather_resid()) return st;
-      std::vector<double> v((size_t)m.nranks);
-      RTB_CUDA(cudaMemcpyAsync(v.data(), all, v.size() * sizeof(double), cudaMemcpyDeviceToHost, s));
-      RTB_CUDA(cudaStreamSynchronize(s));
-      r = *std::max_element(v.begin(), v.end());
-      if (r <= c.scatTol) break;
-    }
-    if (extrapolate) {   // I0..I3 = y_k (Jslab), y_{k-1}, y_{k-2}, y_{k-3} of the slab; every rank solves with all sums
-      if (int st = launch_ng_partials(ngb, cnt, q.Jslab, m.slab, q.rank, s)) return st;
-      if (m.nranks > 1) RTB_NCCL(nccl().AllGather(ngb.sums + 5 * q.rank, ngb.sums, 5, kNcclFloat64, q.comm, s));
-      if (int st = launch_ng_apply(c, ngb, m.nranks, cnt, q.Jslab, Jprev, m.slab, sigmaSlab, etaThSlab, N, stageSlab,
-                                   m.npad, s))
-        return st;
-      if (int st = share_eta()) return st;
-      c.lastLaunches += 4;
-      cycle = 0;
-    }
-    if (k == c.scatMaxIter) break;
-  }
-  if (c.scatTol == 0.)   // read by rtb200_last_scattering: no host round trip in the call
-    if (int st = gather_resid()) return st;
-  RTB_CUDA(cudaEventRecord(c.evStop, s));
-  q.nsegLast = nsTotal;
-  c.lastScatIter = k;
-  c.lastScatResid = r;
-  c.scatResidPending = c.scatTol == 0.;
-  c.lastWarm = false;
-  c.dWarmTaken = warm ? warmTaken : nullptr;   // rtb200_last_scattering_acceleration reads it once the call's work is done
-  c.ngPending = ng;
-  c.scatWarm = true;   // the source pass left y_k in the Jprev slab
-  *iters = k;
-  return RTB200_OK;
+  return source_iteration(c, p, beta, s, iters, &q.nsegLast);
 }
 
 // resident step of one member on stream s: opacities + sweep of the shard + reduce-scatter (+ photo-rates)
@@ -1095,26 +979,38 @@ static int diffuse_resident_member(Multi& m, Member& q, int nAngularLevel, const
   return RTB200_OK;
 }
 
+static int64_t sum_nseg(const Multi& m) {
+  int64_t n = 0;
+  for (const Member* q : m.mem) n += q->nsegLast;
+  return n;
+}
+
+// The frame of a diffuse call of the group: the direction shards, the call's exchange step (a source iteration takes one
+// per iteration), the per-call results reset, `member(q, i, &iterations)` on every member with its device current, and
+// the stored J dropped everywhere when any member fails
+template <class Body>
+static int multi_diffuse(Multi& m, int nAngularLevel, const int32_t* rays, int32_t nrays, int64_t* nseg, Body member) {
+  if (int st = build_shards(m, nAngularLevel, rays, nrays, multi_primary(&m).nx)) return st;
+  m.step++;
+  std::vector<int> iters((size_t)m.nlocal, 1);
+  for (Member* q : m.mem) reset_call_results(q->c);
+  int st = for_each_member(m, [&](Member& q, int i) -> int {
+    RTB_CUDA(cudaSetDevice(q.c.device));
+    return member(q, i, &iters[(size_t)i]);
+  });
+  if (st) drop_stored_j(m);   // a failed solve is no starting guess, on any member
+  m.step += (unsigned long long)(iters[0] - 1);   // the ranks agree on the iteration count
+  if (nseg) *nseg = sum_nseg(m);
+  return st;
+}
+
 int multi_diffuse_resident(Multi* m, int nAngularLevel, const double* uvb, const double* beta, const double* ksi6,
                            int chemistry, void* const* streams, int64_t* nseg) {
   if (m->nleaf == 0 || !uvb || !beta) return RTB200_ERR_ARG;
-  if (int st = build_shards(*m, nAngularLevel, nullptr, 0, multi_primary(m).nx)) return st;
-  m->step++;
-  std::vector<int> iters((size_t)m->nlocal, 1);
-  for (Member* q : m->mem) q->c.lastScatIter = 0, q->c.lastScatResid = 0., q->c.scatResidPending = false, q->c.lastNgCount = 0,
-      q->c.lastWarm = false, q->c.ngPending = false, q->c.dWarmTaken = nullptr;
-  int st = for_each_member(*m, [&](Member& q, int i) -> int {
-    RTB_CUDA(cudaSetDevice(q.c.device));
+  return multi_diffuse(*m, nAngularLevel, nullptr, 0, nseg, [&](Member& q, int i, int* iters) {
     return diffuse_resident_member(*m, q, nAngularLevel, uvb, beta, ksi6, chemistry,
-                                   streams ? (cudaStream_t)streams[i] : q.c.stream, &iters[(size_t)i]);
+                                   streams ? (cudaStream_t)streams[i] : q.c.stream, iters);
   });
-  if (st) drop_stored_j(*m);   // a failed solve is no starting guess, on any member
-  m->step += (unsigned long long)(iters[0] - 1);   // the ranks agree on the iteration count
-  if (nseg) {
-    *nseg = 0;
-    for (Member* q : m->mem) *nseg += q->nsegLast;
-  }
-  return st;
 }
 
 int multi_diffuse_host(Multi* m, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays,
@@ -1125,18 +1021,12 @@ int multi_diffuse_host(Multi* m, int nAngularLevel, const double* uvb, const dou
     drop_stored_j(*m);
     return RTB200_ERR_ARG;
   }
-  if (int st = build_shards(*m, nAngularLevel, rays, nrays, multi_primary(m).nx)) return st;
-  m->step++;
-  std::vector<int> iters((size_t)m->nlocal, 1);
-  for (Member* q : m->mem) q->c.lastScatIter = 0, q->c.lastScatResid = 0., q->c.scatResidPending = false, q->c.lastNgCount = 0,
-      q->c.lastWarm = false, q->c.ngPending = false, q->c.dWarmTaken = nullptr;
-  int st = for_each_member(*m, [&](Member& q, int i) -> int {
+  return multi_diffuse(*m, nAngularLevel, rays, nrays, nseg, [&](Member& q, int, int* iters) -> int {
     Context& c = q.c;
-    RTB_CUDA(cudaSetDevice(c.device));
     const int buf = (int)(m->step & 1);
     PhaseTimer tm("diffuse", q.rank, c.stream);
     if (scatter) {
-      if (int e = scatter_member(*m, q, m->step - 1, nAngularLevel, uvb, beta, Epilogue(), c.stream, &iters[(size_t)i])) return e;
+      if (int e = scatter_member(*m, q, m->step - 1, nAngularLevel, uvb, beta, Epilogue(), c.stream, iters)) return e;
       tm.mark("source iteration");
     } else {
       if (int e = sweep_member(*m, q, buf, nAngularLevel, uvb, beta, c.stream)) return e;
@@ -1157,13 +1047,6 @@ int multi_diffuse_host(Multi* m, int nAngularLevel, const double* uvb, const dou
     tm.mark("status");
     return de;
   });
-  if (st) drop_stored_j(*m);   // a failed solve is no starting guess, on any member
-  m->step += (unsigned long long)(iters[0] - 1);   // the ranks agree on the iteration count
-  if (nseg) {
-    *nseg = 0;
-    for (Member* q : m->mem) *nseg += q->nsegLast;
-  }
-  return st;
 }
 
 // point sources of one member: its share of the source list (round robin over the ranks) into exch[buf][0..5]
@@ -1198,19 +1081,6 @@ static int point_member(Multi& m, Member& q, int buf, const PointInputs& in, std
   return RTB200_OK;
 }
 
-static void scatter_diag(const std::vector<int>& idx, const std::vector<double>& d, double* rem, double* bnd, double* dust,
-                         double* spec, int32_t* hpl) {
-  for (size_t i = 0; i < idx.size(); i++) {
-    const double* p = d.data() + i * 320;
-    const size_t s = (size_t)idx[i];
-    if (rem) memcpy(rem + s * 7, p, 56);
-    if (bnd) memcpy(bnd + s * 7, p + 7, 56);
-    if (dust) dust[s] = p[14];
-    if (hpl) hpl[s] = (int32_t)p[15];
-    if (spec) memcpy(spec + s * 300, p + 16, 2400);
-  }
-}
-
 int multi_point_host(Multi* m, const PointInputs& in, double* const k[6], double* rem, double* bnd, double* dust,
                      double* spec, int32_t* hpl, int64_t* nseg) {
   for (int i = 0; i < 6; i++)
@@ -1238,13 +1108,10 @@ int multi_point_host(Multi* m, const PointInputs& in, double* const k[6], double
       for (int f = 0; f < 6; f++)
         RTB_CUDA(cudaMemcpyAsync(k[f] + off, q.Rslab + (size_t)f * m->slab, nb, cudaMemcpyDeviceToHost, c.stream));
     RTB_CUDA(cudaStreamSynchronize(c.stream));
-    scatter_diag(idx, diag, rem, bnd, dust, spec, hpl);
+    split_diag(diag.data(), idx.size(), idx.data(), rem, bnd, dust, spec, hpl);
     return device_error(c);
   });
-  if (nseg) {
-    *nseg = 0;
-    for (Member* q : m->mem) *nseg += q->nsegLast;
-  }
+  if (nseg) *nseg = sum_nseg(*m);
   return st;
 }
 
@@ -1262,13 +1129,10 @@ int multi_point_resident(Multi* m, const PointInputs& in, void* const* streams, 
     if (int e = point_member(*m, q, buf, in, idx, diag, s)) return e;
     if (int e = reduce_member(*m, q, buf, m->step, 6, q.Rslab, Epilogue(), s)) return e;
     q.haveR = true;
-    scatter_diag(idx, diag, rem, bnd, dust, spec, hpl);
+    split_diag(diag.data(), idx.size(), idx.data(), rem, bnd, dust, spec, hpl);
     return RTB200_OK;
   });
-  if (nseg) {
-    *nseg = 0;
-    for (Member* q : m->mem) *nseg += q->nsegLast;
-  }
+  if (nseg) *nseg = sum_nseg(*m);
   return st;
 }
 
@@ -1442,10 +1306,8 @@ int rtb200_multi_point_resident(rtb200_ctx* h, int nWave, const double* waveleng
                                 double* ndotBoundary, double* ndotDust, double* ndotSpectrum, int32_t* highestPixelLevel,
                                 int64_t* nseg) {
   if (!h || !h->m) return RTB200_ERR_ARG;
-  PointInputs in;
-  in.nWave = nWave; in.wavelength = wavelength; in.lum = lum; in.metallicity = metallicity; in.coefSpectrum = coefSpectrum;
-  in.aDust = aDust; in.dust = dustApproximation; in.maxPixelLevel = maxPixelLevel; in.nsrc = nsrc; in.srcLeaf = srcLeaf;
-  in.srcWeight = srcWeight;
+  PointInputs in = make_point_inputs(nWave, wavelength, lum, metallicity, coefSpectrum, aDust, dustApproximation,
+                                     maxPixelLevel, nsrc, srcLeaf, srcWeight);
   return multi_point_resident(h->m, in, streams, ndotRemaining, ndotBoundary, ndotDust, ndotSpectrum, highestPixelLevel, nseg);
 }
 

@@ -149,18 +149,12 @@ int launch_ng_apply(const Context& c, const NgBuffers& b, int nranks, int64_t cn
   return RTB200_OK;
 }
 
-// frees the Ng history; a count the latest call left on the device is read first
-static void free_history(Context& c) {
+void free_history(Context& c) {
   if (c.ngPending) {
     if (cudaMemcpy(&c.lastNgCount, c.dNg + kNgCount, sizeof(int32_t), cudaMemcpyDeviceToHost) != cudaSuccess) c.lastNgCount = 0;
     c.ngPending = false;
   }
   cudaFree(c.dNg); c.dNg = nullptr; c.ngBytes = 0;
-}
-
-void release_acceleration(Context& c) {
-  c.scatWarm = false;
-  free_history(c);
 }
 
 int set_scattering_acceleration(Context& c, int32_t flags) {

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 
 #include <cstdint>
+#include <functional>
 #include <string>
 #include <vector>
 
@@ -156,13 +157,16 @@ struct Context {
   // uniform plan and the captured graph stay valid across the iterations and the calls
   double* dSigma = nullptr;
   double* dEtaEff = nullptr;
-  double* dScatScratch = nullptr;   // J of the previous iteration [3][nleaf] + the residual word (lazily allocated)
+  double* dScatScratch = nullptr;   // scratch of the source iteration, laid out by source_scratch (lazily allocated)
   size_t scatScratchBytes = 0;
   int32_t scatMaxIter = 1;
   double scatTol = 0;
   int32_t lastScatIter = 0;         // sweeps and last residual of the latest diffuse call
   double lastScatResid = 0;
-  bool scatResidPending = false;    // tolerance 0: the residual is still on the device (read by last_scattering)
+  // tolerance 0: the residual is still on the device, as the max of these words (the context's own residual word, or
+  // every rank's in a device group), read by last_scattering
+  const double* dScatResid = nullptr;
+  int nScatResid = 0;
   // acceleration of the source iteration (rtb200_grid_set_scattering_acceleration, ng.cu): RTB200_SCATTER_* flags
   int32_t scatAccel = 0;
   bool scatWarm = false;            // the J of the previous iteration (Jprev) is the J the latest completed solve returned
@@ -224,6 +228,9 @@ struct Context {
   double lastAlgBytes = 0;
 };
 
+// an entry of a per-leaf field the library accepts (emission, sigma, dust cross-sections): >= 0 and finite
+__host__ __device__ inline bool finite_nonneg(double v) { return v >= 0. && v <= 1.7976931348623157e308; }
+
 int ensure_buffer(void** p, size_t* have, size_t need);
 int context_init(Context& c, int device);
 void context_destroy(Context& c);
@@ -243,6 +250,8 @@ int set_scattering(Context& c, const double* sigma, bool device, int32_t maxIter
 // the diffuse call: one sweep, or the source iteration while scattering is set (a direction subset is refused then)
 int run_diffuse(Context& c, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays, int32_t nrays,
                 double* dJ, cudaStream_t s, int64_t* nseg);
+// forget the scattering results of the previous diffuse call (every diffuse call starts with it)
+void reset_call_results(Context& c);
 // one sweep of the given directions with the context's current source.  iter <= 1: opacities first (+ sigma while
 // scattering is set) and the call's timing starts; iter > 1: stats add up to the earlier sweeps of the call
 int run_sweep(Context& c, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays, int32_t nrays,
@@ -250,6 +259,25 @@ int run_sweep(Context& c, int nAngularLevel, const double* uvb, const double* be
 // scattering.cu: source iteration of a single context over the full direction set
 int scatter_solve(Context& c, int nAngularLevel, const double* uvb, const double* beta, double* dJ, cudaStream_t s,
                   int64_t* nseg);
+// The part of the grid a context iterates and the exchanges around it: the whole grid for a single context (stageStride
+// 0, hooks empty), a slab for a member of a device group.  source_iteration (scattering.cu) is the one loop for both.
+struct SourcePart {
+  int rank = 0, nranks = 1;
+  int64_t off = 0, cnt = 0;      // leaves [off, off + cnt): sigma and eta_th are read at + off
+  double* J = nullptr;           // y_k after sweep(k), [3][jStride]; Jprev and the Ng history use the same stride
+  int64_t jStride = 0;
+  std::function<int(int k, int64_t* ns)> sweep;   // sweep k with the current dEtaEff, its result in J
+  // a member of a device group: the source pass writes this rank's slice (at rank * jStride) of a stage [3][stageStride]
+  // instead of dEtaEff, share_source all-gathers the stage into every rank's dEtaEff, and allgather gathers every
+  // rank's n words at words + n * rank into every rank's words, in place
+  int64_t stageStride = 0;
+  std::function<int(double* stage)> share_source;
+  std::function<int(double* words, int n)> allgather;
+};
+int source_iteration(Context& c, const SourcePart& p, const double* beta, cudaStream_t s, int* iters, int64_t* nseg);
+// frees dEtaEff, the scratch and the Ng history and drops the stored J; results the latest call left on the device are
+// read first (scattering cleared, grid replaced)
+void release_source_iteration(Context& c);
 // eta_out[g * oStride + i] = eta_th + sigma * J, Jprev = J and the residual max |J - Jprev| / J folded into *resid (the
 // bits of a non-negative double) for i < cnt, g < 3; J and Jprev with stride jStride, sigma / eta_th (may be nullptr)
 // with stride sStride
@@ -280,7 +308,7 @@ struct NgBuffers {
 };
 int ng_buffers(Context& c, int64_t stride, NgBuffers* b);
 int set_scattering_acceleration(Context& c, int32_t flags);
-void release_acceleration(Context& c);   // drops the stored J and the Ng history (scattering cleared)
+void free_history(Context& c);   // frees the Ng history (a count the latest call left on the device is read first)
 // the five sums of this rank's cnt entries of I0..I3 (stride jStride) into b.sums[5 * rank ..]
 int launch_ng_partials(const NgBuffers& b, int64_t cnt, const double* I0, int64_t jStride, int rank, cudaStream_t s);
 // from the sums of nranks ranks: a, b and the decision; when it applies, x = max(0, (1-a-b) I0 + a I1 + b I2) into
@@ -320,6 +348,13 @@ int chemistry_run_slab(Context& c, int64_t first, int64_t count, const double* d
 // hDiag = host [nsrc][320] (remaining[7], boundary[7], dust, pad, spectrum[300]) or NULL
 int point_solve(Context& c, const PointInputs& in, double* dRates, double* hDiag, int64_t* nseg, long long* hTrace,
                 long long traceCap, long long* traceLen, double* hRawTables, cudaStream_t s);
+PointInputs make_point_inputs(int nWave, const double* wavelength, const double* lum, const double* metallicity,
+                              double coefSpectrum, const double* aDust, int dust, int maxPixelLevel, int nsrc,
+                              const int32_t* srcLeaf, const int32_t* srcWeight);
+// hDiag records of n sources into the caller's per-source arrays (any may be NULL): record i belongs to source
+// idx[i], or to source i without idx
+void split_diag(const double* d, size_t n, const int* idx, double* rem, double* bnd, double* dust, double* spec,
+                int32_t* hpl);
 
 int set_math(Context& c, int mode);
 int device_error(Context& c);
@@ -335,7 +370,6 @@ int multi_grid_set(Multi* m, int nx, int64_t nleaf, const int8_t* level, const d
 int multi_update_species(Multi* m, const double* HI, const double* HeI, const double* HeII);
 int multi_set_emission(Multi* m, const double* eta);
 int multi_set_scattering(Multi* m, const double* sigma, int32_t maxIterations, double tolerance);
-int multi_last_scattering(Multi* m, int32_t* iterations, double* residual);
 int multi_set_scattering_acceleration(Multi* m, int32_t flags);
 int multi_set_dust(Multi* m, int mode, const double* betaDust, const double* albedo, int32_t maxIterations, double tolerance);
 int multi_get_species(Multi* m, double* HI, double* HeI, double* HeII);

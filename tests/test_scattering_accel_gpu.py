@@ -268,7 +268,9 @@ def test_device_group_equals_plain_context(rt, uvbg, ndev, gname, tol):
         for scale in (1.0, 1.01):   # the second call starts warm
             t.set_scattering(sigma * scale, max_iterations=mi, tolerance=tol)
             J, n = t.diffuse(uvb, beta)
-            out.append((J, n, t.last_scattering()["iterations"], t.last_scattering_acceleration()))
+            st = t.last_stats()
+            out.append((J, n, t.last_scattering()["iterations"], t.last_scattering_acceleration(),
+                        (st["launches"], st["algorithmic_bytes"])))
         return out
 
     one = rt.Transport(device=0, math=rt.MATH_FAITHFUL)
@@ -287,10 +289,11 @@ def test_device_group_equals_plain_context(rt, uvbg, ndev, gname, tol):
             assert np.array_equal(Js, J3[:, off:off + cnt]) if ndev == 1 else rel_err(Js, J3[:, off:off + cnt]) < 1e-12
     finally:
         m.close()
-    for (Jr, nr, ir, ar), (Jg, ng, ig, ag) in zip(ref, got):
+    for (Jr, nr, ir, ar, sr), (Jg, ng, ig, ag, sg) in zip(ref, got):
         print(f"group of {ndev} {gname} tol {tol}: {ig} sweeps {ag} (single {ir} {ar}), err {rel_err(Jg, Jr):.3e}")
         assert nr == ng and ir == ig and ar == ag
         assert np.array_equal(Jg, Jr) if ndev == 1 else rel_err(Jg, Jr) < 1e-12
+        assert sg == sr or ndev > 1   # launches and algorithmic bytes: the same bookkeeping of the source iteration
     assert ref[1][3]["warm_start"] and (tol == 0 or ref[1][2] < ref[0][2])
 
 
