@@ -113,7 +113,7 @@ int rtb200_set_math(rtb200_ctx* ctx, int math_mode);
 /* Launch tuning knobs; results do not depend on them (tests/test_diffuse_gpu.py, test_point_gpu.py).  Keys:
  *   uniform sweep  "slots" (zone tasks per launch, 0 = all), "graph" (CUDA graph replay, 1), "dirs_per_task" (0 = chosen
  *                  from a wave model), "cells" (cells of a layer per thread: 1, 2, or 0 = by grid size and zone tasks per
- *                  launch; an emissive sweep always runs one-cell threads), "block_warps" (rows per block 8 / 4 / 2,
+ *                  launch; an emissive sweep always runs one-cell threads), "block_warps" (warps per block 8 / 4 / 2,
  *                  0 = by the number of blocks a launch has), "transpose_z" (z-major copy for
  *                  the zones sweeping along the contiguous axis, 1), "pdl" (programmatic dependent launch of layer
  *                  l+1 on layer l, also used by the nested-grid waves, 1), "l2_mb"

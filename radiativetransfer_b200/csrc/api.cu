@@ -20,14 +20,15 @@ __global__ void portable_math_kernel(const double* __restrict__ x, int64_t n, do
   }
 }
 
-// the sweeps' FAST exponential (segment_math.cuh: table + short polynomial) for n host values: e^-tau and 1 - e^-tau
+// the sweeps' FAST exponential (segment_math.cuh: table + short polynomial) for n host values: e^-tau and 1 - e^-tau,
+// evaluated as the sweeps do with kappa = tau and the scaled path of a unit length, kExpScale
 __global__ void fast_exp_kernel(const double* __restrict__ tau, int64_t n, double* __restrict__ e, double* __restrict__ ome) {
   __shared__ double sT[kExpTableSize];
   if (threadIdx.x < kExpTableSize) sT[threadIdx.x] = kExpTable32[threadIdx.x];
   __syncthreads();
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     double Ts, p;
-    exp_neg_parts32<true>(tau[i], sT, Ts, p);
+    exp_neg_parts32<true>(tau[i], kExpScale, sT, Ts, p);
     e[i] = fma(Ts, p, Ts);
     ome[i] = fma(-Ts, p, 1.0 - Ts);
   }

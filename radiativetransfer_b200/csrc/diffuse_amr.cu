@@ -468,11 +468,12 @@ __device__ __forceinline__ bool amr_transport_leaf(const AmrParams& P, const Amr
       for (int g = 0; g < 3; g++) { out[g] = t.out[g]; Jthin[g] = __dadd_rn(Jthin[g], t.J[g]); }
     } else {
       const double cs = pat.cs[ray][lane];
+      const double ds = dpath[ray] * kExpScale;   // the exponential's scaled path, once for the three groups
 #pragma unroll
       for (int g = 0; g < 3; g++)
-        out[g] = EMIT ? segment_fast_emit<true>(Iin[ray][g], kap[g] * dpath[ray], cs, sT, Jm[g], eta[g], invk[g],
-                                                dpath[ray], dpath[ray] * wn, E[g])
-                      : segment_fast<true>(Iin[ray][g], kap[g] * dpath[ray], cs, sT, Jm[g]);
+        out[g] = EMIT ? segment_fast_emit<true>(Iin[ray][g], kap[g], ds, cs, sT, Jm[g], eta[g], invk[g], dpath[ray],
+                                                dpath[ray] * wn, E[g])
+                      : segment_fast<true>(Iin[ray][g], kap[g], ds, cs, sT, Jm[g]);
     }
     if (ray == 0) { xy[0] = out[0]; xy[1] = out[1]; xy[2] = out[2]; }
     imean++;

@@ -8,9 +8,10 @@
 //    cell per zone instead of one per direction.
 //  * Within a layer every cell carries the same 1..3 segments (its "pattern"); a characteristic that leaves a
 //    cell sideways continues in the k+1 and/or j+1 neighbour of the SAME layer.  Along the lane axis that hand-over
-//    is a warp shuffle of the neighbour lane's own result (a warp covers 31 cells + 1 recomputed halo cell); along
-//    the row axis the thread recomputes what the (b-1) cell emits from the previous layer's plane value and that
-//    cell's kappa.  No shared-memory exchange, no barrier in the loop, no inter-block communication.
+//    is a warp shuffle of the neighbour lane's own result (a warp covers 31 positions + 1 recomputed halo, and the
+//    positions of a layer run end to end across rows and warps: lane_position); along the row axis the thread
+//    recomputes what the (b-1) cell emits from the previous layer's plane value and that cell's kappa.  No
+//    shared-memory exchange, no barrier in the loop, no inter-block communication.
 //  * The only inter-layer state is the intensity leaving each cell through its top face: one padded plane of
 //    3 doubles per cell per direction ([row][column][group]), ping-ponged in global memory.
 //  * One launch per layer covers every zone task of the batch (gridDim.z); each task owns a private J accumulator
@@ -99,17 +100,20 @@ struct Em {
   double invk[3], invkR[3];  // FAST arithmetic: 1 / kappa with kappa floored as in the segment
 };
 
+// `d` is the layer table's path: the scaled path d * kExpScale for the plain sweep, the path itself for the emissive one
+// (emission needs tau = kappa d; the scaled path is formed here, as the same product the host forms for the plain
+// sweep, so that eta = 0 reproduces it bit for bit).  See fill_step_segs.
 template <bool GUARD, bool EMIT>
 __device__ __forceinline__ double seg_fast(double Iin, double kap, double d, double cs, const double* __restrict__ T,
                                            double& A, double eta, double invk, double dw, double& E) {
-  if (EMIT) return segment_fast_emit<GUARD>(Iin, kap * d, cs, T, A, eta, invk, d, dw, E);
-  return segment_fast<GUARD>(Iin, kap * d, cs, T, A);
+  if (EMIT) return segment_fast_emit<GUARD>(Iin, kap, d * kExpScale, cs, T, A, eta, invk, d, dw, E);
+  return segment_fast<GUARD>(Iin, kap, d, cs, T, A);
 }
 template <bool GUARD, bool EMIT>
 __device__ __forceinline__ double att_fast(double Iin, double kap, double d, const double* __restrict__ T, double eta,
                                            double invk) {
-  if (EMIT) return attenuate_fast_emit<GUARD>(Iin, kap * d, T, eta, invk, d);
-  return attenuate_fast<GUARD>(Iin, kap * d, T);
+  if (EMIT) return attenuate_fast_emit<GUARD>(Iin, kap, d * kExpScale, T, eta, invk, d);
+  return attenuate_fast<GUARD>(Iin, kap, d, T);
 }
 
 template <int NSEG, bool SECL, bool GUARD, bool EMIT = false>
@@ -289,8 +293,38 @@ __device__ __forceinline__ void prefetch_l1(const double* p) { asm volatile("pre
 constexpr double kKappaFloor = 1e-100;  // FAST mode: kappa = 0 is evaluated as this (every formula takes its limit)
 constexpr double kTwoM200 = 6.223015277861141707e-61;  // 2^-200
 
-// block = 8 warps; a warp covers 31 cells of one row plus, in lane 0, the recomputed last cell of the strip to its
-// left (for strip 0 that is the pad column, which behaves as "no neighbour").
+// Lanes and cells.  Per task and layer the positions q = 0 .. R (n+1) - 1 run over R rows (row pairs for two-cell
+// threads) of n + 1 columns: row r = q / (n+1), column a = q mod (n+1) - 1, where a = -1 is the pad column (plane
+// value = boundary intensity, kappa = 0: "no neighbour").  Warp w, lane L takes q = 31 w + L, so the positions run end
+// to end across rows and warps and no lane idles past a row's end:
+//  * lane 0 is a halo: it recomputes the position that lane 31 of warp w - 1 writes, or a pad;
+//  * the writers are lanes 1..31 at a real cell (a >= 0);
+//  * lanes past the last position evaluate the last row's pad and only take part in the shuffles.
+// Invariant that makes this correct without a per-lane select after a shuffle: every value a lane takes from lane - 1
+// is of depth 1 -- the neighbour's xy-segment output (a1 / b1 / I1) or its recomputed (b-1) output (rup, or a2 / I2
+// fed by rup), each a function of the neighbour's OWN plane values and opacities only, never of a shuffled value.  So
+// a halo or pad lane whose own shuffled inputs are garbage (the end of the previous row, or a pad in mid-warp at the
+// start of a row) still hands over exactly what the cell to its right needs.  The per-cell arithmetic and the
+// summation order do not depend on where a cell sits in a warp; only the warp-wide guard vote does, and the guarded
+// and unguarded exponentials agree bit for bit where the vote lets a warp skip the guard (segment_math.cuh).
+struct LanePos {
+  int a, r;       // column (-1 = pad) and row (pair) of this lane's position
+  bool warpLive;  // warp-uniform: the warp holds at least one writer
+};
+__device__ __forceinline__ LanePos lane_position(int rows, int np1) {
+  const int P = rows * np1;                                   // positions per task and layer
+  const int w = blockIdx.x * blockDim.y + threadIdx.y;
+  LanePos lp;
+  lp.warpLive = 31 * w < P - 1;
+  int q = 31 * w + (int)threadIdx.x;
+  if (q >= P) q = P - np1;                                    // past the end: the last row's pad
+  lp.r = q / np1;
+  lp.a = q - lp.r * np1 - 1;
+  return lp;
+}
+// warps per task and layer (host side of lane_position)
+static inline int warps_per_layer(int n, int rows) { return (rows * (n + 1) - 2) / 31 + 1; }
+
 constexpr int kMaxBatch = 40;  // tasks per launch: 40 x 728 B of parameters (the limit is 32764 B since CUDA 12.1)
 struct BatchParams {
   StepParams t[kMaxBatch];
@@ -323,11 +357,11 @@ __device__ __forceinline__ void sweep_cell_body(const BatchParams& bp, const dou
   asm volatile("griddepcontrol.launch_dependents;");
   if (threadIdx.y * 32 + threadIdx.x < kExpTableSize) sT[threadIdx.y * 32 + threadIdx.x] = kExpTable32[threadIdx.y * 32 + threadIdx.x];
   __syncthreads();
-  const int a = blockIdx.x * 31 - 1 + (int)threadIdx.x, b = blockIdx.y * blockDim.y + threadIdx.y;
-  if (b >= n) return;                                          // warp-uniform
-  const bool inRow = a < n;                                    // lanes beyond the row only take part in the shuffles
-  const bool writer = inRow && threadIdx.x >= 1;
-  const bool cell = inRow && a >= 0;                           // a real cell (not the pad column)
+  const LanePos lp = lane_position(n, np1);
+  if (!lp.warpLive) return;                                    // warp-uniform
+  const int a = lp.a, b = lp.r;
+  const bool cell = a >= 0;                                    // a real cell (not the pad column)
+  const bool writer = cell && threadIdx.x >= 1;
   const int laneIsK = sp.laneIsK;
   const int sA = laneIsK ? sp.sk : sp.sj, sB = laneIsK ? sp.sj : sp.sk;
   const int leaf = sp.origin + a * sA + b * sB;
@@ -353,7 +387,7 @@ __device__ __forceinline__ void sweep_cell_body(const BatchParams& bp, const dou
       em.invkR[g] = FAITHFUL ? 0. : 1.0 / (kR[g] > 0. ? kR[g] : kKappaFloor);   // as the (b-1) cell's own thread
     }
   }
-  const int pidx = (b + 1) * np1 + (inRow ? a + 1 : 0);
+  const int pidx = (b + 1) * np1 + a + 1;
   const int ndir = sp.ndir;
   const int dstride = npl3;                                    // one direction's plane (3 groups per cell)
   const int up = 3 * np1;                                      // one row up
@@ -430,29 +464,29 @@ __device__ __forceinline__ void direction_fast2(const LayerSeg& P, const double 
   const unsigned full = 0xffffffffu;
 #pragma unroll
   for (int g = 0; g < 3; g++) {
-    const double a1 = segment_fast<GUARD>(cur0[g], kap0[g] * P.d[0], P.cs[0], T, A0[g]);
-    const double b1 = segment_fast<GUARD>(cur1[g], kap1[g] * P.d[0], P.cs[0], T, A1[g]);
+    const double a1 = segment_fast<GUARD>(cur0[g], kap0[g], P.d[0], P.cs[0], T, A0[g]);
+    const double b1 = segment_fast<GUARD>(cur1[g], kap1[g], P.d[0], P.cs[0], T, A1[g]);
     I0[g] = a1; I1[g] = b1;
     if (NSEG >= 2) {
       double rup = 0.;  // xy-segment output of the (b0 - 1) cell, recomputed (lower cell only)
-      if (!SECL || NSEG == 3) rup = attenuate_fast<GUARD>(upR[g], kR[g] * P.d[0], T);
+      if (!SECL || NSEG == 3) rup = attenuate_fast<GUARD>(upR[g], kR[g], P.d[0], T);
       const double a_in2 = SECL ? __shfl_up_sync(full, a1, 1) : rup;
       const double b_in2 = SECL ? __shfl_up_sync(full, b1, 1) : a1;   // the lower cell's own xy output
-      const double a2 = segment_fast<GUARD>(a_in2, kap0[g] * P.d[1], P.cs[1], T, A0[g]);
-      const double b2 = segment_fast<GUARD>(b_in2, kap1[g] * P.d[1], P.cs[1], T, A1[g]);
+      const double a2 = segment_fast<GUARD>(a_in2, kap0[g], P.d[1], P.cs[1], T, A0[g]);
+      const double b2 = segment_fast<GUARD>(b_in2, kap1[g], P.d[1], P.cs[1], T, A1[g]);
       I0[g] = a2; I1[g] = b2;
       if (NSEG == 3) {
         double a_in3, b_in3;
         if (SECL) {
           const double x = __shfl_up_sync(full, rup, 1);
-          a_in3 = attenuate_fast<GUARD>(x, kR[g] * P.d[1], T);
+          a_in3 = attenuate_fast<GUARD>(x, kR[g], P.d[1], T);
           b_in3 = a2;                                                 // the lower cell's second segment
         } else {
           a_in3 = __shfl_up_sync(full, a2, 1);
           b_in3 = __shfl_up_sync(full, b2, 1);
         }
-        I0[g] = segment_fast<GUARD>(a_in3, kap0[g] * P.d[2], P.cs[2], T, A0[g]);
-        I1[g] = segment_fast<GUARD>(b_in3, kap1[g] * P.d[2], P.cs[2], T, A1[g]);
+        I0[g] = segment_fast<GUARD>(a_in3, kap0[g], P.d[2], P.cs[2], T, A0[g]);
+        I1[g] = segment_fast<GUARD>(b_in3, kap1[g], P.d[2], P.cs[2], T, A1[g]);
       }
     }
   }
@@ -475,8 +509,8 @@ __device__ __forceinline__ void direction_kinds_fast2(const LayerSeg& P, bool se
   }
 }
 
-// block = 8 warps; a warp covers 31 cells (+ the recomputed halo cell in lane 0) of TWO rows.  Register budget: 2 blocks of
-// 256 threads per SM (124 registers, no spills; as many cells in flight as the one-cell kernel at 4 blocks).
+// Positions are row pairs (see lane_position): a lane holds the cell (a, b0) and the one above it.  Register budget: 2
+// blocks of 256 threads per SM (124 registers, no spills; as many cells in flight as the one-cell kernel at 4 blocks).
 __global__ void __launch_bounds__(256, 2)
 sweep_cell2_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1, int npl3) {
   const StepParams& sp = bp.t[blockIdx.z];
@@ -485,12 +519,12 @@ sweep_cell2_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1
   asm volatile("griddepcontrol.launch_dependents;");
   if (threadIdx.y * 32 + threadIdx.x < kExpTableSize) sT[threadIdx.y * 32 + threadIdx.x] = kExpTable32[threadIdx.y * 32 + threadIdx.x];
   __syncthreads();
-  const int a = blockIdx.x * 31 - 1 + (int)threadIdx.x, b0 = 2 * (blockIdx.y * blockDim.y + threadIdx.y);
-  if (b0 >= n) return;                                         // warp-uniform
-  const bool row1 = b0 + 1 < n;                                // warp-uniform: the upper row exists
-  const bool inRow = a < n;
-  const bool writer0 = inRow && threadIdx.x >= 1, writer1 = writer0 && row1;
-  const bool cell0 = inRow && a >= 0, cell1 = cell0 && row1;
+  const LanePos lp = lane_position((n + 1) / 2, np1);
+  if (!lp.warpLive) return;                                    // warp-uniform
+  const int a = lp.a, b0 = 2 * lp.r;
+  const bool row1 = b0 + 1 < n;                                // the upper row exists (not in the last pair of odd n)
+  const bool cell0 = a >= 0, cell1 = cell0 && row1;
+  const bool writer0 = cell0 && threadIdx.x >= 1, writer1 = writer0 && row1;
   const int laneIsK = sp.laneIsK;
   const int sA = laneIsK ? sp.sk : sp.sj, sB = laneIsK ? sp.sj : sp.sk;
   const int leaf0 = sp.origin + a * sA + b0 * sB;
@@ -507,7 +541,7 @@ sweep_cell2_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1
   const double kmax = fmax(fmax(fmax(fmax(kap0[0], kap0[1]), fmax(kap0[2], kR[0])), fmax(kR[1], kR[2])),
                            fmax(fmax(kap1[0], kap1[1]), kap1[2]));
   double A0[3] = {0., 0., 0.}, A1[3] = {0., 0., 0.}, acc0[3] = {0., 0., 0.}, acc1[3] = {0., 0., 0.};
-  const int pidx = (b0 + 1) * np1 + (inRow ? a + 1 : 0);
+  const int pidx = (b0 + 1) * np1 + a + 1;
   const int ndir = sp.ndir;
   const int dstride = npl3;
   const int up = 3 * np1;                                      // one row up in the plane
@@ -656,6 +690,17 @@ int launch_diffuse_rates(Context& c, const double* J, const double* ksi24, const
 // 0.2% of the (direction, layer) pairs take this branch.
 constexpr double kThinLen = 1e-3;
 
+// The layer table a launch reads.  The plan holds the paths d; the FAST layers of the plain sweep read the scaled path
+// d * kExpScale that their exponential takes (segment_math.cuh, exp_neg_parts32), in the same slots.  Thin layers
+// (the reference's operation sequence), FAITHFUL mode and the emissive sweep read d.
+static void fill_step_segs(LayerSeg* P, const LayerSeg* plan, int ndir, bool scaled) {
+  for (int q = 0; q < ndir; q++) {
+    P[q] = plan[q];
+    if (scaled && !P[q].thin)
+      for (int s = 0; s < 3; s++) P[q].d[s] = plan[q].d[s] * kExpScale;
+  }
+}
+
 static LayerSeg make_layer_seg(const RayPattern& p, double cellSize, double weight) {
   LayerSeg L;
   std::memset(&L, 0, sizeof(L));
@@ -687,9 +732,8 @@ static LayerSeg make_layer_seg(const RayPattern& p, double cellSize, double weig
 }
 
 
-// `warps` = rows of the layer a block covers with one warp each (8, 4 or 2): small direction shards (multi-GPU ranks) put
-// only a few hundred 8-warp blocks on the device per layer, 1.5 "waves" of which cost as much as 2; smaller blocks
-// spread the same rows evenly over the SMs
+// `warps` = warps per block (8, 4 or 2): small direction shards (multi-GPU ranks) put only a few hundred 8-warp blocks on
+// the device per layer, 1.5 "waves" of which cost as much as 2; smaller blocks spread the same warps evenly over the SMs
 template <class Kernel, class... Extra>
 static cudaError_t launch_layer(Kernel kern, dim3 grid, cudaStream_t s, bool pdl, const BatchParams& bp, int N, int n,
                                 int warps, const Extra&... extra) {
@@ -716,14 +760,15 @@ static cudaError_t launch_cells(bool faithful, bool pdl, dim3 grid, cudaStream_t
   // (measured on the shards of an 8-GPU run: 7.03 against 7.21 ms mean, 7.31 against 7.93 ms for the slowest rank)
   if (cells == 0) cells = (n >= 192 && grid.z >= 6) ? 2 : 1;
   if (faithful || ep) cells = 1;
-  const int rowsTotal = cells == 2 ? (n + 1) / 2 : n;           // rows of threads per task and layer
+  const int wpl = warps_per_layer(n, cells == 2 ? (n + 1) / 2 : n);   // warps per task and layer
   if (warps != 8 && warps != 4 && warps != 2) {
     // automatic: the largest block that still gives the device ~6 blocks per resident 8-warp slot
     const long long slots = (long long)smCount * (cells == 2 ? 2 : 4);
     warps = 8;
-    while (warps > 2 && (long long)grid.x * ((rowsTotal + warps - 1) / warps) * grid.z < 6 * slots) warps /= 2;
+    while (warps > 2 && (long long)((wpl + warps - 1) / warps) * grid.z < 6 * slots) warps /= 2;
   }
-  grid.y = (unsigned)((rowsTotal + warps - 1) / warps);
+  grid.x = (unsigned)((wpl + warps - 1) / warps);
+  grid.y = 1;
   if (ep) {
     if (faithful) return launch_layer(sweep_cell_emit_kernel<true>, grid, s, pdl, bp, N, n, warps, *ep);
     return launch_layer(sweep_cell_emit_kernel<false>, grid, s, pdl, bp, N, n, warps, *ep);
@@ -766,7 +811,7 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
     if (c.tune.dirsPerTask <= 0) {
       int perZone[25] = {0};
       for (int d = 0; d < ndir; d++) perZone[dirs[d].izone]++;
-      const int64_t bpt = (int64_t)((n + 30) / 31) * ((n + 7) / 8);
+      const int64_t bpt = (warps_per_layer(n, n) + 7) / 8;   // one-cell threads, 8-warp blocks
       const int64_t cap = (int64_t)c.smCount * 4;   // resident blocks: 4 per SM (sweep_cell_kernel's register budget)
       double best = 1e300;
       for (int d = kMaxDirPerTask; d >= 2; d--) {
@@ -872,7 +917,7 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
 
   if (int st = ensure_buffer((void**)&c.dAcc, &c.accBytes, (size_t)c.uniSlots * 3 * N * sizeof(double))) return st;
   if (int st = ensure_buffer((void**)&c.dPlanes, &c.planeBytes, (size_t)2 * std::max(ndir, 1) * 3 * npl * sizeof(double))) return st;
-  dim3 grid((n + 30) / 31, (n + 7) / 8, 1);
+  dim3 grid(1, 1, 1);                                        // launch_cells sizes x; z = tasks of the batch
   double* planeA = c.dPlanes;
   double* planeB = c.dPlanes + (size_t)ndir * 3 * npl;
   const bool faithful = c.mathMode == RTB200_MATH_FAITHFUL;
@@ -901,7 +946,7 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
       sp.planeIn = ((step & 1) ? planeA : planeB) + (size_t)T.planeFirst * 3 * npl;
       sp.planeOut = ((step & 1) ? planeB : planeA) + (size_t)T.planeFirst * 3 * npl;
       sp.origin = (int32_t)(T.origin + step * T.si);
-      for (int q = 0; q < T.ndir; q++) sp.P[q] = T.seg[(size_t)step * kMaxDirPerTask + q];
+      fill_step_segs(sp.P, &T.seg[(size_t)step * kMaxDirPerTask], T.ndir, !faithful && !emit);
       sp.ndir = T.ndir;
       sp.firstInSlot = first;
       return T.ndir;

@@ -34,7 +34,8 @@ const char* last_cuda_error();
 // The second segment of kinds 1,2 (a yz ray) is fed by the cell at k-1, of kinds 3,4 (an xz ray) by the cell at
 // j-1; the third segment by the other one.
 struct LayerSeg {
-  double d[3];     // path length [cm]: cellSize * len
+  double d[3];     // path length [cm]: cellSize * len (a FAST launch of the plain uniform sweep reads d * kExpScale
+                   // in non-thin layers: diffuse_uniform.cu, fill_step_segs)
   double cs[3];    // fast mode: 2^200 * (weight / nseg) / d   (segment_math.cuh, segment_fast)
   double dmax;     // longest segment of the layer [cm] (fast mode: decides whether the overflow guards can be skipped)
   double w;        // weight          (faithful mode divides by nseg first, transportRoutinesModule.f90:953)
@@ -76,7 +77,7 @@ struct Tuning {
   int amrBatch = 0;      // directions per AMR batch (0 = as many as fit in half of the free memory)
   double l2BudgetMB = 96.0;
   int pdl = 1;           // uniform sweep: programmatic dependent launch of layer l+1 on layer l (its prologue overlaps the tail)
-  int blockWarps = 0;    // uniform sweep: rows (warps) per block: 8, 4, 2, or 0 = chosen from the number of blocks per launch
+  int blockWarps = 0;    // uniform sweep: warps per block: 8, 4, 2, or 0 = chosen from the number of blocks per launch
   int cells = 0;         // uniform sweep, FAST arithmetic: cells of a layer per thread (2: two rows per warp, see
                          // sweep_cell2_kernel; 0 = 2 from n = 192 on, where it measured 1-2% faster, else 1: 6% faster at 128^3)
   int transposeZ = 1;    // uniform sweep: zones sweeping along the contiguous axis use a z-major copy of kappa / J

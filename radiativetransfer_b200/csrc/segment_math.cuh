@@ -72,16 +72,31 @@ __device__ __forceinline__ void exp_neg_parts(double tau, const double* __restri
 // Measured at 256^3 on one box, 20 solves back to back under the power cap: 16 entries / r^7 53.8 ms, 32 / r^5
 // 50.7 ms, 64 / r^4 49.8 ms (the 4-way bank conflicts of the larger table cost less than the DFMA saves).
 // (The point-source kernels keep the 16-entry / r^7 version above: their deposits are differences of exponentials.)
+//
+// Round 3: the path length is folded into the range reduction.  The caller passes kappa and the SCALED path
+// d' = d * 64/ln2 (kExpScale: a per-(layer, direction, segment) constant from the host), and the reduction works in
+// units of ln2/64:
+//   t = fma(kappa, d', M),  k = round(kappa d') in t's low word,  r' = fma(kappa, d', -(t - M)) = kappa d' - k
+// with ONE rounding (|r'| <= 1/2), and p = e^(-r' ln2/64) - 1 = r' (a1 + r' (a2 + r' (a3 + r' a4))),
+// a_i = (-ln2/64)^i / i!.  7 FP64 instructions instead of 9 (tau = kappa d and a two-constant Cody-Waite reduction):
+// a segment update takes 12, a recomputed attenuation 9.  fl(64/ln2) is off by -1.4e-17 relative; over
+// 1e-12 <= tau <= 630 the largest relative error is 4.7e-14 on e^-tau and 7.2e-12 on 1 - e^-tau (the truncation bound
+// above), and tau = 0 gives exactly 1 and 0.
 constexpr int kExpTableSize = 64;   // |r| <= ln2/128, polynomial through r^4
-static __constant__ double kExpC32[12] = {
-    0., 4.16666666666666666667e-02, -1.66666666666666666667e-01, 0.5, -1.0,
-    92.33248261689366,            // [5]  64/ln2
-    6755399441055744.0,
-    -0.010830424493178725,        // [7]  -ln2/64 hi
-    -2.030704202170295e-10,       // [8]  -ln2/64 lo
-    0., 0., 0.};
-constexpr int kExpDeg = 3;
+constexpr double kExpScale = 92.33248261689366;   // 64/ln2 (host and device)
+static __constant__ double kExpC32[5] = {
+    5.732851688640402e-10,        // [0] a4 = (ln2/64)^4 / 24
+    -2.1173137155464776e-07,      // [1] a3
+    5.86490495505617e-05,         // [2] a2
+    -0.010830424696249145,        // [3] a1 = -ln2/64
+    6755399441055744.0};          // [4] 1.5 * 2^52: adding it rounds to nearest integer
 constexpr int kExpShift = 6;
+// GUARD: kappa d' is clamped at 65279 (~ tau = 707, the 16-entry version's clamp), where 2^-(k>>6) still leaves
+// Ts = 2^(-k/64) a normal number; beyond it k = 65279 and r' = 0.  The test is one integer compare on the high word of
+// kappa d' (0x40EFDFE0 = 65279.0), and below the clamp the two FMAs are the unguarded body's, so the guarded and
+// unguarded forms give the same bits wherever kappa d <= 64 (the warp vote in the sweeps relies on that).
+constexpr int kExpClampHi = 0x40EFDFE0;
+constexpr int kExpClampK = 65279;
 static __constant__ double kExpTable32[64] = {
     1.00000000000000000000e+00, 9.89228013193975463935e-01, 9.78572062087700089705e-01, 9.68030896746147173637e-01,
     9.57603280698573700036e-01, 9.47287990793482803653e-01, 9.37083817055149981279e-01, 9.26989562541692735387e-01,
@@ -100,19 +115,23 @@ static __constant__ double kExpTable32[64] = {
     5.45253866332628844837e-01, 5.39380398878559930154e-01, 5.33570200338411848584e-01, 5.27822589180278578525e-01,
     5.22136891213706877402e-01, 5.16512439510614207450e-01, 5.10948574327058313571e-01, 5.05444643025850237628e-01};
 
+// e^-(kappa d) from kappa >= 0 and ds = d * kExpScale > 0; Ts and p as for exp_neg_parts
 template <bool GUARD = true>
-__device__ __forceinline__ void exp_neg_parts32(double tau, const double* __restrict__ T, double& Ts, double& p) {
-  if (GUARD) tau = __hiloint2double(min(__double2hiint(tau), 0x40861800), __double2loint(tau));
-  double t = fma(tau, kExpC32[5], kExpC32[6]);
+__device__ __forceinline__ void exp_neg_parts32(double kappa, double ds, const double* __restrict__ T, double& Ts,
+                                                double& p) {
+  const double t = fma(kappa, ds, kExpC32[4]);
   int k = __double2loint(t);
-  double fn = t - kExpC32[6];
-  double r = fma(fn, kExpC32[7], tau);
-  r = fma(fn, kExpC32[8], r);
-  double q = kExpC32[4 - kExpDeg];
+  double r = fma(kappa, ds, -(t - kExpC32[4]));
+  if (GUARD) {
+    const bool clamp = __double2hiint(kappa * ds) > kExpClampHi;
+    k = clamp ? kExpClampK : k;
+    r = clamp ? 0. : r;
+  }
+  double q = kExpC32[0];
 #pragma unroll
-  for (int i = 5 - kExpDeg; i <= 4; i++) q = fma(q, r, kExpC32[i]);
+  for (int i = 1; i <= 3; i++) q = fma(q, r, kExpC32[i]);
   p = q * r;
-  double Tj = T[k & (kExpTableSize - 1)];
+  const double Tj = T[k & (kExpTableSize - 1)];
   Ts = __hiloint2double(__double2hiint(Tj) - ((k >> kExpShift) << 20), __double2loint(Tj));
 }
 
@@ -122,14 +141,15 @@ __device__ __forceinline__ void exp_neg_parts32(double tau, const double* __rest
 // the caller applies ONCE per layer to the sum A over all directions and segments (the power of two keeps every
 // intermediate far from the subnormal range, including the kappa -> 0 limit).  With Ts = 2^(-k/16), p = e^-r - 1:
 //   X = Iin Ts,  Iout = X + X p,  Iin (1 - e^-tau) = (Iin - X) - X p      (Iin - X is exact for k = 0: no cancellation)
-// 5 FP64 instructions after the exponential's 12, instead of 8.
+// kappa and ds = d * kExpScale enter the exponential directly; with its 7 FP64 instructions a segment update is 12.
 // GUARD = false (tau <= 64 for every segment of the warp): no clamp, and no test for Iout underflowing to 0 -- with
 // tau <= 64 that can only happen where Iin < 5e-324 e^64 = 3e-296, i.e. where the segment's contribution to Jmean
 // (< Iin) is itself below every tolerance floor (the parity tests compare with a floor of 1e-290).
 template <bool GUARD = true>
-__device__ __forceinline__ double segment_fast(double Iin, double tau, double cs, const double* __restrict__ T, double& A) {
+__device__ __forceinline__ double segment_fast(double Iin, double kappa, double ds, double cs, const double* __restrict__ T,
+                                               double& A) {
   double Ts, p;
-  exp_neg_parts32<GUARD>(tau, T, Ts, p);
+  exp_neg_parts32<GUARD>(kappa, ds, T, Ts, p);
   const double X = Iin * Ts;
   const double Iout = fma(X, p, X);
   const double Z = fma(-X, p, Iin - X);
@@ -139,9 +159,9 @@ __device__ __forceinline__ double segment_fast(double Iin, double tau, double cs
 }
 
 template <bool GUARD = true>
-__device__ __forceinline__ double attenuate_fast(double Iin, double tau, const double* __restrict__ T) {
+__device__ __forceinline__ double attenuate_fast(double Iin, double kappa, double ds, const double* __restrict__ T) {
   double Ts, p;
-  exp_neg_parts32<GUARD>(tau, T, Ts, p);
+  exp_neg_parts32<GUARD>(kappa, ds, T, Ts, p);
   const double X = Iin * Ts;
   return fma(X, p, X);
 }
@@ -186,11 +206,14 @@ __device__ __forceinline__ double emission_t(double tau, double ome, double invk
 
 // FAST-mode segment with emission: as segment_fast, plus E += phi(tau) * dw (dw = dpath * weight / nseg; the caller
 // adds eta * E to the cell's sum once per layer) and the emitted part of Iout.  invk = 1 / kappa (kappa floored).
+// The attenuation is segment_fast's (the same exponential of kappa and ds); tau = kappa d is formed here only for phi
+// and the small-tau test of the emitted part, so eta = 0 reproduces segment_fast bit for bit.
 template <bool GUARD = true>
-__device__ __forceinline__ double segment_fast_emit(double Iin, double tau, double cs, const double* __restrict__ T, double& A,
-                                                    double eta, double invk, double d, double dw, double& E) {
+__device__ __forceinline__ double segment_fast_emit(double Iin, double kappa, double ds, double cs, const double* __restrict__ T,
+                                                    double& A, double eta, double invk, double d, double dw, double& E) {
   double Ts, p;
-  exp_neg_parts32<GUARD>(tau, T, Ts, p);
+  exp_neg_parts32<GUARD>(kappa, ds, T, Ts, p);
+  const double tau = kappa * d;
   const double X = Iin * Ts;
   const double Iatt = fma(X, p, X);
   const double Z = fma(-X, p, Iin - X);
@@ -202,10 +225,11 @@ __device__ __forceinline__ double segment_fast_emit(double Iin, double tau, doub
 
 // the outgoing intensity alone, bit for bit what segment_fast_emit returns for the same arguments
 template <bool GUARD = true>
-__device__ __forceinline__ double attenuate_fast_emit(double Iin, double tau, const double* __restrict__ T, double eta,
-                                                      double invk, double d) {
+__device__ __forceinline__ double attenuate_fast_emit(double Iin, double kappa, double ds, const double* __restrict__ T,
+                                                      double eta, double invk, double d) {
   double Ts, p;
-  exp_neg_parts32<GUARD>(tau, T, Ts, p);
+  exp_neg_parts32<GUARD>(kappa, ds, T, Ts, p);
+  const double tau = kappa * d;
   const double X = Iin * Ts;
   const double Iatt = fma(X, p, X);
   const double ome = fma(-Ts, p, 1.0 - Ts);
