@@ -250,6 +250,40 @@ int rtb200_grid_set_dust(rtb200_ctx* ctx, int dustApproximation, const double* b
 int rtb200_grid_set_scattering_acceleration(rtb200_ctx* ctx, int32_t flags);
 int rtb200_last_scattering_acceleration(rtb200_ctx* ctx, int32_t* extrapolations, int32_t* warmStarted);
 
+/* Photo-heating and dust absorption of the diffuse field (an extension without a reference value, DESIGN.md 4.10).
+ * While heating is set, every diffuse call ends with one pass over the J it returns (for a scattering solve the J of
+ * the last sweep) that fills five per-leaf fields [5][nleaf] in leaf order.  With t_g = fourPi * J_g (fourPi = 4 * pi
+ * as in the diffuse photo-rates) and every operation rounded on its own (no FMA):
+ *   f = 0, 1, 2  Gamma_s = ((t_1 * gamma[1][s]) + (t_2 * gamma[2][s])) + (t_3 * gamma[3][s])   photo-heating per
+ *                absorber HI, HeI, HeII [erg/s]; gamma[g][s] = gammaHI, gammaHeI, gammaHeII of group g (table57)
+ *   f = 3        H_gas  = ((HI * Gamma_HI) + (HeI * Gamma_HeI)) + (HeII * Gamma_HeII)   [erg/s/cm^3], with the
+ *                species the call's sweep used (a resident call with chemistry: those before chemistry)
+ *   f = 4        H_dust = (u_1 + u_2) + u_3,  u_g = ((1 - albedo_g) * kd_g) * (t_g * W_g)   [erg/s/cm^3]: the power
+ *                the dust of rtb200_grid_set_dust absorbs (kd_g its opacity, exactly as the sweep used it); 0 without
+ *                dust.  W_g is the band width in Hz of rtb200_uvb_band_width, so betaDust_g * W_g is the band integral
+ *                of (nu/nu_g)^-alpha_g sigma_d(nu) d nu and 4 pi kd_g W_g J_g the power absorbed from the power-law band.
+ * Every field is linear in J: the fields of a direction subset are that shard's share, and the shares add up.
+ *   rtb200_grid_set_heating  gamma9 = [group][gammaHI, gammaHeI, gammaHeII] (NULL clears the setting and frees the
+ *                            buffer), width3 = band widths [Hz].  An entry that is negative, NaN or Inf is refused with
+ *                            RTB200_ERR_ARG and the previous state stays.  Queued work completes first.  rtb200_grid_set
+ *                            clears it; rtb200_grid_update_species, emission, scattering, dust and the acceleration keep
+ *                            it.  A device group calls it collectively and stores it on every member.
+ *   rtb200_last_heating      heat5 = host [5][nleaf]: the fields of the latest diffuse call (a device group in rank mode
+ *                            writes its slab only, as the J of the host call).  RTB200_ERR_ARG while heating is not set,
+ *                            when no diffuse call has completed since the setting or the grid changed, or after a
+ *                            failed call.
+ *   rtb200_heating_device    the library's device buffer [5][stride]: offset 0, count = stride = nleaf for a single
+ *                            context (local 0); leaves [offset, offset + count) of local device `local` of a group, as
+ *                            rtb200_multi_slab.  Valid until the next diffuse call or setting change; ERR_ARG while
+ *                            heating is not set.
+ * rtb200_diffuse reads its J, rtb200_diffuse_device the caller's J_device on the caller's stream, the group calls every
+ * member's reduced slab of J (once, after a source iteration).  rtb200_last_stats counts the pass in launches and the
+ * device time; the sweep figures stay the sweep's. */
+int rtb200_grid_set_heating(rtb200_ctx* ctx, const double* gamma9, const double* width3);
+int rtb200_last_heating(rtb200_ctx* ctx, double* heat5);
+int rtb200_heating_device(rtb200_ctx* ctx, int local, int64_t* offset, int64_t* count, int64_t* stride,
+                          double** H_device);
+
 /* Diffuse (UV background) sweep: replaces equiSources.f90:1372-1808 (computeOpacities :4956, the loop over
  * 12*4**(nAngularLevel-1) HEALPix directions, pattern set-up, neighbour threading, transport).
  *   uvb[3]      boundary intensities uvb1..3 (definitionsModule.f90:53)
@@ -289,7 +323,11 @@ int rtb200_diffuse_rates_device(rtb200_ctx* ctx, const double* J_device, const d
  *                           * (e_i - e_{i-1}), sD = the 7-term fit of aDust[7][5] (dustModule.f90:30-73) at the bin's
  *                           wavelength, as the point path evaluates it.  Group 3 runs to wavelengths below the fit's
  *                           range (down to ~1e-4 A at nfreq 400); the fit is extrapolated there as in the point tables.
- *                           Input to rtb200_grid_set_dust.  ERR_ARG for NULL pointers or nfreq < 2. */
+ *                           Input to rtb200_grid_set_dust.  ERR_ARG for NULL pointers or nfreq < 2.
+ *   rtb200_uvb_band_width   width3[g] = shape_g * nu_g * eVtoHz, the band width in Hz of group g (shape_g the band
+ *                           integral of the beta24 normalisation): betaDust3[g] * width3[g] is the band integral of the
+ *                           dust cross-section.  Input to rtb200_grid_set_heating.  ERR_ARG for NULL pointers. */
+int rtb200_uvb_band_width(const double* alpha, double* width3);
 int rtb200_uvb_dust_beta(int nfreq, double freqdel, const double* alpha, const double* aDust, double* betaDust3);
 int rtb200_uvb_amplitudes(double currentRedshift, double uvbCoefficient, double* uvb, double* alpha);
 int rtb200_uvb_beta_table(int nfreq, double freqdel, const double* alpha, double* table57);

@@ -7,7 +7,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "librtb200.so")
-SOURCES = ["api.cu", "diffuse_uniform.cu", "diffuse_amr.cu", "point_source.cu", "chemistry.cu", "multi.cu", "scattering.cu", "ng.cu", "dust.cu", "octree_build.cu", "geometry.cpp", "point_host.cpp", "uvb_host.cpp"]
+SOURCES = ["api.cu", "diffuse_uniform.cu", "diffuse_amr.cu", "point_source.cu", "chemistry.cu", "multi.cu", "scattering.cu", "ng.cu", "dust.cu", "heating.cu", "octree_build.cu", "geometry.cpp", "point_host.cpp", "uvb_host.cpp"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "--use_fast_math=false", "-Xcompiler", "-fPIC,-O2,-ffp-contract=off,-fno-fast-math", "-Xptxas", "-v",

@@ -71,6 +71,7 @@ static void free_grid(Context& c) {
   cudaFree(c.dDustSigma); c.dDustSigma = nullptr;
   c.dustMode = 0;
   for (int g = 0; g < 3; g++) c.dustBeta[g] = c.dustAlbedo[g] = 0.;
+  free_heating(c);
   cudaFree(c.dLogT); c.dLogT = nullptr;
   for (auto& sl : c.pointPool) cudaFree(sl.first);
   c.pointPool.clear();
@@ -208,17 +209,23 @@ void reset_call_results(Context& c) {
   c.lastWarm = false;
   c.ngPending = false;
   c.dWarmTaken = nullptr;
+  c.heatValid = false;
 }
 
 int run_diffuse(Context& c, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays,
                 int32_t nrays, double* dJ, cudaStream_t s, int64_t* nseg) {
   reset_call_results(c);
-  if (!c.scatterSigma()) return run_sweep(c, nAngularLevel, uvb, beta, rays, nrays, dJ, s, nseg, 0);
-  if (rays) {   // the J of a direction subset is not the mean intensity the source needs
+  int st = RTB200_OK;
+  if (!c.scatterSigma()) {
+    st = run_sweep(c, nAngularLevel, uvb, beta, rays, nrays, dJ, s, nseg, 0);
+  } else if (rays) {   // the J of a direction subset is not the mean intensity the source needs
     c.scatWarm = false;
     return RTB200_ERR_ARG;
+  } else {
+    st = scatter_solve(c, nAngularLevel, uvb, beta, dJ, s, nseg);
   }
-  return scatter_solve(c, nAngularLevel, uvb, beta, dJ, s, nseg);
+  if (st || !c.dHeat) return st;
+  return launch_heating(c, 0, c.nleaf, dJ, c.nleaf, s);
 }
 
 // number of entries that are negative, NaN or Inf (the emission check of rtb200_grid_set_emission_device)
@@ -557,6 +564,34 @@ int rtb200_grid_set_scattering_acceleration(rtb200_ctx* h, int32_t flags) {
   return set_scattering_acceleration(h->c, flags);
 }
 
+int rtb200_grid_set_heating(rtb200_ctx* h, const double* gamma9, const double* width3) {
+  if (!h) return RTB200_ERR_ARG;
+  if (h->m) return multi_set_heating(h->m, gamma9, width3);
+  return set_heating(h->c, gamma9, width3, h->c.nleaf);
+}
+
+int rtb200_last_heating(rtb200_ctx* h, double* heat5) {
+  if (!h || !heat5) return RTB200_ERR_ARG;
+  if (h->m) return multi_last_heating(h->m, heat5);
+  Context& c = h->c;
+  if (!c.dHeat || !c.heatValid) return RTB200_ERR_ARG;
+  RTB_CUDA(cudaSetDevice(c.device));
+  RTB_CUDA(cudaDeviceSynchronize());   // the pass of a *_device call runs on the caller's stream
+  RTB_CUDA(cudaMemcpy(heat5, c.dHeat, (size_t)5 * c.nleaf * sizeof(double), cudaMemcpyDeviceToHost));
+  return RTB200_OK;
+}
+
+int rtb200_heating_device(rtb200_ctx* h, int local, int64_t* offset, int64_t* count, int64_t* stride, double** H_device) {
+  if (!h) return RTB200_ERR_ARG;
+  if (h->m) return multi_heating_device(h->m, local, offset, count, stride, H_device);
+  if (local != 0 || !h->c.dHeat) return RTB200_ERR_ARG;
+  if (offset) *offset = 0;
+  if (count) *count = h->c.nleaf;
+  if (stride) *stride = h->c.heatStride;
+  if (H_device) *H_device = h->c.dHeat;
+  return RTB200_OK;
+}
+
 int rtb200_last_scattering_acceleration(rtb200_ctx* h, int32_t* extrapolations, int32_t* warmStarted) {
   if (!h) return RTB200_ERR_ARG;
   return last_scattering_acceleration(h->m ? multi_primary(h->m) : h->c, extrapolations, warmStarted);
@@ -590,6 +625,7 @@ int rtb200_diffuse(rtb200_ctx* h, int nAngularLevel, const double* uvb, const do
   if (err) {
     cudaMemset(c.dErr, 0, 64);
     c.scatWarm = false;   // a failed solve is no starting guess
+    c.heatValid = false;
     return err;
   }
   return RTB200_OK;

@@ -8,6 +8,7 @@
 #include <algorithm>
 #include <cmath>
 
+#include "dust_model.cuh"
 #include "rtb200_internal.h"
 
 namespace rtb {
@@ -20,17 +21,17 @@ struct DustParams {
 };
 
 // kappa_g = kappa_abs,g + kd_g (the gas sequence of compute_opacities_kernel, then kd added and rounded once) and, with
-// sigmaSrc, sigmaSrc_g = albedo_g * kd_g.  Every step rounded on its own (no FMA), so that numpy repeats it bit for bit:
-//   mode 1: kd = ((HI * bd) * abun2) / 0.2f,   mode 2: kd = (((((0.76f * rho) / m_H) * bd) * abun2) / 0.2f
+// sigmaSrc, sigmaSrc_g = albedo_g * kd_g.  Every step rounded on its own (no FMA), so that numpy repeats it bit for bit;
+// kd is dust_kd of dust_model.cuh
 __global__ void compute_opacities_dust_kernel(const double* __restrict__ HI, const double* __restrict__ HeI,
                                               const double* __restrict__ HeII, const double* __restrict__ rho,
                                               const double* __restrict__ abun2, double* __restrict__ kappa,
                                               double* __restrict__ sigmaSrc, int64_t n, DustParams p) {
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     const double h = HI[i], he1 = HeI[i], he2 = HeII[i], a = abun2[i];
-    const double col = p.mode == 1 ? h : __ddiv_rn(__dmul_rn((double)0.76f, rho[i]), (double)1.6726231e-24f);
+    const double col = dust_column(p.mode, h, rho, i);
     double kd[3];
-    for (int g = 0; g < 3; g++) kd[g] = __ddiv_rn(__dmul_rn(__dmul_rn(col, p.bd[g]), a), (double)0.2f);
+    for (int g = 0; g < 3; g++) kd[g] = dust_kd(col, p.bd[g], a);
     kappa[i] = __dadd_rn(__dmul_rn(h, p.b0), kd[0]);
     kappa[n + i] = __dadd_rn(__dadd_rn(__dmul_rn(h, p.b3), __dmul_rn(he1, p.b4)), kd[1]);
     kappa[2 * n + i] = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(h, p.b6), __dmul_rn(he1, p.b7)), __dmul_rn(he2, p.b8)), kd[2]);

@@ -876,6 +876,40 @@ int multi_set_dust(Multi* m, int mode, const double* betaDust, const double* alb
   return for_each_member(*m, [&](Member& q, int) { return set_dust(q.c, mode, betaDust, albedo, maxIterations, tolerance); });
 }
 
+// scalars only, checked on the host before any member changes: every member stores them with a [5][slab] buffer for its
+// slab's fields, and ranks given the same arguments return the same status
+int multi_set_heating(Multi* m, const double* gamma9, const double* width3) {
+  if (m->nleaf == 0 || (gamma9 && !heating_args_ok(gamma9, width3))) return RTB200_ERR_ARG;
+  return for_each_member(*m, [&](Member& q, int) { return set_heating(q.c, gamma9, width3, m->slab); });
+}
+
+// every local member copies its slab of the fields into heat5 [5][nleaf]
+int multi_last_heating(Multi* m, double* heat5) {
+  for (Member* q : m->mem)
+    if (!q->c.dHeat || !q->c.heatValid) return RTB200_ERR_ARG;
+  const int64_t N = m->nleaf;
+  return for_each_member(*m, [&](Member& q, int) -> int {
+    RTB_CUDA(cudaSetDevice(q.c.device));
+    RTB_CUDA(cudaDeviceSynchronize());   // the pass of a resident call runs on the caller's streams
+    const int64_t off = slab_off(*m, q.rank), cnt = slab_cnt(*m, q.rank);
+    if (cnt > 0)
+      for (int f = 0; f < 5; f++)
+        RTB_CUDA(cudaMemcpy(heat5 + f * N + off, q.c.dHeat + f * m->slab, (size_t)cnt * sizeof(double), cudaMemcpyDeviceToHost));
+    return RTB200_OK;
+  });
+}
+
+int multi_heating_device(Multi* m, int local, int64_t* offset, int64_t* count, int64_t* stride, double** H) {
+  if (local < 0 || local >= m->nlocal) return RTB200_ERR_ARG;
+  Member& q = *m->mem[local];
+  if (!q.c.dHeat) return RTB200_ERR_ARG;
+  if (offset) *offset = slab_off(*m, q.rank);
+  if (count) *count = slab_cnt(*m, q.rank);
+  if (stride) *stride = m->slab;
+  if (H) *H = q.c.dHeat;
+  return RTB200_OK;
+}
+
 int multi_get_species(Multi* m, double* HI, double* HeI, double* HeII) {
   if (m->nleaf == 0) return RTB200_ERR_ARG;
   return for_each_member(*m, [&](Member& q, int) -> int {
@@ -909,10 +943,20 @@ int multi_device_error(Multi* m) {
   return first;
 }
 
-// the stored J of the warm start goes on every local member (in rank mode the other ranks learn it from the holding
-// flags all-gathered at the start of their next call)
-static void drop_stored_j(Multi& m) {
-  for (Member* q : m.mem) q->c.scatWarm = false;
+// the heating pass over this member's slab of the reduced J (species at + off), while heating is set
+static int heat_member(Multi& m, Member& q, cudaStream_t s) {
+  if (!q.c.dHeat) return RTB200_OK;
+  return launch_heating(q.c, slab_off(m, q.rank), slab_cnt(m, q.rank), q.Jslab, m.slab, s);
+}
+
+// a failed call of the group: its stored J is no starting guess and its heating fields are not the call's, on every
+// local member (in rank mode the other ranks learn of a lost stored J from the holding flags all-gathered at the start
+// of their next call)
+static void call_failed(Multi& m) {
+  for (Member* q : m.mem) {
+    q->c.scatWarm = false;
+    q->c.heatValid = false;
+  }
 }
 
 // Source iteration of one member (scattering set) over its slab: the loop of source_iteration (scattering.cu), with
@@ -968,6 +1012,7 @@ static int diffuse_resident_member(Multi& m, Member& q, int nAngularLevel, const
     if (int st = sweep_member(m, q, buf, nAngularLevel, uvb, beta, s)) return st;
     if (int st = reduce_member(m, q, buf, m.step, 3, q.Jslab, ep, s)) return st;
   }
+  if (int st = heat_member(m, q, s)) return st;   // from the species the sweep used, before chemistry changes them
   if (chemistry) {
     if (!ksi6) return RTB200_ERR_ARG;
     const int64_t off = slab_off(m, q.rank), cnt = slab_cnt(m, q.rank);
@@ -998,7 +1043,7 @@ static int multi_diffuse(Multi& m, int nAngularLevel, const int32_t* rays, int32
     RTB_CUDA(cudaSetDevice(q.c.device));
     return member(q, i, &iters[(size_t)i]);
   });
-  if (st) drop_stored_j(m);   // a failed solve is no starting guess, on any member
+  if (st) call_failed(m);
   m.step += (unsigned long long)(iters[0] - 1);   // the ranks agree on the iteration count
   if (nseg) *nseg = sum_nseg(m);
   return st;
@@ -1018,7 +1063,7 @@ int multi_diffuse_host(Multi* m, int nAngularLevel, const double* uvb, const dou
   if (m->nleaf == 0 || !uvb || !beta) return RTB200_ERR_ARG;
   const bool scatter = multi_primary(m).scatterSigma() != nullptr;
   if (scatter && rays) {   // the J of a direction subset is not the mean intensity the source needs
-    drop_stored_j(*m);
+    call_failed(*m);
     return RTB200_ERR_ARG;
   }
   return multi_diffuse(*m, nAngularLevel, rays, nrays, nseg, [&](Member& q, int, int* iters) -> int {
@@ -1034,6 +1079,7 @@ int multi_diffuse_host(Multi* m, int nAngularLevel, const double* uvb, const dou
       if (int e = reduce_member(*m, q, buf, m->step, 3, q.Jslab, Epilogue(), c.stream)) return e;
       tm.mark("reduce-scatter");
     }
+    if (int e = heat_member(*m, q, c.stream)) return e;
     const int64_t off = slab_off(*m, q.rank), cnt = slab_cnt(*m, q.rank);
     const size_t nb = (size_t)cnt * sizeof(double);
     if (cnt > 0) {

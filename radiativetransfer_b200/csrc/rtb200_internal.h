@@ -185,6 +185,13 @@ struct Context {
   const double* scatterSigma() const { return dSigma ? dSigma : dDustSigma; }
   // the source the sweeps read: the effective one while the context scatters, else the emission (nullptr: none)
   const double* sweepEta() const { return scatterSigma() ? dEtaEff : dEta; }
+  // photo-heating and dust absorption (rtb200_grid_set_heating, heating.cu): while dHeat is set, every diffuse call ends
+  // with one pass over the J it returns into dHeat [5][heatStride] (nleaf, or the slab of a device-group member)
+  double heatGamma[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};   // [group][gammaHI, gammaHeI, gammaHeII]
+  double heatWidth[3] = {0, 0, 0};                    // band widths [Hz]
+  double* dHeat = nullptr;
+  int64_t heatStride = 0;
+  bool heatValid = false;   // dHeat holds the fields of a diffuse call that completed since the setting or the grid changed
   int uniStdSlots = 0;      // slots [0, uniStdSlots) are in leaf order, the rest z-major
   DevTree tree;
   std::vector<int32_t> hChild;               // host copy of the linear octree
@@ -293,6 +300,13 @@ int set_dust(Context& c, int mode, const double* betaDust, const double* albedo,
 bool dust_args_ok(int mode, const double* betaDust, const double* albedo, int32_t maxIterations, double tolerance);
 int launch_compute_opacities_dust(Context& c, const double* beta, cudaStream_t s);
 int last_scattering(Context& c, int32_t* iterations, double* residual);
+// heating.cu: the heating setting (gamma9 = nullptr clears; stride = entries per field of dHeat) and its pass
+bool heating_args_ok(const double* gamma9, const double* width3);
+int set_heating(Context& c, const double* gamma9, const double* width3, int64_t stride);
+void free_heating(Context& c);
+// the heating pass over leaves [off, off + cnt) into dHeat [f * heatStride + i - off], from J [g * jStride + i - off]
+// and the species at + off; counted in the call's launches and device time
+int launch_heating(Context& c, int64_t off, int64_t cnt, const double* J, int64_t jStride, cudaStream_t s);
 
 // ng.cu: acceleration of the source iteration (DESIGN.md 4.9)
 constexpr int kNgBlocks = 1024;    // fixed grid of the partial-sum pass: its sums do not depend on the device
@@ -373,6 +387,9 @@ int multi_set_emission(Multi* m, const double* eta);
 int multi_set_scattering(Multi* m, const double* sigma, int32_t maxIterations, double tolerance);
 int multi_set_scattering_acceleration(Multi* m, int32_t flags);
 int multi_set_dust(Multi* m, int mode, const double* betaDust, const double* albedo, int32_t maxIterations, double tolerance);
+int multi_set_heating(Multi* m, const double* gamma9, const double* width3);
+int multi_last_heating(Multi* m, double* heat5);
+int multi_heating_device(Multi* m, int local, int64_t* offset, int64_t* count, int64_t* stride, double** H);
 int multi_get_species(Multi* m, double* HI, double* HeI, double* HeII);
 int multi_diffuse_host(Multi* m, int nAngularLevel, const double* uvb, const double* beta, const int32_t* rays,
                        int32_t nrays, double* J1, double* J2, double* J3, int64_t* nseg);

@@ -3,6 +3,7 @@
 //   * group cross-sections beta24..31, rate weights ksi24..31 and heating weights gammaHI/HeI/HeII of the three
 //     frequency groups                                               uvbBetaTable.f90:31-296
 //   * band-mean dust cross-sections of the groups with the same weights (an extension, DESIGN.md 4.8)
+//   * band widths of the groups in Hz, the dust absorption of the heating pass (an extension, DESIGN.md 4.10)
 // They are what computeOpacities (equiSources.f90:4956-4983) and the diffuse photo-rates (:3546-3553) consume, i.e.
 // the `beta[9]` / `ksi*` arguments of rtb200_diffuse* and rtb200_chemistry_device.
 // Every Fortran real literal without a d-exponent is single precision and is widened where it meets a double; integer
@@ -193,6 +194,14 @@ int rtb200_uvb_dust_beta(int nfreq, double freqdel, const double* alpha, const d
   double shape[3];
   band_shapes(alpha, shape);
   for (int g = 0; g < 3; g++) betaDust3[g] = G[g] / (shape[g] * kNu[g]);
+  return RTB200_OK;
+}
+
+int rtb200_uvb_band_width(const double* alpha, double* width3) {
+  if (!alpha || !width3) return RTB200_ERR_ARG;
+  double shape[3];
+  band_shapes(alpha, shape);
+  for (int g = 0; g < 3; g++) width3[g] = shape[g] * kNu[g] * kEvToHz;
   return RTB200_OK;
 }
 

@@ -81,6 +81,18 @@ module rtb200_shim
        integer(c_int32_t), value :: maxIterations
        real(c_double), value :: tolerance
      end function rtb200_grid_set_dust
+     integer(c_int) function rtb200_grid_set_heating(ctx, gamma9, width3) bind(C, name='rtb200_grid_set_heating')
+       import :: c_int, c_ptr
+       type(c_ptr), value :: ctx, gamma9, width3
+     end function rtb200_grid_set_heating
+     integer(c_int) function rtb200_last_heating(ctx, heat5) bind(C, name='rtb200_last_heating')
+       import :: c_int, c_ptr
+       type(c_ptr), value :: ctx, heat5
+     end function rtb200_last_heating
+     integer(c_int) function rtb200_uvb_band_width(alpha, width3) bind(C, name='rtb200_uvb_band_width')
+       import :: c_int, c_ptr
+       type(c_ptr), value :: alpha, width3
+     end function rtb200_uvb_band_width
      integer(c_int) function rtb200_uvb_dust_beta(nfreq, freqdel, alpha, aDust, betaDust) bind(C, name='rtb200_uvb_dust_beta')
        import :: c_ptr, c_int, c_double
        integer(c_int), value :: nfreq
@@ -514,5 +526,31 @@ contains
     call rtbCheck(rtb200_grid_set_dust(rtbContext, int(dustApproximation, c_int), c_loc(betaDust), c_loc(albedoC), &
          int(maxIterations, c_int32_t), tolerance), 'rtb200_grid_set_dust')
   end subroutine rtbSetDust
+
+  ! Photo-heating and dust absorption per leaf (extension, DESIGN.md 4.10): every later rtbDiffuse ends with one pass
+  ! over the J it returns, with the heating weights gammaHI / gammaHeI / gammaHeII of group1..3 (uvbBetaTable) and the
+  ! band widths in Hz of the slopes alpha(3).  The dust absorption uses the dust of rtbSetDust.  rtbSetGrid clears it.
+  subroutine rtbSetHeating()
+    real(c_double), dimension(9), target :: gamma9
+    real(c_double), dimension(3), target :: alphaC, width3
+    gamma9 = (/ group1%gammaHI, group1%gammaHeI, group1%gammaHeII, &
+                group2%gammaHI, group2%gammaHeI, group2%gammaHeII, &
+                group3%gammaHI, group3%gammaHeI, group3%gammaHeII /)
+    alphaC = real(alpha(1:3), c_double)
+    call rtbCheck(rtb200_uvb_band_width(c_loc(alphaC), c_loc(width3)), 'rtb200_uvb_band_width')
+    call rtbCheck(rtb200_grid_set_heating(rtbContext, c_loc(gamma9), c_loc(width3)), 'rtb200_grid_set_heating')
+  end subroutine rtbSetHeating
+
+  ! the fields of the latest rtbDiffuse, heat(leaf, f) in the leaf order of rtbSetGrid (= C [5][nleaf]): f = 1..3
+  ! photo-heating per HI, HeI, HeII atom [erg/s], 4 gas heating, 5 dust absorption [erg/s/cm^3].  zoneType has no field
+  ! for them, so they stay in the flat order (scatter them with the driver's own walk of the leaves).
+  subroutine rtbDiffuseHeating(heat)
+    real(c_double), dimension(:,:), target, contiguous, intent(out) :: heat
+    if (size(heat, 1).ne.rtbLeaves .or. size(heat, 2).ne.5) then
+       write(*,*) 'rtb200: heat must be (nleaf, 5)'
+       stop
+    endif
+    call rtbCheck(rtb200_last_heating(rtbContext, c_loc(heat)), 'rtb200_last_heating')
+  end subroutine rtbDiffuseHeating
 
 end module rtb200_shim

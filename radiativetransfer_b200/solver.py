@@ -266,6 +266,34 @@ class Transport:
                    "rtb200_last_scattering_acceleration")
         return {"extrapolations": n.value, "warm_start": bool(w.value)}
 
+    def set_heating(self, gamma, band_width=None):
+        """Photo-heating and dust absorption per leaf (DESIGN.md 4.10): `gamma` [3, 3] = [group][gammaHI, gammaHeI,
+        gammaHeII] and `band_width[3]` in Hz, as workloads.uvb_heating returns them; None clears the setting.  Every
+        diffuse call then ends with one pass over the J it returns (read back with last_heating / heating_device).
+        Negative, NaN or Inf entries raise and keep the previous state.  set_grid clears it."""
+        if gamma is None:
+            _lib.check(self.L.rtb200_grid_set_heating(self.h, None, None), "rtb200_grid_set_heating")
+            return
+        g, w = _f64(gamma), _f64(band_width)
+        if g.size != 9 or w is None or w.size != 3:
+            raise ValueError("gamma takes [3][3] values and band_width one per frequency group")
+        _lib.check(self.L.rtb200_grid_set_heating(self.h, _ptr(g), _ptr(w)), "rtb200_grid_set_heating")
+
+    def last_heating(self):
+        """The heating fields of the latest diffuse call, each [nleaf]: {"gamma_HI", "gamma_HeI", "gamma_HeII"} in erg/s
+        per absorber, {"gas", "dust"} in erg/s/cm^3 (a device group in rank mode fills its slab only, the rest is 0)."""
+        H = np.zeros((5, self.nleaf))
+        _lib.check(self.L.rtb200_last_heating(self.h, _ptr(H)), "rtb200_last_heating")
+        return dict(gamma_HI=H[0], gamma_HeI=H[1], gamma_HeII=H[2], gas=H[3], dust=H[4])
+
+    def heating_device(self, local=0):
+        """(ptr, offset, count, stride): the library's device buffer [5][stride] of local device `local`, holding leaves
+        [offset, offset + count); valid until the next diffuse call or setting change."""
+        off, cnt, stride, H = C.c_int64(0), C.c_int64(0), C.c_int64(0), C.c_void_p()
+        _lib.check(self.L.rtb200_heating_device(self.h, int(local), C.byref(off), C.byref(cnt), C.byref(stride), C.byref(H)),
+                   "rtb200_heating_device")
+        return H.value, off.value, cnt.value, stride.value
+
     def diffuse(self, uvb, beta, n_angular_level=3, rays=None, out=None):
         """Host-buffer call (H2D of nothing but tables, D2H of J): returns (J[3, nleaf], nseg)."""
         uvb, beta = _f64(uvb), _f64(np.asarray(beta).reshape(9))

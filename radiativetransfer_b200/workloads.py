@@ -75,6 +75,21 @@ def uvb_dust_beta(alpha, a_dust, nfreq=400, freqdel=None):
     return out
 
 
+def uvb_heating(table, alpha):
+    """(gamma9, width3), the inputs of Transport.set_heating (DESIGN.md 4.10): gamma9 [3, 3] = [group][gammaHI, gammaHeI,
+    gammaHeII] from the background's table[3][19] (columns 16-18), width3[3] = the band widths in Hz of
+    rtb200_uvb_band_width for the effective slopes alpha[3] (uvb_background()["table"], ["alpha"])."""
+    import ctypes as C
+
+    from . import _lib
+    gamma = np.ascontiguousarray(np.asarray(table, dtype=np.float64).reshape(3, 19)[:, 16:19])
+    al = np.ascontiguousarray(alpha, dtype=np.float64).reshape(3)
+    width = np.zeros(3)
+    p = lambda a: a.ctypes.data_as(C.c_void_p)
+    _lib.check(_lib.lib().rtb200_uvb_band_width(p(al), p(width)), "rtb200_uvb_band_width")
+    return gamma, width
+
+
 # ------------------------------------------------------------------------------------------------------
 # grids
 # ------------------------------------------------------------------------------------------------------
