@@ -114,7 +114,7 @@ int rtb200_set_math(rtb200_ctx* ctx, int math_mode);
  *   uniform sweep  "slots" (zone tasks per launch, 0 = all), "graph" (CUDA graph replay, 1), "dirs_per_task" (0 = chosen
  *                  from a wave model), "cells" (cells of a layer per thread: 1, 2, or 0 = by grid size and zone tasks per
  *                  launch; an emissive sweep always runs one-cell threads), "block_warps" (warps per block 8 / 4 / 2,
- *                  0 = by the number of blocks a launch has), "transpose_z" (z-major copy for
+ *                  at most 4 for two-cell threads, 0 = by the number of blocks a launch has), "transpose_z" (z-major copy for
  *                  the zones sweeping along the contiguous axis, 1), "pdl" (programmatic dependent launch of layer
  *                  l+1 on layer l, also used by the nested-grid waves, 1), "l2_mb"
  *   nested grids   "force_amr" (general octree path on a uniform grid), "amr_batch" (directions per batch, 0 = as many

@@ -70,6 +70,7 @@ struct StepParams {
   int32_t origin;          // leaf index of rotated (step, 0, 0)
   int32_t sj, sk;
   int32_t ndir, laneIsK, firstInSlot, n;
+  int32_t anyThin;         // a direction of this layer is thin (LayerSeg::thin)
 };
 
 // Planes carry one extra row and column on the upstream side (index -1) that permanently hold the boundary
@@ -509,9 +510,65 @@ __device__ __forceinline__ void direction_kinds_fast2(const LayerSeg& P, bool se
   }
 }
 
-// Positions are row pairs (see lane_position): a lane holds the cell (a, b0) and the one above it.  Register budget: 2
-// blocks of 256 threads per SM (124 registers, no spills; as many cells in flight as the one-cell kernel at 4 blocks).
-__global__ void __launch_bounds__(256, 2)
+// The thin layers of the two-cell kernel (P.thin: 0.2% of the direction-layers): the reference's operation sequence,
+// cell by cell, on the unfloored opacities; the upper cell takes the lower one as its (b-1) cell exactly as the
+// single-cell kernel does.  Returns the two cells' sums.  Out of line and reloading what it needs, so that none of its
+// state is live in the FAST loop.
+struct FaithOut2 {
+  Tri acc0, acc1;
+};
+__device__ __noinline__ FaithOut2 thin_pass2(const StepParams& sp, int pidx, int up, int up1, int dstride,
+                                             const double* __restrict__ kg, int N, int sB, bool cell0, bool cell1,
+                                             bool hasR, bool writer0, bool writer1) {
+  double kF0[3], kF1[3], kR[3], acc0[3] = {0., 0., 0.}, acc1[3] = {0., 0., 0.};
+#pragma unroll
+  for (int g = 0; g < 3; g++) {
+    const double* k = kg + (int64_t)g * N;
+    kF0[g] = cell0 ? k[0] : 0.;
+    kF1[g] = cell1 ? k[sB] : 0.;
+    kR[g] = hasR ? k[-sB] : 0.;
+  }
+  const double* pin = sp.planeIn + 3 * pidx;
+  double* pout = sp.planeOut + 3 * pidx;
+  for (int q = 0; q < sp.ndir; q++, pin += dstride, pout += dstride) {
+    const LayerSeg& P = sp.P[q];
+    if (!P.thin) continue;
+    const int kind = P.kind;
+    double cur0[3], cur1[3], upR[3] = {0., 0., 0.}, I0[3], I1[3];
+#pragma unroll
+    for (int g = 0; g < 3; g++) { cur0[g] = pin[g]; cur1[g] = pin[g + up1]; }
+    const bool secL = (kind <= 2) == (sp.laneIsK != 0);
+    if (kind == 2 || kind == 4 || (kind != 0 && !secL)) {
+#pragma unroll
+      for (int g = 0; g < 3; g++) upR[g] = pin[g - up];
+    }
+    direction_dispatch_faithful(P, secL, cur0, upR, kF0, kR, I0, acc0);
+    direction_dispatch_faithful(P, secL, cur1, cur0, kF1, kF0, I1, acc1);
+    if (writer0) {
+#pragma unroll
+      for (int g = 0; g < 3; g++) pout[g] = I0[g];
+    }
+    if (writer1) {
+#pragma unroll
+      for (int g = 0; g < 3; g++) pout[g + up] = I1[g];
+    }
+  }
+  FaithOut2 o;
+#pragma unroll
+  for (int g = 0; g < 3; g++) { o.acc0.v[g] = acc0[g]; o.acc1.v[g] = acc1[g]; }
+  return o;
+}
+
+// Positions are row pairs (see lane_position): a lane holds the cell (a, b0) and the one above it.  Register budget: 6
+// blocks of 128 threads per SM (80 registers): 24 resident warps per SM instead of 16 at 124 registers, for a kernel
+// that is latency-bound (dependent FP64 and shuffle chains; DESIGN.md 4.1, 4.2: 5 blocks at 96 registers gained nothing).  The few spill slots ptxas uses hold
+// loop-invariant values: stored before the direction loop, one 4-byte reload per direction, the rest around the call
+// of thin_pass2 -- none inside the segment arithmetic.
+// The thin layers (P.thin) are swept in a second pass over the directions, after the FAST ones: their sums and the
+// FAST sums A0/A1 are separate until the final fma, and every direction has its own plane, so the order of the two
+// passes changes no bit.
+constexpr int kCell2Warps = 4;  // warps per block at most
+__global__ void __launch_bounds__(32 * kCell2Warps, 6)
 sweep_cell2_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1, int npl3) {
   const StepParams& sp = bp.t[blockIdx.z];
   const double* __restrict__ kappa = sp.kappa;
@@ -528,19 +585,18 @@ sweep_cell2_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1
   const int laneIsK = sp.laneIsK;
   const int sA = laneIsK ? sp.sk : sp.sj, sB = laneIsK ? sp.sj : sp.sk;
   const int leaf0 = sp.origin + a * sA + b0 * sB;
-  double kap0[3], kap1[3], kF0[3], kF1[3], kR[3];
+  double kap0[3], kap1[3], kR[3];
 #pragma unroll
   for (int g = 0; g < 3; g++) {
     const double* kg = kappa + (int64_t)g * N + leaf0;
-    kF0[g] = cell0 ? kg[0] : 0.;
-    kF1[g] = cell1 ? kg[sB] : 0.;
+    const double kF0 = cell0 ? kg[0] : 0., kF1 = cell1 ? kg[sB] : 0.;
     kR[g] = (cell0 && b0 > 0) ? kg[-sB] : 0.;                  // kappa = 0 outside: exp(-0) = 1 exactly
-    kap0[g] = kF0[g] > 0. ? kF0[g] : kKappaFloor;
-    kap1[g] = kF1[g] > 0. ? kF1[g] : kKappaFloor;
+    kap0[g] = kF0 > 0. ? kF0 : kKappaFloor;
+    kap1[g] = kF1 > 0. ? kF1 : kKappaFloor;
   }
   const double kmax = fmax(fmax(fmax(fmax(kap0[0], kap0[1]), fmax(kap0[2], kR[0])), fmax(kR[1], kR[2])),
                            fmax(fmax(kap1[0], kap1[1]), kap1[2]));
-  double A0[3] = {0., 0., 0.}, A1[3] = {0., 0., 0.}, acc0[3] = {0., 0., 0.}, acc1[3] = {0., 0., 0.};
+  double A0[3] = {0., 0., 0.}, A1[3] = {0., 0., 0.};
   const int pidx = (b0 + 1) * np1 + a + 1;
   const int ndir = sp.ndir;
   const int dstride = npl3;
@@ -557,6 +613,7 @@ sweep_cell2_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1
       prefetch_l1(pin + dstride + up1);
       prefetch_l1(pin + dstride - up);
     }
+    if (P.thin) continue;                                      // second pass
     double cur0[3], cur1[3], upR[3] = {0., 0., 0.}, I0[3], I1[3];
 #pragma unroll
     for (int g = 0; g < 3; g++) { cur0[g] = pin[g]; cur1[g] = pin[g + up1]; }
@@ -565,16 +622,10 @@ sweep_cell2_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1
 #pragma unroll
       for (int g = 0; g < 3; g++) upR[g] = pin[g - up];
     }
-    if (P.thin) {
-      // rare (0.2% of the direction-layers): the reference's operation sequence, cell by cell; the upper cell takes
-      // the lower one as its (b-1) cell exactly as the single-cell kernel does
-      direction_dispatch_faithful(P, secL, cur0, upR, kF0, kR, I0, acc0);
-      direction_dispatch_faithful(P, secL, cur1, cur0, kF1, kF0, I1, acc1);
-    } else if (__any_sync(0xffffffffu, kmax * P.dmax > 64.)) {
+    if (__any_sync(0xffffffffu, kmax * P.dmax > 64.))
       direction_kinds_fast2<true>(P, secL, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, sT);
-    } else {
+    else
       direction_kinds_fast2<false>(P, secL, cur0, cur1, upR, kap0, kap1, kR, I0, I1, A0, A1, sT);
-    }
     if (writer0) {
 #pragma unroll
       for (int g = 0; g < 3; g++) pout[g] = I0[g];
@@ -584,10 +635,13 @@ sweep_cell2_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1
       for (int g = 0; g < 3; g++) pout[g + up] = I1[g];
     }
   }
+  FaithOut2 acc = {};
+  if (sp.anyThin)
+    acc = thin_pass2(sp, pidx, up, up1, dstride, kappa + leaf0, N, sB, cell0, cell1, cell0 && b0 > 0, writer0, writer1);
   if (writer0) {
 #pragma unroll
     for (int g = 0; g < 3; g++) {
-      const double v = fma(A0[g], kTwoM200 / kap0[g], acc0[g]);
+      const double v = fma(A0[g], kTwoM200 / kap0[g], acc.acc0.v[g]);
       double* p = sp.acc + (int64_t)g * N + leaf0;
       *p = sp.firstInSlot ? v : __dadd_rn(*p, v);
     }
@@ -595,7 +649,7 @@ sweep_cell2_kernel(const __grid_constant__ BatchParams bp, int N, int n, int np1
   if (writer1) {
 #pragma unroll
     for (int g = 0; g < 3; g++) {
-      const double v = fma(A1[g], kTwoM200 / kap1[g], acc1[g]);
+      const double v = fma(A1[g], kTwoM200 / kap1[g], acc.acc1.v[g]);
       double* p = sp.acc + (int64_t)g * N + leaf0 + sB;
       *p = sp.firstInSlot ? v : __dadd_rn(*p, v);
     }
@@ -750,32 +804,61 @@ static cudaError_t launch_layer(Kernel kern, dim3 grid, cudaStream_t s, bool pdl
   return cudaLaunchKernelEx(&cfg, kern, bp, N, n, n + 1, 3 * (n + 1) * (n + 1), extra...);
 }
 
+// The layer kernels, the largest block each takes (warps), and how many of its warps an SM holds at that block size --
+// from the occupancy calculator, once per context, so that the wave arithmetic below follows the register budgets.
+enum SweepKernel { kCell1, kCell1Faithful, kCell2, kEmit, kEmitFaithful };
+static int max_block_warps(int k) { return k == kCell2 ? kCell2Warps : 8; }
+static cudaError_t resident_warps(Context& c, int k, int* out) {
+  int& w = c.uniResidentWarps[k];
+  if (w == 0) {
+    const int warps = max_block_warps(k), threads = 32 * warps;
+    int blocks = 0;
+    cudaError_t e = cudaSuccess;
+    switch (k) {
+      case kCell1: e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, sweep_cell_kernel<false>, threads, 0); break;
+      case kCell1Faithful: e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, sweep_cell_kernel<true>, threads, 0); break;
+      case kCell2: e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, sweep_cell2_kernel, threads, 0); break;
+      case kEmit: e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, sweep_cell_emit_kernel<false>, threads, 0); break;
+      default: e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, sweep_cell_emit_kernel<true>, threads, 0); break;
+    }
+    if (e != cudaSuccess) return e;
+    w = std::max(1, blocks) * warps;
+  }
+  *out = w;
+  return cudaSuccess;
+}
+
 // `pdl`: programmatic dependent launch on the previous launch of the stream (only for a layer whose predecessor in
 // the stream is the previous layer's sweep kernel)
 // `ep` != nullptr: the emissive sweep (sweep_cell_emit_kernel: one cell per thread)
-static cudaError_t launch_cells(bool faithful, bool pdl, dim3 grid, cudaStream_t s, const BatchParams& bp, int N, int n,
-                                int cells, int warps, int smCount, const EtaParams* ep = nullptr) {
+// `warps` (set_tuning "block_warps"): 8, 4 or 2, at most the kernel's largest block; anything else = automatic
+static cudaError_t launch_cells(Context& c, bool faithful, bool pdl, dim3 grid, cudaStream_t s, const BatchParams& bp,
+                                int N, int n, int cells, int warps, const EtaParams* ep = nullptr) {
   // automatic: two cells per thread pay (1-2%) when the launch has many zone tasks; a small direction shard (3 zone
   // tasks on each of 8 GPUs) is 1.3 waves of two-cell threads but fills the device evenly with one-cell threads
   // (measured on the shards of an 8-GPU run: 7.03 against 7.21 ms mean, 7.31 against 7.93 ms for the slowest rank)
   if (cells == 0) cells = (n >= 192 && grid.z >= 6) ? 2 : 1;
   if (faithful || ep) cells = 1;
+  const int k = ep ? (faithful ? kEmitFaithful : kEmit) : faithful ? kCell1Faithful : cells == 2 ? kCell2 : kCell1;
   const int wpl = warps_per_layer(n, cells == 2 ? (n + 1) / 2 : n);   // warps per task and layer
   if (warps != 8 && warps != 4 && warps != 2) {
-    // automatic: the largest block that still gives the device ~6 blocks per resident 8-warp slot
-    const long long slots = (long long)smCount * (cells == 2 ? 2 : 4);
-    warps = 8;
+    // automatic: the largest block that still gives the device ~6 blocks per resident 8 warps
+    int resident = 0;
+    if (cudaError_t e = resident_warps(c, k, &resident)) return e;
+    const long long slots = (long long)c.smCount * resident / 8;
+    warps = max_block_warps(k);
     while (warps > 2 && (long long)((wpl + warps - 1) / warps) * grid.z < 6 * slots) warps /= 2;
   }
+  warps = std::min(warps, max_block_warps(k));
   grid.x = (unsigned)((wpl + warps - 1) / warps);
   grid.y = 1;
-  if (ep) {
-    if (faithful) return launch_layer(sweep_cell_emit_kernel<true>, grid, s, pdl, bp, N, n, warps, *ep);
-    return launch_layer(sweep_cell_emit_kernel<false>, grid, s, pdl, bp, N, n, warps, *ep);
+  switch (k) {
+    case kEmitFaithful: return launch_layer(sweep_cell_emit_kernel<true>, grid, s, pdl, bp, N, n, warps, *ep);
+    case kEmit: return launch_layer(sweep_cell_emit_kernel<false>, grid, s, pdl, bp, N, n, warps, *ep);
+    case kCell1Faithful: return launch_layer(sweep_cell_kernel<true>, grid, s, pdl, bp, N, n, warps);
+    case kCell2: return launch_layer(sweep_cell2_kernel, grid, s, pdl, bp, N, n, warps);
+    default: return launch_layer(sweep_cell_kernel<false>, grid, s, pdl, bp, N, n, warps);
   }
-  if (faithful) return launch_layer(sweep_cell_kernel<true>, grid, s, pdl, bp, N, n, warps);
-  if (cells == 2) return launch_layer(sweep_cell2_kernel, grid, s, pdl, bp, N, n, warps);
-  return launch_layer(sweep_cell_kernel<false>, grid, s, pdl, bp, N, n, warps);
 }
 
 int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std::vector<Direction>& dirs,
@@ -811,8 +894,11 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
     if (c.tune.dirsPerTask <= 0) {
       int perZone[25] = {0};
       for (int d = 0; d < ndir; d++) perZone[dirs[d].izone]++;
-      const int64_t bpt = (warps_per_layer(n, n) + 7) / 8;   // one-cell threads, 8-warp blocks
-      const int64_t cap = (int64_t)c.smCount * 4;   // resident blocks: 4 per SM (sweep_cell_kernel's register budget)
+      // in units of one-cell threads in 8-warp blocks (the shard shapes this choice serves run one-cell threads)
+      int resident = 0;
+      RTB_CUDA(resident_warps(c, kCell1, &resident));
+      const int64_t bpt = (warps_per_layer(n, n) + 7) / 8;
+      const int64_t cap = (int64_t)c.smCount * resident / 8;   // resident 8-warp blocks
       double best = 1e300;
       for (int d = kMaxDirPerTask; d >= 2; d--) {
         int64_t T = 0;
@@ -947,6 +1033,8 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
       sp.planeOut = ((step & 1) ? planeB : planeA) + (size_t)T.planeFirst * 3 * npl;
       sp.origin = (int32_t)(T.origin + step * T.si);
       fill_step_segs(sp.P, &T.seg[(size_t)step * kMaxDirPerTask], T.ndir, !faithful && !emit);
+      sp.anyThin = 0;
+      for (int q = 0; q < T.ndir; q++) sp.anyThin |= sp.P[q].thin;
       sp.ndir = T.ndir;
       sp.firstInSlot = first;
       return T.ndir;
@@ -965,7 +1053,7 @@ int diffuse_uniform(Context& c, int nAngularLevel, const double* uvb, const std:
         }
         dim3 gz = grid;
         gz.z = nb;
-        RTB_CUDA(launch_cells(faithful, c.tune.pdl && step > 0, gz, st, bp, (int)N, n, c.tune.cells, c.tune.blockWarps, c.smCount, epp));
+        RTB_CUDA(launch_cells(c, faithful, c.tune.pdl && step > 0, gz, st, bp, (int)N, n, c.tune.cells, c.tune.blockWarps, epp));
         nLaunched++;
       }
     }

@@ -226,6 +226,7 @@ struct Context {
   int uniSlots = 0;
   std::vector<UniTaskHost> uniTasks;
   int64_t uniNseg = 0, uniLaunches = 0;
+  int uniResidentWarps[5] = {0, 0, 0, 0, 0};  // resident warps per SM of each uniform sweep kernel (diffuse_uniform.cu)
   std::string amrPlanKey;
   bool statsPending = false, sweepTimed = false;
 
